@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — LightGCN_SPEX propagation throughput (GEdges/s) + full-rank top-20 users/s on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scale S]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scale S] [--dump-outputs DIR]
 
 One "step" = one computer() forward of the reference model
 (/root/reference/LightGCN_SPEX/code/utility1/model.py:66-97): K_layers = 3 propagation layers over
@@ -63,7 +63,15 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--cpu-sample-scale", type=float, default=0.01)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned to DIR/*.npy (see dump_outputs), so that two builds "
+                         "can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU step (--impl ours)")
+    return args
 
 
 def peaks():
@@ -241,6 +249,38 @@ def table_hash(t, row0, torch):
             torch.arange(1, D + 1, device=t.device, dtype=torch.int64)[None, :]
         h += (x * idx).sum()
     return h
+
+
+DUMP_ROWS = 1 << 17   # 32 MB of fp32 rows at D = 64: the whole dump stays under 64 MB
+
+
+def dump_outputs(path, res, bounds, rank, world, torch, dist):
+    """Write what the timed step returned (the propagated [N, D] fp32 table; this rank holds global rows
+    bounds[rank]:bounds[rank + 1] of it) to `path`, on rank 0:
+      propagated_sample.npy       fp32 [S, D]  S = min(N, DUMP_ROWS) rows drawn with seed 0, in row order
+      propagated_sample_rows.npy  fp64 [S]     their global row ids
+      propagated_col_sum.npy      fp64 [D]     column sums over all N rows, so that no row goes unchecked
+    The inputs are seeded, so the same arguments give the same files on the same build."""
+    import numpy as np
+
+    n_rows = bounds[-1]
+    rows = np.sort(np.random.default_rng(0).choice(n_rows, min(n_rows, DUMP_ROWS), replace=False))
+    owner = np.searchsorted(bounds, rows, side="right") - 1
+    dev = res.device
+    sample = torch.zeros(rows.size, res.shape[1], dtype=res.dtype, device=dev)
+    mine = owner == rank
+    sample[torch.from_numpy(mine).to(dev)] = res[torch.from_numpy(rows[mine] - bounds[rank]).to(dev)]
+    col_sum = res.sum(0, dtype=torch.float64)
+    if world > 1:
+        parts = torch.empty(world * rows.size, res.shape[1], dtype=res.dtype, device=dev)
+        dist.all_gather_into_tensor(parts, sample)
+        sample = parts.view(world, rows.size, -1)[torch.from_numpy(owner).to(dev), torch.arange(rows.size, device=dev)]
+        dist.all_reduce(col_sum)
+    if rank == 0:
+        os.makedirs(path, exist_ok=True)
+        np.save(os.path.join(path, "propagated_sample.npy"), sample.cpu().numpy())
+        np.save(os.path.join(path, "propagated_sample_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(path, "propagated_col_sum.npy"), col_sum.cpu().numpy())
 
 
 # ---- CPU legs (oracle = the reference's torch CPU path restated; the checker, not the product) -------
@@ -789,6 +829,8 @@ def run_ours(args):
     ms_step = float(t.item()) / args.steps
     value = nnz * K_LAYERS / (ms_step * 1e-3) / 1e9
     launches_timed = _capi.launch_count() - launches0
+    if args.dump_outputs:   # before the parity check below reuses the work buffers
+        dump_outputs(args.dump_outputs, res, [0, N] if world == 1 else bounds, rank, world, torch, dist)
     # parity at full size, untimed: D^-1/2 A D^-1/2 has the eigenvector sqrt(deg) (eigenvalue 1), so
     # propagating a table whose columns are multiples of sqrt(deg) must return it unchanged
     gsrc = g if world == 1 else lg

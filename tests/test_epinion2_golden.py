@@ -63,7 +63,7 @@ def test_loader_and_adjacency_match_reference(ep2, G):
     assert len(ep2.trainUser) == 209304 and len(ep2.testRatings) == 3185
     A = ep2.getSparseGraph()
     assert A.is_coalesced() and A._nnz() == int(G["adj_nnz"]) == 418608
-    idx, val = A.indices().numpy(), A.values().numpy()
+    idx, val = A.indices().cpu().numpy(), A.values().cpu().numpy()   # on the GPU when there is one
     pick = G["adj_pick"]
     assert np.array_equal(idx[:, pick], G["adj_pick_rc"])
     assert np.array_equal(val[pick], G["adj_pick_val"]), "adjacency values must be bit-equal"

@@ -46,14 +46,15 @@ def test_adjacency_bit_equal_to_reference(tiny, G):
     A = tiny.getSparseGraph()
     assert A.is_coalesced() and A.dtype == torch.float32 and A.indices().dtype == torch.int64
     assert tuple(A.shape) == (tiny.n_users + 1 + tiny.m_items,) * 2
-    assert np.array_equal(A.indices().numpy(), G["adj_indices"])
-    assert np.array_equal(A.values().numpy(), G["adj_values"]), "values must be bit-equal"
+    # the Loader puts the graph on the GPU when there is one
+    assert np.array_equal(A.indices().cpu().numpy(), G["adj_indices"])
+    assert np.array_equal(A.values().cpu().numpy(), G["adj_values"]), "values must be bit-equal"
     # second load goes through the s_pre_adj_mat.npz cache and must give the same matrix
     from spex_b200.dataloader import Loader
 
     again = Loader(make_args(dataset="tiny", data_path=os.path.dirname(os.path.dirname(tiny.path))))
     A2 = again.getSparseGraph()
-    assert np.array_equal(A2.values().numpy(), G["adj_values"])
+    assert np.array_equal(A2.values().cpu().numpy(), G["adj_values"])
     # oracle restatement of the builder
     Ao = O.to_sparse_tensor(O.norm_adj_scipy(tiny.trainUser, tiny.trainItem, tiny.n_users + 1, tiny.m_items))
     assert np.array_equal(Ao.indices().numpy(), G["adj_indices"])
