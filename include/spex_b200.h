@@ -85,6 +85,9 @@ typedef struct spex_long_plan {
   float* hot_partial;         /* fp32  [n_split_rows, D] workspace of pass A                   */
   int64_t n_split_rows;       /* rows [0, n_split_rows) take part in pass A                    */
   int64_t interleave_split;   /* SPEX_PLAN_INTERLEAVE: first row of the second class           */
+  int32_t n_hub_seg;          /* column-blocked list: segments [0, n_hub_seg) are hub-row cells, gathered
+                                 with the default L2 priority so that their window stays resident; the
+                                 rest are mid-row segments (no reuse: evict_first under COL_HOTBIT)     */
 } spex_long_plan;
 
 /*

@@ -36,6 +36,7 @@ class LongPlan(C.Structure):
         ("hot_partial", _p),
         ("n_split_rows", _i64),
         ("interleave_split", _i64),
+        ("n_hub_seg", _i32),
     ]
 
 

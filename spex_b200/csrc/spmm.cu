@@ -19,7 +19,7 @@
 //     summation order is a pure function of the row => bit-reproducible, no atomics;
 //   * rows longer than plan->seg_len are skipped here and reduced by two extra launches (warp per segment ->
 //     partial rows -> warp per long row), hub rows cut at column-block boundaries and listed block-major so
-//     that the table window they gather from stays in L2;
+//     that the table window they gather from stays in L2 (a warp reduces a run of such cells back to back);
 //   * epilogue: Y = acc (next layer's input) and/or Z = (addend*a + acc)*b (running layer mean forward,
 //     g + A^T G backward), optionally stored into every peer's table (P2P or one NVLS multicast store), with the
 //     next call's table or a dense Adam step riding on the last layer (row-partitioned modes);
@@ -148,18 +148,75 @@ __device__ __forceinline__ f8 ld_gather_f8_first(const float* p) {
       : "l"(p));
   return v;
 }
-template <int D, bool kHot>
+// kCold: the L2 priority of a column without the hot bit - evict_first (kCold) or the default one.  Hot columns
+// (kHot and bit 31 set) always load with evict_last.
+template <int D, bool kHot, bool kCold = kHot>
 __device__ __forceinline__ f8 gather_row8(const float* Xs, int cc) {
   // one IMAD.WIDE.U32 (left to itself the compiler builds the 64-bit product from two shifts, two masks and
   // a carry chain: 6 instructions per gather)
   const float* p;
   asm("mad.wide.u32 %0, %1, %2, %3;" : "=l"(p) : "r"(kHot ? (uint32_t)cc & 0x7fffffffu : (uint32_t)cc), "n"(D * 4), "l"(Xs));
-  if (kHot) return cc < 0 ? ld_gather_f8_last(p) : ld_gather_f8_first(p);
-  return ld_gather_f8(p);
+  if (kHot) return cc < 0 ? ld_gather_f8_last(p) : (kCold ? ld_gather_f8_first(p) : ld_gather_f8(p));
+  return kCold ? ld_gather_f8_first(p) : ld_gather_f8(p);
 }
 __device__ __forceinline__ void f8_fma(f8& acc, float s, const f8& x) {
   f4_fma(acc.a, s, x.a);
   f4_fma(acc.b, s, x.b);
+}
+
+// One 32-edge batch of a row or segment: rem (> 0) = edges left from the batch's first edge on, (c, v) = this
+// lane's edge of the batch.  Group g adds batch edges [g*LPR8, (g+1)*LPR8) to acc in edge order.
+template <int D, int U, bool kHot, bool kCold = kHot>
+__device__ __forceinline__ void batch_accumulate8(f8& acc, const float* Xs, int c, float v, int rem, int grp) {
+  constexpr int LPR8 = D / 8;          // lanes per row = edges per group per batch = shuffle width
+  static_assert(LPR8 % U == 0, "U must divide the group's share of a batch");
+  if (rem >= 32) {
+#pragma unroll
+    for (int k0 = 0; k0 < LPR8; k0 += U) {
+      f8 x[U];
+      float vv[U];
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int cc = __shfl_sync(kFull, c, k0 + u, LPR8);
+        vv[u] = __shfl_sync(kFull, v, k0 + u, LPR8);
+        x[u] = gather_row8<D, kHot, kCold>(Xs, cc);
+      }
+#pragma unroll
+      for (int u = 0; u < U; ++u) f8_fma(acc, vv[u], x[u]);
+    }
+  } else {
+    const int ng = rem - grp * LPR8;              // edges of this group (<= 0: none)
+    const int nmax = rem < LPR8 ? rem : LPR8;     // group 0 holds the most
+#pragma unroll 1
+    for (int k0 = 0; k0 < nmax; k0 += U) {
+      f8 x[U];
+      float vv[U];
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int cc = __shfl_sync(kFull, c, k0 + u, LPR8);
+        vv[u] = __shfl_sync(kFull, v, k0 + u, LPR8);
+        if (k0 + u < ng) {
+          x[u] = gather_row8<D, kHot, kCold>(Xs, cc);
+        } else {
+          x[u].a = f4_zero();
+          x[u].b = f4_zero();
+          vv[u] = 0.f;
+        }
+      }
+#pragma unroll
+      for (int u = 0; u < U; ++u) f8_fma(acc, vv[u], x[u]);
+    }
+  }
+}
+
+// the fixed xor tree over the lane groups: afterwards every group holds the whole row
+template <int D>
+__device__ __forceinline__ void groups_reduce8(f8& acc) {
+#pragma unroll
+  for (int m = D / 8; m < 32; m <<= 1) {
+    f4_add(acc.a, f4_shfl_xor(acc.a, m));
+    f4_add(acc.b, f4_shfl_xor(acc.b, m));
+  }
 }
 
 // Sum over CSR edges [start, end) of val[e] * X[col[e], :]; returns, in the 128-bit kernels' layout (lane l <
@@ -169,8 +226,7 @@ __device__ __forceinline__ float4 warp_row_accumulate8(const int32_t* __restrict
                                                        const float* __restrict__ val,
                                                        const float* __restrict__ X, int64_t start,
                                                        int64_t end, int lane) {
-  constexpr int LPR8 = D / 8;          // lanes per row = edges per group per batch = shuffle width
-  static_assert(LPR8 % U == 0, "U must divide the group's share of a batch");
+  constexpr int LPR8 = D / 8;
   const int grp = lane / LPR8, sub = lane % LPR8;
   const float* Xs = X + sub * 8;
   f8 acc;
@@ -192,54 +248,14 @@ __device__ __forceinline__ float4 warp_row_accumulate8(const int32_t* __restrict
       cn = ld_stream_s32(cp + 32);
       vn = ld_stream_f32(vp + 32);
     }
-    if (rem >= 32) {
-#pragma unroll
-      for (int k0 = 0; k0 < LPR8; k0 += U) {
-        f8 x[U];
-        float vv[U];
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-          const int cc = __shfl_sync(kFull, c, k0 + u, LPR8);
-          vv[u] = __shfl_sync(kFull, v, k0 + u, LPR8);
-          x[u] = gather_row8<D, kHot>(Xs, cc);
-        }
-#pragma unroll
-        for (int u = 0; u < U; ++u) f8_fma(acc, vv[u], x[u]);
-      }
-    } else {
-      const int ng = rem - grp * LPR8;              // edges of this group (<= 0: none)
-      const int nmax = rem < LPR8 ? rem : LPR8;     // group 0 holds the most
-#pragma unroll 1
-      for (int k0 = 0; k0 < nmax; k0 += U) {
-        f8 x[U];
-        float vv[U];
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-          const int cc = __shfl_sync(kFull, c, k0 + u, LPR8);
-          vv[u] = __shfl_sync(kFull, v, k0 + u, LPR8);
-          if (k0 + u < ng) {
-            x[u] = gather_row8<D, kHot>(Xs, cc);
-          } else {
-            x[u].a = f4_zero();
-            x[u].b = f4_zero();
-            vv[u] = 0.f;
-          }
-        }
-#pragma unroll
-        for (int u = 0; u < U; ++u) f8_fma(acc, vv[u], x[u]);
-      }
-    }
+    batch_accumulate8<D, U, kHot>(acc, Xs, c, v, rem, grp);
     c = cn;
     v = vn;
     cp += 32;
     vp += 32;
     rem -= 32;
   }
-#pragma unroll
-  for (int m = LPR8; m < 32; m <<= 1) {
-    f4_add(acc.a, f4_shfl_xor(acc.a, m));
-    f4_add(acc.b, f4_shfl_xor(acc.b, m));
-  }
+  groups_reduce8<D>(acc);
   // lane l of the 128-bit layout takes half (l & 1) of lane l / 2
   const int src = (lane >> 1) & (LPR8 - 1);
   float4 lo, hi;
@@ -577,6 +593,106 @@ spmm_seg_list_kernel(const int32_t* __restrict__ col, const float* __restrict__ 
   if (lane < LPR) *reinterpret_cast<float4*>(partial + (int64_t)seg * D + lane * 4) = acc;
 }
 
+// Segments of the column-blocked list per warp: a run of kHubRun consecutive hub cells (segments
+// [0, n_hub_seg), block-major, so a run gathers from one window), or of kMidRun mid-row segments.  A hub cell
+// has a median of ~31 edges: as a CTA of its own it was one partial batch, the tree and a store with nothing
+// else in flight (and a CTA launch per cell).  Here the run's (start, count) pairs are loaded once, and the
+// last batch of a cell loads the next cell's first (col, val) batch, so it is in flight during the current
+// gathers, tree and store.
+#ifndef SPEX_SEG_HUB_RUN
+#define SPEX_SEG_HUB_RUN 8
+#endif
+#ifndef SPEX_SEG_MID_RUN
+#define SPEX_SEG_MID_RUN 2
+#endif
+constexpr int kHubRun = SPEX_SEG_HUB_RUN, kMidRun = SPEX_SEG_MID_RUN;
+static_assert(kHubRun <= 32 && kMidRun <= 32, "a run's segment extents are held one per lane");
+
+// Segments [first, first + n) into their partial rows, each summed exactly as warp_row_accumulate8 sums it.
+// kCold: L2 priority of the gathers (evict_first for mid rows, which have no reuse; the default priority for
+// hub cells, whose window the block-major order exists to keep in L2).
+template <int D, bool kHot, bool kCold>
+__device__ __forceinline__ void seg_run8(const int32_t* __restrict__ col, const float* __restrict__ val,
+                                         const float* __restrict__ X, const int64_t* __restrict__ seg_start,
+                                         const int32_t* __restrict__ seg_count, int first, int n,
+                                         float* __restrict__ partial, int lane) {
+  constexpr int LPR8 = D / 8, U = D >= 64 ? SPEX_V8_U : D / 8;
+  const int grp = lane / LPR8, sub = lane % LPR8;
+  const float* Xs = X + sub * 8;
+  int64_t my_start = 0;      // lane k < n: extent of segment first + k
+  int my_cnt = 0;
+  if (lane < n) {
+    my_start = seg_start[first + lane];
+    my_cnt = seg_count[first + lane];
+  }
+  int64_t start = __shfl_sync(kFull, my_start, 0);
+  int rem = __shfl_sync(kFull, my_cnt, 0);
+  int c = 0;
+  float v = 0.f;
+  if (lane < rem) {
+    c = ld_stream_s32(col + start + lane);
+    v = ld_stream_f32(val + start + lane);
+  }
+#pragma unroll 1
+  for (int k = 0; k < n; ++k) {
+    const int64_t nstart = __shfl_sync(kFull, my_start, (k + 1) & 31);
+    const int ncnt = k + 1 < n ? __shfl_sync(kFull, my_cnt, (k + 1) & 31) : 0;
+    f8 acc;
+    acc.a = f4_zero();
+    acc.b = f4_zero();
+    int64_t e = start + lane;
+#pragma unroll 1
+    while (rem > 0) {
+      int cn = 0;
+      float vn = 0.f;
+      if (rem > 32) {                  // next batch of this segment
+        if (lane + 32 < rem) {
+          cn = ld_stream_s32(col + e + 32);
+          vn = ld_stream_f32(val + e + 32);
+        }
+      } else if (lane < ncnt) {        // first batch of the next segment
+        cn = ld_stream_s32(col + nstart + lane);
+        vn = ld_stream_f32(val + nstart + lane);
+      }
+      batch_accumulate8<D, U, kHot, kCold>(acc, Xs, c, v, rem, grp);
+      c = cn;
+      v = vn;
+      e += 32;
+      rem -= 32;
+    }
+    groups_reduce8<D>(acc);
+    // group 0 stores the row (lane l: floats [8l, 8l+8)), streaming: the partials are read once by the fix-up
+    // and must not push the window out of L2
+    if (lane < LPR8) {
+      float* p = partial + (int64_t)(first + k) * D + lane * 8;
+      st_stream_f4(p, acc.a);
+      st_stream_f4(p + 4, acc.b);
+    }
+    start = nstart;
+    rem = ncnt;
+  }
+}
+
+template <int D, bool kHot>
+__global__ void __launch_bounds__(32, SPEX_V8_MINB)
+spmm_seg_runs_kernel(const int32_t* __restrict__ col, const float* __restrict__ val, const float* __restrict__ X,
+                     const int64_t* __restrict__ seg_start, const int32_t* __restrict__ seg_count, int32_t n_seg,
+                     int32_t n_hub_seg, float* __restrict__ partial) {
+  const int lane = threadIdx.x;
+  const int hub_warps = (n_hub_seg + kHubRun - 1) / kHubRun;
+  const int w = blockIdx.x;
+  if (w < hub_warps) {
+    const int first = w * kHubRun;
+    const int n = min(kHubRun, n_hub_seg - first);
+    seg_run8<D, kHot, false>(col, val, X, seg_start, seg_count, first, n, partial, lane);
+  } else {
+    const int first = n_hub_seg + (w - hub_warps) * kMidRun;
+    if (first >= n_seg) return;
+    const int n = min(kMidRun, n_seg - first);
+    seg_run8<D, kHot, kHot>(col, val, X, seg_start, seg_count, first, n, partial, lane);
+  }
+}
+
 // warp per long row: sum its partial rows in column-block order (fixed order), then the epilogue
 template <int D, int U>
 __global__ void __launch_bounds__(kRowsPerCta * 32)
@@ -653,6 +769,14 @@ spmm_rows_generic_kernel(const int64_t* __restrict__ rowptr, const int32_t* __re
 
 static bool g_rows_only = false;   // spex_debug_spmm_rows: launch the short-row kernel alone
 
+// SPEX_SPMM_SEG_LEGACY=1: column-blocked segment lists take spmm_seg_list_kernel (one segment per CTA, every
+// non-hot gather evict_first) instead of spmm_seg_runs_kernel - same bits, the A/B reference.  Read at every
+// launch so that one process can compare the two.
+static bool seg_legacy() {
+  const char* e = getenv("SPEX_SPMM_SEG_LEGACY");
+  return e && e[0] == '1';
+}
+
 // Row subset of one layer (spex_spmm_csr_rows_f32): only the listed rows are computed.  `rows` lists them all
 // (the rows kernel skips the long ones exactly as in a full layer); the listed rows that take the long-row path
 // are given again as slots into plan->long_rows, together with the ids of their segments, so that they run
@@ -712,8 +836,15 @@ static int launch_vec_h(const int64_t* rowptr, const int32_t* col, const float* 
     const int gs = (n_seg + kRowsPerCta - 1) / kRowsPerCta;
     const int gf = (n_long + kRowsPerCta - 1) / kRowsPerCta;
     if (plan->seg_start) {   // explicit segment list (column-blocked hubs + fixed-length rest)
-      spmm_seg_list_kernel<D, U, kHot, kV8, kMask><<<gs, kRowsPerCta * 32, 0, st>>>(
-          col, val, X, plan->seg_start, plan->seg_count, n_seg, plan->partial, seg_sel, nz);
+      if (kV8 && !kMask && !sub && !seg_legacy()) {
+        const int n_mid = n_seg - plan->n_hub_seg;
+        const int gr = (plan->n_hub_seg + kHubRun - 1) / kHubRun + (n_mid + kMidRun - 1) / kMidRun;
+        spmm_seg_runs_kernel<D, kHot><<<gr, 32, 0, st>>>(col, val, X, plan->seg_start, plan->seg_count, n_seg,
+                                                         plan->n_hub_seg, plan->partial);
+      } else {
+        spmm_seg_list_kernel<D, U, kHot, kV8, kMask><<<gs, kRowsPerCta * 32, 0, st>>>(
+            col, val, X, plan->seg_start, plan->seg_count, n_seg, plan->partial, seg_sel, nz);
+      }
       spmm_long_fix_list_kernel<D, U><<<gf, kRowsPerCta * 32, 0, st>>>(
           plan->long_rows, plan->long_segptr, plan->row_seg, n_long, plan->partial, ep, slot_sel);
     } else {                 // fixed-length segmentation
@@ -765,6 +896,7 @@ int spmm_launch(const int64_t* rowptr, const int32_t* col, const float* val, con
                        !plan->partial || plan->n_seg < plan->n_long,
                    SPEX_E_BADARG);
     SPEX_RETURN_IF(plan->seg_start && (!plan->seg_count || !plan->row_seg), SPEX_E_BADARG);
+    SPEX_RETURN_IF(plan->n_hub_seg < 0 || plan->n_hub_seg > plan->n_seg, SPEX_E_BADARG);
     SPEX_RETURN_IF(!aligned16(plan->partial), SPEX_E_ALIGN);
   }
   if (n_rows == 0) return 0;

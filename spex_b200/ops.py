@@ -175,6 +175,7 @@ class DeviceGraph:
         self.n_long = int(long_rows.numel())
         self.long_rows = long_rows.to(torch.int32)
         self.seg_start = self.seg_count = self.row_seg = None
+        self.n_hub_seg = 0
         self._plan_D = 0
         if self.n_long == 0:
             self.long_segptr = torch.zeros(1, dtype=torch.int32, device=dev)
@@ -207,6 +208,7 @@ class DeviceGraph:
         hub_slots = torch.nonzero(is_hub).flatten()       # indices into long_rows
         mid_slots = torch.nonzero(~is_hub).flatten()
         parts_start, parts_cnt, parts_row = [], [], []
+        n_hub_cells = 0                                   # hub cells come first in the list
         if hub_slots.numel():
             hrows = long_rows[hub_slots]
             nh = hrows.numel()
@@ -227,6 +229,7 @@ class DeviceGraph:
             cr = hub_slots.repeat(n_cb)
             keep = cc > 0
             parts_start.append(cs[keep]); parts_cnt.append(cc[keep]); parts_row.append(cr[keep])
+            n_hub_cells = int(parts_cnt[0].numel())
         if mid_slots.numel():
             mrows = long_rows[mid_slots]
             parts_start.append(self.rowptr[mrows]); parts_cnt.append(deg[mrows]); parts_row.append(mid_slots)
@@ -242,6 +245,7 @@ class DeviceGraph:
         seg_row = cell_row[seg_cell]
         self.n_seg = int(seg_start.numel())
         self.n_hub = int(hub_slots.numel())
+        self.n_hub_seg = int(pieces[:n_hub_cells].sum())
         if self.n_seg >= 2 ** 31:
             raise ValueError("too many long-row segments")
         # per row, segments in ascending edge order = fixed summation order
@@ -377,7 +381,8 @@ class DeviceGraph:
                               self.long_segptr.data_ptr(), partial.data_ptr(),
                               self.seg_start.data_ptr() if self.seg_start is not None else None,
                               self.seg_count.data_ptr() if self.seg_count is not None else None,
-                              self.row_seg.data_ptr() if self.row_seg is not None else None, *tail)
+                              self.row_seg.data_ptr() if self.row_seg is not None else None, *tail,
+                              self.n_hub_seg)
                 self._plan_tensors = (partial, hot_partial)
             self._plan_struct = st
             self._plan_D = D
