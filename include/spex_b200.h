@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define SPEX_ABI_VERSION 1
+#define SPEX_ABI_VERSION 2
 
 /* argument errors (negative; positive values are cudaError_t) */
 #define SPEX_E_BADARG   (-1)  /* null pointer / negative size */
@@ -43,32 +43,25 @@ int spex_device_check(int* sm_count, int* cc_major, int* cc_minor);
 int64_t spex_launch_count(void);
 
 /* ------------------------------------------------------------------------------------------
- * Long-row plan.  Rows with more than `seg_len` non-zeros are cut into segments; each segment is
- * reduced by one warp into a partial row and the partials of a row are summed in a fixed order
- * (deterministic two-pass — no atomics).  Two segmentations:
- *   fixed-length   (seg_start == NULL): segments of seg_len consecutive edges; segment j of long
- *                  row r is partial row long_segptr[r] + j;
- *   column-blocked (seg_start != NULL): segments are (row, column block) pairs listed in
- *                  BLOCK-MAJOR order so that concurrently running warps gather from one L2-sized
- *                  window of the table; row_seg lists each row's segments in column order.
+ * Long-row plan.  Rows with more than `seg_len` non-zeros are cut into segments of at most seg_len
+ * edges; each segment is reduced by one warp into a partial row and the partials of a row are
+ * summed in a fixed order (deterministic two-pass — no atomics).  The segments form one list:
+ *   [0, n_hub_seg)     hub-row cells: a hub row is cut at column-block boundaries (and a cell longer
+ *                      than seg_len every seg_len edges), and the cells are listed BLOCK-MAJOR so that
+ *                      concurrently running warps gather from one L2-sized window of the table;
+ *   [n_hub_seg, n_seg) mid-row segments: every other long row is cut every seg_len edges from its
+ *                      first edge, listed in ascending row order.
+ * A table that fits in L2 has no hub rows (n_hub_seg == 0).  row_seg lists each long row's segments
+ * in edge order: long row r owns row_seg[long_segptr[r] .. long_segptr[r+1]), and its partials are
+ * summed in that order.
  * The plan is built once per graph by the host (spex_b200/ops.py: DeviceGraph) and passed to every
  * SpMM as a HOST struct holding device pointers; NULL (or n_long == 0) means "no long rows".
  * ------------------------------------------------------------------------------------------ */
 /* flags: bit 31 of every col[] entry marks a HOT table row (one that is gathered so often that it
  * should stay in L2): the kernels strip the bit and gather hot rows with the L2 evict_last policy,
- * all others with evict_first.  A plan with n_long == 0 may still carry this flag. */
+ * all others with evict_first.  A plan with n_long == 0 may still carry this flag.  No other flag
+ * bit is defined: a plan that sets one is rejected with SPEX_E_BADARG. */
 #define SPEX_PLAN_COL_HOTBIT 1
-/* two-pass rows: inside every short row of [0, n_split_rows) the hot edges were moved to the
- * front (rowmid[r] = first cold edge).  Pass A reduces only hot edges - its working set is the hot
- * part of the table plus streamed (col, val), so it stays L2-resident by construction - into
- * hot_partial; pass B reduces the cold edges (pure streaming) and adds the partial row.  Needs
- * SPEX_PLAN_COL_HOTBIT. */
-#define SPEX_PLAN_TWO_PASS 2
-/* rows [0, interleave_split) and [interleave_split, n_rows) are two classes with different
- * bottlenecks (user rows gather popular item rows out of L2, item rows gather random user rows out
- * of DRAM): the short-row kernel visits them interleaved in proportion, so that L2-bound and
- * DRAM-bound work overlap instead of running one after the other. */
-#define SPEX_PLAN_INTERLEAVE 4
 
 typedef struct spex_long_plan {
   int32_t seg_len;            /* rows with degree > seg_len take the long-row path (>= 32)    */
@@ -78,16 +71,12 @@ typedef struct spex_long_plan {
   const int32_t* long_rows;   /* int32 [n_long]    row ids, ascending                         */
   const int32_t* long_segptr; /* int32 [n_long+1]  exclusive scan of segments per long row    */
   float* partial;             /* fp32  [n_seg, D]  workspace                                  */
-  const int64_t* seg_start;   /* int64 [n_seg]  first edge of each segment (NULL: fixed-length) */
+  const int64_t* seg_start;   /* int64 [n_seg]  first edge of each segment                    */
   const int32_t* seg_count;   /* int32 [n_seg]  edges in each segment                         */
-  const int32_t* row_seg;     /* int32 [n_seg]  segment ids grouped by long row, column order */
-  const int64_t* rowmid;      /* int64 [n_rows]  SPEX_PLAN_TWO_PASS: first cold edge of every row */
-  float* hot_partial;         /* fp32  [n_split_rows, D] workspace of pass A                   */
-  int64_t n_split_rows;       /* rows [0, n_split_rows) take part in pass A                    */
-  int64_t interleave_split;   /* SPEX_PLAN_INTERLEAVE: first row of the second class           */
-  int32_t n_hub_seg;          /* column-blocked list: segments [0, n_hub_seg) are hub-row cells, gathered
-                                 with the default L2 priority so that their window stays resident; the
-                                 rest are mid-row segments (no reuse: evict_first under COL_HOTBIT)     */
+  const int32_t* row_seg;     /* int32 [n_seg]  segment ids grouped by long row, edge order   */
+  int32_t n_hub_seg;          /* segments [0, n_hub_seg) are hub-row cells, gathered with the default L2
+                                 priority so that their window stays resident; the rest are mid-row
+                                 segments (no reuse: evict_first under COL_HOTBIT)                   */
 } spex_long_plan;
 
 /*

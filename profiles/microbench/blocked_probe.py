@@ -15,7 +15,7 @@ del keys
 D = 64
 N = g.n_rows
 X = synthetic.xavier_table(nu + 1, m, D, 1, dev)
-print("n_long", g.n_long, "n_seg", g.n_seg, "blocked", g.seg_start is not None)
+print("n_long", g.n_long, "n_seg", g.n_seg, "blocked", g.n_hub_seg > 0)
 cnt = g.seg_count.long()
 print("segment edges: mean %.1f  median %d  p90 %d  max %d  total %d" % (
     cnt.float().mean(), cnt.median(), cnt.float().quantile(0.9), cnt.max(), cnt.sum()))

@@ -32,10 +32,6 @@ class LongPlan(C.Structure):
         ("seg_start", _p),
         ("seg_count", _p),
         ("row_seg", _p),
-        ("rowmid", _p),
-        ("hot_partial", _p),
-        ("n_split_rows", _i64),
-        ("interleave_split", _i64),
         ("n_hub_seg", _i32),
     ]
 

@@ -13,13 +13,14 @@
 //     FMA; the batch's edges are dealt to the lane groups in consecutive runs so that a segmented shuffle with
 //     an immediate lane delivers them; hot columns (bit 31 of col) load with L2::evict_last, the rest with
 //     evict_first (static qualifiers, 256-bit loads only).  4.2 instructions per edge.
-//     Fallback for 16-byte aligned tables / SPEX_SPMM_LDG128=1: the 128-bit loop of round 1
+//     Fallback for tables that are only 16-byte aligned: the 128-bit loop of round 1
 //     (warp_row_accumulate: 16 lanes per row, policy descriptors);
 //   * lane groups accumulate disjoint edge runs in edge order and are combined by a fixed xor-shuffle tree: the
 //     summation order is a pure function of the row => bit-reproducible, no atomics;
-//   * rows longer than plan->seg_len are skipped here and reduced by two extra launches (warp per segment ->
-//     partial rows -> warp per long row), hub rows cut at column-block boundaries and listed block-major so
-//     that the table window they gather from stays in L2 (a warp reduces a run of such cells back to back);
+//   * rows longer than plan->seg_len are skipped here and reduced by two extra launches over the plan's segment
+//     list (warp per run of segments -> partial rows -> warp per long row): hub rows cut at column-block
+//     boundaries and listed block-major so that the table window they gather from stays in L2, the other long
+//     rows cut every seg_len edges;
 //   * epilogue: Y = acc (next layer's input) and/or Z = (addend*a + acc)*b (running layer mean forward,
 //     g + A^T G backward), optionally stored into every peer's table (P2P or one NVLS multicast store), with the
 //     next call's table or a dense Adam step riding on the last layer (row-partitioned modes);
@@ -28,7 +29,6 @@
 //     keep every computed row bit-identical to the full dense layer.
 #include "common.cuh"
 #include <math.h>
-#include <stdlib.h>
 
 namespace spex {
 
@@ -42,18 +42,14 @@ struct RowShape {
 };
 
 // Sum over edges e in [start,end) of val[e] * X[col[e], :], returned in every lane for the
-// float4 slot `lane % LPR`.  kMode 0: CSR edges; 1: col[e] = e, val[e] = 1 (sum of consecutive
-// partial rows); 2: col[e] from the list, val[e] = 1 (sum of listed partial rows).
-// kFirst: the first 32 edges' (col, val) were loaded by the caller (c0, v0) while the previous row
-// was being reduced (software prefetch in the persistent kernels).
+// float4 slot `lane % LPR`.  kList: col[e] lists partial rows of X and val[e] = 1 (val is not read).
 // kHot: bit 31 of a column index flags a hot table row (spex_long_plan.flags & SPEX_PLAN_COL_HOTBIT):
 // hot rows are gathered with the L2 evict_last policy, the rest with evict_first.
-template <int D, int U, int kMode, bool kFirst = false, bool kHot = false>
+template <int D, int U, bool kList, bool kHot = false>
 __device__ __forceinline__ float4 warp_row_accumulate(const int32_t* __restrict__ col,
                                                       const float* __restrict__ val,
                                                       const float* __restrict__ X, int64_t start,
-                                                      int64_t end, int lane, int c0 = 0,
-                                                      float v0 = 0.f) {
+                                                      int64_t end, int lane) {
   constexpr int LPR = RowShape<D>::LPR, G = RowShape<D>::G;
   const int grp = lane / LPR, sub = lane % LPR;
   const float* Xs = X + sub * 4;
@@ -67,20 +63,9 @@ __device__ __forceinline__ float4 warp_row_accumulate(const int32_t* __restrict_
     const int64_t e = base + lane;
     int c = 0;
     float v = 0.f;
-    if (kFirst && base == start) {
-      c = c0;
-      v = v0;
-    } else if (e < end) {
-      if (kMode == 1) {
-        c = (int)e;
-        v = 1.f;
-      } else if (kMode == 2) {
-        c = ld_stream_s32(col + e);
-        v = 1.f;
-      } else {
-        c = ld_stream_s32(col + e);
-        v = ld_stream_f32(val + e);
-      }
+    if (e < end) {
+      c = ld_stream_s32(col + e);
+      v = kList ? 1.f : ld_stream_f32(val + e);
     }
     const int n = (int)((end - base) < 32 ? (end - base) : 32);
 #pragma unroll 1
@@ -389,7 +374,7 @@ __device__ __forceinline__ float4 row_sum(const int32_t* __restrict__ col, const
                                           const uint8_t* __restrict__ nz = nullptr) {
   if (kV8 && kMask) return warp_row_accumulate8_masked<D, kHot>(col, val, X, nz, start, end, lane);
   if (kV8) return warp_row_accumulate8<D, (D >= 64 ? SPEX_V8_U : D / 8), kHot>(col, val, X, start, end, lane);
-  return warp_row_accumulate<D, U, 0, false, kHot>(col, val, X, start, end, lane);
+  return warp_row_accumulate<D, U, false, kHot>(col, val, X, start, end, lane);
 }
 
 struct Epilogue {
@@ -405,9 +390,6 @@ struct Epilogue {
   // or ONE store to an NVSwitch multicast mapping of the peers' tables (NVLS): the switch
   // replicates it into every GPU's copy, so the row leaves this GPU once instead of P-1 times
   float* mcast;
-  // two-pass rows (SPEX_PLAN_TWO_PASS): partial row of the hot pass, added before anything else
-  const float* partial_in;
-  int64_t n_partial;
   // piggy-backed publish (row partition, last layer): the warp that finishes output row r also copies
   // row r of `pub_src` (this rank's slice of the NEXT call's table) into every rank's table - one
   // multimem.st to `pub_mcast`, or P2P stores to `pub_peer[]` - so the E^(0) exchange of the next
@@ -437,7 +419,6 @@ __device__ __forceinline__ void row_epilogue(const Epilogue& ep, float4 acc, int
   constexpr int LPR = RowShape<D>::LPR;
   if (lane < LPR) {
     const int64_t off = row * D + lane * 4;
-    if (ep.partial_in && row < ep.n_partial) f4_add(acc, ld_stream_f4(ep.partial_in + off));
     if (ep.Y) *reinterpret_cast<float4*>(ep.Y + off) = acc;
     if (ep.mcast) {
       st_multimem_f4(ep.mcast + (row + ep.peer_row_offset) * D + lane * 4, acc);
@@ -499,25 +480,14 @@ template <int D, int U, bool kHot, bool kV8, bool kMask>
 __global__ void __launch_bounds__(kRowsPerCta * 32, SPEX_V8_MINB / kRowsPerCta)
 spmm_rows_kernel(const int64_t* __restrict__ rowptr, const int32_t* __restrict__ col,
                  const float* __restrict__ val, const float* __restrict__ X, int64_t n_rows,
-                 int32_t skip_longer_than, Epilogue ep, const int64_t* __restrict__ rowmid, int pass,
-                 int64_t split, const int32_t* __restrict__ row_sel, const uint8_t* __restrict__ nz) {
+                 int32_t skip_longer_than, Epilogue ep, const int32_t* __restrict__ row_sel,
+                 const uint8_t* __restrict__ nz) {
   const int lane = threadIdx.x & 31;
   int64_t row = (int64_t)blockIdx.x * kRowsPerCta + (threadIdx.x >> 5);
   if (row >= n_rows) return;
-  if (row_sel) {
-    row = row_sel[row];        // row subset (spex_spmm_csr_rows_f32): n_rows = length of the list
-  } else if (split > 0) {
-    // SPEX_PLAN_INTERLEAVE: slot b -> rows of class A = [0, split) and class B = [split, n_rows)
-    // taken in proportion (B gets slot b iff floor((b+1) nb / n) > floor(b nb / n)); a bijection
-    const int64_t nb = n_rows - split;
-    const int64_t kb = (row * nb) / n_rows, kb1 = ((row + 1) * nb) / n_rows;
-    row = (kb1 > kb) ? split + kb : row - kb;
-  }
-  int64_t start = rowptr[row], end = rowptr[row + 1];
-  if (skip_longer_than > 0 && end - start > skip_longer_than) return;  // long-row path
-  // two-pass rows: pass 1 = hot edges [start, rowmid), pass 2 = cold edges [rowmid, end)
-  if (pass == 1) end = rowmid[row];
-  if (pass == 2) start = rowmid[row];
+  if (row_sel) row = row_sel[row];   // row subset (spex_spmm_csr_rows_f32): n_rows = length of the list
+  const int64_t start = rowptr[row], end = rowptr[row + 1];
+  if (skip_longer_than > 0 && end > start + skip_longer_than) return;  // long-row path
   // sparse-input layers are bound by the per-row latency chain (rowptr -> col/val -> mask -> gathers -> addend):
   // ask L2 for the epilogue's addend row now (in the dense layers, which are throughput-bound, the same prefetch
   // measured no gain: profiles/r02_spmm_ldg256.md)
@@ -527,56 +497,12 @@ spmm_rows_kernel(const int64_t* __restrict__ rowptr, const int32_t* __restrict__
   row_epilogue<D>(ep, acc, row, lane);
 }
 
-// warp per segment of a long row -> partial[seg, :]
-template <int D, int U, bool kHot, bool kV8, bool kMask>
-__global__ void __launch_bounds__(kRowsPerCta * 32, SPEX_V8_MINB / kRowsPerCta)
-spmm_long_seg_kernel(const int64_t* __restrict__ rowptr, const int32_t* __restrict__ col,
-                     const float* __restrict__ val, const float* __restrict__ X,
-                     const int32_t* __restrict__ long_rows,
-                     const int32_t* __restrict__ long_segptr, int32_t n_long, int32_t n_seg,
-                     int32_t seg_len, float* __restrict__ partial, const int32_t* __restrict__ seg_sel,
-                     const uint8_t* __restrict__ nz) {
-  constexpr int LPR = RowShape<D>::LPR;
-  const int lane = threadIdx.x & 31;
-  int seg = blockIdx.x * kRowsPerCta + (threadIdx.x >> 5);
-  if (seg >= n_seg) return;
-  if (seg_sel) seg = seg_sel[seg];   // subset: n_seg = length of the list
-  // largest r with long_segptr[r] <= seg
-  int lo = 0, hi = n_long;
-  while (hi - lo > 1) {
-    const int mid = (lo + hi) >> 1;
-    if (long_segptr[mid] <= seg) lo = mid; else hi = mid;
-  }
-  const int64_t row = long_rows[lo];
-  const int k = seg - long_segptr[lo];
-  const int64_t rs = rowptr[row], re = rowptr[row + 1];
-  const int64_t start = rs + (int64_t)k * seg_len;
-  const int64_t end = (start + seg_len < re) ? start + seg_len : re;
-  const float4 acc = row_sum<D, U, kHot, kV8, kMask>(col, val, X, start, end, lane, nz);
-  if (lane < LPR) *reinterpret_cast<float4*>(partial + (int64_t)seg * D + lane * 4) = acc;
-}
-
-// warp per long row: sum its partial rows in segment order, then the usual epilogue
-template <int D, int U>
-__global__ void __launch_bounds__(kRowsPerCta * 32)
-spmm_long_fix_kernel(const int32_t* __restrict__ long_rows,
-                     const int32_t* __restrict__ long_segptr, int32_t n_long,
-                     const float* __restrict__ partial, Epilogue ep, const int32_t* __restrict__ slot_sel) {
-  const int lane = threadIdx.x & 31;
-  int r = blockIdx.x * kRowsPerCta + (threadIdx.x >> 5);
-  if (r >= n_long) return;
-  if (slot_sel) r = slot_sel[r];     // subset: n_long = length of the list
-  const float4 acc = warp_row_accumulate<D, U, 1>(nullptr, nullptr, partial, long_segptr[r],
-                                                  long_segptr[r + 1], lane);
-  row_epilogue<D>(ep, acc, (int64_t)long_rows[r], lane);
-}
-
-// ---- column-blocked long rows ----------------------------------------------------------------
-// Long rows (hub items: thousands of edges, columns spread over the whole table) are cut at fixed
-// COLUMN-block boundaries instead of fixed edge counts, and the segments are launched in
-// block-major order: at any moment the resident warps gather from one ~32 MB window of the
-// table, which the 126 MB L2 keeps resident, so each table row of the window comes from HBM once
-// instead of once per edge.  warp per (row, column block) segment -> partial[seg, :]
+// ---- long rows: the segment list of spex_long_plan ----------------------------------------------
+// Hub rows (thousands of edges, columns spread over the whole table) are cut at fixed COLUMN-block
+// boundaries, and these cells are listed in block-major order: at any moment the resident warps gather
+// from one ~32 MB window of the table, which the 126 MB L2 keeps resident, so each table row of the
+// window comes from HBM once instead of once per edge.  The other long rows (mid rows) are cut every
+// seg_len edges.  warp per segment -> partial[seg, :]
 template <int D, int U, bool kHot, bool kV8, bool kMask>
 __global__ void __launch_bounds__(kRowsPerCta * 32, SPEX_V8_MINB / kRowsPerCta)
 spmm_seg_list_kernel(const int32_t* __restrict__ col, const float* __restrict__ val,
@@ -593,7 +519,7 @@ spmm_seg_list_kernel(const int32_t* __restrict__ col, const float* __restrict__ 
   if (lane < LPR) *reinterpret_cast<float4*>(partial + (int64_t)seg * D + lane * 4) = acc;
 }
 
-// Segments of the column-blocked list per warp: a run of kHubRun consecutive hub cells (segments
+// Segments of the list per warp: a run of kHubRun consecutive hub cells (segments
 // [0, n_hub_seg), block-major, so a run gathers from one window), or of kMidRun mid-row segments.  A hub cell
 // has a median of ~31 edges: as a CTA of its own it was one partial batch, the tree and a store with nothing
 // else in flight (and a CTA launch per cell).  Here the run's (start, count) pairs are loaded once, and the
@@ -693,7 +619,7 @@ spmm_seg_runs_kernel(const int32_t* __restrict__ col, const float* __restrict__ 
   }
 }
 
-// warp per long row: sum its partial rows in column-block order (fixed order), then the epilogue
+// warp per long row: sum its partial rows in edge order (row_seg: a fixed order), then the epilogue
 template <int D, int U>
 __global__ void __launch_bounds__(kRowsPerCta * 32)
 spmm_long_fix_list_kernel(const int32_t* __restrict__ long_rows,
@@ -704,8 +630,8 @@ spmm_long_fix_list_kernel(const int32_t* __restrict__ long_rows,
   int r = blockIdx.x * kRowsPerCta + (threadIdx.x >> 5);
   if (r >= n_long) return;
   if (slot_sel) r = slot_sel[r];     // subset: n_long = length of the list
-  const float4 acc = warp_row_accumulate<D, U, 2>(row_seg, nullptr, partial, long_segptr[r],
-                                                  long_segptr[r + 1], lane);
+  const float4 acc = warp_row_accumulate<D, U, true>(row_seg, nullptr, partial, long_segptr[r],
+                                                     long_segptr[r + 1], lane);
   row_epilogue<D>(ep, acc, (int64_t)long_rows[r], lane);
 }
 
@@ -769,14 +695,6 @@ spmm_rows_generic_kernel(const int64_t* __restrict__ rowptr, const int32_t* __re
 
 static bool g_rows_only = false;   // spex_debug_spmm_rows: launch the short-row kernel alone
 
-// SPEX_SPMM_SEG_LEGACY=1: column-blocked segment lists take spmm_seg_list_kernel (one segment per CTA, every
-// non-hot gather evict_first) instead of spmm_seg_runs_kernel - same bits, the A/B reference.  Read at every
-// launch so that one process can compare the two.
-static bool seg_legacy() {
-  const char* e = getenv("SPEX_SPMM_SEG_LEGACY");
-  return e && e[0] == '1';
-}
-
 // Row subset of one layer (spex_spmm_csr_rows_f32): only the listed rows are computed.  `rows` lists them all
 // (the rows kernel skips the long ones exactly as in a full layer); the listed rows that take the long-row path
 // are given again as slots into plan->long_rows, together with the ids of their segments, so that they run
@@ -800,30 +718,9 @@ static int launch_vec_h(const int64_t* rowptr, const int32_t* col, const float* 
   const int64_t n_work = sub ? sub->n_rows : n_rows;
   const int64_t grid = (n_work + kRowsPerCta - 1) / kRowsPerCta;
   if (grid > 0x7fffffffLL) return SPEX_E_TOOBIG;
-  const int64_t split = (!sub && plan && (plan->flags & SPEX_PLAN_INTERLEAVE) && plan->interleave_split > 0 &&
-                         plan->interleave_split < n_rows)
-                            ? plan->interleave_split
-                            : 0;
-  const int32_t* row_sel = sub ? sub->rows : nullptr;
-  if (!sub && !kMask && kHot && plan && (plan->flags & SPEX_PLAN_TWO_PASS) && plan->rowmid && plan->hot_partial) {
-    const int64_t nA = plan->n_split_rows < n_rows ? plan->n_split_rows : n_rows;
-    Epilogue epA{};
-    epA.Y = plan->hot_partial;
-    const int64_t gridA = (nA + kRowsPerCta - 1) / kRowsPerCta;
-    if (gridA > 0) {
-      spmm_rows_kernel<D, U, kHot, kV8, false><<<(unsigned)gridA, kRowsPerCta * 32, 0, st>>>(
-          rowptr, col, val, X, nA, has_long ? plan->seg_len : 0, epA, plan->rowmid, 1, 0, nullptr, nullptr);
-      count_launch();
-    }
-    Epilogue epB = ep;
-    epB.partial_in = plan->hot_partial;
-    epB.n_partial = nA;
-    spmm_rows_kernel<D, U, kHot, kV8, false><<<(unsigned)grid, kRowsPerCta * 32, 0, st>>>(
-        rowptr, col, val, X, n_rows, has_long ? plan->seg_len : 0, epB, plan->rowmid, 2, split, nullptr, nullptr);
-    count_launch();
-  } else if (grid > 0) {
+  if (grid > 0) {
     spmm_rows_kernel<D, U, kHot, kV8, kMask><<<(unsigned)grid, kRowsPerCta * 32, 0, st>>>(
-        rowptr, col, val, X, n_work, has_long ? plan->seg_len : 0, ep, nullptr, 0, split, row_sel, nz);
+        rowptr, col, val, X, n_work, has_long ? plan->seg_len : 0, ep, sub ? sub->rows : nullptr, nz);
     count_launch();
   }
   if (rows_only) return check_last();
@@ -835,25 +732,20 @@ static int launch_vec_h(const int64_t* rowptr, const int32_t* col, const float* 
     if (n_long == 0) return check_last();
     const int gs = (n_seg + kRowsPerCta - 1) / kRowsPerCta;
     const int gf = (n_long + kRowsPerCta - 1) / kRowsPerCta;
-    if (plan->seg_start) {   // explicit segment list (column-blocked hubs + fixed-length rest)
-      if (kV8 && !kMask && !sub && !seg_legacy()) {
-        const int n_mid = n_seg - plan->n_hub_seg;
-        const int gr = (plan->n_hub_seg + kHubRun - 1) / kHubRun + (n_mid + kMidRun - 1) / kMidRun;
-        spmm_seg_runs_kernel<D, kHot><<<gr, 32, 0, st>>>(col, val, X, plan->seg_start, plan->seg_count, n_seg,
-                                                         plan->n_hub_seg, plan->partial);
-      } else {
-        spmm_seg_list_kernel<D, U, kHot, kV8, kMask><<<gs, kRowsPerCta * 32, 0, st>>>(
-            col, val, X, plan->seg_start, plan->seg_count, n_seg, plan->partial, seg_sel, nz);
-      }
-      spmm_long_fix_list_kernel<D, U><<<gf, kRowsPerCta * 32, 0, st>>>(
-          plan->long_rows, plan->long_segptr, plan->row_seg, n_long, plan->partial, ep, slot_sel);
-    } else {                 // fixed-length segmentation
-      spmm_long_seg_kernel<D, U, kHot, kV8, kMask><<<gs, kRowsPerCta * 32, 0, st>>>(
-          rowptr, col, val, X, plan->long_rows, plan->long_segptr, plan->n_long, n_seg,
-          plan->seg_len, plan->partial, seg_sel, nz);
-      spmm_long_fix_kernel<D, U><<<gf, kRowsPerCta * 32, 0, st>>>(
-          plan->long_rows, plan->long_segptr, n_long, plan->partial, ep, slot_sel);
+    // Runs of segments per warp pay off on a list with hub cells (a table larger than L2: millions of segments,
+    // throughput-bound).  A list of mid-row segments only (a table that fits in L2) is short and on the layer's
+    // critical path, so each of its segments gets a warp of its own (same bits either way).
+    if (kV8 && !kMask && !sub && plan->n_hub_seg > 0) {
+      const int n_mid = n_seg - plan->n_hub_seg;
+      const int gr = (plan->n_hub_seg + kHubRun - 1) / kHubRun + (n_mid + kMidRun - 1) / kMidRun;
+      spmm_seg_runs_kernel<D, kHot><<<gr, 32, 0, st>>>(col, val, X, plan->seg_start, plan->seg_count, n_seg,
+                                                       plan->n_hub_seg, plan->partial);
+    } else {
+      spmm_seg_list_kernel<D, U, kHot, kV8, kMask><<<gs, kRowsPerCta * 32, 0, st>>>(
+          col, val, X, plan->seg_start, plan->seg_count, n_seg, plan->partial, seg_sel, nz);
     }
+    spmm_long_fix_list_kernel<D, U><<<gf, kRowsPerCta * 32, 0, st>>>(
+        plan->long_rows, plan->long_segptr, plan->row_seg, n_long, plan->partial, ep, slot_sel);
     count_launch(2);
   }
   return check_last();
@@ -863,13 +755,8 @@ template <int D, int U>
 static int launch_vec(const int64_t* rowptr, const int32_t* col, const float* val, const float* X,
                       int64_t n_rows, const Epilogue& ep, const spex_long_plan* plan,
                       cudaStream_t st, const RowSubset* sub, const uint8_t* nz) {
-  // 256-bit gathers need a 32-byte aligned table (row pitch D*4 is a multiple of 32 for these D);
-  // SPEX_SPMM_LDG128=1 forces the 128-bit kernels (A/B measurements)
-  static const bool force128 = [] {
-    const char* e = getenv("SPEX_SPMM_LDG128");
-    return e && e[0] == '1';
-  }();
-  const bool v8 = !force128 && (reinterpret_cast<uintptr_t>(X) & 31u) == 0;
+  // 256-bit gathers need a 32-byte aligned table (row pitch D*4 is a multiple of 32 for these D)
+  const bool v8 = (reinterpret_cast<uintptr_t>(X) & 31u) == 0;
   const bool hot = plan && (plan->flags & SPEX_PLAN_COL_HOTBIT);
   if (nz && v8) {   // sparse-input variant (only with the 256-bit kernels; otherwise the mask is simply not used)
     if (hot) return launch_vec_h<D, U, true, true, true>(rowptr, col, val, X, n_rows, ep, plan, st, sub, nz);
@@ -891,11 +778,12 @@ int spmm_launch(const int64_t* rowptr, const int32_t* col, const float* val, con
   SPEX_RETURN_IF(D <= 0 || (D & 3) || D > 512, SPEX_E_BADDIM);
   SPEX_RETURN_IF(!aligned16(X) || !aligned16(ep.Y) || !aligned16(ep.Z) || !aligned16(ep.addend),
                  SPEX_E_ALIGN);
+  SPEX_RETURN_IF(plan && (plan->flags & ~SPEX_PLAN_COL_HOTBIT), SPEX_E_BADARG);
   if (plan && plan->n_long > 0) {
     SPEX_RETURN_IF(plan->seg_len < 32 || !plan->long_rows || !plan->long_segptr ||
                        !plan->partial || plan->n_seg < plan->n_long,
                    SPEX_E_BADARG);
-    SPEX_RETURN_IF(plan->seg_start && (!plan->seg_count || !plan->row_seg), SPEX_E_BADARG);
+    SPEX_RETURN_IF(!plan->seg_start || !plan->seg_count || !plan->row_seg, SPEX_E_BADARG);
     SPEX_RETURN_IF(plan->n_hub_seg < 0 || plan->n_hub_seg > plan->n_seg, SPEX_E_BADARG);
     SPEX_RETURN_IF(!aligned16(plan->partial), SPEX_E_ALIGN);
   }
@@ -908,7 +796,7 @@ int spmm_launch(const int64_t* rowptr, const int32_t* col, const float* val, con
   }
   SPEX_RETURN_IF(sub != nullptr, SPEX_E_BADDIM);   // row subsets: D in {32, 64, 128} only (a mask is just ignored)
   SPEX_RETURN_IF(plan && (plan->flags & SPEX_PLAN_COL_HOTBIT), SPEX_E_BADDIM);  // D in {32,64,128} only
-  SPEX_RETURN_IF(ep.partial_in != nullptr || ep.pub_src != nullptr || ep.adam_p != nullptr, SPEX_E_BADDIM);  // same
+  SPEX_RETURN_IF(ep.pub_src != nullptr || ep.adam_p != nullptr, SPEX_E_BADDIM);  // same
   // generic path handles long rows serially (no plan needed; still deterministic)
   const int64_t grid = (n_rows + kRowsPerCta - 1) / kRowsPerCta;
   if (grid > 0x7fffffffLL) return SPEX_E_TOOBIG;

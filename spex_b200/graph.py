@@ -170,24 +170,6 @@ def transpose_positions(g: CSRGraph) -> np.ndarray:
     return tpos
 
 
-def plan_long_rows(rowptr: np.ndarray, seg_len: int = DEFAULT_SEG_LEN):
-    """Rows with more than seg_len edges -> (long_rows int32, long_segptr int32).
-
-    Mirrors spex_long_plan in include/spex_b200.h: long_segptr is the exclusive scan of
-    ceil(deg / seg_len) over the long rows.
-    """
-    if seg_len < 32:
-        raise ValueError("seg_len must be >= 32")
-    deg = np.diff(np.asarray(rowptr, dtype=np.int64))
-    long_rows = np.nonzero(deg > seg_len)[0].astype(np.int32)
-    nseg = (deg[long_rows] + seg_len - 1) // seg_len
-    segptr = np.zeros(long_rows.size + 1, dtype=np.int64)
-    np.cumsum(nseg, out=segptr[1:])
-    if segptr[-1] >= 2**31:
-        raise ValueError("too many long-row segments")
-    return long_rows, segptr.astype(np.int32)
-
-
 def partition_rows_by_nnz(rowptr: np.ndarray, parts: int, row_cost: float = 2.0) -> List[int]:
     """Contiguous row ranges with balanced work = nnz + row_cost * rows (SURVEY §8e).
 

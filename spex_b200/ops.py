@@ -23,7 +23,7 @@ import torch
 
 from . import _capi
 from ._capi import LongPlan, call, ptr, stream_ptr
-from .graph import CSRGraph, DEFAULT_SEG_LEN, plan_long_rows
+from .graph import CSRGraph, DEFAULT_SEG_LEN
 
 
 class _Workspaces:
@@ -114,6 +114,8 @@ class DeviceGraph:
     for the 1B-edge graph that is 16 GB for (col,val) and 120 MB for rowptr.
     """
 
+    interleave_split = 0   # always 0: bench.py still reports it (config.interleaved_row_classes)
+
     def __init__(self, rowptr, col, val, n_cols: int, tpos=None, seg_len: int = DEFAULT_SEG_LEN,
                  row_offset: int = 0, symmetric: bool = True, D_hint: int = 64, col_hot: bool = False):
         _need_cuda(rowptr, col, val)
@@ -130,9 +132,6 @@ class DeviceGraph:
         self._plan_struct = None
         self._plan_D = 0
         self._plan_tensors = None
-        self.interleave_split = 0     # first row of the second row class (SPEX_PLAN_INTERLEAVE)
-        self.rowmid = None            # first cold edge of every row (SPEX_PLAN_TWO_PASS)
-        self.n_split_rows = 0
         self.col_hot = False          # bit 31 of col flags hot table rows (SPEX_PLAN_COL_HOTBIT)
         if col_hot:                   # a row block cut from an already marked graph
             self.col_hot = True
@@ -169,94 +168,90 @@ class DeviceGraph:
     HUB_EDGES_PER_BLOCK = 16     # average edges per (row, column block) that make blocking pay (r02 sweep, ms per layer / GB of DRAM reads of the segment kernel: 64 -> 52.4 / 118, 32 -> 51.3 / 98, 16 -> 51.4 / 84)
 
     def _build_plan(self, D: int):
-        dev = self.device
-        deg = self.rowptr[1:] - self.rowptr[:-1]
-        long_rows = torch.nonzero(deg > self.seg_len).flatten()
-        self.n_long = int(long_rows.numel())
-        self.long_rows = long_rows.to(torch.int32)
-        self.seg_start = self.seg_count = self.row_seg = None
-        self.n_hub_seg = 0
+        self.__dict__.update(self.long_row_plan(self.rowptr, self.col, self.n_cols, self.seg_len, D))
         self._plan_D = 0
-        if self.n_long == 0:
-            self.long_segptr = torch.zeros(1, dtype=torch.int32, device=dev)
-            self.n_seg = 0
-            return
-        table_bytes = self.n_cols * D * 4
-        if table_bytes <= 4 * self.L2_WINDOW_BYTES:
-            # fixed-length segments (the whole table fits in L2 anyway)
-            nseg = (deg[long_rows] + self.seg_len - 1) // self.seg_len
-            segptr = torch.zeros(self.n_long + 1, dtype=torch.int64, device=dev)
-            torch.cumsum(nseg, 0, out=segptr[1:])
-            self.long_segptr = segptr.to(torch.int32)
-            self.n_seg = int(segptr[-1].item())
-            return
-        # Explicit segment list (include/spex_b200.h: spex_long_plan, column-blocked form):
-        #   hub rows  (>= HUB_EDGES_PER_BLOCK edges per column block on average) are cut at column-
-        #             block boundaries and listed BLOCK-MAJOR: concurrently running warps gather
-        #             from one ~32 MB window of the table, which L2 keeps resident.  Measured
-        #             (profiles/microbench/l2_window.py): 12.7 TB/s for 128-edge rows in a 32 MB
-        #             window vs 6.8 TB/s over the whole table - but only 6.7 TB/s for 16-edge rows,
-        #             so rows too short to fill their blocks stay on
-        #   mid rows  fixed-length segments of seg_len consecutive edges.
-        import os as _os
-        win = int(_os.environ.get("SPEX_L2_WINDOW_MB", 0)) << 20 or self.L2_WINDOW_BYTES
-        epb = int(_os.environ.get("SPEX_HUB_EPB", 0)) or self.HUB_EDGES_PER_BLOCK
-        cb_cols = max(win // (D * 4), self.MIN_CB_COLS)
-        n_cb = (self.n_cols + cb_cols - 1) // cb_cols
+
+    @classmethod
+    def long_row_plan(cls, rowptr: torch.Tensor, col: torch.Tensor, n_cols: int, seg_len: int, D: int) -> dict:
+        """The segment list of spex_long_plan (include/spex_b200.h) for a CSR (int64 rowptr, int32 col, which
+        may carry the hot flag in bit 31) and embedding width D, built on the tensors' device: the tensors
+        long_rows, long_segptr (int32), seg_start (int64), seg_count, row_seg (int32) and the counts n_long,
+        n_seg, n_hub (hub rows), n_hub_seg (hub cells, listed first).
+
+        Rows with more than seg_len edges are long.  Hub rows (>= HUB_EDGES_PER_BLOCK edges per column block
+        on average) are cut at column-block boundaries and their cells listed BLOCK-MAJOR: concurrently
+        running warps gather from one ~32 MB window of the table, which L2 keeps resident.  Measured
+        (profiles/microbench/l2_window.py): 12.7 TB/s for 128-edge rows in a 32 MB window vs 6.8 TB/s over
+        the whole table - but only 6.7 TB/s for 16-edge rows, so rows too short to fill their blocks are mid
+        rows.  A table that fits in L2 has no hub rows.  Mid rows follow, in ascending row order, and every
+        cell is cut every seg_len edges from its first edge.
+        """
+        if seg_len < 32:
+            raise ValueError("seg_len must be >= 32")
+        dev = rowptr.device
+        nnz = col.numel()
+        deg = rowptr[1:] - rowptr[:-1]
+        long_rows = torch.nonzero(deg > seg_len).flatten()
+        n_long = int(long_rows.numel())
         ldeg = deg[long_rows]
-        is_hub = ldeg >= epb * n_cb
-        hub_slots = torch.nonzero(is_hub).flatten()       # indices into long_rows
-        mid_slots = torch.nonzero(~is_hub).flatten()
+        is_hub = torch.zeros_like(ldeg, dtype=torch.bool)
         parts_start, parts_cnt, parts_row = [], [], []
         n_hub_cells = 0                                   # hub cells come first in the list
-        if hub_slots.numel():
-            hrows = long_rows[hub_slots]
-            nh = hrows.numel()
-            lo = self.rowptr[hrows].unsqueeze(1).expand(nh, n_cb + 1).clone()
-            hi = self.rowptr[hrows + 1].unsqueeze(1).expand(nh, n_cb + 1).clone()
-            target = (torch.arange(n_cb + 1, device=dev, dtype=torch.int64) * cb_cols).unsqueeze(0)
-            steps = int(ldeg.max().item()).bit_length() + 1
-            last = self.nnz - 1
-            for _ in range(steps):  # vectorised lower_bound of every block boundary in every hub row
-                mid = (lo + hi) >> 1
-                go = ((self.col[mid.clamp(max=last)] & 0x7FFFFFFF).to(torch.int64) < target) & (lo < hi)
-                lo = torch.where(go, mid + 1, lo)
-                hi = torch.where(go, hi, mid)
-            pos = lo  # [nh, n_cb+1]: first edge of the row with column >= b * cb_cols
-            del lo, hi, mid, go
-            cs = pos[:, :-1].t().reshape(-1)               # block-major flattening
-            cc = (pos[:, 1:] - pos[:, :-1]).t().reshape(-1)
-            cr = hub_slots.repeat(n_cb)
-            keep = cc > 0
-            parts_start.append(cs[keep]); parts_cnt.append(cc[keep]); parts_row.append(cr[keep])
-            n_hub_cells = int(parts_cnt[0].numel())
-        if mid_slots.numel():
-            mrows = long_rows[mid_slots]
-            parts_start.append(self.rowptr[mrows]); parts_cnt.append(deg[mrows]); parts_row.append(mid_slots)
+        if n_cols * D * 4 > 4 * cls.L2_WINDOW_BYTES:
+            import os as _os
+            win = int(_os.environ.get("SPEX_L2_WINDOW_MB", 0)) << 20 or cls.L2_WINDOW_BYTES
+            epb = int(_os.environ.get("SPEX_HUB_EPB", 0)) or cls.HUB_EDGES_PER_BLOCK
+            cb_cols = max(win // (D * 4), cls.MIN_CB_COLS)
+            n_cb = (n_cols + cb_cols - 1) // cb_cols
+            is_hub = ldeg >= epb * n_cb
+            hub_slots = torch.nonzero(is_hub).flatten()   # indices into long_rows
+            if hub_slots.numel():
+                hrows = long_rows[hub_slots]
+                nh = hrows.numel()
+                lo = rowptr[hrows].unsqueeze(1).expand(nh, n_cb + 1).clone()
+                hi = rowptr[hrows + 1].unsqueeze(1).expand(nh, n_cb + 1).clone()
+                target = (torch.arange(n_cb + 1, device=dev, dtype=torch.int64) * cb_cols).unsqueeze(0)
+                steps = int(ldeg.max().item()).bit_length() + 1
+                last = nnz - 1
+                for _ in range(steps):  # vectorised lower_bound of every block boundary in every hub row
+                    mid = (lo + hi) >> 1
+                    go = ((col[mid.clamp(max=last)] & 0x7FFFFFFF).to(torch.int64) < target) & (lo < hi)
+                    lo = torch.where(go, mid + 1, lo)
+                    hi = torch.where(go, hi, mid)
+                pos = lo  # [nh, n_cb+1]: first edge of the row with column >= b * cb_cols
+                del lo, hi, mid, go
+                cs = pos[:, :-1].t().reshape(-1)               # block-major flattening
+                cc = (pos[:, 1:] - pos[:, :-1]).t().reshape(-1)
+                cr = hub_slots.repeat(n_cb)
+                keep = cc > 0
+                parts_start.append(cs[keep]); parts_cnt.append(cc[keep]); parts_row.append(cr[keep])
+                n_hub_cells = int(parts_cnt[0].numel())
+        mid_slots = torch.nonzero(~is_hub).flatten()
+        mrows = long_rows[mid_slots]
+        parts_start.append(rowptr[mrows]); parts_cnt.append(deg[mrows]); parts_row.append(mid_slots)
         cell_start = torch.cat(parts_start)
         cell_cnt = torch.cat(parts_cnt)
         cell_row = torch.cat(parts_row)
-        pieces = (cell_cnt + self.seg_len - 1) // self.seg_len   # cap a segment at seg_len edges
+        pieces = (cell_cnt + seg_len - 1) // seg_len   # cap a segment at seg_len edges
         seg_cell = torch.repeat_interleave(torch.arange(cell_cnt.numel(), device=dev), pieces)
         first = torch.cumsum(pieces, 0) - pieces
         piece_idx = torch.arange(seg_cell.numel(), device=dev) - first[seg_cell]
-        seg_start = cell_start[seg_cell] + piece_idx * self.seg_len
-        seg_end = torch.minimum(seg_start + self.seg_len, (cell_start + cell_cnt)[seg_cell])
+        seg_start = cell_start[seg_cell] + piece_idx * seg_len
+        seg_end = torch.minimum(seg_start + seg_len, (cell_start + cell_cnt)[seg_cell])
         seg_row = cell_row[seg_cell]
-        self.n_seg = int(seg_start.numel())
-        self.n_hub = int(hub_slots.numel())
-        self.n_hub_seg = int(pieces[:n_hub_cells].sum())
-        if self.n_seg >= 2 ** 31:
+        n_seg = int(seg_start.numel())
+        if n_seg >= 2 ** 31:
             raise ValueError("too many long-row segments")
         # per row, segments in ascending edge order = fixed summation order
-        order = torch.sort(seg_row * (self.nnz + 1) + seg_start, stable=True).indices
-        counts = torch.bincount(seg_row, minlength=self.n_long)
-        segptr = torch.zeros(self.n_long + 1, dtype=torch.int64, device=dev)
+        order = torch.sort(seg_row * (nnz + 1) + seg_start, stable=True).indices
+        counts = torch.bincount(seg_row, minlength=n_long)
+        segptr = torch.zeros(n_long + 1, dtype=torch.int64, device=dev)
         torch.cumsum(counts, 0, out=segptr[1:])
-        self.long_segptr = segptr.to(torch.int32)
-        self.seg_start = seg_start.contiguous()
-        self.seg_count = (seg_end - seg_start).to(torch.int32).contiguous()
-        self.row_seg = order.to(torch.int32).contiguous()
+        return {"n_long": n_long, "n_seg": n_seg, "n_hub": int(is_hub.sum()),
+                "n_hub_seg": int(pieces[:n_hub_cells].sum()),
+                "long_rows": long_rows.to(torch.int32), "long_segptr": segptr.to(torch.int32),
+                "seg_start": seg_start.contiguous(), "seg_count": (seg_end - seg_start).to(torch.int32).contiguous(),
+                "row_seg": order.to(torch.int32).contiguous()}
 
     HOT_L2_BYTES = 48 << 20   # table bytes flagged hot (kept in L2 by the evict_last policy)
 
@@ -294,96 +289,25 @@ class DeviceGraph:
         self._plan_D = 0
         return int(hot.sum())
 
-    def split_hot_cold(self, n_split_rows: Optional[int] = None, chunk_edges: int = 1 << 27) -> int:
-        """Two-pass rows (SPEX_PLAN_TWO_PASS): inside every short row of [0, n_split_rows) move the
-        edges whose column is flagged hot to the front (stable, in place) and remember the first
-        cold edge in `rowmid`.  The SpMM then reduces the hot edges of all those rows first - a pass
-        whose table working set is the hot set only, so it stays in L2 - and the cold edges in a
-        second, purely streaming pass.  Long rows keep their column order (their segment lists
-        depend on it).  Only the summation order inside a row changes.  Returns the hot edges moved.
-        """
-        if not self.col_hot:
-            return 0
-        if self.tpos is not None:
-            raise ValueError("split_hot_cold would invalidate the transpose map (edge dropout graphs)")
-        n_split = self.n_rows if n_split_rows is None else min(int(n_split_rows), self.n_rows)
-        dev = self.device
-        rowptr = self.rowptr
-        rowmid = rowptr[:-1].clone()
-        total_hot = 0
-        rp_host = rowptr[: n_split + 1].cpu()
-        a = 0
-        while a < n_split:
-            # rows [a, b) with at most chunk_edges edges (at least one row)
-            limit = int(rp_host[a]) + chunk_edges
-            b = int(torch.searchsorted(rp_host, torch.tensor(limit), right=True)) - 1
-            b = max(min(b, n_split), a + 1)
-            ea, eb = int(rp_host[a]), int(rp_host[b])
-            if eb > ea:
-                c, v = self.col[ea:eb], self.val[ea:eb]
-                lrp = rowptr[a: b + 1] - ea
-                d = lrp[1:] - lrp[:-1]
-                rid = torch.repeat_interleave(torch.arange(b - a, device=dev), d)
-                h = (c < 0) & (d <= self.seg_len)[rid]
-                cs0 = torch.zeros(eb - ea + 1, dtype=torch.int64, device=dev)
-                cs0[1:] = torch.cumsum(h, 0, dtype=torch.int64)
-                hot_before = cs0[:-1] - cs0[lrp[:-1]][rid]            # hot edges of the row before e
-                hot_cnt = cs0[lrp[1:]] - cs0[lrp[:-1]]
-                pos = torch.arange(eb - ea, device=dev) - lrp[:-1][rid]
-                newpos = lrp[:-1][rid] + torch.where(h, hot_before, hot_cnt[rid] + (pos - hot_before))
-                cn, vn = torch.empty_like(c), torch.empty_like(v)
-                cn[newpos] = c
-                vn[newpos] = v
-                c.copy_(cn)
-                v.copy_(vn)
-                rowmid[a:b] += hot_cnt
-                total_hot += int(hot_cnt.sum())
-                del rid, h, cs0, hot_before, hot_cnt, pos, newpos, cn, vn
-            a = b
-        self.rowmid = rowmid
-        self.n_split_rows = n_split
-        self._plan_D = 0
-        return total_hot
-
-    def set_row_classes(self, split: int):
-        """SPEX_PLAN_INTERLEAVE: rows [0, split) (users) and [split, n_rows) (items) are visited
-        interleaved in proportion by the short-row kernel.  0 turns it off.  Results are unchanged
-        (only the order in which rows are scheduled moves)."""
-        self.interleave_split = int(split)
-        self._plan_D = 0
-
     def clean_col(self) -> torch.Tensor:
         """Column indices without the hot flag."""
         return (self.col & 0x7FFFFFFF) if self.col_hot else self.col
 
     def plan(self, D: int):
         """ctypes pointer to a spex_long_plan for embedding width D (NULL if nothing to say)."""
-        inter = 0 < self.interleave_split < self.n_rows
-        if self.n_long == 0 and not self.col_hot and not inter:
+        if self.n_long == 0 and not self.col_hot:
             return None
-        flags = 1 if self.col_hot else 0
-        two = self.col_hot and self.rowmid is not None
-        if two:
-            flags |= 2
-        if inter:
-            flags |= 4
         if self._plan_D != D:
-            hot_partial = (torch.empty(self.n_split_rows * D, dtype=torch.float32, device=self.device)
-                           if two else None)
-            tail = (self.rowmid.data_ptr() if two else None, hot_partial.data_ptr() if two else None,
-                    self.n_split_rows if two else 0, self.interleave_split if inter else 0)
+            flags = 1 if self.col_hot else 0
             if self.n_long == 0:
-                st = LongPlan(self.seg_len, 0, 0, flags, None, None, None, None, None, None, *tail)
-                self._plan_tensors = (None, hot_partial)
+                st = LongPlan(self.seg_len, 0, 0, flags)
+                self._plan_tensors = None
             else:
                 partial = torch.empty(self.n_seg * D, dtype=torch.float32, device=self.device)
                 st = LongPlan(self.seg_len, self.n_long, self.n_seg, flags, self.long_rows.data_ptr(),
-                              self.long_segptr.data_ptr(), partial.data_ptr(),
-                              self.seg_start.data_ptr() if self.seg_start is not None else None,
-                              self.seg_count.data_ptr() if self.seg_count is not None else None,
-                              self.row_seg.data_ptr() if self.row_seg is not None else None, *tail,
-                              self.n_hub_seg)
-                self._plan_tensors = (partial, hot_partial)
+                              self.long_segptr.data_ptr(), partial.data_ptr(), self.seg_start.data_ptr(),
+                              self.seg_count.data_ptr(), self.row_seg.data_ptr(), self.n_hub_seg)
+                self._plan_tensors = partial
             self._plan_struct = st
             self._plan_D = D
         return C.byref(self._plan_struct)
@@ -429,7 +353,7 @@ class DeviceGraph:
         total = int(cnt.sum().item())
         first = torch.cumsum(cnt, 0) - cnt
         pos = torch.repeat_interleave(a - first, cnt, output_size=total) + torch.arange(total, device=self.device)
-        seg_ids = self.row_seg[pos] if self.row_seg is not None else pos.to(torch.int32)
+        seg_ids = self.row_seg[pos]
         return r32, slots.to(torch.int32).contiguous(), seg_ids.to(torch.int32).contiguous()
 
     # -- derived graphs -------------------------------------------------------------------------

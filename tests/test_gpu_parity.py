@@ -110,7 +110,7 @@ def test_spmm_column_blocked_long_rows(cuda_device, seg_len, monkeypatch):
 
 
 @pytest.mark.parametrize("seg_len", [32, 1024])
-def test_hot_column_hints_do_not_change_results(cuda_device, seg_len):
+def test_hot_column_flags_give_bit_identical_results(cuda_device, seg_len):
     """Bit 31 of col flags hot table rows (L2 evict_last gathers): a cache hint only, so results
     are bit-identical to the unflagged graph."""
     from spex_b200 import ops
@@ -129,43 +129,39 @@ def test_hot_column_hints_do_not_change_results(cuda_device, seg_len):
     assert torch.equal(ops.propagate_mean(E, g1, 3), ops.propagate_mean(E, g0, 3))
     A = g1.to_sparse_coo()
     assert int(A.indices()[1].max()) < nu + 1 + m
-    # SPEX_PLAN_INTERLEAVE only changes the order in which rows are scheduled
-    g1.set_row_classes(nu + 1)
-    assert torch.equal(ops.spmm(g1, X), ops.spmm(g0, X))
-    assert torch.equal(ops.propagate_mean(E, g1, 3), ops.propagate_mean(E, g0, 3))
-    g2 = _dev_graph(u, i, nu + 1, m, cuda_device, seg_len)
-    g2.set_row_classes(nu + 1)                      # without hot flags: plan carries only the split
-    assert torch.equal(ops.spmm(g2, X), ops.spmm(g0, X))
 
 
-@pytest.mark.parametrize("seg_len", [32, 1024])
-def test_two_pass_hot_cold_rows(cuda_device, seg_len):
-    """SPEX_PLAN_TWO_PASS: hot edges of every short user row are reduced in a first pass, cold
-    edges in a second one that adds the partial row.  Same matrix, only the summation order inside
-    a row changes: parity with torch.sparse.mm at the fp32 bar, reproducible, long rows untouched."""
-    from spex_b200 import ops
+def test_spmm_rejects_a_plan_without_segment_list_or_with_unknown_flags(cuda_device):
+    """spex_long_plan has one segment list and one flag bit (SPEX_PLAN_COL_HOTBIT): a plan with long rows but no
+    seg_start / seg_count / row_seg, or with any other flag bit set, is refused with SPEX_E_BADARG before a launch."""
+    import ctypes
 
-    nu, m, D = 900, 500, 64
-    u, i = random_graph(nu, m, 12000, 17, hub_items=4, hub_degree=700)
-    g0 = _dev_graph(u, i, nu + 1, m, cuda_device, seg_len)
-    g1 = _dev_graph(u, i, nu + 1, m, cuda_device, seg_len)
-    g1.tpos = None
-    assert g1.mark_hot_columns(D, budget_bytes=32 * 1024) > 0
-    moved = g1.split_hot_cold(nu + 1, chunk_edges=3000)
-    assert moved > 0 and g1.rowmid is not None
-    deg = g1.rowptr[1:] - g1.rowptr[:-1]
-    assert bool((g1.rowmid >= g1.rowptr[:-1]).all()) and bool((g1.rowmid <= g1.rowptr[1:]).all())
-    assert bool((g1.rowmid[nu + 1:] == g1.rowptr[nu + 1: -1]).all())          # item rows: no hot pass
-    assert bool((g1.rowmid[: nu + 1][deg[: nu + 1] > seg_len] == g1.rowptr[: nu + 1][deg[: nu + 1] > seg_len]).all())
-    torch.manual_seed(0)
-    X = torch.randn(nu + 1 + m, D, device=cuda_device)
-    A = g0.to_sparse_coo()
-    want = torch.sparse.mm(A, X)
-    got = ops.spmm(g1, X)
-    assert rel_err(got, want) < TOL
-    assert torch.equal(got, ops.spmm(g1, X))
-    E = X * 0.1
-    assert rel_err(ops.propagate_mean(E, g1, 3), ops.propagate_mean(E, g0, 3)) < TOL
+    from spex_b200 import _capi, ops
+
+    nu, m, D = 700, 400, 64
+    u, i = random_graph(nu, m, 9000, 11, hub_items=3, hub_degree=500)
+    g = _dev_graph(u, i, nu + 1, m, cuda_device, 32)
+    assert g.n_long > 0
+    X = torch.randn(g.n_cols, D, device=cuda_device)
+    Y = torch.empty(g.n_rows, D, device=cuda_device)
+    g.plan(D)
+
+    def run(plan):
+        rc = _capi.lib.spex_spmm_csr_f32(_capi.ptr(g.rowptr), _capi.ptr(g.col), _capi.ptr(g.val), _capi.ptr(X),
+                                         g.n_rows, D, _capi.ptr(Y), None, 1.0, None, 1.0, ctypes.byref(plan),
+                                         _capi.stream_ptr())
+        torch.cuda.synchronize()
+        return rc
+
+    assert run(_capi.LongPlan.from_buffer_copy(g._plan_struct)) == 0
+    for flag in (2, 4, 1 << 30):
+        bad = _capi.LongPlan.from_buffer_copy(g._plan_struct)
+        bad.flags |= flag
+        assert run(bad) == -1, flag                      # SPEX_E_BADARG
+    for field in ("seg_start", "seg_count", "row_seg"):
+        bad = _capi.LongPlan.from_buffer_copy(g._plan_struct)
+        setattr(bad, field, None)
+        assert run(bad) == -1, field
 
 
 @pytest.mark.parametrize("K", [0, 1, 2, 3, 4])

@@ -21,7 +21,7 @@ def _graph(dev, seg_len, nu=20000, m=8000, n_inter=120000, hubs=6, hub_degree=90
 
 
 @pytest.mark.parametrize("blocked", [False, True])
-def test_row_subset_layer_is_bit_identical(cuda_device, blocked, monkeypatch):
+def test_row_subset_layer_is_bit_identical_on_both_plan_shapes(cuda_device, blocked, monkeypatch):
     """One layer on a row list (short rows, long rows through their segments, an empty row) = the same rows of
     the full layer; the rows outside the list are left untouched.  Both long-row plans."""
     from spex_b200 import ops
@@ -31,7 +31,7 @@ def test_row_subset_layer_is_bit_identical(cuda_device, blocked, monkeypatch):
         monkeypatch.setattr(ops.DeviceGraph, "MIN_CB_COLS", 64)
         monkeypatch.setattr(ops.DeviceGraph, "HUB_EDGES_PER_BLOCK", 4)
     g, nur, m = _graph(cuda_device, seg_len=32)
-    assert g.n_long > 0 and (g.seg_start is not None) == blocked
+    assert g.n_long > 0 and (g.n_hub_seg > 0) == blocked
     N, D = nur + m, 64
     torch.manual_seed(3)
     X = torch.randn(N, D, device=cuda_device)

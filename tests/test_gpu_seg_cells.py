@@ -1,6 +1,7 @@
 """Column-blocked long rows, several segments per warp (spmm_seg_runs_kernel: hub cells at the default L2 priority,
-mid-row segments evict_first) against the one-segment-per-CTA kernel, which SPEX_SPMM_SEG_LEGACY=1 selects.  Only
-cache priorities and scheduling differ, so every output must be bit-identical."""
+mid-row segments evict_first) against the one-segment-per-CTA kernel (spmm_seg_list_kernel), which the row-list
+entry point runs for every segment when every row is listed.  Only cache priorities and scheduling differ, so every
+output must be bit-identical."""
 import numpy as np
 import pytest
 import torch
@@ -37,10 +38,9 @@ def test_seg_runs_bit_identical_to_one_segment_per_cta(cuda_device, seg_len, hot
     monkeypatch.setattr(ops.DeviceGraph, "L2_WINDOW_BYTES", (16 if seg_len == 32 else 64) * 1024)
     monkeypatch.setattr(ops.DeviceGraph, "MIN_CB_COLS", 48)
     monkeypatch.setattr(ops.DeviceGraph, "HUB_EDGES_PER_BLOCK", 10 if seg_len == 32 else 100)
-    monkeypatch.delenv("SPEX_SPMM_SEG_LEGACY", raising=False)
     g = _graph(cuda_device, seg_len)
     H = g.n_hub_seg
-    assert g.seg_start is not None and 0 < H < g.n_seg
+    assert 0 < H < g.n_seg
     assert H % HUB_RUN != 0 and g.n_seg % HUB_RUN != 0            # runs cut short at both list boundaries
     cnt = g.seg_count.cpu()
     assert bool((cnt[:H] > 0).all()) and bool((cnt <= seg_len).all())
@@ -81,12 +81,45 @@ def test_seg_runs_bit_identical_to_one_segment_per_cta(cuda_device, seg_len, hot
         torch.cuda.synchronize()
         return r
 
+    every_row = g.row_subset(torch.arange(N, device=cuda_device))
+
+    def one_segment_per_cta():
+        """The same outputs with every row listed, so that every segment takes spmm_seg_list_kernel."""
+        def layer(x, Y=None, **kw):
+            if Y is None and kw.get("Z") is None:
+                Y = torch.zeros_like(x)
+            ops.spmm_rows(g, x, every_row, Y=Y, **kw)
+            return Y
+
+        r = {f"spmm{D}": layer(x) for D, x in X.items()}
+        # the K=3 mean and its backward layer by layer, with the epilogues of spex_propagate_mean_f32 / _bwd_f32
+        E0 = X[64] * 0.1
+        out, grad = torch.empty_like(E0), torch.empty_like(E0)
+        tmp = [torch.empty_like(E0), torch.empty_like(E0)]
+        x = E0
+        for k in range(3):
+            last = k == 2
+            layer(x, Y=None if last else tmp[k & 1], addend=E0 if k == 0 else out, Z=out, z_scale=0.25 if last else 1.0)
+            x = tmp[k & 1]
+        x = W                                                     # d sum(out * W) / d out
+        for j in range(1, 4):
+            last = j == 3
+            layer(x, addend=W, Z=grad if last else tmp[(j - 1) & 1], z_scale=0.25 if last else 1.0)
+            x = tmp[(j - 1) & 1]
+        r["mean"], r["grad"] = out, grad
+        r["all_rows"] = r["spmm64"]
+        r["subset"] = torch.zeros_like(X[64])
+        r["subset"][sel] = r["spmm64"][sel]
+        r["masked"] = layer(Xs, x_nonzero=ops.nonzero_mask(N, act))
+        r["dense_of_sparse"] = layer(Xs)
+        torch.cuda.synchronize()
+        return r
+
     new = run()
-    monkeypatch.setenv("SPEX_SPMM_SEG_LEGACY", "1")
-    old = run()
-    monkeypatch.delenv("SPEX_SPMM_SEG_LEGACY")
+    ref = one_segment_per_cta()
+    assert set(new) == set(ref)
     for k in new:
-        assert torch.equal(new[k], old[k]), k
+        assert torch.equal(new[k], ref[k]), k
     # the row subset and the sparse-input layer keep the one-segment kernel: their rows equal the new full layer's
     assert torch.equal(new["subset"][sel], new["spmm64"][sel])
     assert torch.equal(new["masked"], new["dense_of_sparse"])

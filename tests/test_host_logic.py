@@ -42,17 +42,79 @@ def test_empty_graph_and_single_edge():
     assert g.nnz == 2 and g.val.tolist() == [1.0, 1.0] and g.col.tolist() == [5, 2]
 
 
-def test_long_row_plan():
-    from spex_b200.graph import plan_long_rows
+def _plan_segments(p):
+    """(segment -> long-row slot) and the (start, count) pairs of a DeviceGraph.long_row_plan result."""
+    segptr, row_seg = p["long_segptr"].tolist(), p["row_seg"].tolist()
+    seg_slot = [0] * p["n_seg"]
+    for k in range(p["n_long"]):
+        for j in row_seg[segptr[k]: segptr[k + 1]]:
+            seg_slot[j] = k
+    return seg_slot, list(zip(p["seg_start"].tolist(), p["seg_count"].tolist()))
 
-    rowptr = np.array([0, 10, 10, 110, 174, 1200])
-    rows, segptr = plan_long_rows(rowptr, 64)
-    assert rows.tolist() == [2, 4]
-    assert segptr.tolist() == [0, 2, 2 + 17]
-    rows, segptr = plan_long_rows(rowptr, 2048)
-    assert rows.size == 0 and segptr.tolist() == [0]
+
+def test_long_row_plan_segment_list_fits_in_l2():
+    """DeviceGraph.long_row_plan on CPU tensors.  A table that fits in L2 has no hub rows: every long row is cut
+    every seg_len edges, in ascending row order, and row_seg is the identity."""
+    from spex_b200.ops import DeviceGraph
+
+    rowptr = torch.tensor([0, 10, 10, 110, 174, 1200])
+    col = torch.cat([torch.arange(int(d), dtype=torch.int32) for d in rowptr.diff()])
+    p = DeviceGraph.long_row_plan(rowptr, col, 2000, 64, 64)
+    assert p["long_rows"].tolist() == [2, 4] and p["n_long"] == 2
+    assert p["long_segptr"].tolist() == [0, 2, 2 + 17] and p["n_seg"] == 19
+    assert p["n_hub"] == 0 and p["n_hub_seg"] == 0
+    cuts = [(s, min(64, int(rowptr[r + 1]) - s)) for r in (2, 4) for s in range(int(rowptr[r]), int(rowptr[r + 1]), 64)]
+    assert _plan_segments(p)[1] == cuts
+    assert p["row_seg"].tolist() == list(range(19))
+    p = DeviceGraph.long_row_plan(rowptr, col, 2000, 2048, 64)
+    assert p["n_long"] == 0 and p["n_seg"] == 0 and p["long_segptr"].tolist() == [0]
     with pytest.raises(ValueError):
-        plan_long_rows(rowptr, 16)
+        DeviceGraph.long_row_plan(rowptr, col, 2000, 16, 64)
+
+
+def test_long_row_plan_segment_list_column_blocked(monkeypatch):
+    """A window far smaller than the table: hub rows are cut at column-block boundaries and their cells listed
+    first, block-major; every long-row edge is in exactly one segment; each row's segments ascend; the hot flag
+    in bit 31 of col does not change the plan."""
+    from spex_b200.ops import DeviceGraph
+
+    monkeypatch.setattr(DeviceGraph, "L2_WINDOW_BYTES", 16 * 1024)    # 64 columns per block at D = 64
+    monkeypatch.setattr(DeviceGraph, "MIN_CB_COLS", 48)
+    monkeypatch.setattr(DeviceGraph, "HUB_EDGES_PER_BLOCK", 10)       # 4000 columns = 63 blocks: hub from 630 edges
+    monkeypatch.delenv("SPEX_L2_WINDOW_MB", raising=False)
+    monkeypatch.delenv("SPEX_HUB_EPB", raising=False)
+    n_cols, cb, seg_len = 4000, 64, 64
+    rng = np.random.default_rng(0)
+    degs = [10, 3000, 200, 5, 1500, 700, 100, 64, 65, 500, 2500, 0]
+    col = torch.from_numpy(np.concatenate([np.sort(rng.choice(n_cols, d, replace=False)) for d in degs]).astype(np.int32))
+    rowptr = torch.from_numpy(np.concatenate([[0], np.cumsum(degs)]).astype(np.int64))
+    p = DeviceGraph.long_row_plan(rowptr, col, n_cols, seg_len, 64)
+    long_rows = [r for r, d in enumerate(degs) if d > seg_len]
+    hubs = [r for r, d in enumerate(degs) if d >= 630]
+    assert p["long_rows"].tolist() == long_rows and p["n_hub"] == len(hubs)
+    H = p["n_hub_seg"]
+    seg_slot, segs = _plan_segments(p)
+    assert 0 < H < p["n_seg"]
+    assert all(0 < c <= seg_len for _, c in segs)
+    seg_row = [long_rows[k] for k in seg_slot]
+    assert all(r in hubs for r in seg_row[:H]) and not any(r in hubs for r in seg_row[H:])
+    c = col.numpy()
+    blocks = [int(c[s]) // cb for s, _ in segs[:H]]
+    assert blocks == sorted(blocks)                                     # hub cells block-major
+    assert all(int(c[s]) // cb == int(c[s + n - 1]) // cb for s, n in segs[:H])   # a cell stays in its block
+    mid = [(s, min(seg_len, int(rowptr[r + 1]) - s)) for r in long_rows if r not in hubs
+           for s in range(int(rowptr[r]), int(rowptr[r + 1]), seg_len)]
+    assert segs[H:] == mid                                              # mid rows: seg_len cuts, row order
+    edges = sorted(e for s, n in segs for e in range(s, s + n))
+    assert edges == [e for r in long_rows for e in range(int(rowptr[r]), int(rowptr[r + 1]))]
+    segptr, row_seg = p["long_segptr"].tolist(), p["row_seg"].tolist()
+    for k, r in enumerate(long_rows):                                   # each row's segments tile it in order
+        own = [segs[j] for j in row_seg[segptr[k]: segptr[k + 1]]]
+        assert own[0][0] == int(rowptr[r]) and own[-1][0] + own[-1][1] == int(rowptr[r + 1])
+        assert all(a[0] + a[1] == b[0] for a, b in zip(own, own[1:]))
+    hot = col | torch.where(torch.from_numpy(rng.random(col.numel()) < 0.3), -(2 ** 31), 0).to(torch.int32)
+    q = DeviceGraph.long_row_plan(rowptr, hot, n_cols, seg_len, 64)
+    assert all(torch.equal(q[k], v) if torch.is_tensor(v) else q[k] == v for k, v in p.items())
 
 
 def test_partition_balances_nnz():
@@ -141,7 +203,7 @@ def test_negative_sampler_consumes_the_reference_stream():
     assert not ps.contains(users[len(feats):], items[len(feats):]).any()
 
 
-def test_capi_exports_every_declared_symbol():
+def test_capi_exports_every_declared_symbol_at_abi_2():
     hdr = open(os.path.join(ROOT, "include", "spex_b200.h")).read()
     hdr = re.sub(r"/\*.*?\*/", "", hdr, flags=re.S)
     declared = set(re.findall(r"\b(spex_[a-z0-9_]+)\s*\(", hdr))
@@ -152,7 +214,7 @@ def test_capi_exports_every_declared_symbol():
     from spex_b200 import _capi
 
     assert declared == set(_capi.SIGNATURES), declared ^ set(_capi.SIGNATURES)
-    assert _capi.abi_version() == 1
+    assert _capi.abi_version() == 2
     assert "SPEX_E_ALIGN" in _capi.error_string(-3)
 
 
