@@ -154,6 +154,30 @@ int spex_gather_f32(const float* src, const int64_t* idx, const float* scale, fl
                     float* out, int64_t n, void* stream);
 
 /*
+ * Edge dropout with a counter-based mask generated on the device: the values of A_drop and A_drop^T in one
+ * pass, with no host random numbers and no mask to copy.  The mask is a pure function of (seed, global row,
+ * global column); for the edge at global row r = row_offset + local row and column c (bit 31 of col stripped):
+ *      key  = ((uint64)r << 32) | (uint32)c
+ *      h    = splitmix64(seed ^ key)            (SplitMix64 finaliser, including its += 0x9E3779B97F4A7C15)
+ *      u    = (float)(h >> 40) * 0x1p-24f       (exact: 24 bits, in [0, 1))
+ *      keep = (int)(u + keep_prob) != 0         (fp32 add, round to nearest: (torch.rand(n) + keep_prob).int())
+ *      val_out[e]  = (val[e] * (keep(r, c) ? 1 : 0)) / keep_prob
+ *      valT_out[e] = (vt     * (keep(c, r) ? 1 : 0)) / keep_prob,   vt = tpos ? val[tpos[e]] : val[e]
+ * (no division when keep_prob == 1): the operations of spex_gather_f32 in the same order, so the same mask fed
+ * through it gives the same bits.  The two directions of an interaction are independent draws, as in the
+ * reference (model.py:46-55 draws every stored entry on its own) - but from a different generator: the
+ * reference's torch.rand stream is replaced, so other edges are dropped, with the same distribution.
+ *   rowptr/col/val  a CSR or a row block of one (rows r of the block are global rows row_offset + r)
+ *   tpos            int64 [nnz] positions of the transposed entries in this CSR; NULL = the values are
+ *                   symmetric bit for bit (val of (c, r) == val of (r, c))
+ *   valT_out        NULL: only val_out is written
+ * keep_prob must be in (0, 1]; n_rows == 0 is a no-op.
+ */
+int spex_edge_dropout_f32(const int64_t* rowptr, const int32_t* col, const float* val, const int64_t* tpos,
+                          int64_t n_rows, int64_t row_offset, uint64_t seed, float keep_prob,
+                          float* val_out, float* valT_out, void* stream);
+
+/*
  * BCE step (reference loss): gamma[b] = <U[users[b]], I[items[b]]>  (model.py:115-118),
  * loss = mean BCEWithLogits(gamma, labels) (model.py:23,120).
  *   U, I      propagated user / item tables (views of `out` above), row stride D

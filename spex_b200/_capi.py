@@ -52,6 +52,7 @@ SIGNATURES = {
     "spex_propagate_mean_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _i32, _p, _p, _p, _PLAN, _p]),
     "spex_propagate_mean_bwd_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _i32, _p, _p, _p, _PLAN, _p]),
     "spex_gather_f32": (C.c_int, [_p, _p, _p, _f, _p, _i64, _p]),
+    "spex_edge_dropout_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i64, C.c_uint64, _f, _p, _p, _p]),
     "spex_bce_fwd_f32": (C.c_int, [_p, _p, _i32, _p, _p, _p, _i64, _p, _p, _p, _p]),
     "spex_bce_bwd_f32": (C.c_int, [_p, _p, _i32, _p, _p, _p, _p, _i64, _p, _p, _p]),
     "spex_scatter_workspace_bytes": (_i64, [_i64]),

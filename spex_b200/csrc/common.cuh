@@ -87,6 +87,15 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
+// SplitMix64 finaliser (Steele, Lea, Flood 2014): the counter-based hash of the device samplers
+// (sampler.cu) and of the edge-dropout mask (spmm.cu).
+__device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
+  x += 0x9E3779B97F4A7C15ull;
+  x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
+  x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
+  return x ^ (x >> 31);
+}
+
 __device__ __forceinline__ float4 f4_zero() { return make_float4(0.f, 0.f, 0.f, 0.f); }
 __device__ __forceinline__ void f4_fma(float4& a, float s, const float4& x) {
   a.x = fmaf(s, x.x, a.x);

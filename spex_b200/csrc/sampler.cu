@@ -17,12 +17,6 @@
 
 namespace spex {
 
-__device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
-  x += 0x9E3779B97F4A7C15ull;
-  x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
-  x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
-  return x ^ (x >> 31);
-}
 // unbiased enough for m << 2^32: high 32 bits of a 64-bit hash, multiply-shift into [0, m)
 __device__ __forceinline__ int32_t draw_below(uint64_t h, int32_t m) {
   return (int32_t)(((h >> 32) * (uint64_t)(uint32_t)m) >> 32);

@@ -865,6 +865,80 @@ __global__ void gather_scale_kernel(const float* __restrict__ src, const int64_t
   }
 }
 
+// The 24-bit draw (h >> 40) of edge (r, c) of the counter-based dropout mask (spex_edge_dropout_f32).
+__device__ __forceinline__ uint32_t edge_draw(uint64_t seed, uint32_t r, uint32_t c) {
+  return (uint32_t)(splitmix64(seed ^ (((uint64_t)r << 32) | c)) >> 40);
+}
+
+constexpr int kDropChunk = 1024;   // contiguous edges per warp and chunk: one row search per chunk
+constexpr int kDropUnroll = 4;     // edges per lane in flight
+
+// val_out / valT_out of the edge-dropped graph in one pass.  A warp takes a chunk of kDropChunk edges, finds the
+// row of its first edge by binary search and walks forward from there: each lane advances its row over the row
+// ends it passes, so an empty row costs one step and a hub row none.  col, val, tpos and both outputs are read
+// and written coalesced, 32 consecutive edges per warp instruction.
+template <bool kT, bool kTpos>
+__global__ void __launch_bounds__(256)
+edge_dropout_kernel(const int64_t* __restrict__ rowptr, const int32_t* __restrict__ col,
+                    const float* __restrict__ val, const int64_t* __restrict__ tpos, int64_t n_rows,
+                    int64_t row_offset, uint64_t seed, float keep_prob, float* __restrict__ val_out,
+                    float* __restrict__ valT_out) {
+  // keep = int(RN(u + keep_prob)) != 0 with u = draw * 2^-24 is nondecreasing in the draw, so it is the test
+  // draw >= k_min; k_min (2^24: nothing kept) is found by bisection with the same fp32 operations.
+  uint32_t k_min = 0, k_hi = 1u << 24;
+  while (k_min < k_hi) {
+    const uint32_t mid = (k_min + k_hi) >> 1;
+    if (__float2int_rz(__fadd_rn(__uint2float_rn(mid) * 0x1p-24f, keep_prob)) != 0) k_hi = mid; else k_min = mid + 1;
+  }
+  // (v * keep) / keep_prob is v / keep_prob for a kept edge and v * 0 (the same signed zero) for a dropped one
+  const bool divide = keep_prob != 1.f;
+  const int lane = threadIdx.x & (kWarp - 1);
+  const int64_t warps = (int64_t)gridDim.x * (blockDim.x / kWarp);
+  const int64_t e_end = __ldg(rowptr + n_rows);
+  for (int64_t c0 = __ldg(rowptr) + ((int64_t)blockIdx.x * (blockDim.x / kWarp) + threadIdx.x / kWarp) * kDropChunk;
+       c0 < e_end; c0 += warps * kDropChunk) {
+    int64_t lo = 0, hi = n_rows;   // rowptr[lo] <= c0 < rowptr[hi]: lo ends at the last row starting at or before c0
+    while (hi - lo > 1) {
+      const int64_t mid = (lo + hi) >> 1;
+      if (__ldg(rowptr + mid) <= c0) lo = mid; else hi = mid;
+    }
+    int64_t row = lo;
+    int32_t row_end = (int32_t)(__ldg(rowptr + row + 1) - c0);   // chunk-relative from here on
+    const int n = (int)min((int64_t)kDropChunk, e_end - c0);
+    const int32_t* cc = col + c0;
+    const float* vc = val + c0;
+    float* oc = val_out + c0;
+    float* ot = kT ? valT_out + c0 : nullptr;
+    for (int i0 = lane; i0 < n; i0 += kDropUnroll * kWarp) {
+      uint32_t cv[kDropUnroll];   // the loads of kDropUnroll edges are issued before any of them is used
+      float v[kDropUnroll], vt[kDropUnroll];
+#pragma unroll
+      for (int k = 0; k < kDropUnroll; ++k) {
+        const int i = i0 + k * kWarp;
+        if (i < n) {
+          cv[k] = (uint32_t)ld_stream_s32(cc + i) & 0x7fffffffu;
+          v[k] = ld_stream_f32(vc + i);
+          if (kT && kTpos) vt[k] = __ldg(val + __ldcs(tpos + c0 + i));
+        }
+      }
+#pragma unroll
+      for (int k = 0; k < kDropUnroll; ++k) {
+        const int i = i0 + k * kWarp;
+        if (i >= n) break;
+        while (row_end <= i) row_end = (int32_t)(__ldg(rowptr + (++row) + 1) - c0);
+        const uint32_t r = (uint32_t)(row + row_offset);
+        const float q = divide ? v[k] / keep_prob : v[k];   // IEEE fp32 division, as gather_scale_kernel
+        __stcs(oc + i, edge_draw(seed, r, cv[k]) >= k_min ? q : v[k] * 0.f);
+        if (kT) {
+          const float w = kTpos ? vt[k] : v[k];
+          const float qt = !kTpos ? q : divide ? w / keep_prob : w;
+          __stcs(ot + i, edge_draw(seed, cv[k], r) >= k_min ? qt : w * 0.f);
+        }
+      }
+    }
+  }
+}
+
 }  // namespace spex
 
 using namespace spex;
@@ -1173,6 +1247,25 @@ extern "C" int spex_gather_f32(const float* src, const int64_t* idx, const float
   int64_t blocks = (n + 255) / 256;
   if (blocks > 148 * 16) blocks = 148 * 16;
   gather_scale_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(src, idx, scale, divisor, out, n);
+  count_launch();
+  return check_last();
+}
+
+extern "C" int spex_edge_dropout_f32(const int64_t* rowptr, const int32_t* col, const float* val, const int64_t* tpos,
+                                     int64_t n_rows, int64_t row_offset, uint64_t seed, float keep_prob,
+                                     float* val_out, float* valT_out, void* stream) {
+  SPEX_RETURN_IF(!rowptr || !col || !val || !val_out || n_rows < 0 || row_offset < 0 ||
+                     !(keep_prob > 0.f && keep_prob <= 1.f),
+                 SPEX_E_BADARG);
+  if (n_rows == 0) return 0;
+  // the edge count lives on the device (rowptr[n_rows]): one resident wave of CTAs strides over the chunks
+  auto kernel = !valT_out ? edge_dropout_kernel<false, false>
+                : tpos    ? edge_dropout_kernel<true, true> : edge_dropout_kernel<true, false>;
+  int ctas_per_sm = 0;
+  cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, kernel, 256, 0);
+  if (e != cudaSuccess) return (int)e;
+  kernel<<<148 * ctas_per_sm, 256, 0, (cudaStream_t)stream>>>(rowptr, col, val, tpos, n_rows, row_offset, seed,
+                                                             keep_prob, val_out, valT_out);
   count_launch();
   return check_last();
 }

@@ -17,7 +17,7 @@ _FLAGS = (
     ("recdim", int, 64, "embedding width D (the sm_100a fast paths are built for 32/64/128)"),
     ("layer", int, 3, "propagation depth K of computer()"),
     ("lr", float, 0.001, "Adam step size"),
-    ("dropout", int, 0, "1 = edge dropout on the normalised adjacency while training"),
+    ("dropout", int, 0, "1 = reference RNG stream, 2 = counter-based mask generated on the GPU"),
     ("keepprob", float, 0.6, "probability that an edge survives the dropout"),
     ("a_fold", int, 100, "row folds of the adjacency when A_split is on"),
     ("epochs", int, 50, "training epochs"),

@@ -99,7 +99,7 @@ def main_distributed(args):
     from .graph import partition_rows_by_nnz
 
     if args.dropout:
-        raise SystemExit("--dropout 1 is not supported with torchrun (row-partitioned backward needs the symmetric graph)")
+        raise SystemExit(f"--dropout {args.dropout} is not supported with torchrun (row-partitioned backward needs the symmetric graph)")
     rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
     local_rank = int(os.environ.get("LOCAL_RANK", rank))
     torch.cuda.set_device(local_rank)

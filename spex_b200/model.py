@@ -15,8 +15,10 @@ Differences in HOW (not in WHAT):
   * K layers = K launches of the CSR SpMM, the layer mean rides in the epilogue: no stack/mean
     temporaries (model.py:94-95);
   * edge dropout (model.py:46-55) keeps the CSR structure and scales values by mask/keep_prob;
-    the mask is drawn by the same CPU ``torch.rand(nnz)`` call so a shared seed drops the same
-    edges;
+    with ``dropout=1`` the mask is drawn by the same CPU ``torch.rand(nnz)`` call so a shared seed
+    drops the same edges; ``dropout=2`` generates it on the GPU from a hash of (seed, row, column)
+    (ops.DeviceGraph.device_dropout_values): other edges than the reference drops, with the same
+    distribution, and no host random numbers or copies at any graph size;
   * the backward is explicit (A^T SpMMs + deterministic segmented scatter), no atomics.
 """
 from __future__ import annotations
@@ -138,6 +140,8 @@ class LightGCN(BasicModel):
         return self._dev_graph
 
     def _dropout_values(self, g: ops.DeviceGraph):
+        if self.args_r.dropout == 2:
+            return g.device_dropout_values(dropout_seed(), self.keep_prob)
         # model.py:50-53: keep edge e iff int(rand[e] + keep_prob) != 0; kept values / keep_prob.
         # Same CPU generator call as the reference, in coalesced (= CSR) edge order.
         keep = (torch.rand(g.nnz) + self.keep_prob).int().bool()
@@ -300,6 +304,12 @@ class LightGCN(BasicModel):
                 ops.score_topk_bf16(Ub, ub.numel(), b_pad, Ib, self.num_items, m_pad, k, ub, mrp, mcol,
                                     idx[s: s + ub.numel()], val[s: s + ub.numel()])
         return idx, val
+
+
+def dropout_seed() -> int:
+    """Seed of one training forward's device dropout mask (dropout=2), drawn from torch's default CPU generator so
+    that torch.manual_seed reproduces a run."""
+    return int(torch.randint(1 << 62, (1,)))
 
 
 def _stack_row_folds(folds):

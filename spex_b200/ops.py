@@ -117,7 +117,8 @@ class DeviceGraph:
     interleave_split = 0   # always 0: bench.py still reports it (config.interleaved_row_classes)
 
     def __init__(self, rowptr, col, val, n_cols: int, tpos=None, seg_len: int = DEFAULT_SEG_LEN,
-                 row_offset: int = 0, symmetric: bool = True, D_hint: int = 64, col_hot: bool = False):
+                 row_offset: int = 0, symmetric: bool = True, D_hint: int = 64, col_hot: bool = False,
+                 values_symmetric: bool = False):
         _need_cuda(rowptr, col, val)
         assert rowptr.dtype == torch.int64 and col.dtype == torch.int32 and val.dtype == torch.float32
         self.rowptr, self.col, self.val = rowptr, col, val
@@ -127,6 +128,9 @@ class DeviceGraph:
         self.tpos = tpos
         self.row_offset = int(row_offset)
         self.symmetric = symmetric
+        # val of (c, r) == val of (r, c) bit for bit (no tpos needed for the transposed values).  Not implied by
+        # `symmetric`: a weighted build computes (d_u*w)*d_i one way and (d_i*w)*d_u the other.
+        self.values_symmetric = values_symmetric
         self.device = val.device
         self.seg_len = int(seg_len)
         self._plan_struct = None
@@ -379,6 +383,19 @@ class DeviceGraph:
         call("spex_gather_f32", ptr(self.val), None, ptr(scale), float(keep_prob), ptr(out), self.nnz,
              stream_ptr())
         return out
+
+    def device_dropout_values(self, seed: int, keep_prob: float):
+        """(val, valT) of the edge-dropped graph under the counter-based mask of spex_edge_dropout_f32: edge (r, c)
+        is kept by a hash of (seed, global row, column), so no host random numbers and no mask copy.  Fresh
+        tensors: autograd holds valT until the backward runs."""
+        if self.tpos is None and not self.values_symmetric:
+            raise RuntimeError("edge dropout needs the transpose map of the adjacency or bit-symmetric values; "
+                               "build the graph through spex_b200.dataloader (getCSR) or synthetic.build_norm_adj_device")
+        val = torch.empty_like(self.val)
+        valT = torch.empty_like(self.val)
+        call("spex_edge_dropout_f32", ptr(self.rowptr), ptr(self.col), ptr(self.val), ptr(self.tpos), self.n_rows,
+             self.row_offset, int(seed), float(keep_prob), ptr(val), ptr(valT), stream_ptr())
+        return val, valT
 
     def to_sparse_coo(self) -> torch.Tensor:
         deg = self.rowptr[1:] - self.rowptr[:-1]

@@ -95,7 +95,8 @@ def build_norm_adj_device(keys: torch.Tensor, n_users: int, m_items: int,
     col[nR:] = u2.to(torch.int32)
     val[nR:] = d[nur + i2] * d[u2]
     del i2, u2
-    g = DeviceGraph(rowptr, col, val, N, None, seg_len)
+    # values d[u]*d[i] both ways and no duplicate pairs: symmetric bit for bit, so dropout needs no tpos
+    g = DeviceGraph(rowptr, col, val, N, None, seg_len, values_symmetric=True)
     return g, mask_rowptr, mask_col
 
 
