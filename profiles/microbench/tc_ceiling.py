@@ -22,7 +22,7 @@ for _ in range(3):
 e1.record()
 torch.cuda.synchronize()
 ms = e0.elapsed_time(e1) / 3
-print(f"dbg={os.environ.get('SPEX_TC_DBG', '0')} {ms:.2f} ms  {2.0 * n_u * m * D / ms / 1e9:.0f} TFLOP/s")
+print(f"{ms:.2f} ms  {2.0 * n_u * m * D / ms / 1e9:.0f} TFLOP/s")
 
 if os.environ.get("CLOCKS"):
     # SM clock and board power while the scorer runs back to back for ~1.5 s

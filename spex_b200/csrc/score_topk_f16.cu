@@ -40,97 +40,17 @@
 //     outputs, NGCF_SPEX/code/main_rec.py:85; one CTA per SM).
 //   * warp roles as in round 1: warp 0 bulk-copy producer, warp 1 TMEM allocator + MMA issuer
 //     (elect.sync, back-to-back polls), warps 2-5 epilogue (TMEM lane quarter = warp % 4).
-#include "topk.cuh"
+#include "tcgen05.cuh"
 #include <cuda_fp16.h>
 #include <stdlib.h>
 
 namespace spex {
 namespace tf {
 
-constexpr int BM = 128;            // users per CTA  (UMMA M)
-constexpr int BN = 128;            // items per tile (UMMA N)
-constexpr int UMMA_K = 16;
-constexpr int kThreads = 32 * 6;
-constexpr int kMaxStages = 4;
-constexpr int kTmemCols = 256;     // 2 accumulator buffers x 128 columns (fp16 accumulators still
-                                   // occupy one 32-bit cell each); two CTAs share an SM at D = 64
-constexpr int KMAX_TC = 64;
-constexpr uint32_t kSpinLimit = 1u << 26;   // bounded waits: trap instead of hanging the GPU
+using namespace tcgen05;
+
 constexpr float kEpsRel = 1.0f / 512.0f;    // 2^-9, see the header comment
 constexpr float kEpsAbs = 1.0f / 1024.0f;   // subnormal flush of tiny operands (bound 2^-11)
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) {
-  return (uint32_t)__cvta_generic_to_shared(p);
-}
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)),
-               "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t spins = 0;
-  while (!mbar_try_wait(bar, parity)) {
-    if (++spins > kSpinLimit) __trap();
-  }
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-          smem_u32(dst)),
-      "l"(src), "r"(bytes), "r"(smem_u32(bar))
-      : "memory");
-}
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred;
-  asm volatile(
-      "{\n\t.reg .pred P1;\n\t"
-      "elect.sync _|P1, 0xffffffff;\n\t"
-      "selp.u32 %0, 1, 0, P1;\n\t}"
-      : "=r"(pred));
-  return pred != 0;
-}
-__device__ __forceinline__ void tc_fence_before() {
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-}
-__device__ __forceinline__ void tc_fence_after() {
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-}
-__device__ __forceinline__ void tc_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(
-                   smem_u32(bar))
-               : "memory");
-}
-// D[tmem] (+)= A[smem] * B[smem]^T, fp16 x fp16 -> fp16 accumulator
-__device__ __forceinline__ void tc_mma(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc,
-                                       uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
-  return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)((lbo >> 4) & 0x3FFFu) << 16) |
-         ((uint64_t)((sbo >> 4) & 0x3FFFu) << 32) | (1ull << 46);
-}
 
 // tcgen05.ld 32 lanes x 128 columns of 16-bit accumulators packed two per register (column 2i in
 // the low half of register i), without waiting
@@ -182,10 +102,6 @@ struct MaskCursor {
   const int32_t* cur[BM];
   const int32_t* end[BM];
 };
-
-__device__ __forceinline__ unsigned long long pack_state(int n, float tau) {
-  return ((unsigned long long)(unsigned)n << 32) | (unsigned long long)__float_as_uint(tau);
-}
 
 // exact score of (this row, item id): fp32 FMA chain over the fp16 operands, d = 0 .. DK-1
 template <int DK>
@@ -379,7 +295,6 @@ score_topk_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict_
   // difference), bit 1 = the epilogue only hands the accumulator back (MMA side alone)
   constexpr int CAP = 32 * EPL;
   constexpr int A_BYTES = BM * DK * 2, B_BYTES = BN * DK * 2;
-  constexpr uint32_t lbo = 128, sbo = 16 * DK;   // layout written by spex_pack_f16
   extern __shared__ uint8_t smem_raw[];
   __shared__ __align__(8) uint64_t bar_full[kMaxStages];
   __shared__ __align__(8) uint64_t bar_empty[kMaxStages];
@@ -399,89 +314,17 @@ score_topk_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict_
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t tile_m = blockIdx.x;
 
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < stages; ++s) {
-      mbar_init(&bar_full[s], 1);
-      mbar_init(&bar_empty[s], 1);
-    }
-    for (int b = 0; b < 2; ++b) {
-      mbar_init(&bar_tfull[b], 1);
-      mbar_init(&bar_tempty[b], 4);   // one arrive per epilogue warp
-    }
-    mbar_init(&bar_a, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-                     smem_u32(&tmem_slot)),
-                 "r"((uint32_t)kTmemCols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = tmem_slot;
+  const uint32_t tmem_base =
+      pipeline_init(warp, stages, bar_full, bar_empty, bar_tfull, bar_tempty, &bar_a, &tmem_slot);
 
   if (warp == 0) {
-    // ===== producer: one thread streams the user tile once, then every item tile =====
-    if (elect_one()) {
-      mbar_arrive_expect_tx(&bar_a, A_BYTES);
-      bulk_g2s(sA, Uh + tile_m * A_BYTES, A_BYTES, &bar_a);
-      int s = 0;
-      uint32_t ph = 0;
-      for (int t = 0; t < n_item_tiles; ++t) {
-        mbar_wait(&bar_empty[s], ph ^ 1u);
-        mbar_arrive_expect_tx(&bar_full[s], B_BYTES);
-        bulk_g2s(sB + (size_t)s * B_BYTES, Ih + (size_t)t * B_BYTES, B_BYTES, &bar_full[s]);
-        if (++s == stages) {
-          s = 0;
-          ph ^= 1u;
-        }
-      }
-    }
+    producer_role<DK>(Uh, Ih, tile_m, n_item_tiles, stages, sA, sB, bar_full, bar_empty, &bar_a);
   } else if (warp == 1) {
-    // ===== MMA issuer: one thread drives the tensor core =====
-    if (elect_one()) {
-      // instruction descriptor: c = f16 (0 at [4,6)), a = b = f16 (0 at [7,10), [10,13)), K-major
-      // A and B, N>>3 at [17,23), M>>4 at [24,29)
-      const uint32_t idesc = ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
-      const uint32_t a_addr = smem_u32(sA);
-      constexpr uint32_t kstep = 2 * lbo;  // 16 halves along K = two 8-element core matrices
-      mbar_wait(&bar_a, 0);
-      int s = 0;
-      uint32_t ph = 0;
-      for (int t = 0; t < n_item_tiles; ++t) {
-        const int buf = t & 1;
-        const uint32_t use = (uint32_t)(t >> 1) & 1u;
-        // both polls of a tile (operands landed, accumulator drained) are issued back to back:
-        // while the tensor pipe is busy a poll costs ~200 cycles even when its phase is complete
-        bool have_b = mbar_try_wait(&bar_full[s], ph);
-        bool have_d = mbar_try_wait(&bar_tempty[buf], use ^ 1u);
-        uint32_t spins = 0;
-        while (!have_b) {
-          have_b = mbar_try_wait(&bar_full[s], ph);
-          if (++spins > kSpinLimit) __trap();
-        }
-        while (!have_d) {
-          have_d = mbar_try_wait(&bar_tempty[buf], use ^ 1u);
-          if (++spins > kSpinLimit) __trap();
-        }
-        tc_fence_after();
-        const uint32_t b_addr = smem_u32(sB + (size_t)s * B_BYTES);
-#pragma unroll
-        for (int kk = 0; kk < DK / UMMA_K; ++kk) {
-          tc_mma(tmem_base + (uint32_t)(buf * BN), make_desc(a_addr + kk * kstep, lbo, sbo),
-                 make_desc(b_addr + kk * kstep, lbo, sbo), idesc, kk > 0 ? 1u : 0u);
-        }
-        tc_commit(&bar_empty[s]);     // smem stage reusable once these MMAs have read it
-        tc_commit(&bar_tfull[buf]);   // accumulator ready for the epilogue
-        if (++s == stages) {
-          s = 0;
-          ph ^= 1u;
-        }
-      }
-    }
+    // instruction descriptor: c = f16 (0 at [4,6)), a = b = f16 (0 at [7,10), [10,13)), K-major
+    // A and B, N>>3 at [17,23), M>>4 at [24,29)
+    constexpr uint32_t idesc = ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
+    mma_role<DK>(idesc, sA, sB, tmem_base, n_item_tiles, stages, bar_full, bar_empty, bar_tfull,
+                 bar_tempty, &bar_a);
   } else {
     // ===== epilogue: thread owns one user row; warp = TMEM lane quarter =====
     const int q = warp & 3;
@@ -671,14 +514,7 @@ score_topk_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict_
       atomicAdd(stats + 2, c_slow);
     }
   }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base),
-                 "r"((uint32_t)kTmemCols)
-                 : "memory");
-  }
+  pipeline_teardown(warp, tmem_base);
 }
 
 // ---- operand packing ---------------------------------------------------------------------------
@@ -725,42 +561,15 @@ __global__ void finish_meta_kernel(float* __restrict__ meta) {
   meta[2] = sqrtf(n2) * sc * 1.0001f;
 }
 
-// fp32 [rows, D] -> fp16(x * scale) in the core-matrix-tiled layout:
-//   byte offset of (r, k) = (r/8) * (16*D) + (k/8) * 128 + (r%8) * 16 + (k%8) * 2
-// optional row gather; rows in [n, n_pad) are zero.  Thread per (row, 8-element chunk).
+// fp32 [rows, D] -> fp16(x * scale) in the layout of pack_rows, scale = meta[0]
 __global__ void __launch_bounds__(256)
 pack_f16_kernel(const float* __restrict__ src, const int64_t* __restrict__ rows, int64_t n,
                 int64_t n_pad, int D, const float* __restrict__ meta, uint8_t* __restrict__ dst) {
   const float sc = meta[0];
-  const int D8 = D >> 3;
-  const int64_t total = n_pad * D8;
-  int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  for (; i < total; i += stride) {
-    const int64_t r = i / D8;
-    const int kc = (int)(i - r * D8);
-    float4 a = f4_zero(), b = f4_zero();
-    if (r < n) {
-      const int64_t sr = rows ? rows[r] : r;
-      a = *reinterpret_cast<const float4*>(src + sr * D + kc * 8);
-      b = *reinterpret_cast<const float4*>(src + sr * D + kc * 8 + 4);
-    }
-    uint4 pk;
-    auto h2 = [sc](float x, float y) -> uint32_t {
-      const __half2 h = __floats2half2_rn(x * sc, y * sc);
-      return *reinterpret_cast<const uint32_t*>(&h);
-    };
-    pk.x = h2(a.x, a.y);
-    pk.y = h2(a.z, a.w);
-    pk.z = h2(b.x, b.y);
-    pk.w = h2(b.z, b.w);
-    const int64_t off = (r >> 3) * (16 * (int64_t)D) + (int64_t)kc * 128 + (r & 7) * 16;
-    *reinterpret_cast<uint4*>(dst + off) = pk;
-  }
-}
-
-static size_t smem_bytes(int DK, int cap, int stages) {
-  return 128 + (size_t)BM * DK * 2 + (size_t)stages * BN * DK * 2 + (size_t)cap * BM * 8;
+  pack_rows(src, rows, n, n_pad, D, dst, [sc](float x, float y) -> uint32_t {
+    const __half2 h = __floats2half2_rn(x * sc, y * sc);
+    return *reinterpret_cast<const uint32_t*>(&h);
+  });
 }
 
 static unsigned long long* g_stats = nullptr;
@@ -772,9 +581,7 @@ static int launch(const void* Uh, const void* Ih, int64_t B, int64_t B_pad, int6
                   float* out_val, cudaStream_t st) {
   // D = 64: two CTAs per SM need <= ~113 KB each (228 KB per SM, 1 KB reserved per CTA, static
   // shared memory ~7 KB); D = 128: one CTA per SM, up to 227 KB
-  const size_t budget = (DK == 64) ? 115712 - 7600 : 227 * 1024 - 7600;
-  int stages = kMaxStages;
-  while (stages > 2 && smem_bytes(DK, 32 * EPL, stages) > budget) --stages;
+  int stages = choose_stages(DK, 32 * EPL, (DK == 64) ? 115712 - 7600 : 227 * 1024 - 7600);
   if (const char* e = getenv("SPEX_TF_STAGES")) stages = atoi(e);   // bring-up experiment
   SPEX_RETURN_IF(stages < 2 || stages > kMaxStages, SPEX_E_BADARG);
   const size_t smem = smem_bytes(DK, 32 * EPL, stages);

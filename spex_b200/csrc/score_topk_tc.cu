@@ -34,105 +34,19 @@
 //     elect.sync (straight-line UTCHMMA/UTCBAR/UBLKCP instead of one ELECT + BRA.U.ANY loop per
 //     instruction) and the MMA thread issues its two mbarrier polls of a tile back to back:
 //     together 1134 -> 1699 TFLOP/s for the MMA side alone, 895 -> 935 with the epilogue.
-#include "topk.cuh"
+#include "tcgen05.cuh"
 #include <cuda_bf16.h>
-#include <stdlib.h>
 
 namespace spex {
 namespace tc {
 
-constexpr int BM = 128;            // users per CTA  (UMMA M)
-constexpr int BN = 128;            // items per tile (UMMA N)
+using namespace tcgen05;
+
 constexpr int DK = 64;             // embedding dim  (4 x UMMA K)
-constexpr int UMMA_K = 16;
 constexpr int A_BYTES = BM * DK * 2;
 constexpr int B_BYTES = BN * DK * 2;
-constexpr int kThreads = 32 * 6;
-constexpr int kMaxStages = 4;
-constexpr int kTmemCols = 256;     // 2 accumulator buffers x 128 columns; two CTAs share an SM
-constexpr int KMAX_TC = 64;
 constexpr int kGroup = 8;          // appends are capacity-checked every 8 scores
-constexpr uint32_t kSpinLimit = 1u << 26;   // bounded waits: trap instead of hanging the GPU
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) {
-  return (uint32_t)__cvta_generic_to_shared(p);
-}
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)),
-               "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t spins = 0;
-  while (!mbar_try_wait(bar, parity)) {
-    if (++spins > kSpinLimit) __trap();
-  }
-}
-// 1-D bulk async copy global -> shared, completion counted in bytes on `bar`
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-          smem_u32(dst)),
-      "l"(src), "r"(bytes), "r"(smem_u32(bar))
-      : "memory");
-}
-// Elect one thread of a converged warp.  With elect.sync the compiler knows that exactly one thread
-// runs the guarded block and issues tcgen05.mma / tcgen05.commit / cp.async.bulk straight from
-// uniform registers; with `lane == 0` it wraps every such instruction in an ELECT + BRA.U.ANY
-// loop with R2UR moves (~61 cycles per MMA issue, measured: profiles/microbench/mma_pipe.cu).
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred;
-  asm volatile(
-      "{\n\t.reg .pred P1;\n\t"
-      "elect.sync _|P1, 0xffffffff;\n\t"
-      "selp.u32 %0, 1, 0, P1;\n\t}"
-      : "=r"(pred));
-  return pred != 0;
-}
-__device__ __forceinline__ void tc_fence_before() {
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-}
-__device__ __forceinline__ void tc_fence_after() {
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-}
-__device__ __forceinline__ void tc_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(
-                   smem_u32(bar))
-               : "memory");
-}
-// D[tmem] (+)= A[smem] * B[smem]^T, bf16 x bf16 -> fp32
-__device__ __forceinline__ void tc_mma(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc,
-                                       uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// UMMA shared-memory descriptor, SWIZZLE_NONE, K-major canonical layout
-//   bits [0,14) start>>4 | [16,30) LBO>>4 | [32,46) SBO>>4 | [46,48) version=1 | [61,64) layout=0
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
-  return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)((lbo >> 4) & 0x3FFFu) << 16) |
-         ((uint64_t)((sbo >> 4) & 0x3FFFu) << 32) | (1ull << 46);
-}
 // tcgen05.ld 32 lanes x 32 columns (one 32-bit word per lane per column) WITHOUT waiting: the
 // registers are only valid after tmem_wait32() on the same array.
 #define SPEX_R32(r)                                                                            \
@@ -193,10 +107,6 @@ struct MaskCursor {
   const int32_t* end[BM];
   int next[BM];                // smallest training item id not yet passed (INT_MAX: none left)
 };
-
-__device__ __forceinline__ unsigned long long pack_state(int n, float tau) {
-  return ((unsigned long long)(unsigned)n << 32) | (unsigned long long)__float_as_uint(tau);
-}
 
 // One column of a chunk has at least one survivor in this warp (lanes in `b`).  Called by the
 // whole warp (convergent), out of line.  Each surviving lane runs the mask cursor and appends
@@ -320,26 +230,8 @@ __global__ void __launch_bounds__(kThreads, 2)
 score_topk_tc_kernel(const uint8_t* __restrict__ Ub, const uint8_t* __restrict__ Ib, int64_t B,
                      int m_items, int n_item_tiles, const int64_t* __restrict__ user_ids,
                      const int64_t* __restrict__ mask_rowptr, const int32_t* __restrict__ mask_col,
-                     int k, int32_t* __restrict__ out_idx, float* __restrict__ out_val, int stages,
-                     long long* __restrict__ trace, int dbg) {
+                     int k, int32_t* __restrict__ out_idx, float* __restrict__ out_val, int stages) {
   constexpr int CAP = 32 * EPL;
-  // bring-up instrumentation (trace == nullptr in production): CTA 0 records clock64 stamps of
-  // tiles [kTraceT0, kTraceT0 + 64): MMA thread [t][5] loop top, [6] B tile landed, [0] TMEM
-  // buffer free, [1] chain issued; epilogue warp 2 [t][2] accumulator ready, [3] drained
-  // (compiled in only with -DSPEX_TC_TRACE: the stamps lengthen the MMA thread's loop; the same
-  // builds read SPEX_TC_DBG: bit 0 = nothing survives, i.e. the cost of the survivor path)
-#ifdef SPEX_TC_TRACE
-  constexpr int kTraceT0 = 2000;
-  const bool tracing = trace != nullptr && blockIdx.x == 0;
-#define SPEX_TC_STAMP(t, slot)                                                       \
-  do {                                                                               \
-    if (tracing && (t) >= kTraceT0 && (t) < kTraceT0 + 64)                           \
-      trace[((t) - kTraceT0) * 8 + (slot)] = clock64();                              \
-  } while (0)
-#else
-#define SPEX_TC_STAMP(t, slot) do { } while (0)
-#endif
-  constexpr uint32_t lbo = 128, sbo = 1024;   // layout written by spex_pack_bf16 (D = 64)
   extern __shared__ uint8_t smem_raw[];
   __shared__ __align__(8) uint64_t bar_full[kMaxStages];
   __shared__ __align__(8) uint64_t bar_empty[kMaxStages];
@@ -359,95 +251,18 @@ score_topk_tc_kernel(const uint8_t* __restrict__ Ub, const uint8_t* __restrict__
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t tile_m = blockIdx.x;
 
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < stages; ++s) {
-      mbar_init(&bar_full[s], 1);
-      mbar_init(&bar_empty[s], 1);
-    }
-    for (int b = 0; b < 2; ++b) {
-      mbar_init(&bar_tfull[b], 1);
-      mbar_init(&bar_tempty[b], 4);   // one arrive per epilogue warp
-    }
-    mbar_init(&bar_a, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-                     smem_u32(&tmem_slot)),
-                 "r"((uint32_t)kTmemCols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = tmem_slot;
+  const uint32_t tmem_base =
+      pipeline_init(warp, stages, bar_full, bar_empty, bar_tfull, bar_tempty, &bar_a, &tmem_slot);
 
   if (warp == 0) {
-    // ===== producer: one thread streams the user tile once, then every item tile =====
-    if (elect_one()) {
-      mbar_arrive_expect_tx(&bar_a, A_BYTES);
-      bulk_g2s(sA, Ub + tile_m * A_BYTES, A_BYTES, &bar_a);
-      int s = 0;
-      uint32_t ph = 0;
-      for (int t = 0; t < n_item_tiles; ++t) {
-        mbar_wait(&bar_empty[s], ph ^ 1u);
-        mbar_arrive_expect_tx(&bar_full[s], B_BYTES);
-        bulk_g2s(sB + (size_t)s * B_BYTES, Ib + (size_t)t * B_BYTES, B_BYTES, &bar_full[s]);
-        if (++s == stages) {
-          s = 0;
-          ph ^= 1u;
-        }
-      }
-    }
+    producer_role<DK>(Ub, Ib, tile_m, n_item_tiles, stages, sA, sB, bar_full, bar_empty, &bar_a);
   } else if (warp == 1) {
-    // ===== MMA issuer: one thread drives the tensor core =====
-    if (elect_one()) {
-      // instruction descriptor: c=f32 (1<<4), a=bf16 (1<<7), b=bf16 (1<<10), K-major A and B,
-      // N>>3 at [17,23), M>>4 at [24,29)
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN >> 3) << 17) |
-                             ((uint32_t)(BM >> 4) << 24);
-      const uint32_t a_addr = smem_u32(sA);
-      constexpr uint32_t kstep = 2 * lbo;  // 16 bf16 along K = two 8-element core matrices
-      mbar_wait(&bar_a, 0);
-      int s = 0;
-      uint32_t ph = 0;
-      for (int t = 0; t < n_item_tiles; ++t) {
-        const int buf = t & 1;
-        const uint32_t use = (uint32_t)(t >> 1) & 1u;
-        SPEX_TC_STAMP(t, 5);
-        // While the tensor pipe is busy a poll of an mbarrier takes ~200 cycles even when its
-        // phase is long complete (profiles/microbench/mma_pipe.cu), so the two polls of a tile
-        // (operands landed, accumulator drained) are issued back to back and overlap.
-        bool have_b = mbar_try_wait(&bar_full[s], ph);
-        bool have_d = mbar_try_wait(&bar_tempty[buf], use ^ 1u);
-        uint32_t spins = 0;
-        while (!have_b) {
-          have_b = mbar_try_wait(&bar_full[s], ph);
-          if (++spins > kSpinLimit) __trap();
-        }
-        SPEX_TC_STAMP(t, 6);
-        while (!have_d) {
-          have_d = mbar_try_wait(&bar_tempty[buf], use ^ 1u);
-          if (++spins > kSpinLimit) __trap();
-        }
-        tc_fence_after();
-        SPEX_TC_STAMP(t, 0);
-        const uint32_t b_addr = smem_u32(sB + (size_t)s * B_BYTES);
-#pragma unroll
-        for (int kk = 0; kk < DK / UMMA_K; ++kk) {
-          tc_mma(tmem_base + (uint32_t)(buf * BN), make_desc(a_addr + kk * kstep, lbo, sbo),
-                 make_desc(b_addr + kk * kstep, lbo, sbo), idesc, kk > 0 ? 1u : 0u);
-        }
-        tc_commit(&bar_empty[s]);     // smem stage reusable once these MMAs have read it
-        tc_commit(&bar_tfull[buf]);   // accumulator ready for the epilogue
-        SPEX_TC_STAMP(t, 1);
-        if (++s == stages) {
-          s = 0;
-          ph ^= 1u;
-        }
-      }
-    }
+    // instruction descriptor: c=f32 (1<<4), a=bf16 (1<<7), b=bf16 (1<<10), K-major A and B,
+    // N>>3 at [17,23), M>>4 at [24,29)
+    constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN >> 3) << 17) |
+                               ((uint32_t)(BM >> 4) << 24);
+    mma_role<DK>(idesc, sA, sB, tmem_base, n_item_tiles, stages, bar_full, bar_empty, bar_tfull,
+                 bar_tempty, &bar_a);
   } else {
     // ===== epilogue: thread owns one user row; warp = TMEM lane quarter =====
     const int q = warp & 3;
@@ -457,7 +272,6 @@ score_topk_tc_kernel(const uint8_t* __restrict__ Ub, const uint8_t* __restrict__
     int* ci_warp = ci + q * 32 * CAP;
     int n = 0;
     float tau = (grow < B) ? -INFINITY : INFINITY;   // +inf: padded row, nothing survives
-    if (dbg & 1) tau = INFINITY;                     // bring-up builds only
     {
       const int32_t* c = mask_col;
       const int32_t* e = mask_col;
@@ -478,7 +292,6 @@ score_topk_tc_kernel(const uint8_t* __restrict__ Ub, const uint8_t* __restrict__
       const uint32_t use = (uint32_t)(t >> 1) & 1u;
       mbar_wait(&bar_tfull[buf], use);
       tc_fence_after();
-      if (warp == 2 && lane == 0) SPEX_TC_STAMP(t, 2);
       const uint32_t tbase = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * BN);
       const int item0 = t * BN;
       // software pipeline over the four 32-column chunks with three register buffers: two
@@ -500,7 +313,6 @@ score_topk_tc_kernel(const uint8_t* __restrict__ Ub, const uint8_t* __restrict__
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&bar_tempty[buf]);
-      if (warp == 2 && lane == 0) SPEX_TC_STAMP(t, 3);
     }
     // final compaction of every row (sorted best-first), then each thread writes its own row
     n = (int)(tc_column<EPL>(kFull, 0.f, 0, n, tau, k, m_items, lane, row, cv_warp, ci_warp, &mc, true) >> 32);
@@ -512,47 +324,17 @@ score_topk_tc_kernel(const uint8_t* __restrict__ Ub, const uint8_t* __restrict__
       }
     }
   }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base),
-                 "r"((uint32_t)kTmemCols)
-                 : "memory");
-  }
+  pipeline_teardown(warp, tmem_base);
 }
 
-// fp32 [rows, D] -> bf16 core-matrix-tiled layout:
-//   byte offset of (r, k) = (r/8) * (16*D) + (k/8) * 128 + (r%8) * 16 + (k%8) * 2
-// optional row gather; rows in [n, n_pad) are zero.  Thread per (row, 8-element chunk).
+// fp32 [rows, D] -> bf16 in the layout of pack_rows
 __global__ void __launch_bounds__(256)
 pack_bf16_kernel(const float* __restrict__ src, const int64_t* __restrict__ rows, int64_t n,
                  int64_t n_pad, int D, uint8_t* __restrict__ dst) {
-  const int D8 = D >> 3;
-  const int64_t total = n_pad * D8;
-  int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  for (; i < total; i += stride) {
-    const int64_t r = i / D8;
-    const int kc = (int)(i - r * D8);
-    float4 a = f4_zero(), b = f4_zero();
-    if (r < n) {
-      const int64_t sr = rows ? rows[r] : r;
-      a = *reinterpret_cast<const float4*>(src + sr * D + kc * 8);
-      b = *reinterpret_cast<const float4*>(src + sr * D + kc * 8 + 4);
-    }
-    uint4 pk;
-    pk.x = (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(a.x)) |
-           ((uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(a.y)) << 16);
-    pk.y = (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(a.z)) |
-           ((uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(a.w)) << 16);
-    pk.z = (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(b.x)) |
-           ((uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(b.y)) << 16);
-    pk.w = (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(b.z)) |
-           ((uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(b.w)) << 16);
-    const int64_t off = (r >> 3) * (16 * (int64_t)D) + (int64_t)kc * 128 + (r & 7) * 16;
-    *reinterpret_cast<uint4*>(dst + off) = pk;
-  }
+  pack_rows(src, rows, n, n_pad, D, dst, [](float x, float y) -> uint32_t {
+    return (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(x)) |
+           ((uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(y)) << 16);
+  });
 }
 
 }  // namespace tc
@@ -574,24 +356,14 @@ extern "C" int spex_pack_bf16(const float* src, const int64_t* rows, int64_t n, 
   return check_last();
 }
 
-static long long* g_tc_trace = nullptr;
-// bring-up only (not part of the declared ABI): device buffer of 64*8 int64 clock stamps
-extern "C" void spex_debug_tc_trace(void* dev_buf) { g_tc_trace = (long long*)dev_buf; }
-
-static size_t tc_smem_bytes(int cap, int stages) {
-  return 128 + (size_t)tc::A_BYTES + (size_t)stages * tc::B_BYTES + (size_t)cap * tc::BM * 8;
-}
-
 template <int EPL>
 static int tc_launch(const void* Ub, const void* Ib, int64_t B, int64_t B_pad, int64_t m_items,
                      int64_t m_pad, const int64_t* user_ids, const int64_t* mask_rowptr,
                      const int32_t* mask_col, int32_t k, int32_t* out_idx, float* out_val,
                      cudaStream_t st) {
   // two CTAs per SM need <= ~113 KB each (228 KB per SM, 1 KB reserved per CTA, static smem)
-  int stages = tc::kMaxStages;
-  while (stages > 2 && tc_smem_bytes(32 * EPL, stages) + 2800 > 115712) --stages;
-  if (const char* e = getenv("SPEX_TC_STAGES")) stages = atoi(e);   // bring-up experiment
-  const size_t smem = tc_smem_bytes(32 * EPL, stages);
+  const int stages = tcgen05::choose_stages(tc::DK, 32 * EPL, 115712 - 2800);
+  const size_t smem = tcgen05::smem_bytes(tc::DK, 32 * EPL, stages);
   SPEX_RETURN_IF(smem > 226 * 1024, SPEX_E_TOOBIG);
   // per device and per function, and the size depends on `stages`: set on every launch (cheap)
   {
@@ -601,13 +373,9 @@ static int tc_launch(const void* Ub, const void* Ib, int64_t B, int64_t B_pad, i
   }
   const int64_t grid = B_pad / tc::BM;
   SPEX_RETURN_IF(grid > 0x7fffffffLL, SPEX_E_TOOBIG);
-  int dbg = 0;
-#ifdef SPEX_TC_TRACE
-  if (const char* e = getenv("SPEX_TC_DBG")) dbg = atoi(e);
-#endif
   tc::score_topk_tc_kernel<EPL><<<(unsigned)grid, tc::kThreads, smem, st>>>(
       (const uint8_t*)Ub, (const uint8_t*)Ib, B, (int)m_items, (int)(m_pad / tc::BN), user_ids,
-      mask_rowptr, mask_col, k, out_idx, out_val, stages, g_tc_trace, dbg);
+      mask_rowptr, mask_col, k, out_idx, out_val, stages);
   count_launch();
   return check_last();
 }

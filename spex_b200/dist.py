@@ -724,41 +724,15 @@ class ShardedEvaluator:
         self.k, self.group, self.scorer = int(k), group, scorer
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
-        self.D = I_all.shape[1]
         if scorer == "f16" and not ops.f16_filter_is_selective(U_all, I_all, torch.arange(U_all.shape[0], device=I_all.device)):
             scorer = self.scorer = "fp32"      # near-equal scores: the exact scorer is the faster exact path
-        if scorer == "f16":
-            self.Ih, self.m_pad, self.imeta = ops.pack_f16(I_all, None, ops.TC_ITEM_MULTIPLE)
-        elif scorer == "bf16":
-            self.Ib, self.m_pad = ops.pack_bf16(I_all, None, ops.TC_ITEM_MULTIPLE)
-        elif scorer != "fp32":
-            raise ValueError("scorer must be 'f16', 'bf16' or 'fp32'")
+        self.ranker = ops.FullRanker(I_all, scorer)
 
     def rank_topk(self, users: torch.Tensor, block: int = 148 * 2 * 128 * 4):
         """(idx int32 [n_local, k], val fp32 [n_local, k], (lo, hi)) for this rank's shard of `users`."""
-        from . import ops
-
         lo, hi = shard_range(users.numel(), self.rank, self.world)
         mine = users[lo:hi].to(torch.int64).contiguous()
-        dev = self.I.device
-        idx = torch.empty(hi - lo, self.k, dtype=torch.int32, device=dev)
-        val = torch.empty(hi - lo, self.k, dtype=torch.float32, device=dev)
-        m = self.I.shape[0]
-        for a in range(0, hi - lo, block):
-            ub = mine[a: a + block]
-            o_i, o_v = idx[a: a + ub.numel()], val[a: a + ub.numel()]
-            if self.scorer == "f16":
-                Uh, b_pad, umeta = ops.pack_f16(self.U, ub, ops.TC_USER_MULTIPLE)
-                ops.score_topk_f16(Uh, umeta, ub.numel(), b_pad, self.Ih, self.imeta, m, self.m_pad, self.D, self.k,
-                                   ub, self.mrp, self.mcol, o_i, o_v)
-            elif self.scorer == "bf16":
-                Ub, b_pad = ops.pack_bf16(self.U, ub, ops.TC_USER_MULTIPLE)
-                ops.score_topk_bf16(Ub, ub.numel(), b_pad, self.Ib, m, self.m_pad, self.k, ub, self.mrp, self.mcol,
-                                    o_i, o_v)
-            else:
-                i32, v32 = ops.score_topk_f32(self.U, self.I, ub, self.k, self.mrp, self.mcol)
-                o_i.copy_(i32)
-                o_v.copy_(v32)
+        idx, val = self.ranker.topk(self.U, mine, self.k, self.mrp, self.mcol, block)
         return idx, val, (lo, hi)
 
     def recall_ndcg(self, users: torch.Tensor, truth_rowptr, truth_col):

@@ -87,7 +87,7 @@ class LightGCN(BasicModel):
         self._mask_csr = None
         self._frozen_out: Optional[torch.Tensor] = None
         self._freeze = False
-        self._item_pack = None
+        self._ranker: Optional[ops.FullRanker] = None
         self._fuse()
 
     # ---- fused table ---------------------------------------------------------------------------
@@ -112,12 +112,12 @@ class LightGCN(BasicModel):
         self._dev_graph = None
         self._mask_csr = None
         self._frozen_out = None
-        self._item_pack = None
+        self._ranker = None
         return self
 
     def train(self, mode: bool = True):
         self._frozen_out = None
-        self._item_pack = None
+        self._ranker = None
         return super().train(mode)
 
     # ---- graph ---------------------------------------------------------------------------------
@@ -271,39 +271,14 @@ class LightGCN(BasicModel):
         mrp = mcol = None
         if exclude_train:
             mrp, mcol = self.train_mask_csr()
-        if precision == "fp32":
-            return ops.score_topk_f32(all_users, all_items, users, k, mrp, mcol)
-        if precision not in ("f16", "bf16"):
-            raise ValueError("precision must be 'f16', 'bf16' or 'fp32'")
-        if precision == "bf16" and self.latent_dim != 64:
-            raise RuntimeError("the bf16 tcgen05 scorer is built for recdim == 64")
-        if precision == "f16" and self.latent_dim not in (64, 128):
-            raise RuntimeError("the f16 tcgen05 scorer is built for recdim 64 or 128")
+        # the packed item table is reused across eval-mode calls; fp32 reads the current table as it is
+        r = self._ranker
+        if r is None or self.training or r.precision != precision or precision == "fp32":
+            r = self._ranker = ops.FullRanker(all_items, precision)
         if precision == "f16" and probe and not ops.f16_filter_is_selective(all_users, all_items, users):
             # degenerate score distribution (near-ties everywhere): the exact scorer is the faster exact path
             return ops.score_topk_f32(all_users, all_items, users, k, mrp, mcol)
-        if self._item_pack is None or self.training or self._item_pack[0] != precision:
-            if precision == "f16":
-                self._item_pack = (precision,) + ops.pack_f16(all_items, None, ops.TC_ITEM_MULTIPLE)
-            else:
-                self._item_pack = (precision,) + ops.pack_bf16(all_items, None, ops.TC_ITEM_MULTIPLE)
-        B = users.numel()
-        idx = torch.empty(B, k, dtype=torch.int32, device=dev)
-        val = torch.empty(B, k, dtype=torch.float32, device=dev)
-        for s in range(0, B, user_block):
-            ub = users[s: s + user_block]
-            if precision == "f16":
-                _, Ih, m_pad, imeta = self._item_pack
-                Uh, b_pad, umeta = ops.pack_f16(all_users, ub, ops.TC_USER_MULTIPLE)
-                ops.score_topk_f16(Uh, umeta, ub.numel(), b_pad, Ih, imeta, self.num_items, m_pad,
-                                   self.latent_dim, k, ub, mrp, mcol, idx[s: s + ub.numel()],
-                                   val[s: s + ub.numel()])
-            else:
-                _, Ib, m_pad = self._item_pack
-                Ub, b_pad = ops.pack_bf16(all_users, ub, ops.TC_USER_MULTIPLE)
-                ops.score_topk_bf16(Ub, ub.numel(), b_pad, Ib, self.num_items, m_pad, k, ub, mrp, mcol,
-                                    idx[s: s + ub.numel()], val[s: s + ub.numel()])
-        return idx, val
+        return r.topk(all_users, users, k, mrp, mcol, user_block)
 
 
 def dropout_seed() -> int:

@@ -114,7 +114,7 @@ class LightGCN(_RecLightGCN):
         self._mask_csr = None
         self._frozen_out = None
         self._freeze = False
-        self._item_pack = None
+        self._ranker = None
         self._fuse()
 
     # ---- recommendation branch -----------------------------------------------------------------

@@ -211,10 +211,7 @@ class Model_Wrapper(nn.Module):
         if precision == "fp32" or Dk not in (64, 128) or (probe and not ops.f16_filter_is_selective(ua, ia, users)):
             # (an untrained NGCF's normalised outputs are almost parallel: near-ties everywhere, no filter helps)
             return ops.score_topk_f32(ua, ia, users, k, mask_rowptr, mask_col)
-        Ih, m_pad, imeta = ops.pack_f16(ia, None, ops.TC_ITEM_MULTIPLE)
-        Uh, b_pad, umeta = ops.pack_f16(ua, users, ops.TC_USER_MULTIPLE)
-        return ops.score_topk_f16(Uh, umeta, users.numel(), b_pad, Ih, imeta, ia.shape[0], m_pad, Dk, k, users,
-                                  mask_rowptr, mask_col)
+        return ops.FullRanker(ia, "f16").topk(ua, users, k, mask_rowptr, mask_col)
 
     @torch.no_grad()
     def rate_all_items(self, users):

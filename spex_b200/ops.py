@@ -867,6 +867,58 @@ def score_topk_f16(Uh, u_meta, B, B_pad, Ih, i_meta, m_items, m_pad, D, k, user_
     return out_idx, out_val
 
 
+class FullRanker:
+    """Full-ranking top-k of user rows against one item table, (idx int32 [B, k], score fp32 [B, k]): score
+    descending, ties by ascending item id, the items of each user's mask row excluded.
+
+    precision "f16":  tcgen05 fp16-accumulator filter + exact fp32 re-score (score_topk_f16; D 64 or 128);
+    precision "bf16": tcgen05 bf16 operands / fp32 accumulators (score_topk_bf16; D = 64);
+    precision "fp32": exact CUDA-core scorer (score_topk_f32; any D).
+    The item table is packed once, here (the fp32 scorer reads it as it is); the users are packed block by
+    block in topk()."""
+
+    def __init__(self, I_all, precision: str = "f16"):
+        D = I_all.shape[1]
+        if precision not in ("f16", "bf16", "fp32"):
+            raise ValueError("precision must be 'f16', 'bf16' or 'fp32'")
+        if precision == "bf16" and D != 64:
+            raise RuntimeError("the bf16 tcgen05 scorer is built for recdim == 64")
+        if precision == "f16" and D not in (64, 128):
+            raise RuntimeError("the f16 tcgen05 scorer is built for recdim 64 or 128")
+        self.precision, self.device = precision, I_all.device
+        self.m_items, self.D = I_all.shape
+        self._I = I_all if precision == "fp32" else None
+        if precision == "f16":
+            self._Ih, self._m_pad, self._imeta = pack_f16(I_all, None, TC_ITEM_MULTIPLE)
+        elif precision == "bf16":
+            self._Ib, self._m_pad = pack_bf16(I_all, None, TC_ITEM_MULTIPLE)
+
+    def topk(self, U_all, users, k, mask_rowptr=None, mask_col=None, user_block=None):
+        """Rank U_all[users] in blocks of `user_block` users (None: one block)."""
+        dev, m, D = self.device, self.m_items, self.D
+        users = _i64c(users, dev)
+        B = users.numel()
+        idx = torch.empty(B, k, dtype=torch.int32, device=dev)
+        val = torch.empty(B, k, dtype=torch.float32, device=dev)
+        step = user_block or max(B, 1)
+        for s in range(0, B, step):
+            ub = users[s: s + step]
+            o_i, o_v = idx[s: s + ub.numel()], val[s: s + ub.numel()]
+            if self.precision == "f16":
+                Uh, b_pad, umeta = pack_f16(U_all, ub, TC_USER_MULTIPLE)
+                score_topk_f16(Uh, umeta, ub.numel(), b_pad, self._Ih, self._imeta, m, self._m_pad, D, k, ub,
+                               mask_rowptr, mask_col, o_i, o_v)
+            elif self.precision == "bf16":
+                Ub, b_pad = pack_bf16(U_all, ub, TC_USER_MULTIPLE)
+                score_topk_bf16(Ub, ub.numel(), b_pad, self._Ib, m, self._m_pad, k, ub, mask_rowptr, mask_col,
+                                o_i, o_v)
+            else:
+                i32, v32 = score_topk_f32(U_all, self._I, ub, k, mask_rowptr, mask_col)
+                o_i.copy_(i32)
+                o_v.copy_(v32)
+        return idx, val
+
+
 GATE_BWD_BLOCKS = 1184  # SPEX_GATE_BWD_BLOCKS in include/spex_b200.h
 
 
