@@ -6,6 +6,7 @@ Also prints the slow-path statistics of the f16 kernel (tiles that entered the s
 """
 import argparse
 import ctypes as C
+import hashlib
 import json
 import os
 import sys
@@ -69,6 +70,8 @@ def main():
                   "block_calls_per_warp": st[1] / nw, "slow_path_cycles_per_warp": st[2] / nw,
                   "inserts_per_warp": st[3] / nw, "exact_settlements_per_warp": st[4] / nw,
                   "exact_settlement_cycles_per_warp": st[5] / nw}
+    # digest of the f16 result bits: two builds of the exact scorer must agree on it
+    out["f16"]["out_sha256"] = hashlib.sha256(idx.cpu().numpy().tobytes() + val.cpu().numpy().tobytes()).hexdigest()
     i16 = idx.clone()
     if args.D == 64:
         Ib, m_pad2 = ops.pack_bf16(I, None, ops.TC_ITEM_MULTIPLE)

@@ -13,10 +13,14 @@
 //     every row norm is below 2^7: no overflow, |score| < 2^14), same UMMA no-swizzle K-major
 //     canonical layout as before (8-row x 16-byte core matrices, one bulk copy per tile);
 //   * the tensor core accumulates in fp16 (tcgen05.mma.kind::f16, c_format = F16).  That result
-//     `a` is only a FILTER: |a - s| <= eps_u = 2^-9 |u| Vmax + 2^-10 for the exact score s of the
-//     same fp16 operands (four K=16 steps, each rounding a partial sum bounded by sum|u_d v_d| <=
-//     |u||v| to fp16: 4 * 2^-12 with round-to-nearest, 4 * 2^-11 = 2^-9 even with truncation;
-//     measured ~2^-14 |u||v|, profiles/microbench/f16acc_b200.txt);
+//     `a` is only a FILTER: |a - s| <= eps_u = (DK/16) 2^-11 |u| Vmax + 2^-10 for the exact score s
+//     of the same fp16 operands.  Each of the DK/16 K=16 MMAs of a tile reads the fp16 accumulator
+//     and writes it back rounded to fp16; the partial sum it rounds is bounded by sum|u_d v_d| <=
+//     |u||v|, so with round-to-nearest (unit roundoff 2^-11) each step adds at most 2^-11 |u||v|:
+//     2^-9 at D = 64 (4 steps), 2^-8 at D = 128 (8 steps); 2^-10 covers fp16 subnormals.  The bound
+//     is nearly reached: tests/test_gpu_ranking_edges.py builds items that lose (DK/16 - 0.6) 2^-11
+//     |u| Vmax (a margin of 2^-9 dropped them at D = 128).  Truncation would need twice the margin.
+//     One random tile shows ~2^-14 |u||v| (profiles/microbench/f16acc_b200.txt);
 //   * an epilogue thread owns one user row: ONE tcgen05.ld.x64.pack::16b brings the 128 scores of
 //     its row into 64 registers, the accumulator buffer is handed back to the MMA warp at once,
 //     63 HMNMX2 + one compare + one vote reject the tile against the row's threshold thr.
@@ -49,7 +53,9 @@ namespace tf {
 
 using namespace tcgen05;
 
-constexpr float kEpsRel = 1.0f / 512.0f;    // 2^-9, see the header comment
+// filter margin per unit |u| Vmax: one fp16 rounding (2^-11) per K=16 step, see the header comment
+template <int DK>
+constexpr float kEpsRel = (DK / 16) * (1.0f / 2048.0f);   // D = 64: 2^-9, D = 128: 2^-8
 constexpr float kEpsAbs = 1.0f / 1024.0f;   // subnormal flush of tiny operands (bound 2^-11)
 
 // tcgen05.ld 32 lanes x 128 columns of 16-bit accumulators packed two per register (column 2i in
@@ -371,7 +377,7 @@ score_topk_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict_
       }
     }
     const float vmax = i_meta[2];                       // max scaled item-row norm
-    const float eps = kEpsRel * sqrtf(un2) * vmax * 1.0001f + kEpsAbs;
+    const float eps = kEpsRel<DK> * sqrtf(un2) * vmax * 1.0001f + kEpsAbs;
     float* cv_row = cv_warp + lane * CAP;
     int* ci_row = ci_warp + lane * CAP;
     __half thr = __float2half_rd(thrf);                 // -inf (or +inf for padded rows)

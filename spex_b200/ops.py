@@ -764,8 +764,8 @@ def rating_dense(U, I, users, apply_sigmoid: bool = True):
 
 def f16_filter_is_selective(U, I, users, n_users: int = 64, n_items: int = 8192, seed: int = 0) -> bool:
     """Probe for spex_score_topk_f16.  Its fp16-accumulated score only FILTERS: everything within 2 eps of a
-    row's k-th best (eps = 2^-9 |u| max|v|) is re-scored exactly, one row at a time.  On tables whose scores are
-    nearly equal across items - an untrained NGCF model, whose normalised layer outputs are almost parallel:
+    row's k-th best (eps = 2^-9 |u| max|v| at D = 64, 2^-8 at D = 128; the probe uses 2^-9) is re-scored
+    exactly, one row at a time.  On tables whose scores are nearly equal across items - an untrained NGCF model, whose normalised layer outputs are almost parallel:
     measured 99 ms against 1.7 ms for random tables of the same shape and 7 ms for the exact fp32 scorer - that
     band holds most items and the filter degenerates.  The probe scores a sample (n_users x n_items, exact fp32,
     spex_rating_f32) and compares the band with the spread of each user's scores: selective iff the median of
@@ -874,8 +874,7 @@ class FullRanker:
     precision "f16":  tcgen05 fp16-accumulator filter + exact fp32 re-score (score_topk_f16; D 64 or 128);
     precision "bf16": tcgen05 bf16 operands / fp32 accumulators (score_topk_bf16; D = 64);
     precision "fp32": exact CUDA-core scorer (score_topk_f32; any D).
-    The item table is packed once, here (the fp32 scorer reads it as it is); the users are packed block by
-    block in topk()."""
+    The item table is packed once, here (the fp32 scorer reads it as it is); the users are packed in topk()."""
 
     def __init__(self, I_all, precision: str = "f16"):
         D = I_all.shape[1]
@@ -894,18 +893,29 @@ class FullRanker:
             self._Ib, self._m_pad = pack_bf16(I_all, None, TC_ITEM_MULTIPLE)
 
     def topk(self, U_all, users, k, mask_rowptr=None, mask_col=None, user_block=None):
-        """Rank U_all[users] in blocks of `user_block` users (None: one block)."""
+        """Rank U_all[users] in blocks of `user_block` users (None: one block).
+
+        f16: the result does not depend on `user_block`.  The users of the call are packed once, so one user
+        scale 2^s, chosen over all of them, rounds every user's operands (a per-block scale would round a user's
+        fp16 subnormal components differently depending on its block-mates); each block is a slice of that
+        buffer, `user_block` rounded up to a multiple of 128 rows."""
         dev, m, D = self.device, self.m_items, self.D
         users = _i64c(users, dev)
         B = users.numel()
         idx = torch.empty(B, k, dtype=torch.int32, device=dev)
         val = torch.empty(B, k, dtype=torch.float32, device=dev)
         step = user_block or max(B, 1)
+        if self.precision == "f16":
+            step = (step + TC_USER_MULTIPLE - 1) // TC_USER_MULTIPLE * TC_USER_MULTIPLE
+            if B:
+                Uh_all, _, umeta = pack_f16(U_all, users, TC_USER_MULTIPLE)
         for s in range(0, B, step):
             ub = users[s: s + step]
             o_i, o_v = idx[s: s + ub.numel()], val[s: s + ub.numel()]
             if self.precision == "f16":
-                Uh, b_pad, umeta = pack_f16(U_all, ub, TC_USER_MULTIPLE)
+                # the canonical layout keeps every 8-row group contiguous: rows [s, s + b_pad) are one slice
+                b_pad = (ub.numel() + TC_USER_MULTIPLE - 1) // TC_USER_MULTIPLE * TC_USER_MULTIPLE
+                Uh = Uh_all[s * D: (s + b_pad) * D]
                 score_topk_f16(Uh, umeta, ub.numel(), b_pad, self._Ih, self._imeta, m, self._m_pad, D, k, ub,
                                mask_rowptr, mask_col, o_i, o_v)
             elif self.precision == "bf16":
