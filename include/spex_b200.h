@@ -378,6 +378,27 @@ int spex_score_topk_f16(const void* Uh, const void* Ih, int32_t D, int64_t B, in
                         void* stream);
 
 /*
+ * The same scorer for 1 <= k <= 512: same operands, filter, mask, user_ids and output contract as
+ * spex_score_topk_f16 (exact top-k of the fp32 scores of the fp16 operands, score descending, ties
+ * by ascending item id, -1 / -inf past the user's unmasked items).  Each user row's candidate
+ * buffer lives in the caller's workspace instead of shared memory: work (device, 16-byte aligned)
+ * of at least spex_score_topk_f16_wide_workspace_bytes(B_pad, k) bytes, B_pad * cap(k) entries of
+ * 8 bytes with cap(k) = 2k + 64 rounded up to 32; its contents on entry do not matter.  Serves
+ * the k above 64 that spex_score_topk_f16 rejects (and above 128, where spex_score_topk_f32 stops).
+ * Errors, before anything is launched: SPEX_E_TOOBIG for k outside [1, 512] or m_pad >= 2^31;
+ * SPEX_E_WORKSPACE for work NULL or smaller than the query; SPEX_E_ALIGN for Uh, Ih or work
+ * misaligned; SPEX_E_BADARG for B_pad or m_pad not a multiple of 128, half a mask, NULL operands
+ * or outputs; SPEX_E_BADDIM for D not 64 or 128.
+ * spex_score_topk_f16_wide_workspace_bytes returns 0 for B_pad < 0 or k outside [1, 512].
+ */
+int64_t spex_score_topk_f16_wide_workspace_bytes(int64_t B_pad, int32_t k);
+int spex_score_topk_f16_wide(const void* Uh, const void* Ih, int32_t D, int64_t B, int64_t B_pad,
+                             int64_t m_items, int64_t m_pad, const float* u_meta, const float* i_meta,
+                             const int64_t* user_ids, const int64_t* mask_rowptr,
+                             const int32_t* mask_col, int32_t k, int32_t* out_idx, float* out_val,
+                             void* work, int64_t work_bytes, void* stream);
+
+/*
  * Sampled-candidate scoring for the reference Test() (batch_test.py:28-40, hoisted):
  *   score[u,c] = <U[users[u]], I[cand[u,c]]>,  cand int32 [n_u, n_c]  ->  score fp32 [n_u, n_c]
  */

@@ -74,6 +74,9 @@ SIGNATURES = {
     "spex_score_topk_bf16": (C.c_int, [_p, _p, _i64, _i64, _i64, _i64, _p, _p, _p, _i32, _p, _p, _p]),
     "spex_pack_f16": (C.c_int, [_p, _p, _i64, _i64, _i32, _p, _p, _p]),
     "spex_score_topk_f16": (C.c_int, [_p, _p, _i32, _i64, _i64, _i64, _i64, _p, _p, _p, _p, _p, _i32, _p, _p, _p]),
+    "spex_score_topk_f16_wide_workspace_bytes": (_i64, [_i64, _i32]),
+    "spex_score_topk_f16_wide": (C.c_int, [_p, _p, _i32, _i64, _i64, _i64, _i64, _p, _p, _p, _p, _p, _i32, _p, _p, _p,
+                                           _i64, _p]),
     "spex_score_candidates_f32": (C.c_int, [_p, _p, _i32, _p, _p, _i64, _i32, _p, _p]),
     "spex_ngcf_epilogue_f32": (C.c_int, [_p, _p, _p, _p, _p, _p, _i64, _i32, _f, _p, _p, _i64, _p]),
     "spex_ngcf_layer_fwd_f32": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _i64, _i32, _f, _p, _p, _i64, _p]),
@@ -99,7 +102,8 @@ SIGNATURES = {
     ),
 }
 
-_NO_STATUS = {"spex_abi_version", "spex_error_string", "spex_launch_count", "spex_scatter_workspace_bytes"}
+_NO_STATUS = {"spex_abi_version", "spex_error_string", "spex_launch_count", "spex_scatter_workspace_bytes",
+              "spex_score_topk_f16_wide_workspace_bytes"}
 
 
 class SpexLibraryMissing(ImportError):

@@ -44,6 +44,9 @@
 //     outputs, NGCF_SPEX/code/main_rec.py:85; one CTA per SM).
 //   * warp roles as in round 1: warp 0 bulk-copy producer, warp 1 TMEM allocator + MMA issuer
 //     (elect.sync, back-to-back polls), warps 2-5 epilogue (TMEM lane quarter = warp % 4).
+//   * k > 64 (spex_score_topk_f16_wide, up to 512): the same kernel with EPL = kWorkspace keeps each
+//     row's buffer of cap = 2k + 64 entries in a global workspace and compacts through a per-warp
+//     shared scratch (tf_compact_ws: radix select instead of the shuffle ranking; DESIGN §4.3).
 #include "tcgen05.cuh"
 #include <cuda_fp16.h>
 #include <stdlib.h>
@@ -289,6 +292,178 @@ __device__ __noinline__ unsigned long long tf_compact(unsigned need, int n, int 
   return pack_state(n | (nsort << 16), thrf);
 }
 
+// ---- wide candidate buffers (k up to KMAX_WIDE) ---------------------------------------------------------------
+// EPL of the kernel whose candidate buffers live in a caller-owned global workspace: row r of the launch owns
+// entries [r * cap, (r + 1) * cap), each a uint2 {score bits, item id | kApprox while the score is a filter value}.
+// Only the row's epilogue thread appends to it; a warp compacts one row at a time through a per-warp shared scratch
+// of cap entries.
+constexpr int kWorkspace = 0;
+constexpr int KMAX_WIDE = 512;
+
+// buffer capacity: the k kept entries, as much room again, and 64 slots for the near-ties of the fast form
+static inline int wide_cap(int k) { return (2 * k + 64 + 31) / 32 * 32; }
+
+// order-preserving uint32 key of a float (-0 as +0, so that key order agrees with `beats`)
+__device__ __forceinline__ unsigned ord_key(unsigned bits) {
+  bits = (bits == 0x80000000u) ? 0u : bits;
+  return (bits & 0x80000000u) ? ~bits : (bits | 0x80000000u);
+}
+// (score desc, id asc) as one descending uint64 key of an exact entry
+__device__ __forceinline__ unsigned long long entry_key(uint2 e) {
+  return ((unsigned long long)ord_key(e.x) << 32) | (unsigned)(0x7fffffff - (int)(e.y & 0x7fffffff));
+}
+
+// k-th largest (1 <= k <= ns) of key(sc[p]), p < ns, on bits [lo, 64): one warp, a bitwise radix select (64 - lo
+// counting passes over the scratch).  The bits below lo of the result are zero.
+template <class Key>
+__device__ __forceinline__ unsigned long long kth_largest(const uint2* sc, int ns, int k, int lo, Key key) {
+  const int lane = threadIdx.x & 31;
+  unsigned long long pre = 0;
+#pragma unroll 1
+  for (int b = 63; b >= lo; --b) {
+    const unsigned long long want = pre | (1ull << b);
+    int c = 0;
+#pragma unroll 4
+    for (int p = lane; p < ns; p += 32) c += ((key(sc[p]) ^ want) >> b) == 0 ? 1 : 0;
+    c = (int)__reduce_add_sync(kFull, (unsigned)c);
+    if (c >= k) pre = want;
+    else k -= c;
+  }
+  return pre;
+}
+
+// the entries p < ns of sc with keep(sc[p]), in their order, to dst[0, count) (dst may be sc); returns count
+template <class Keep>
+__device__ __forceinline__ int warp_compact(uint2* sc, int ns, uint2* dst, Keep keep) {
+  const int lane = threadIdx.x & 31;
+  int c = 0;
+#pragma unroll 1
+  for (int p0 = 0; p0 < ns; p0 += 32) {
+    const int p = p0 + lane;
+    const uint2 e = (p < ns) ? sc[p] : make_uint2(0u, 0u);
+    const bool kp = p < ns && keep(e);
+    const unsigned b = __ballot_sync(kFull, kp);
+    __syncwarp();                                // every read of this chunk precedes any in-place write
+    if (kp) dst[c + __popc(b & ((1u << lane) - 1u))] = e;
+    c += __popc(b);
+  }
+  __syncwarp();
+  return c;
+}
+
+// Compaction of the wide buffers of the rows in `need`, by the whole warp, one row at a time.  The invariants of
+// tf_compact, with a selection in place of the O(cap^2) shuffle ranking:
+// Fast form (no global load of the operands): A = the k-th largest value (radix select on the float bits); the
+// entries >= A - 2 eps are kept in place, the threshold becomes A - 2 eps.
+// Exact form (when the fast form would keep more than half the headroom - near-ties - and in the final pass): the
+// flagged entries are re-scored exactly, the k best under (score desc, id asc) are selected on the 64-bit key of
+// entry_key (so exact ties cannot keep more than k), and the threshold becomes (exact k-th best) - eps.
+// Final pass (`out_idx` != NULL): the exact form, then a bitonic sort of the kept entries in the scratch and the
+// row's output, written by the warp: the k slots of row grow = row_g0 + r (when grow < B), -1 / -inf past the
+// entries held.  Returns this lane's (n, filter threshold).
+template <int DK>
+__device__ __noinline__ unsigned long long tf_compact_ws(unsigned need, int n, float thrf, float eps, int k, int cap,
+                                                         int lane, int row0, const uint8_t* sA, const uint8_t* Ib,
+                                                         uint2* ws_warp, uint2* sc, int64_t row_g0, int64_t B,
+                                                         float inv, int32_t* out_idx, float* out_val,
+                                                         unsigned long long* stats) {
+  const bool final_pass = out_idx != nullptr;
+  __syncwarp();                                  // the lanes' appends to the buffers are visible to the warp
+  while (need) {
+    const long long c0 = stats ? clock64() : 0;
+    const int src = __ffs(need) - 1;
+    need &= need - 1;
+    const int ns = __shfl_sync(kFull, n, src);
+    const float eps_s = __shfl_sync(kFull, eps, src);
+    uint2* wr = ws_warp + (size_t)src * cap;
+    for (int p = lane; p < ns; p += 32) sc[p] = wr[p];
+    __syncwarp();
+    bool exact = final_pass || ns <= k;
+    float new_thr = -INFINITY;
+    int new_n = ns;
+    if (!exact) {
+      const unsigned ka = (unsigned)(kth_largest(sc, ns, k, 32, [](uint2 e) {
+                                       return (unsigned long long)ord_key(e.x) << 32;
+                                     }) >> 32);
+      const float A = __uint_as_float((ka & 0x80000000u) ? (ka & 0x7fffffffu) : ~ka);
+      const float keep = A - 2.f * eps_s;
+      int c_keep = 0;
+      for (int p = lane; p < ns; p += 32) c_keep += (__uint_as_float(sc[p].x) >= keep) ? 1 : 0;
+      c_keep = (int)__reduce_add_sync(kFull, (unsigned)c_keep);
+      if (c_keep <= (cap + k) / 2) {
+        new_n = warp_compact(sc, ns, wr, [keep](uint2 e) { return __uint_as_float(e.x) >= keep; });
+        new_thr = keep;
+      } else {
+        exact = true;                            // too many near-ties: settle them exactly
+      }
+    }
+    if (exact) {
+      const int rr = row0 + src;
+      const uint8_t* a_row = sA + (size_t)(rr >> 3) * (16 * DK) + (size_t)(rr & 7) * 16;
+      for (int p = lane; p < ns; p += 32) {
+        const uint2 e = sc[p];
+        if (e.y & (unsigned)kApprox) {
+          const int id = (int)(e.y & 0x7fffffffu);
+          sc[p] = make_uint2(__float_as_uint(exact_score<DK>(a_row, Ib, id)), (unsigned)id);
+        }
+      }
+      __syncwarp();
+      new_n = ns;
+      if (ns > k) {
+        const unsigned long long kk = kth_largest(sc, ns, k, 0, [](uint2 e) { return entry_key(e); });
+        new_n = warp_compact(sc, ns, final_pass ? sc : wr, [kk](uint2 e) { return entry_key(e) >= kk; });
+        const unsigned ke = (unsigned)(kk >> 32);
+        new_thr = __uint_as_float((ke & 0x80000000u) ? (ke & 0x7fffffffu) : ~ke) - eps_s;
+      } else if (!final_pass) {
+        for (int p = lane; p < ns; p += 32) wr[p] = sc[p];
+      }
+      if (final_pass) {
+        // bitonic sort of the new_n kept entries, best first; the padding up to a power of two never wins
+        int np2 = 1;
+        while (np2 < new_n) np2 <<= 1;
+        for (int p = new_n + lane; p < np2; p += 32) sc[p] = make_uint2(__float_as_uint(-INFINITY), 0x7fffffffu);
+        __syncwarp();
+        for (int size = 2; size <= np2; size <<= 1) {
+          for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            for (int t = lane; t < (np2 >> 1); t += 32) {
+              const int i = 2 * t - (t & (stride - 1)), j = i + stride;
+              const uint2 a = sc[i], b = sc[j];
+              const bool b_first = beats(__uint_as_float(b.x), (int)b.y, __uint_as_float(a.x), (int)a.y);
+              if (b_first == ((i & size) == 0)) {
+                sc[i] = b;
+                sc[j] = a;
+              }
+            }
+            __syncwarp();
+          }
+        }
+        const int64_t grow = row_g0 + src;
+        if (grow < B) {
+          for (int p = lane; p < k; p += 32) {
+            const bool ok = p < new_n;
+            out_idx[grow * k + p] = ok ? (int)sc[p].y : -1;
+            out_val[grow * k + p] = ok ? __uint_as_float(sc[p].x) * inv : -INFINITY;
+          }
+        }
+        __syncwarp();
+      }
+    }
+    __syncwarp();
+    if (lane == src) {
+      n = new_n;
+      thrf = fmaxf(thrf, new_thr);               // thresholds never move down
+    }
+    if (stats && lane == 0) {
+      atomicAdd(stats + 3, 1ull);
+      if (exact) atomicAdd(stats + 4, 1ull);
+      atomicAdd(stats + 5, (unsigned long long)(clock64() - c0));
+    }
+  }
+  return pack_state(n, thrf);
+}
+
+// EPL > 0: candidate buffers of CAP = 32 * EPL entries per row in shared memory (k <= KMAX_TC);
+// EPL == kWorkspace: buffers of `cap` entries per row in the global workspace `ws` (k <= KMAX_WIDE)
 template <int DK, int EPL>
 __global__ void __launch_bounds__(kThreads, DK == 64 ? 2 : 1)
 score_topk_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict__ Ih, int64_t B,
@@ -296,10 +471,11 @@ score_topk_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict_
                       const float* __restrict__ i_meta, const int64_t* __restrict__ user_ids,
                       const int64_t* __restrict__ mask_rowptr, const int32_t* __restrict__ mask_col,
                       int k, int32_t* __restrict__ out_idx, float* __restrict__ out_val, int stages,
-                      unsigned long long* __restrict__ stats, int dbg) {
+                      unsigned long long* __restrict__ stats, int dbg, uint2* __restrict__ ws, int cap) {
   // dbg (bring-up, SPEX_TF_DBG): bit 0 = nothing survives the filter (cost of the survivor path by
   // difference), bit 1 = the epilogue only hands the accumulator back (MMA side alone)
-  constexpr int CAP = 32 * EPL;
+  constexpr bool kWide = EPL == kWorkspace;
+  const int CAP = kWide ? cap : 32 * EPL;
   constexpr int A_BYTES = BM * DK * 2, B_BYTES = BN * DK * 2;
   extern __shared__ uint8_t smem_raw[];
   __shared__ __align__(8) uint64_t bar_full[kMaxStages];
@@ -316,6 +492,7 @@ score_topk_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict_
   uint8_t* sB = smem + A_BYTES;                                          // stages x [128 items][DK]
   float* cv = reinterpret_cast<float*>(sB + (size_t)stages * B_BYTES);   // [BM][CAP]
   int* ci = reinterpret_cast<int*>(cv + (size_t)CAP * BM);               // [BM][CAP]
+  uint2* sc = reinterpret_cast<uint2*>(cv);                              // wide: [4 warps][cap] scratch
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t tile_m = blockIdx.x;
@@ -380,6 +557,8 @@ score_topk_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict_
     const float eps = kEpsRel<DK> * sqrtf(un2) * vmax * 1.0001f + kEpsAbs;
     float* cv_row = cv_warp + lane * CAP;
     int* ci_row = ci_warp + lane * CAP;
+    uint2* ws_warp = kWide ? ws + (size_t)(tile_m * BM + q * 32) * CAP : nullptr;
+    uint2* ws_row = kWide ? ws_warp + (size_t)lane * CAP : nullptr;
     __half thr = __float2half_rd(thrf);                 // -inf (or +inf for padded rows)
     unsigned long long n_hits = 0, n_tiles_slow = 0, c_slow = 0;
     const uint32_t tq = tmem_base + ((uint32_t)(q * 32) << 16);
@@ -460,14 +639,23 @@ score_topk_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict_
               mc.cur[row] = c;
             }
             if (mnext != id) {                         // == id: training item of this user, excluded
-              cv_row[n] = __half2float(a);
-              ci_row[n] = id | kApprox;
+              if constexpr (kWide) {
+                ws_row[n] = make_uint2(__float_as_uint(__half2float(a)), (unsigned)(id | kApprox));
+              } else {
+                cv_row[n] = __half2float(a);
+                ci_row[n] = id | kApprox;
+              }
               ++n;
             }
           };
           auto compact = [&](unsigned need) {
-            const unsigned long long st = tf_compact<DK, EPL>(need, n, nsort, thrf, eps, k, lane, q * 32, sA, Ih,
-                                                             cv_warp, ci_warp, false, stats);
+            unsigned long long st;
+            if constexpr (kWide)
+              st = tf_compact_ws<DK>(need, n, thrf, eps, k, CAP, lane, q * 32, sA, Ih, ws_warp, sc + q * CAP, 0, 0,
+                                     0.f, nullptr, nullptr, stats);
+            else
+              st = tf_compact<DK, EPL>(need, n, nsort, thrf, eps, k, lane, q * 32, sA, Ih, cv_warp, ci_warp, false,
+                                       stats);
             thrf = __uint_as_float((unsigned)(st & 0xffffffffull));
             thr = __float2half_rd(thrf);
             n = (int)(st >> 32) & 0xffff;
@@ -504,14 +692,20 @@ score_topk_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict_
         if (stats) c_slow += (unsigned long long)(clock64() - c0);
       }
     }
-    // final compaction of every row (sorted best-first), then each thread writes its own row
-    n = (int)(tf_compact<DK, EPL>(kFull, n, nsort, thrf, eps, k, lane, q * 32, sA, Ih, cv_warp, ci_warp, true, nullptr) >> 32) & 0xffff;
-    if (grow < B) {
-      const float inv = u_meta[1] * i_meta[1];   // 2^-(s_u + s_i): exact
-      for (int p = 0; p < k; ++p) {
-        const bool ok = p < n;
-        out_idx[grow * k + p] = ok ? ci_warp[lane * CAP + p] : -1;
-        out_val[grow * k + p] = ok ? cv_warp[lane * CAP + p] * inv : -INFINITY;
+    if constexpr (kWide) {
+      // final compaction of every row: the warp writes each row's output
+      tf_compact_ws<DK>(kFull, n, thrf, eps, k, CAP, lane, q * 32, sA, Ih, ws_warp, sc + q * CAP,
+                        tile_m * BM + q * 32, B, u_meta[1] * i_meta[1], out_idx, out_val, nullptr);
+    } else {
+      // final compaction of every row (sorted best-first), then each thread writes its own row
+      n = (int)(tf_compact<DK, EPL>(kFull, n, nsort, thrf, eps, k, lane, q * 32, sA, Ih, cv_warp, ci_warp, true, nullptr) >> 32) & 0xffff;
+      if (grow < B) {
+        const float inv = u_meta[1] * i_meta[1];   // 2^-(s_u + s_i): exact
+        for (int p = 0; p < k; ++p) {
+          const bool ok = p < n;
+          out_idx[grow * k + p] = ok ? ci_warp[lane * CAP + p] : -1;
+          out_val[grow * k + p] = ok ? cv_warp[lane * CAP + p] * inv : -INFINITY;
+        }
       }
     }
     if (stats && lane == 0) {   // bring-up statistics, summed over epilogue warps: slow-path tiles, block
@@ -584,13 +778,17 @@ template <int DK, int EPL>
 static int launch(const void* Uh, const void* Ih, int64_t B, int64_t B_pad, int64_t m_items,
                   int64_t m_pad, const float* u_meta, const float* i_meta, const int64_t* user_ids,
                   const int64_t* mask_rowptr, const int32_t* mask_col, int32_t k, int32_t* out_idx,
-                  float* out_val, cudaStream_t st) {
+                  float* out_val, uint2* ws, int cap, cudaStream_t st) {
+  constexpr bool kWide = EPL == kWorkspace;
+  // shared candidate entries per user row; wide: the four per-warp scratches of cap entries
+  const int cand = kWide ? cap / 32 : 32 * EPL;
   // D = 64: two CTAs per SM need <= ~113 KB each (228 KB per SM, 1 KB reserved per CTA, static
   // shared memory ~7 KB); D = 128: one CTA per SM, up to 227 KB
-  int stages = choose_stages(DK, 32 * EPL, (DK == 64) ? 115712 - 7600 : 227 * 1024 - 7600);
-  if (const char* e = getenv("SPEX_TF_STAGES")) stages = atoi(e);   // bring-up experiment
+  int stages = choose_stages(DK, cand, (DK == 64) ? 115712 - 7600 : 227 * 1024 - 7600);
+  if (!kWide)
+    if (const char* e = getenv("SPEX_TF_STAGES")) stages = atoi(e);   // bring-up experiment
   SPEX_RETURN_IF(stages < 2 || stages > kMaxStages, SPEX_E_BADARG);
-  const size_t smem = smem_bytes(DK, 32 * EPL, stages);
+  const size_t smem = smem_bytes(DK, cand, stages);
   SPEX_RETURN_IF(smem > 227 * 1024 - 7600, SPEX_E_TOOBIG);
   cudaError_t e = cudaFuncSetAttribute(score_topk_f16_kernel<DK, EPL>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -598,10 +796,11 @@ static int launch(const void* Uh, const void* Ih, int64_t B, int64_t B_pad, int6
   const int64_t grid = B_pad / BM;
   SPEX_RETURN_IF(grid > 0x7fffffffLL, SPEX_E_TOOBIG);
   int dbg = 0;
-  if (const char* e = getenv("SPEX_TF_DBG")) dbg = atoi(e);   // bring-up experiment
+  if (!kWide)
+    if (const char* e = getenv("SPEX_TF_DBG")) dbg = atoi(e);   // bring-up experiment
   score_topk_f16_kernel<DK, EPL><<<(unsigned)grid, kThreads, smem, st>>>(
       (const uint8_t*)Uh, (const uint8_t*)Ih, B, (int)m_items, (int)(m_pad / BN), u_meta, i_meta,
-      user_ids, mask_rowptr, mask_col, k, out_idx, out_val, stages, g_stats, dbg);
+      user_ids, mask_rowptr, mask_col, k, out_idx, out_val, stages, g_stats, dbg, ws, cap);
   count_launch();
   return check_last();
 }
@@ -615,10 +814,10 @@ static int launch_k(const void* Uh, const void* Ih, int64_t B, int64_t B_pad, in
   int epl_min = 1;
   if (const char* e = getenv("SPEX_TF_EPL")) epl_min = atoi(e);   // bring-up experiment
   if (k <= 24 && epl_min <= 1)
-    return launch<DK, 1>(Uh, Ih, B, B_pad, m_items, m_pad, u_meta, i_meta, user_ids, mask_rowptr, mask_col, k, out_idx, out_val, st);
+    return launch<DK, 1>(Uh, Ih, B, B_pad, m_items, m_pad, u_meta, i_meta, user_ids, mask_rowptr, mask_col, k, out_idx, out_val, nullptr, 0, st);
   if (k <= 56 && epl_min <= 2)
-    return launch<DK, 2>(Uh, Ih, B, B_pad, m_items, m_pad, u_meta, i_meta, user_ids, mask_rowptr, mask_col, k, out_idx, out_val, st);
-  return launch<DK, 3>(Uh, Ih, B, B_pad, m_items, m_pad, u_meta, i_meta, user_ids, mask_rowptr, mask_col, k, out_idx, out_val, st);
+    return launch<DK, 2>(Uh, Ih, B, B_pad, m_items, m_pad, u_meta, i_meta, user_ids, mask_rowptr, mask_col, k, out_idx, out_val, nullptr, 0, st);
+  return launch<DK, 3>(Uh, Ih, B, B_pad, m_items, m_pad, u_meta, i_meta, user_ids, mask_rowptr, mask_col, k, out_idx, out_val, nullptr, 0, st);
 }
 
 }  // namespace tf
@@ -672,4 +871,34 @@ extern "C" int spex_score_topk_f16(const void* Uh, const void* Ih, int32_t D, in
   if (D == 64)
     return tf::launch_k<64>(Uh, Ih, B, B_pad, m_items, m_pad, u_meta, i_meta, user_ids, mask_rowptr, mask_col, k, out_idx, out_val, st);
   return tf::launch_k<128>(Uh, Ih, B, B_pad, m_items, m_pad, u_meta, i_meta, user_ids, mask_rowptr, mask_col, k, out_idx, out_val, st);
+}
+
+extern "C" int64_t spex_score_topk_f16_wide_workspace_bytes(int64_t B_pad, int32_t k) {
+  if (B_pad < 0 || k < 1 || k > tf::KMAX_WIDE) return 0;
+  return B_pad * tf::wide_cap(k) * (int64_t)sizeof(uint2);
+}
+
+extern "C" int spex_score_topk_f16_wide(const void* Uh, const void* Ih, int32_t D, int64_t B, int64_t B_pad,
+                                        int64_t m_items, int64_t m_pad, const float* u_meta,
+                                        const float* i_meta, const int64_t* user_ids,
+                                        const int64_t* mask_rowptr, const int32_t* mask_col, int32_t k,
+                                        int32_t* out_idx, float* out_val, void* work, int64_t work_bytes,
+                                        void* stream) {
+  SPEX_RETURN_IF(!Uh || !Ih || !u_meta || !i_meta || !out_idx || !out_val || B < 0 || B_pad < B ||
+                     m_items < 0 || m_pad < m_items,
+                 SPEX_E_BADARG);
+  SPEX_RETURN_IF((mask_rowptr == nullptr) != (mask_col == nullptr), SPEX_E_BADARG);
+  SPEX_RETURN_IF((B_pad % tf::BM) || (m_pad % tf::BN), SPEX_E_BADARG);
+  SPEX_RETURN_IF(D != 64 && D != 128, SPEX_E_BADDIM);
+  SPEX_RETURN_IF(k < 1 || k > tf::KMAX_WIDE || m_pad > 0x7fffffffLL, SPEX_E_TOOBIG);
+  SPEX_RETURN_IF(!work || work_bytes < spex_score_topk_f16_wide_workspace_bytes(B_pad, k), SPEX_E_WORKSPACE);
+  SPEX_RETURN_IF(!aligned16(Uh) || !aligned16(Ih) || !aligned16(work), SPEX_E_ALIGN);
+  if (B == 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int cap = tf::wide_cap(k);
+  if (D == 64)
+    return tf::launch<64, tf::kWorkspace>(Uh, Ih, B, B_pad, m_items, m_pad, u_meta, i_meta, user_ids, mask_rowptr,
+                                          mask_col, k, out_idx, out_val, (uint2*)work, cap, st);
+  return tf::launch<128, tf::kWorkspace>(Uh, Ih, B, B_pad, m_items, m_pad, u_meta, i_meta, user_ids, mask_rowptr,
+                                         mask_col, k, out_idx, out_val, (uint2*)work, cap, st);
 }

@@ -724,7 +724,8 @@ class ShardedEvaluator:
         self.k, self.group, self.scorer = int(k), group, scorer
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
-        if scorer == "f16" and not ops.f16_filter_is_selective(U_all, I_all, torch.arange(U_all.shape[0], device=I_all.device)):
+        if (scorer == "f16" and self.k <= ops.F32_MAX_K
+                and not ops.f16_filter_is_selective(U_all, I_all, torch.arange(U_all.shape[0], device=I_all.device))):
             scorer = self.scorer = "fp32"      # near-equal scores: the exact scorer is the faster exact path
         self.ranker = ops.FullRanker(I_all, scorer)
 

@@ -203,12 +203,16 @@ class Model_Wrapper(nn.Module):
                   probe: bool = True):
         """Top-k items per user over the concatenated layer outputs (utility/batch_test.py:158 followed by
         the ranking): tcgen05 fp16-accumulator filter + exact fp32 re-score at D = 64 (L + 1), or the exact
-        fp32 CUDA-core scorer (precision "fp32").  Returns (idx int32 [B, k], score fp32 [B, k])."""
+        fp32 CUDA-core scorer (precision "fp32", k <= 128).  k <= 512 with the f16 scorer; near-equal scores
+        (see ops.f16_filter_is_selective) go to the fp32 scorer when k <= 128.  Returns (idx int32 [B, k],
+        score fp32 [B, k])."""
+        ops.check_k(precision, k)
         ua, ia = self.propagate()
         ua, ia = ua.contiguous(), ia.contiguous()
         users = torch.as_tensor(users, device=ua.device).long().contiguous()
         Dk = ua.shape[1]
-        if precision == "fp32" or Dk not in (64, 128) or (probe and not ops.f16_filter_is_selective(ua, ia, users)):
+        if precision == "fp32" or Dk not in (64, 128) or (probe and k <= ops.F32_MAX_K and
+                                                           not ops.f16_filter_is_selective(ua, ia, users)):
             # (an untrained NGCF's normalised outputs are almost parallel: near-ties everywhere, no filter helps)
             return ops.score_topk_f32(ua, ia, users, k, mask_rowptr, mask_col)
         return ops.FullRanker(ia, "f16").topk(ua, users, k, mask_rowptr, mask_col)

@@ -789,7 +789,9 @@ def f16_filter_is_selective(U, I, users, n_users: int = 64, n_items: int = 8192,
 
 
 TC_USER_MULTIPLE = 128   # users per CTA of the tcgen05 scorer (UMMA M)
-TC_MAX_K = 64            # larger k: score_topk_f32
+TC_MAX_K = 64            # larger k: score_topk_f16_wide (or score_topk_f32 up to F32_MAX_K)
+F32_MAX_K = 128          # k limit of score_topk_f32
+WIDE_MAX_K = 512         # k limit of score_topk_f16_wide
 TC_ITEM_MULTIPLE = 128   # items per tile (UMMA N)
 
 
@@ -867,13 +869,47 @@ def score_topk_f16(Uh, u_meta, B, B_pad, Ih, i_meta, m_items, m_pad, D, k, user_
     return out_idx, out_val
 
 
+def score_topk_f16_wide(Uh, u_meta, B, B_pad, Ih, i_meta, m_items, m_pad, D, k, user_ids=None,
+                        mask_rowptr=None, mask_col=None, out_idx=None, out_val=None):
+    """score_topk_f16 for 1 <= k <= WIDE_MAX_K: the same operands and output contract, each user row's
+    candidate buffer in a device workspace (allocated here, B_pad * (2k + 64) * 8 bytes) instead of shared
+    memory."""
+    _need_cuda(Uh, Ih)
+    if not 1 <= k <= WIDE_MAX_K:
+        raise ValueError(f"score_topk_f16_wide: k must be in [1, {WIDE_MAX_K}]")
+    if D not in (64, 128):
+        raise ValueError("score_topk_f16_wide: D must be 64 or 128 (use score_topk_f32 otherwise)")
+    dev = Uh.device
+    if out_idx is None:
+        out_idx = torch.empty(B, k, dtype=torch.int32, device=dev)
+    if out_val is None:
+        out_val = torch.empty(B, k, dtype=torch.float32, device=dev)
+    uid = None if user_ids is None else _i64c(user_ids, dev)
+    nbytes = int(call("spex_score_topk_f16_wide_workspace_bytes", int(B_pad), int(k)))
+    work = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=dev)
+    call("spex_score_topk_f16_wide", ptr(Uh), ptr(Ih), int(D), B, B_pad, m_items, m_pad, ptr(u_meta),
+         ptr(i_meta), ptr(uid), ptr(mask_rowptr), ptr(mask_col), int(k), ptr(out_idx), ptr(out_val),
+         ptr(work), nbytes, stream_ptr())
+    return out_idx, out_val
+
+
+def check_k(precision: str, k: int):
+    """ValueError unless `precision` serves top-`k`: f16 up to WIDE_MAX_K, bf16 up to TC_MAX_K, fp32 up to
+    F32_MAX_K; the message names the precision that serves a k beyond the limit."""
+    limit = {"bf16": TC_MAX_K, "fp32": F32_MAX_K}.get(precision, WIDE_MAX_K)
+    if not 1 <= k <= limit:
+        hint = f"; precision 'f16' serves k <= {WIDE_MAX_K}" if precision != "f16" and 1 <= k <= WIDE_MAX_K else ""
+        raise ValueError(f"precision '{precision}' serves 1 <= k <= {limit}, got k = {k}{hint}")
+
+
 class FullRanker:
     """Full-ranking top-k of user rows against one item table, (idx int32 [B, k], score fp32 [B, k]): score
     descending, ties by ascending item id, the items of each user's mask row excluded.
 
-    precision "f16":  tcgen05 fp16-accumulator filter + exact fp32 re-score (score_topk_f16; D 64 or 128);
-    precision "bf16": tcgen05 bf16 operands / fp32 accumulators (score_topk_bf16; D = 64);
-    precision "fp32": exact CUDA-core scorer (score_topk_f32; any D).
+    precision "f16":  tcgen05 fp16-accumulator filter + exact fp32 re-score (D 64 or 128): score_topk_f16 for
+                      k <= TC_MAX_K, score_topk_f16_wide up to WIDE_MAX_K;
+    precision "bf16": tcgen05 bf16 operands / fp32 accumulators (score_topk_bf16; D = 64; k <= TC_MAX_K);
+    precision "fp32": exact CUDA-core scorer (score_topk_f32; any D; k <= F32_MAX_K).
     The item table is packed once, here (the fp32 scorer reads it as it is); the users are packed in topk()."""
 
     def __init__(self, I_all, precision: str = "f16"):
@@ -900,6 +936,7 @@ class FullRanker:
         fp16 subnormal components differently depending on its block-mates); each block is a slice of that
         buffer, `user_block` rounded up to a multiple of 128 rows."""
         dev, m, D = self.device, self.m_items, self.D
+        check_k(self.precision, k)
         users = _i64c(users, dev)
         B = users.numel()
         idx = torch.empty(B, k, dtype=torch.int32, device=dev)
@@ -916,8 +953,9 @@ class FullRanker:
                 # the canonical layout keeps every 8-row group contiguous: rows [s, s + b_pad) are one slice
                 b_pad = (ub.numel() + TC_USER_MULTIPLE - 1) // TC_USER_MULTIPLE * TC_USER_MULTIPLE
                 Uh = Uh_all[s * D: (s + b_pad) * D]
-                score_topk_f16(Uh, umeta, ub.numel(), b_pad, self._Ih, self._imeta, m, self._m_pad, D, k, ub,
-                               mask_rowptr, mask_col, o_i, o_v)
+                f16 = score_topk_f16 if k <= TC_MAX_K else score_topk_f16_wide
+                f16(Uh, umeta, ub.numel(), b_pad, self._Ih, self._imeta, m, self._m_pad, D, k, ub, mask_rowptr,
+                    mask_col, o_i, o_v)
             elif self.precision == "bf16":
                 Ub, b_pad = pack_bf16(U_all, ub, TC_USER_MULTIPLE)
                 score_topk_bf16(Ub, ub.numel(), b_pad, self._Ib, m, self._m_pad, k, ub, mask_rowptr, mask_col,
