@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define SPEX_ABI_VERSION 2
+#define SPEX_ABI_VERSION 3
 
 /* argument errors (negative; positive values are cudaError_t) */
 #define SPEX_E_BADARG   (-1)  /* null pointer / negative size */
@@ -96,11 +96,51 @@ int spex_spmm_csr_f32(const int64_t* rowptr, const int32_t* col, const float* va
                       const spex_long_plan* plan, void* stream);
 
 /*
- * The same layer restricted to a ROW SUBSET: only the listed rows of Y / Z are computed and written, each with
- * exactly the value spex_spmm_csr_f32 would give it (same kernels, same summation order).
- * Replaces nothing literal in the reference - it removes work the reference does: main_rec.py:34 calls
- * computer() (model.py:66-97: all N rows of all K layers) for a mini-batch whose loss (model.py:115-120) reads
- * only the batch's ~1.8 k rows of the result; layer K is needed on those rows only, layer K-1 on their
+ * Epilogue of one propagation layer (spex_spmm_layer_f32): what the warp that finishes output row i does with
+ * acc = (A·X)[i,:].  A HOST struct holding device pointers; the *_host members are host arrays of device
+ * pointers.  Zero-initialise it and set what the layer needs: every feature is off when its fields are NULL / 0.
+ * Tables are fp32 [rows, D], 16-byte aligned (SPEX_E_ALIGN otherwise).
+ */
+typedef struct spex_spmm_epilogue {
+  float* Y;                     /* [n_rows, D]: Y[i,:] = acc (NULL: not written) */
+  const float* addend;          /* [n_rows, D]: addend of Z (NULL: 0) */
+  float addend_scale;
+  float* Z;                     /* [n_rows, D]: Z[i,:] = (addend[i,:] * addend_scale + acc) * z_scale (NULL: none) */
+  float z_scale;
+  int64_t out_row_offset;       /* >= 0: row i goes to row out_row_offset + i of the exchange / publish tables */
+  /* Y exchange (at most one of the two ways): acc is also stored into every GPU's next-layer table, by ONE
+   * multimem.st to the NVSwitch multicast mapping y_mcast (cuMulticast*, e.g. torch symmetric memory's
+   * multicast_ptr; NVLS), or by P2P stores to the n_y_peers (0..8) tables of y_peers_host (own table included). */
+  float* y_mcast;
+  float* const* y_peers_host;
+  int32_t n_y_peers;
+  /* publish: row i of pub_src [n_rows, D] (this rank's slice of the NEXT call's table) is stored into every
+   * GPU's table through exactly one of pub_mcast / the n_pub_peers (0..8) tables of pub_peers_host: the E^(0)
+   * exchange of the next propagation rides on this layer's epilogue.  Not with Adam. */
+  const float* pub_src;
+  float* pub_mcast;
+  float* const* pub_peers_host;
+  int32_t n_pub_peers;
+  /* fused dense Adam (adam_p, adam_m, adam_v all set or all NULL; step >= 1): the Z row is the gradient of row
+   * i of adam_p [n_rows, D]; the warp applies torch.optim.Adam's arithmetic (that of spex_adam_f32) to the rows
+   * of (p, m, v) and, if a publish destination is set, publishes the UPDATED p row.  Z may be NULL. */
+  float* adam_p;
+  float* adam_m;
+  float* adam_v;
+  float lr;
+  float beta1;
+  float beta2;
+  float eps;
+  int32_t step;
+} spex_spmm_epilogue;
+
+/*
+ * One propagation layer with any epilogue, optionally restricted to a ROW SUBSET: only the listed rows are
+ * computed and written, each with exactly the value the full layer gives it (same kernels, same summation
+ * order).  The CSR may be a row block of the full matrix: X is the full [n_cols, D] table, the rows are LOCAL.
+ * The subset replaces nothing literal in the reference - it removes work the reference does: main_rec.py:34
+ * calls computer() (model.py:66-97: all N rows of all K layers) for a mini-batch whose loss (model.py:115-120)
+ * reads only the batch's ~1.8 k rows of the result; layer K is needed on those rows only, layer K-1 on their
  * neighbours, ... (the receptive field), and the backward pass has the mirrored sparsity.
  *   rows        int32 [n_sel]       row ids (no duplicates, any order)
  *   long_slots  int32 [n_long_sel]  for the listed rows of degree > plan->seg_len: their positions in
@@ -111,17 +151,20 @@ int spex_spmm_csr_f32(const int64_t* rowptr, const int32_t* col, const float* va
  *                                   H_1 = g + A^T g, non-zero only on the batch's rows and their neighbours.  Those
  *                                   gathers are skipped; the result is bit-identical to the dense layer (the
  *                                   skipped terms are val * (+0)).  Used with 32-byte aligned tables, else ignored.
- * D in {32, 64, 128}.
+ * Subsets, publish and Adam need D in {32, 64, 128}.  Uses of the row partition (spex_b200/dist.py):
+ *   Y exchange   layers 1..K-1 of a propagation: SpMM and all-gather of the next layer's table in one kernel
+ *   publish      the last layer of a propagation whose next call's E^(0) is already known
+ *   Adam         the last backward layer: main_rec.py:35-37's backward tail, the optimiser and the next
+ *                forward's E^(0) all-gather in one kernel
+ * The descriptor is checked in full (SPEX_E_BADARG / SPEX_E_ALIGN) before anything else, n_sel == 0 included.
  */
-int spex_spmm_csr_rows_f32(const int64_t* rowptr, const int32_t* col, const float* val,
-                           const float* X, int64_t n_rows, int32_t D,
-                           const int32_t* rows, int64_t n_sel,
-                           const int32_t* long_slots, int32_t n_long_sel,
-                           const int32_t* seg_ids, int32_t n_seg_sel,
-                           const uint8_t* x_nonzero,
-                           float* Y, const float* addend, float addend_scale,
-                           float* Z, float z_scale,
-                           const spex_long_plan* plan, void* stream);
+int spex_spmm_layer_f32(const int64_t* rowptr, const int32_t* col, const float* val,
+                        const float* X, int64_t n_rows, int32_t D,
+                        const int32_t* rows, int64_t n_sel,
+                        const int32_t* long_slots, int32_t n_long_sel,
+                        const int32_t* seg_ids, int32_t n_seg_sel,
+                        const uint8_t* x_nonzero,
+                        const spex_spmm_epilogue* ep, const spex_long_plan* plan, void* stream);
 
 /*
  * K-layer propagation + layer mean:  out = (E0 + A·E0 + ... + A^K·E0) / (K+1)
@@ -192,18 +235,14 @@ int spex_bce_fwd_f32(const float* U, const float* I, int32_t D,
 /*
  * Backward of the gather-dot: scatter dgamma[b]*I[items[b]] into gU[users[b]] and
  * dgamma[b]*U[users[b]] into gI[items[b]], times upstream scalar *grad_loss (device fp32[1],
- * NULL = 1).  Duplicate indices are reduced in batch order by a segmented scan — no atomics
- * (replaces index_put_(accumulate=True), K6).  gU/gI must be zero-filled by the caller for rows
- * not touched; touched rows are overwritten.
+ * NULL = 1).  Duplicate indices are reduced in batch order — no atomics (replaces
+ * index_put_(accumulate=True), K6).  gU/gI must be zero-filled by the caller for rows not touched;
+ * touched rows are overwritten.
+ * work NULL: a segmented duplicate scan (O(B^2/32), <= 2^18 entries).  Otherwise (device, 16-byte
+ * aligned, >= spex_scatter_workspace_bytes(max list length) bytes; list length: B for BCE, 2B for
+ * BPR): a stable radix sort of (row, position) pairs + one warp per run, which pays from a few
+ * thousand samples on - same summation order (ascending batch position), bit-identical gradients.
  */
-int spex_bce_bwd_f32(const float* U, const float* I, int32_t D,
-                     const int64_t* users, const int64_t* items, const float* dgamma,
-                     const float* grad_loss, int64_t B, float* gU, float* gI, void* stream);
-/* The same with a workspace: from a few thousand samples on, the duplicate scan (O(B^2/32)) is
- * replaced by a stable radix sort of (row, position) pairs + one warp per run - same summation
- * order (ascending batch position), bit-identical gradients.  work: device, 16-byte aligned,
- * >= spex_scatter_workspace_bytes(max list length) bytes (list length: B for BCE, 2B for BPR);
- * NULL selects the scan (<= 2^18 entries). */
 int64_t spex_scatter_workspace_bytes(int64_t total_entries);
 int spex_bce_bwd_ws_f32(const float* U, const float* I, int32_t D,
                         const int64_t* users, const int64_t* items, const float* dgamma,
@@ -245,13 +284,9 @@ int spex_bpr_fwd_f32(const float* U, const float* I, const float* U0, const floa
  * BPR backward.  grad2 (device fp32[2]) = upstream {dL/dloss, dL/dreg}.
  *   gU[u] += gl*dscore*(n-p); gI[p] += -gl*dscore*u; gI[n] += gl*dscore*u   (propagated tables)
  *   gU0[u] += gr*U0[u]/B; gI0[p] += gr*I0[p]/B; gI0[n] += gr*I0[n]/B        (ego tables)
- * Same deterministic segmented reduction as spex_bce_bwd_f32; touched rows are overwritten,
+ * Same deterministic reduction and workspace as spex_bce_bwd_ws_f32; touched rows are overwritten,
  * untouched rows must have been zero-filled by the caller.
  */
-int spex_bpr_bwd_f32(const float* U, const float* I, const float* U0, const float* I0, int32_t D,
-                     const int64_t* users, const int64_t* pos, const int64_t* neg,
-                     const float* dscore, const float* grad2, int64_t B,
-                     float* gU, float* gI, float* gU0, float* gI0, void* stream);
 int spex_bpr_bwd_ws_f32(const float* U, const float* I, const float* U0, const float* I0, int32_t D,
                         const int64_t* users, const int64_t* pos, const int64_t* neg,
                         const float* dscore, const float* grad2, int64_t B,
@@ -442,81 +477,26 @@ int spex_ngcf_layer_bwd_f32(const float* ego, const float* side, const float* W1
 
 /*
  * CUDA-IPC helpers for the row-partitioned multi-GPU path (SURVEY §8e): each rank allocates its
- * exchange buffer with spex_ipc_alloc, publishes the 64-byte handle, and opens its peers'.
- * spex_spmm_csr_f32_push is spex_spmm_csr_f32 whose Y epilogue also stores every output row
- * into up to 8 peer tables (P2P stores over NVLink): SpMM and all-gather in one kernel.
+ * exchange buffer with spex_ipc_alloc, publishes the 64-byte handle, and opens its peers'.  The layer
+ * kernel stores into the mapped tables through spex_spmm_epilogue's Y exchange and publish.
  */
 int spex_ipc_alloc(int64_t bytes, void** dev_ptr, void* handle64_host);
-/* all-gather of this rank's E^(0) rows by P2P stores: src fp32 [n_rows, D] is stored at rows
- * [out_row_offset, out_row_offset + n_rows) of each of the n_peers (<= 8) tables (own included). */
-int spex_push_rows_f32(const float* src, int64_t n_rows, int32_t D, int64_t out_row_offset,
-                       float* const* peer_Y_host, int32_t n_peers, void* stream);
-/* the same with an explicit grid: n_ctas == 0 is the full-speed grid; a small n_ctas (e.g. the SM
- * count) makes it a BACKGROUND exchange that can run next to a layer kernel on a high-priority
- * stream (spex_b200/dist.py: the next call's E^(0) is published while the last layer runs). */
-int spex_push_rows_f32_ex(const float* src, int64_t n_rows, int32_t D, int64_t out_row_offset,
-                          float* const* peer_Y_host, int32_t n_peers, int32_t n_ctas, void* stream);
 int spex_ipc_open(const void* handle64_host, void** dev_ptr);
 int spex_ipc_close(void* dev_ptr);
 int spex_ipc_free(void* dev_ptr);
-/* NVLS variants: `mcast_Y` is the NVSwitch multicast mapping (cuMulticast*, e.g. torch symmetric
- * memory's multicast_ptr) of the peers' tables; every output row / E^(0) element is stored ONCE with
- * multimem.st and the switch replicates it into all GPUs' copies (own included). */
-int spex_spmm_csr_f32_mcast(const int64_t* rowptr, const int32_t* col, const float* val,
-                            const float* X, int64_t n_rows, int32_t D, int64_t out_row_offset,
-                            float* mcast_Y, const float* addend, float addend_scale, float* Z,
-                            float z_scale, const spex_long_plan* plan, void* stream);
-int spex_mcast_rows_f32(const float* src, int64_t n_rows, int32_t D, int64_t out_row_offset,
-                        float* mcast_Y, void* stream);
+/* all-gather of this rank's E^(0) rows: src fp32 [n_rows, D] is stored at rows
+ * [out_row_offset, out_row_offset + n_rows) of each of the n_peers (<= 8) tables (own included) by P2P
+ * stores, or of every GPU's table by ONE multimem.st per element to the multicast mapping mcast_Y.
+ * n_ctas == 0 is the full-speed grid; a small n_ctas (e.g. the SM count) makes it a BACKGROUND exchange
+ * that can run next to a layer kernel on a high-priority stream (spex_b200/dist.py: the next call's
+ * E^(0) is published while the last layer runs). */
+int spex_push_rows_f32_ex(const float* src, int64_t n_rows, int32_t D, int64_t out_row_offset,
+                          float* const* peer_Y_host, int32_t n_peers, int32_t n_ctas, void* stream);
 int spex_mcast_rows_f32_ex(const float* src, int64_t n_rows, int32_t D, int64_t out_row_offset,
                            float* mcast_Y, int32_t n_ctas, void* stream);
-/* spex_spmm_csr_rows_f32 with the fused exchange of the row-partitioned modes: the listed rows (LOCAL ids of the
- * rank's row block) are computed and their Y rows stored at rows out_row_offset + row of every rank's next-layer
- * table - one multimem.st per row to mcast_Y (NVLS) or P2P stores to the n_peers tables of peer_Y_host (at most
- * one of the two).  Forward of dist.PartitionedTrainer: layers 2..K of computer() (main_rec.py:34) restricted to
- * the mini-batch's receptive field on every rank; n_sel < 0 = all rows, x_nonzero as above (second backward
- * layer).  D in {32, 64, 128}. */
-int spex_spmm_csr_rows_exchange_f32(const int64_t* rowptr, const int32_t* col, const float* val,
-                                    const float* X, int64_t n_rows, int32_t D,
-                                    const int32_t* rows, int64_t n_sel,
-                                    const int32_t* long_slots, int32_t n_long_sel,
-                                    const int32_t* seg_ids, int32_t n_seg_sel,
-                                    const uint8_t* x_nonzero,
-                                    int64_t out_row_offset, float* mcast_Y,
-                                    float* const* peer_Y_host, int32_t n_peers,
-                                    const float* addend, float addend_scale, float* Z, float z_scale,
-                                    const spex_long_plan* plan, void* stream);
-/* Last layer of a row-partitioned propagation with the NEXT call's E^(0) piggy-backed on its epilogue:
- * Z = (addend * addend_scale + A.X) * z_scale (no Y output), and the warp that finishes output row r also
- * copies row r of pub_src (this rank's slice of the next table) to rows out_row_offset + r of every rank's
- * table - one multimem.st to pub_mcast (NVLS), or P2P stores to the n_pub_peers tables of pub_peers_host
- * (exactly one of the two).  The E^(0) exchange then costs what the Y rows of the other layers cost,
- * instead of a kernel of its own (spex_b200/dist.py).  D in {32, 64, 128}. */
-int spex_spmm_csr_f32_publish(const int64_t* rowptr, const int32_t* col, const float* val,
-                              const float* X, int64_t n_rows, int32_t D, int64_t out_row_offset,
-                              const float* addend, float addend_scale, float* Z, float z_scale,
-                              const float* pub_src, float* pub_mcast,
-                              float* const* pub_peers_host, int32_t n_pub_peers,
-                              const spex_long_plan* plan, void* stream);
-/* Last layer of the row-partitioned BACKWARD propagation fused with the optimiser and the next exchange
- * (main_rec.py:35-37 + the E^(0) all-gather of the next step in ONE kernel): the warp that finishes row r of
- * dW = (addend * addend_scale + A.X) * z_scale applies dense Adam to row r of (p, m, v) - the arithmetic of
- * spex_adam_f32 / torch.optim.Adam - and stores the UPDATED parameter row at rows out_row_offset + r of every
- * rank's table (pub_mcast, or the n_pub_peers tables of pub_peers_host; none: no publish).  Z may be NULL. */
-int spex_spmm_csr_f32_adam(const int64_t* rowptr, const int32_t* col, const float* val, const float* X,
-                           int64_t n_rows, int32_t D, int64_t out_row_offset, const float* addend,
-                           float addend_scale, float* Z, float z_scale, float* p, float* m, float* v,
-                           float lr, float beta1, float beta2, float eps, int32_t step,
-                           float* pub_mcast, float* const* pub_peers_host, int32_t n_pub_peers,
-                           const spex_long_plan* plan, void* stream);
 /* cudaMemcpyAsync(DeviceToDevice) on `stream`: a copy-engine transfer into an IPC-mapped peer
  * table (dst may be peer memory), used for the E^(0) all-gather so that no SM is involved. */
 int spex_memcpy_peer_async(void* dst, const void* src, int64_t bytes, void* stream);
-int spex_spmm_csr_f32_push(const int64_t* rowptr, const int32_t* col, const float* val,
-                           const float* X, int64_t n_rows, int32_t D,
-                           int64_t out_row_offset, float* const* peer_Y_host, int32_t n_peers,
-                           const float* addend, float addend_scale, float* Z, float z_scale,
-                           const spex_long_plan* plan, void* stream);
 
 #ifdef __cplusplus
 }

@@ -36,6 +36,19 @@ class LongPlan(C.Structure):
     ]
 
 
+class SpmmEpilogue(C.Structure):
+    """spex_spmm_epilogue (include/spex_b200.h)."""
+
+    _fields_ = [
+        ("Y", _p), ("addend", _p), ("addend_scale", _f), ("Z", _p), ("z_scale", _f),
+        ("out_row_offset", _i64),
+        ("y_mcast", _p), ("y_peers_host", C.POINTER(_p)), ("n_y_peers", _i32),
+        ("pub_src", _p), ("pub_mcast", _p), ("pub_peers_host", C.POINTER(_p)), ("n_pub_peers", _i32),
+        ("adam_p", _p), ("adam_m", _p), ("adam_v", _p),
+        ("lr", _f), ("beta1", _f), ("beta2", _f), ("eps", _f), ("step", _i32),
+    ]
+
+
 _PLAN = C.POINTER(LongPlan)
 
 # name -> (restype, argtypes); mirrors include/spex_b200.h declaration by declaration
@@ -45,16 +58,13 @@ SIGNATURES = {
     "spex_device_check": (C.c_int, [C.POINTER(C.c_int)] * 3),
     "spex_launch_count": (_i64, []),
     "spex_spmm_csr_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _p, _p, _f, _p, _f, _PLAN, _p]),
-    "spex_spmm_csr_rows_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _p, _i64, _p, _i32, _p, _i32, _p, _p, _p, _f, _p, _f,
-                                         _PLAN, _p]),
-    "spex_spmm_csr_rows_exchange_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _p, _i64, _p, _i32, _p, _i32, _p, _i64, _p,
-                                                  _p, _i32, _p, _f, _p, _f, _PLAN, _p]),
+    "spex_spmm_layer_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _p, _i64, _p, _i32, _p, _i32, _p,
+                                      C.POINTER(SpmmEpilogue), _PLAN, _p]),
     "spex_propagate_mean_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _i32, _p, _p, _p, _PLAN, _p]),
     "spex_propagate_mean_bwd_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _i32, _p, _p, _p, _PLAN, _p]),
     "spex_gather_f32": (C.c_int, [_p, _p, _p, _f, _p, _i64, _p]),
     "spex_edge_dropout_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i64, C.c_uint64, _f, _p, _p, _p]),
     "spex_bce_fwd_f32": (C.c_int, [_p, _p, _i32, _p, _p, _p, _i64, _p, _p, _p, _p]),
-    "spex_bce_bwd_f32": (C.c_int, [_p, _p, _i32, _p, _p, _p, _p, _i64, _p, _p, _p]),
     "spex_scatter_workspace_bytes": (_i64, [_i64]),
     "spex_bce_bwd_ws_f32": (C.c_int, [_p, _p, _i32, _p, _p, _p, _p, _i64, _p, _p, _p, _i64, _p]),
     "spex_clear_rows_f32": (C.c_int, [_p, _p, _i64, _i32, _p]),
@@ -62,7 +72,6 @@ SIGNATURES = {
     "spex_scatter_rows_f32": (C.c_int, [_p, _p, _p, _p, _f, _i64, _p, _i32, _p, _i64, _i64, _p, _i64, _p]),
     "spex_bpr_bwd_ws_f32": (C.c_int, [_p, _p, _p, _p, _i32, _p, _p, _p, _p, _p, _i64, _p, _p, _p, _p, _p, _i64, _p]),
     "spex_bpr_fwd_f32": (C.c_int, [_p, _p, _p, _p, _i32, _p, _p, _p, _i64, _p, _p, _p, _p]),
-    "spex_bpr_bwd_f32": (C.c_int, [_p, _p, _p, _p, _i32, _p, _p, _p, _p, _p, _i64, _p, _p, _p, _p, _p]),
     "spex_adam_f32": (C.c_int, [_p, _p, _p, _p, _i64, _f, _f, _f, _f, _i32, _p]),
     "spex_sample_negatives": (C.c_int, [_p, _p, _i32, _i32, _p, _i64, _i32, C.c_uint64, _p, _p]),
     "spex_sample_bpr": (C.c_int, [_p, _p, _i32, _i32, _i64, _i64, C.c_uint64, _p, _p, _p, _p]),
@@ -86,20 +95,9 @@ SIGNATURES = {
     "spex_ipc_open": (C.c_int, [_p, C.POINTER(_p)]),
     "spex_ipc_close": (C.c_int, [_p]),
     "spex_ipc_free": (C.c_int, [_p]),
-    "spex_spmm_csr_f32_mcast": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _i64, _p, _p, _f, _p, _f, _PLAN, _p]),
-    "spex_mcast_rows_f32": (C.c_int, [_p, _i64, _i32, _i64, _p, _p]),
     "spex_mcast_rows_f32_ex": (C.c_int, [_p, _i64, _i32, _i64, _p, _i32, _p]),
     "spex_push_rows_f32_ex": (C.c_int, [_p, _i64, _i32, _i64, C.POINTER(_p), _i32, _i32, _p]),
-    "spex_spmm_csr_f32_publish": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _i64, _p, _f, _p, _f, _p, _p,
-                                            C.POINTER(_p), _i32, _PLAN, _p]),
-    "spex_spmm_csr_f32_adam": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _i64, _p, _f, _p, _f, _p, _p, _p, _f, _f, _f, _f,
-                                         _i32, _p, C.POINTER(_p), _i32, _PLAN, _p]),
     "spex_memcpy_peer_async": (C.c_int, [_p, _p, _i64, _p]),
-    "spex_push_rows_f32": (C.c_int, [_p, _i64, _i32, _i64, C.POINTER(_p), _i32, _p]),
-    "spex_spmm_csr_f32_push": (
-        C.c_int,
-        [_p, _p, _p, _p, _i64, _i32, _i64, C.POINTER(_p), _i32, _p, _f, _p, _f, _PLAN, _p],
-    ),
 }
 
 _NO_STATUS = {"spex_abi_version", "spex_error_string", "spex_launch_count", "spex_scatter_workspace_bytes",

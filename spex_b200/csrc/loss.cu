@@ -642,12 +642,6 @@ extern "C" int spex_bce_bwd_ws_f32(const float* U, const float* I, int32_t D, co
   return launch_scatter(L, U, gI, D, work, work_bytes, st);
 }
 
-extern "C" int spex_bce_bwd_f32(const float* U, const float* I, int32_t D, const int64_t* users,
-                                const int64_t* items, const float* dgamma, const float* grad_loss,
-                                int64_t B, float* gU, float* gI, void* stream) {
-  return spex_bce_bwd_ws_f32(U, I, D, users, items, dgamma, grad_loss, B, gU, gI, nullptr, 0, stream);
-}
-
 extern "C" int spex_bpr_fwd_f32(const float* U, const float* I, const float* U0, const float* I0,
                                 int32_t D, const int64_t* users, const int64_t* pos,
                                 const int64_t* neg, int64_t B, float* out2, float* dscore,
@@ -706,15 +700,6 @@ extern "C" int spex_bpr_bwd_ws_f32(const float* U, const float* I, const float* 
   L.idx[0] = pos; L.src_idx[0] = pos; L.sign[0] = 1.f;
   L.idx[1] = neg; L.src_idx[1] = neg; L.sign[1] = 1.f;
   return launch_scatter(L, I0, gI0, D, work, work_bytes, st);
-}
-
-extern "C" int spex_bpr_bwd_f32(const float* U, const float* I, const float* U0, const float* I0,
-                                int32_t D, const int64_t* users, const int64_t* pos,
-                                const int64_t* neg, const float* dscore, const float* grad2,
-                                int64_t B, float* gU, float* gI, float* gU0, float* gI0,
-                                void* stream) {
-  return spex_bpr_bwd_ws_f32(U, I, U0, I0, D, users, pos, neg, dscore, grad2, B, gU, gI, gU0, gI0, nullptr, 0,
-                             stream);
 }
 
 extern "C" int spex_adam_f32(float* p, const float* g, float* m, float* v, int64_t n, float lr,

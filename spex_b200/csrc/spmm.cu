@@ -485,7 +485,7 @@ spmm_rows_kernel(const int64_t* __restrict__ rowptr, const int32_t* __restrict__
   const int lane = threadIdx.x & 31;
   int64_t row = (int64_t)blockIdx.x * kRowsPerCta + (threadIdx.x >> 5);
   if (row >= n_rows) return;
-  if (row_sel) row = row_sel[row];   // row subset (spex_spmm_csr_rows_f32): n_rows = length of the list
+  if (row_sel) row = row_sel[row];   // row subset (spex_spmm_layer_f32): n_rows = length of the list
   const int64_t start = rowptr[row], end = rowptr[row + 1];
   if (skip_longer_than > 0 && end > start + skip_longer_than) return;  // long-row path
   // sparse-input layers are bound by the per-row latency chain (rowptr -> col/val -> mask -> gathers -> addend):
@@ -695,7 +695,7 @@ spmm_rows_generic_kernel(const int64_t* __restrict__ rowptr, const int32_t* __re
 
 static bool g_rows_only = false;   // spex_debug_spmm_rows: launch the short-row kernel alone
 
-// Row subset of one layer (spex_spmm_csr_rows_f32): only the listed rows are computed.  `rows` lists them all
+// Row subset of one layer (spex_spmm_layer_f32): only the listed rows are computed.  `rows` lists them all
 // (the rows kernel skips the long ones exactly as in a full layer); the listed rows that take the long-row path
 // are given again as slots into plan->long_rows, together with the ids of their segments, so that they run
 // through the SAME segment -> partial -> fix-up sequence as in a full layer: a row's result does not depend on
@@ -958,172 +958,77 @@ extern "C" int spex_spmm_csr_f32(const int64_t* rowptr, const int32_t* col, cons
   return spmm_launch(rowptr, col, val, X, n_rows, D, ep, plan, (cudaStream_t)stream);
 }
 
-// One layer restricted to a row subset (the receptive field of a mini-batch: LightGCN_SPEX/code/main_rec.py:34
-// calls computer() - all N rows of all K layers - for a batch of 256 users; the loss reads ~1.8 k rows of the
-// result, which need E^(K-1) only on their neighbours, and so on).  rows: int32 [n_sel] row ids, any order, no
+// Translates a spex_spmm_epilogue into the kernels' Epilogue: the only check of epilogue arguments.
+static int make_epilogue(const spex_spmm_epilogue* d, Epilogue& ep) {
+  SPEX_RETURN_IF(!d || d->out_row_offset < 0, SPEX_E_BADARG);
+  // Y exchange: at most one of a multicast table and up to 8 peer tables
+  SPEX_RETURN_IF(d->y_mcast && d->n_y_peers > 0, SPEX_E_BADARG);
+  SPEX_RETURN_IF(d->n_y_peers < 0 || d->n_y_peers > 8 || (d->n_y_peers > 0 && !d->y_peers_host), SPEX_E_BADARG);
+  // publish: the rows of pub_src or the rows Adam updates, to exactly one destination
+  const bool adam = d->adam_p || d->adam_m || d->adam_v;
+  const bool pub_dst = d->pub_mcast || d->n_pub_peers > 0;
+  SPEX_RETURN_IF(d->n_pub_peers < 0 || d->n_pub_peers > 8 || (d->n_pub_peers > 0 && !d->pub_peers_host),
+                 SPEX_E_BADARG);
+  SPEX_RETURN_IF(d->pub_mcast && d->n_pub_peers > 0, SPEX_E_BADARG);
+  SPEX_RETURN_IF(d->pub_src && (adam || !pub_dst), SPEX_E_BADARG);
+  SPEX_RETURN_IF(pub_dst && !d->pub_src && !adam, SPEX_E_BADARG);
+  SPEX_RETURN_IF(adam && (!d->adam_p || !d->adam_m || !d->adam_v || d->step < 1), SPEX_E_BADARG);
+  for (int p = 0; p < d->n_y_peers; ++p) SPEX_RETURN_IF(!d->y_peers_host[p], SPEX_E_BADARG);
+  for (int p = 0; p < d->n_pub_peers; ++p) SPEX_RETURN_IF(!d->pub_peers_host[p], SPEX_E_BADARG);
+  SPEX_RETURN_IF(!aligned16(d->Y) || !aligned16(d->addend) || !aligned16(d->Z) || !aligned16(d->y_mcast) ||
+                     !aligned16(d->pub_src) || !aligned16(d->pub_mcast) || !aligned16(d->adam_p) ||
+                     !aligned16(d->adam_m) || !aligned16(d->adam_v),
+                 SPEX_E_ALIGN);
+  for (int p = 0; p < d->n_y_peers; ++p) SPEX_RETURN_IF(!aligned16(d->y_peers_host[p]), SPEX_E_ALIGN);
+  for (int p = 0; p < d->n_pub_peers; ++p) SPEX_RETURN_IF(!aligned16(d->pub_peers_host[p]), SPEX_E_ALIGN);
+  ep.Y = d->Y;
+  ep.addend = d->addend;
+  ep.addend_scale = d->addend_scale;
+  ep.Z = d->Z;
+  ep.z_scale = d->z_scale;
+  ep.peer_row_offset = d->out_row_offset;
+  ep.mcast = d->y_mcast;
+  ep.n_peers = d->n_y_peers;
+  for (int p = 0; p < d->n_y_peers; ++p) ep.peer[p] = d->y_peers_host[p];
+  ep.pub_src = d->pub_src;
+  ep.pub_mcast = d->pub_mcast;
+  ep.n_pub_peers = d->n_pub_peers;
+  for (int p = 0; p < d->n_pub_peers; ++p) ep.pub_peer[p] = d->pub_peers_host[p];
+  if (adam) {
+    ep.adam_p = d->adam_p;
+    ep.adam_m = d->adam_m;
+    ep.adam_v = d->adam_v;
+    const double bc1 = 1.0 - pow((double)d->beta1, (double)d->step);
+    const double bc2 = 1.0 - pow((double)d->beta2, (double)d->step);
+    ep.adam_b1 = d->beta1;
+    ep.adam_b2 = d->beta2;
+    ep.adam_eps = d->eps;
+    ep.adam_step_size = (float)((double)d->lr / bc1);
+    ep.adam_bc2_sqrt = (float)sqrt(bc2);
+  }
+  return 0;
+}
+
+// One layer, optionally restricted to a row subset (the receptive field of a mini-batch: main_rec.py:34 calls
+// computer() - all N rows of all K layers - for a batch of 256 users; the loss reads ~1.8 k rows of the result,
+// which need E^(K-1) only on their neighbours, and so on).  rows: int32 [n_sel] row ids, any order, no
 // duplicates; rows with degree > plan->seg_len are skipped by the rows kernel and must be given again as
 // long_slots (their positions in plan->long_rows) with seg_ids = the ids of all their segments.  Every listed
-// row gets exactly the value a full spex_spmm_csr_f32 would give it; the other rows of Y / Z are not touched.
-extern "C" int spex_spmm_csr_rows_f32(const int64_t* rowptr, const int32_t* col, const float* val,
-                                      const float* X, int64_t n_rows, int32_t D, const int32_t* rows,
-                                      int64_t n_sel, const int32_t* long_slots, int32_t n_long_sel,
-                                      const int32_t* seg_ids, int32_t n_seg_sel, const uint8_t* x_nonzero,
-                                      float* Y, const float* addend, float addend_scale, float* Z, float z_scale,
-                                      const spex_long_plan* plan, void* stream) {
+// row gets exactly the value the full layer would give it; the other rows of the outputs are not touched.
+extern "C" int spex_spmm_layer_f32(const int64_t* rowptr, const int32_t* col, const float* val, const float* X,
+                                   int64_t n_rows, int32_t D, const int32_t* rows, int64_t n_sel,
+                                   const int32_t* long_slots, int32_t n_long_sel, const int32_t* seg_ids,
+                                   int32_t n_seg_sel, const uint8_t* x_nonzero, const spex_spmm_epilogue* epilogue,
+                                   const spex_long_plan* plan, void* stream) {
   SPEX_RETURN_IF(n_long_sel < 0 || n_seg_sel < 0 || (n_sel > 0 && !rows), SPEX_E_BADARG);
   SPEX_RETURN_IF(n_long_sel > 0 && (!long_slots || !seg_ids || !plan || n_seg_sel < n_long_sel), SPEX_E_BADARG);
-  if (n_sel == 0) return 0;
   Epilogue ep{};
-  ep.Y = Y;
-  ep.addend = addend;
-  ep.addend_scale = addend_scale;
-  ep.Z = Z;
-  ep.z_scale = z_scale;
+  const int rc = make_epilogue(epilogue, ep);
+  if (rc) return rc;
+  if (n_sel == 0) return 0;
   RowSubset sub{rows, n_sel, long_slots, n_long_sel, seg_ids, n_seg_sel};
   return spmm_launch(rowptr, col, val, X, n_rows, D, ep, plan, (cudaStream_t)stream, n_sel < 0 ? nullptr : &sub,
                      x_nonzero);
-}
-
-// The row-subset layer with the fused exchange of the row-partitioned modes: the listed rows (LOCAL ids of this
-// rank's row block) are computed as in spex_spmm_csr_rows_f32 and their Y rows stored into every rank's
-// next-layer table - one multimem.st per row to mcast_Y (NVLS), or P2P stores to the n_peers tables of
-// peer_Y_host (at most one of the two; neither: local outputs only) - at rows out_row_offset + row.
-// Forward of dist.PartitionedTrainer: layers 2..K of main_rec.py:34's computer() restricted to the batch's
-// receptive field on every rank.
-extern "C" int spex_spmm_csr_rows_exchange_f32(const int64_t* rowptr, const int32_t* col, const float* val,
-                                               const float* X, int64_t n_rows, int32_t D, const int32_t* rows,
-                                               int64_t n_sel, const int32_t* long_slots, int32_t n_long_sel,
-                                               const int32_t* seg_ids, int32_t n_seg_sel, const uint8_t* x_nonzero,
-                                               int64_t out_row_offset, float* mcast_Y, float* const* peer_Y_host,
-                                               int32_t n_peers, const float* addend, float addend_scale, float* Z,
-                                               float z_scale, const spex_long_plan* plan, void* stream) {
-  SPEX_RETURN_IF(n_long_sel < 0 || n_seg_sel < 0 || (n_sel > 0 && !rows) || out_row_offset < 0, SPEX_E_BADARG);
-  SPEX_RETURN_IF(n_long_sel > 0 && (!long_slots || !seg_ids || !plan || n_seg_sel < n_long_sel), SPEX_E_BADARG);
-  SPEX_RETURN_IF(mcast_Y && n_peers > 0, SPEX_E_BADARG);
-  SPEX_RETURN_IF(n_peers < 0 || n_peers > 8 || (n_peers > 0 && !peer_Y_host), SPEX_E_BADARG);
-  SPEX_RETURN_IF(mcast_Y && !aligned16(mcast_Y), SPEX_E_ALIGN);
-  if (n_sel == 0) return 0;
-  Epilogue ep{};
-  ep.addend = addend;
-  ep.addend_scale = addend_scale;
-  ep.Z = Z;
-  ep.z_scale = z_scale;
-  ep.peer_row_offset = out_row_offset;
-  ep.mcast = mcast_Y;
-  ep.n_peers = mcast_Y ? 0 : n_peers;
-  for (int p = 0; p < ep.n_peers; ++p) {
-    SPEX_RETURN_IF(!peer_Y_host[p] || !aligned16(peer_Y_host[p]), SPEX_E_BADARG);
-    ep.peer[p] = peer_Y_host[p];
-  }
-  RowSubset sub{rows, n_sel, long_slots, n_long_sel, seg_ids, n_seg_sel};
-  return spmm_launch(rowptr, col, val, X, n_rows, D, ep, plan, (cudaStream_t)stream, n_sel < 0 ? nullptr : &sub,
-                     x_nonzero);
-}
-
-extern "C" int spex_spmm_csr_f32_push(const int64_t* rowptr, const int32_t* col, const float* val,
-                                      const float* X, int64_t n_rows, int32_t D,
-                                      int64_t out_row_offset, float* const* peer_Y_host,
-                                      int32_t n_peers, const float* addend, float addend_scale,
-                                      float* Z, float z_scale, const spex_long_plan* plan,
-                                      void* stream) {
-  SPEX_RETURN_IF(n_peers < 0 || n_peers > 8 || (n_peers > 0 && !peer_Y_host), SPEX_E_BADARG);
-  Epilogue ep{};
-  ep.Y = nullptr;
-  ep.addend = addend;
-  ep.addend_scale = addend_scale;
-  ep.Z = Z;
-  ep.z_scale = z_scale;
-  ep.n_peers = n_peers;
-  ep.peer_row_offset = out_row_offset;
-  for (int p = 0; p < n_peers; ++p) {
-    SPEX_RETURN_IF(!peer_Y_host[p] || !aligned16(peer_Y_host[p]), SPEX_E_BADARG);
-    ep.peer[p] = peer_Y_host[p];
-  }
-  return spmm_launch(rowptr, col, val, X, n_rows, D, ep, plan, (cudaStream_t)stream);
-}
-
-extern "C" int spex_spmm_csr_f32_mcast(const int64_t* rowptr, const int32_t* col, const float* val,
-                                       const float* X, int64_t n_rows, int32_t D,
-                                       int64_t out_row_offset, float* mcast_Y, const float* addend,
-                                       float addend_scale, float* Z, float z_scale,
-                                       const spex_long_plan* plan, void* stream) {
-  SPEX_RETURN_IF(!mcast_Y || !aligned16(mcast_Y) || out_row_offset < 0, SPEX_E_BADARG);
-  Epilogue ep{};
-  ep.addend = addend;
-  ep.addend_scale = addend_scale;
-  ep.Z = Z;
-  ep.z_scale = z_scale;
-  ep.peer_row_offset = out_row_offset;
-  ep.mcast = mcast_Y;
-  return spmm_launch(rowptr, col, val, X, n_rows, D, ep, plan, (cudaStream_t)stream);
-}
-
-// Last layer of a row-partitioned propagation with the NEXT call's E^(0) piggy-backed on its epilogue
-// (see Epilogue::pub_src): Z = (addend * addend_scale + A.X) * z_scale as usual, no Y output, and row r of
-// pub_src goes to rows out_row_offset + r of every rank's table through pub_mcast (NVLS) or pub_peers.
-extern "C" int spex_spmm_csr_f32_publish(const int64_t* rowptr, const int32_t* col, const float* val,
-                                         const float* X, int64_t n_rows, int32_t D, int64_t out_row_offset,
-                                         const float* addend, float addend_scale, float* Z, float z_scale,
-                                         const float* pub_src, float* pub_mcast,
-                                         float* const* pub_peers_host, int32_t n_pub_peers,
-                                         const spex_long_plan* plan, void* stream) {
-  SPEX_RETURN_IF(!pub_src || !aligned16(pub_src) || out_row_offset < 0, SPEX_E_BADARG);
-  SPEX_RETURN_IF((pub_mcast == nullptr) == (n_pub_peers <= 0), SPEX_E_BADARG);   // exactly one of the two ways
-  SPEX_RETURN_IF(pub_mcast && !aligned16(pub_mcast), SPEX_E_ALIGN);
-  SPEX_RETURN_IF(n_pub_peers < 0 || n_pub_peers > 8 || (n_pub_peers > 0 && !pub_peers_host), SPEX_E_BADARG);
-  Epilogue ep{};
-  ep.addend = addend;
-  ep.addend_scale = addend_scale;
-  ep.Z = Z;
-  ep.z_scale = z_scale;
-  ep.peer_row_offset = out_row_offset;
-  ep.pub_src = pub_src;
-  ep.pub_mcast = pub_mcast;
-  ep.n_pub_peers = pub_mcast ? 0 : n_pub_peers;
-  for (int p = 0; p < ep.n_pub_peers; ++p) {
-    SPEX_RETURN_IF(!pub_peers_host[p] || !aligned16(pub_peers_host[p]), SPEX_E_BADARG);
-    ep.pub_peer[p] = pub_peers_host[p];
-  }
-  return spmm_launch(rowptr, col, val, X, n_rows, D, ep, plan, (cudaStream_t)stream);
-}
-
-// Last layer of the row-partitioned BACKWARD propagation fused with the optimiser and the next exchange:
-// the warp that finishes row r of  dW = (addend * addend_scale + A.X) * z_scale  applies dense Adam to row r of
-// (p, m, v) (spex_adam_f32 arithmetic) and stores the updated parameter row into every rank's table (NVLS
-// multicast or P2P peers; both NULL/0: no publish).  dW itself is written only if Z != NULL.
-extern "C" int spex_spmm_csr_f32_adam(const int64_t* rowptr, const int32_t* col, const float* val, const float* X,
-                                      int64_t n_rows, int32_t D, int64_t out_row_offset, const float* addend,
-                                      float addend_scale, float* Z, float z_scale, float* p, float* m, float* v,
-                                      float lr, float beta1, float beta2, float eps, int32_t step,
-                                      float* pub_mcast, float* const* pub_peers_host, int32_t n_pub_peers,
-                                      const spex_long_plan* plan, void* stream) {
-  SPEX_RETURN_IF(!p || !m || !v || step < 1 || out_row_offset < 0, SPEX_E_BADARG);
-  SPEX_RETURN_IF(!aligned16(p) || !aligned16(m) || !aligned16(v) || (pub_mcast && !aligned16(pub_mcast)), SPEX_E_ALIGN);
-  SPEX_RETURN_IF(pub_mcast && n_pub_peers > 0, SPEX_E_BADARG);
-  SPEX_RETURN_IF(n_pub_peers < 0 || n_pub_peers > 8 || (n_pub_peers > 0 && !pub_peers_host), SPEX_E_BADARG);
-  Epilogue ep{};
-  ep.addend = addend;
-  ep.addend_scale = addend_scale;
-  ep.Z = Z;
-  ep.z_scale = z_scale;
-  ep.peer_row_offset = out_row_offset;
-  ep.pub_mcast = pub_mcast;
-  ep.n_pub_peers = pub_mcast ? 0 : n_pub_peers;
-  for (int q = 0; q < ep.n_pub_peers; ++q) {
-    SPEX_RETURN_IF(!pub_peers_host[q] || !aligned16(pub_peers_host[q]), SPEX_E_BADARG);
-    ep.pub_peer[q] = pub_peers_host[q];
-  }
-  ep.adam_p = p;
-  ep.adam_m = m;
-  ep.adam_v = v;
-  const double bc1 = 1.0 - pow((double)beta1, (double)step);
-  const double bc2 = 1.0 - pow((double)beta2, (double)step);
-  ep.adam_b1 = beta1;
-  ep.adam_b2 = beta2;
-  ep.adam_eps = eps;
-  ep.adam_step_size = (float)((double)lr / bc1);
-  ep.adam_bc2_sqrt = (float)sqrt(bc2);
-  return spmm_launch(rowptr, col, val, X, n_rows, D, ep, plan, (cudaStream_t)stream);
 }
 
 // n_ctas == 0: the full-speed grid (8 CTAs per SM); > 0: a small grid for a BACKGROUND exchange that
@@ -1140,11 +1045,6 @@ extern "C" int spex_mcast_rows_f32_ex(const float* src, int64_t n_rows, int32_t 
                                                             mcast_Y + out_row_offset * D);
   count_launch();
   return check_last();
-}
-
-extern "C" int spex_mcast_rows_f32(const float* src, int64_t n_rows, int32_t D, int64_t out_row_offset,
-                                   float* mcast_Y, void* stream) {
-  return spex_mcast_rows_f32_ex(src, n_rows, D, out_row_offset, mcast_Y, 0, stream);
 }
 
 extern "C" int spex_push_rows_f32_ex(const float* src, int64_t n_rows, int32_t D, int64_t out_row_offset,
@@ -1166,11 +1066,6 @@ extern "C" int spex_push_rows_f32_ex(const float* src, int64_t n_rows, int32_t D
   push_rows_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>((const float4*)src, n4, out_row_offset * D / 4, pt);
   count_launch();
   return check_last();
-}
-
-extern "C" int spex_push_rows_f32(const float* src, int64_t n_rows, int32_t D, int64_t out_row_offset,
-                                  float* const* peer_Y_host, int32_t n_peers, void* stream) {
-  return spex_push_rows_f32_ex(src, n_rows, D, out_row_offset, peer_Y_host, n_peers, 0, stream);
 }
 
 extern "C" int spex_propagate_mean_f32(const int64_t* rowptr, const int32_t* col, const float* val,

@@ -12,21 +12,22 @@ is that partition with one process per GPU: rank p owns the contiguous node rang
 Three exchange modes:
   "nccl"  one all-gather of the [rows_p, D] slices per layer (torch.distributed over NCCL/NVLink);
   "push"  the SpMM epilogue itself stores every output row into all peers' next-layer tables with
-          P2P stores over NVLink (spex_spmm_csr_f32_push): transfer overlaps the gather-bound
-          math row by row; layers are separated by a stream-ordered 4-byte all-reduce (barrier).
+          P2P stores over NVLink (the Y exchange of spex_spmm_layer_f32's epilogue): transfer overlaps
+          the gather-bound math row by row; layers are separated by a stream-ordered 4-byte all-reduce
+          (barrier).
           E^(0) has no producing kernel to fuse with and travels by NCCL all-gather (measured
           faster than P2P stores or copy engines, which stay selectable: e0_exchange).
 
   "mcast" the same fusion with ONE store per row to an NVSwitch multicast mapping of the tables
           (NVLS; torch symmetric memory provides the mapping): a row leaves the GPU once instead of
-          P-1 times, which removes the NVLink egress bound of "push" (spex_spmm_csr_f32_mcast,
-          spex_mcast_rows_f32 for E^(0)).
+          P-1 times, which removes the NVLink egress bound of "push" (the epilogue's y_mcast,
+          spex_mcast_rows_f32_ex for E^(0)).
 
 In the two fused modes the tables are a ring of THREE buffers: E^(0) of a call lives in slot a, layer k
 reads slot a+k and writes slot a+k+1 (mod 3), the next call's E^(0) goes to slot a+K.  That slot is idle
 while the LAST layer runs (which stores nothing over NVLink), so `propagate(E0, next_E0_local=...)`
 publishes the next call's table DURING the last layer - from that layer's own epilogue (the warp that
-finishes output row r also multicasts row r of the next table: spex_spmm_csr_f32_publish), or from a
+finishes output row r also multicasts row r of the next table: the epilogue's publish), or from a
 small high-priority side-stream kernel (fuse_publish = False): the E^(0) exchange (5.4 ms + 2.5 ms of
 skew at 8 GPUs in round 1, un-overlapped) disappears from the critical path, and the ring makes the "everybody is done reading the buffer" barrier of round 1
 unnecessary (every slot's previous readers are separated from its next writer by a barrier that
@@ -197,22 +198,11 @@ class PartitionedPropagator:
 
     # ---- one layer --------------------------------------------------------------------------------
     def _layer(self, X_full, Y_local, addend, Z_local, z_scale, push_buf=None, publish=None, subset=None,
-               x_nonzero=None):
-        if subset is not None or x_nonzero is not None:
-            # restricted to a row list (receptive field of a mini-batch) and / or reading a table that is zero
-            # outside the rows x_nonzero marks; same fused exchange
-            from ._capi import call, ptr, stream_ptr
-
-            rows, slots, segs = subset if subset is not None else (None, None, None)
-            mc = C.c_void_p(self._mc[push_buf]) if (push_buf is not None and self.mode == "mcast") else None
-            peers = self._peer_ptrs[push_buf] if (push_buf is not None and self.mode == "push") else None
-            call("spex_spmm_csr_rows_exchange_f32", ptr(self.g.rowptr), ptr(self.g.col), ptr(self.g.val), ptr(X_full),
-                 self.g.n_rows, self.D, ptr(rows), -1 if rows is None else rows.numel(), ptr(slots),
-                 0 if slots is None else slots.numel(), ptr(segs), 0 if segs is None else segs.numel(),
-                 ptr(x_nonzero), self.r0, mc, peers,
-                 self.world if peers is not None else 0, ptr(addend), 1.0, ptr(Z_local), float(z_scale),
-                 self.g.plan(self.D), stream_ptr())
-            return
+               x_nonzero=None, adam=None):
+        """One layer over the local rows (ops.spmm_rows), restricted to `subset` / reading a table that is zero
+        outside the rows `x_nonzero` marks.  Fused modes: `push_buf` = ring slot into which the Y rows go on every
+        rank; `publish` = (src, slot): the rows of src - or, with `adam` ({p, m, v, lr, beta1, beta2, eps, step},
+        src None), the rows of p updated with the Z rows as gradient - go to ring slot `slot` on every rank."""
         if self.local_spmm is not None:
             acc = self.local_spmm(self.g, X_full)
             if Y_local is not None:
@@ -220,41 +210,18 @@ class PartitionedPropagator:
             Z_local.copy_((addend + acc) * z_scale)
             return
         from . import ops
-        from ._capi import call, ptr, stream_ptr
 
-        if publish is not None:   # last layer + the next call's E^(0) on its epilogue
-            src, slot = publish
-            mc = C.c_void_p(self._mc[slot]) if self.mode == "mcast" else None
-            peers = None if self.mode == "mcast" else self._peer_ptrs[slot]
-            call("spex_spmm_csr_f32_publish", ptr(self.g.rowptr), ptr(self.g.col), ptr(self.g.val), ptr(X_full),
-                 self.g.n_rows, self.D, self.r0, ptr(addend), 1.0, ptr(Z_local), float(z_scale), ptr(src), mc,
-                 peers, 0 if self.mode == "mcast" else self.world, self.g.plan(self.D), stream_ptr())
-            return
-        if push_buf is None:
-            ops.spmm(self.g, X_full, Y=Y_local, addend=addend, addend_scale=1.0, Z=Z_local, z_scale=z_scale)
-            return
-        if self.mode == "mcast":   # fused SpMM + all-gather, one multicast store per row
-            call("spex_spmm_csr_f32_mcast", ptr(self.g.rowptr), ptr(self.g.col), ptr(self.g.val), ptr(X_full),
-                 self.g.n_rows, self.D, self.r0, C.c_void_p(self._mc[push_buf]),
-                 ptr(addend), 1.0, ptr(Z_local), float(z_scale), self.g.plan(self.D), stream_ptr())
-            return
-        # fused SpMM + all-gather: rows go to every peer's (and our own) next-layer table
-        call("spex_spmm_csr_f32_push", ptr(self.g.rowptr), ptr(self.g.col), ptr(self.g.val), ptr(X_full),
-             self.g.n_rows, self.D, self.r0, self._peer_ptrs[push_buf], self.world,
-             ptr(addend), 1.0, ptr(Z_local), float(z_scale), self.g.plan(self.D), stream_ptr())
+        def dest(slot):   # how an epilogue reaches ring slot `slot` of every rank: (multicast address, peers)
+            if slot is None:
+                return None, None
+            return (self._mc[slot], None) if self.mode == "mcast" else (None, self._peer_ptrs[slot])
 
-    def _layer_adam(self, X_full, addend, z_scale, adam, slot):
-        """Last layer of the backward propagation + dense Adam on the owned rows + publish of the updated
-        rows into ring slot `slot` of every rank (spex_spmm_csr_f32_adam)."""
-        from ._capi import call, ptr, stream_ptr
-
-        mc = C.c_void_p(self._mc[slot]) if self.mode == "mcast" else None
-        peers = None if self.mode == "mcast" else self._peer_ptrs[slot]
-        call("spex_spmm_csr_f32_adam", ptr(self.g.rowptr), ptr(self.g.col), ptr(self.g.val), ptr(X_full),
-             self.g.n_rows, self.D, self.r0, ptr(addend), 1.0, None, float(z_scale), ptr(adam["p"]), ptr(adam["m"]),
-             ptr(adam["v"]), float(adam["lr"]), float(adam["beta1"]), float(adam["beta2"]), float(adam["eps"]),
-             int(adam["step"]), mc, peers, 0 if self.mode == "mcast" else self.world, self.g.plan(self.D),
-             stream_ptr())
+        y_mcast, y_peers = dest(push_buf)
+        pub_src, pub_slot = publish if publish is not None else (None, None)
+        pub_mcast, pub_peers = dest(pub_slot)
+        ops.spmm_rows(self.g, X_full, subset, Y=Y_local, addend=addend, Z=Z_local, z_scale=float(z_scale),
+                      x_nonzero=x_nonzero, out_row_offset=self.r0, y_mcast=y_mcast, y_peers=y_peers,
+                      pub_src=pub_src, pub_mcast=pub_mcast, pub_peers=pub_peers, adam=adam)
 
     def _mark(self, name):
         if self.timing is not None:
@@ -396,7 +363,7 @@ class PartitionedPropagator:
         training step: zero but for the batch's rows, which every rank can compute).
         `adam` (fused modes): {p, m, v, lr, beta1, beta2, eps, step} - the result is not returned but consumed
         as the gradient of `p` by a dense Adam fused into the last layer's epilogue, and the updated rows of
-        `p` are published as the next call's table (spex_spmm_csr_f32_adam).
+        `p` are published as the next call's table (the fused Adam of spex_spmm_layer_f32's epilogue).
         `row_sets` (fused modes; from receptive_sets(S)): layer k computes - and exchanges - only the rows
         row_sets[k] (None = all); only the rows S = row_sets[K] of the result are then valid.
         `x_masks` (fused modes): x_masks[k] = uint8 [N] marking the rows of layer k's INPUT table that may be
@@ -435,7 +402,7 @@ class PartitionedPropagator:
             if last and adam is not None:
                 if not fused:
                     raise ValueError("the fused Adam epilogue needs a fused exchange mode")
-                self._layer_adam(X_full, addend, inv, adam, (a + K) % nt)
+                self._layer(X_full, None, addend, None, inv, publish=(None, (a + K) % nt), adam=adam)
                 self._mark(f"layer{k + 1}")
                 done = torch.cuda.Event()
                 done.record()
@@ -445,7 +412,7 @@ class PartitionedPropagator:
             publish = None
             if last and next_E0_local is not None and self.can_prefetch():
                 if fused and self.fuse_publish and self.D in (32, 64, 128) and next_E0_local.is_contiguous():
-                    # the next table rides on this layer's epilogue (spex_spmm_csr_f32_publish)
+                    # the next table rides on this layer's epilogue (its publish)
                     if next_ready is not None:
                         torch.cuda.current_stream().wait_event(next_ready)
                     publish = (next_E0_local, (a + K) % nt)
@@ -526,9 +493,9 @@ class PartitionedPropagator:
 #   optimiser row-owned dense Adam (spex_adam_f32 on the local slice): no collective.
 # With a fused exchange (push / mcast) the tail of the step is ONE kernel per rank: the last backward layer
 # applies Adam to each owned row in its epilogue and stores the updated row into every rank's table
-# (spex_spmm_csr_f32_adam), so the next forward starts without an E^(0) exchange; and the first backward
-# layer reads a gradient table every rank assembles locally (all batch rows are known everywhere): of the
-# four exchanges of round-partitioned step only the per-layer ones remain.
+# (the fused Adam of spex_spmm_layer_f32), so the next forward starts without an E^(0) exchange; and the first
+# backward layer reads a gradient table every rank assembles locally (all batch rows are known everywhere): of
+# the four exchanges of round-partitioned step only the per-layer ones remain.
 # ---------------------------------------------------------------------------------------------------
 class _CudaTrainOps:
     """The CUDA entry points behind PartitionedTrainer (no fallback: CPU tensors are rejected)."""

@@ -22,7 +22,7 @@ import numpy as np
 import torch
 
 from . import _capi
-from ._capi import LongPlan, call, ptr, stream_ptr
+from ._capi import LongPlan, SpmmEpilogue, call, ptr, stream_ptr
 from .graph import CSRGraph, DEFAULT_SEG_LEN
 
 
@@ -340,7 +340,7 @@ class DeviceGraph:
         return torch.unique(c.to(torch.int64))
 
     def row_subset(self, rows: torch.Tensor):
-        """(rows int32, long_slots int32 | None, seg_ids int32 | None) for spex_spmm_csr_rows_f32: the listed
+        """(rows int32, long_slots int32 | None, seg_ids int32 | None) for spex_spmm_layer_f32: the listed
         rows, and - for those on the long-row path - their slots in the plan with all their segments."""
         rows = rows.to(torch.int64)
         r32 = rows.to(torch.int32).contiguous()
@@ -432,26 +432,39 @@ def nonzero_mask(n: int, rows: torch.Tensor) -> torch.Tensor:
 def spmm_rows(g: DeviceGraph, X: torch.Tensor, subset, Y: Optional[torch.Tensor] = None,
               addend: Optional[torch.Tensor] = None, addend_scale: float = 1.0,
               Z: Optional[torch.Tensor] = None, z_scale: float = 1.0, val: Optional[torch.Tensor] = None,
-              x_nonzero: Optional[torch.Tensor] = None):
+              x_nonzero: Optional[torch.Tensor] = None, out_row_offset: int = 0, y_mcast: Optional[int] = None,
+              y_peers=None, pub_src: Optional[torch.Tensor] = None, pub_mcast: Optional[int] = None,
+              pub_peers=None, adam: Optional[dict] = None):
     """spmm() restricted to the rows of `subset` (= g.row_subset(rows); None = all rows): the listed rows of
     Y / Z get exactly the values a full layer gives them, the other rows are left untouched.  `x_nonzero`
     (uint8 [n_cols]): X is exactly zero on the rows it marks 0 - those gathers are skipped, the result is
-    bit-identical."""
+    bit-identical.  The other arguments are the exchange epilogues of a row partition (spex_spmm_epilogue, whose
+    rows out_row_offset + i they write): the Y rows to every rank's table through the multicast address `y_mcast`
+    or the ctypes array of peer tables `y_peers`; the rows of `pub_src` (or, with `adam`, the updated rows of
+    adam["p"]) likewise through `pub_mcast` / `pub_peers`; `adam` = {p, m, v, lr, beta1, beta2, eps, step}: dense
+    Adam on the rows of p with the Z row as gradient."""
     _need_cuda(X)
     X = _f32c(X)
     D = X.shape[1]
     if X.shape[0] != g.n_cols:
         raise ValueError(f"X has {X.shape[0]} rows, graph has {g.n_cols} columns")
-    if Y is None and Z is None:
-        raise ValueError("spmm_rows writes into caller-provided Y and/or Z")
+    if Y is None and Z is None and adam is None:
+        raise ValueError("spmm_rows writes into caller-provided Y, Z or Adam state")
     rows, slots, segs = subset if subset is not None else (None, None, None)
     v = g.val if val is None else val
     if x_nonzero is not None and (x_nonzero.dtype != torch.uint8 or x_nonzero.numel() != g.n_cols):
         raise ValueError("x_nonzero must be uint8 [n_cols]")
-    call("spex_spmm_csr_rows_f32", ptr(g.rowptr), ptr(g.col), ptr(v), ptr(X), g.n_rows, D, ptr(rows),
+    ep = SpmmEpilogue(Y=ptr(Y), addend=ptr(addend), addend_scale=addend_scale, Z=ptr(Z), z_scale=z_scale,
+                      out_row_offset=out_row_offset, y_mcast=y_mcast, y_peers_host=y_peers,
+                      n_y_peers=0 if y_peers is None else len(y_peers), pub_src=ptr(pub_src), pub_mcast=pub_mcast,
+                      pub_peers_host=pub_peers, n_pub_peers=0 if pub_peers is None else len(pub_peers))
+    if adam is not None:
+        ep.adam_p, ep.adam_m, ep.adam_v = ptr(adam["p"]), ptr(adam["m"]), ptr(adam["v"])
+        ep.lr, ep.beta1, ep.beta2, ep.eps, ep.step = (adam["lr"], adam["beta1"], adam["beta2"], adam["eps"],
+                                                     adam["step"])
+    call("spex_spmm_layer_f32", ptr(g.rowptr), ptr(g.col), ptr(v), ptr(X), g.n_rows, D, ptr(rows),
          -1 if rows is None else rows.numel(), ptr(slots), 0 if slots is None else slots.numel(), ptr(segs),
-         0 if segs is None else segs.numel(), ptr(x_nonzero), ptr(Y), ptr(addend), float(addend_scale), ptr(Z),
-         float(z_scale), g.plan(D), stream_ptr())
+         0 if segs is None else segs.numel(), ptr(x_nonzero), C.byref(ep), g.plan(D), stream_ptr())
 
 
 # A layer's input is treated as sparse (x_nonzero mask, gathers of zero rows skipped) while the rows that may be

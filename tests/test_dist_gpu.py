@@ -1,6 +1,6 @@
 """Row-partitioned propagation on real GPUs (needs >= 2 devices, skipped otherwise): the NCCL
-all-gather exchange and the fused SpMM + P2P push exchange (spex_spmm_csr_f32_push,
-spex_push_rows_f32) against the single-GPU kernel on the same graph.  Same row partition as the
+all-gather exchange and the fused SpMM + P2P push exchange (the Y exchange of spex_spmm_layer_f32's
+epilogue, spex_push_rows_f32_ex) against the single-GPU kernel on the same graph.  Same row partition as the
 reference's serial folds (/root/reference/LightGCN_SPEX/code/utility1/dataloader.py:167-177)."""
 import os
 import socket

@@ -203,7 +203,7 @@ def test_negative_sampler_consumes_the_reference_stream():
     assert not ps.contains(users[len(feats):], items[len(feats):]).any()
 
 
-def test_capi_exports_every_declared_symbol_at_abi_2():
+def test_capi_exports_every_declared_symbol_at_abi_3():
     hdr = open(os.path.join(ROOT, "include", "spex_b200.h")).read()
     hdr = re.sub(r"/\*.*?\*/", "", hdr, flags=re.S)
     declared = set(re.findall(r"\b(spex_[a-z0-9_]+)\s*\(", hdr))
@@ -214,7 +214,7 @@ def test_capi_exports_every_declared_symbol_at_abi_2():
     from spex_b200 import _capi
 
     assert declared == set(_capi.SIGNATURES), declared ^ set(_capi.SIGNATURES)
-    assert _capi.abi_version() == 2
+    assert _capi.abi_version() == 3
     assert "SPEX_E_ALIGN" in _capi.error_string(-3)
 
 
@@ -249,6 +249,73 @@ def test_ctypes_signatures_match_the_header_prototypes():
     for name, (_res, argtypes) in _capi.SIGNATURES.items():
         params = [p for p in protos[name].split(",") if p.strip() and p.strip() != "void"]
         assert [kind_c(p) for p in params] == [kind_py(t) for t in argtypes], name
+
+
+# spex_spmm_epilogue rules.  The addresses are never dereferenced: with n_rows = 0 the library returns after its
+# argument checks, so these run without a GPU.
+_A, _B = 0x10000, 0x20000          # 16-byte aligned
+_MIS = _A + 4                      # misaligned
+
+
+def _peers(*p):
+    return (ctypes.c_void_p * len(p))(*p)
+
+
+_ADAM = dict(adam_p=_A, adam_m=_B, adam_v=_A + 0x100, lr=1e-3, beta1=0.9, beta2=0.999, eps=1e-8, step=1)
+_BADARG, _ALIGN = -1, -3
+_EPILOGUE_CASES = [
+    # one valid descriptor of each epilogue kind
+    ("plain", dict(Y=_A, addend=_B, addend_scale=1.0, Z=_B, z_scale=0.5), 0),
+    ("y_peers", dict(Z=_B, out_row_offset=7, y_peers_host=_peers(_A, _B), n_y_peers=2), 0),
+    ("y_mcast", dict(Z=_B, out_row_offset=7, y_mcast=_A), 0),
+    ("publish_peers", dict(Z=_B, pub_src=_A, pub_peers_host=_peers(_A, _B), n_pub_peers=2), 0),
+    ("publish_mcast", dict(Z=_B, pub_src=_A, pub_mcast=_B), 0),
+    ("adam", dict(_ADAM), 0),
+    ("adam_publish_peers", dict(_ADAM, pub_peers_host=_peers(_A), n_pub_peers=1), 0),
+    ("adam_publish_mcast", dict(_ADAM, Z=_B, pub_mcast=_B), 0),
+    # one violating descriptor per rule
+    ("negative_out_row_offset", dict(Z=_B, y_mcast=_A, out_row_offset=-1), _BADARG),
+    ("y_mcast_and_peers", dict(Z=_B, y_mcast=_A, y_peers_host=_peers(_A), n_y_peers=1), _BADARG),
+    ("y_peers_negative", dict(Z=_B, y_peers_host=_peers(_A), n_y_peers=-1), _BADARG),
+    ("y_peers_over_8", dict(Z=_B, y_peers_host=_peers(*[_A] * 9), n_y_peers=9), _BADARG),
+    ("y_peers_null_array", dict(Z=_B, n_y_peers=1), _BADARG),
+    ("y_peers_null_peer", dict(Z=_B, y_peers_host=_peers(_A, None), n_y_peers=2), _BADARG),
+    ("pub_peers_over_8", dict(Z=_B, pub_src=_A, pub_peers_host=_peers(*[_A] * 9), n_pub_peers=9), _BADARG),
+    ("pub_peers_null_peer", dict(Z=_B, pub_src=_A, pub_peers_host=_peers(None), n_pub_peers=1), _BADARG),
+    ("pub_src_without_destination", dict(Z=_B, pub_src=_A), _BADARG),
+    ("pub_src_with_two_destinations", dict(Z=_B, pub_src=_A, pub_mcast=_B, pub_peers_host=_peers(_A),
+                                           n_pub_peers=1), _BADARG),
+    ("pub_mcast_without_source", dict(Z=_B, pub_mcast=_B), _BADARG),
+    ("pub_peers_without_source", dict(Z=_B, pub_peers_host=_peers(_A), n_pub_peers=1), _BADARG),
+    ("pub_src_with_adam", dict(_ADAM, pub_src=_A, pub_mcast=_B), _BADARG),
+    ("adam_partial", dict(_ADAM, adam_v=None), _BADARG),
+    ("adam_step_0", dict(_ADAM, step=0), _BADARG),
+    ("misaligned_Y", dict(Y=_MIS), _ALIGN),
+    ("misaligned_addend", dict(Z=_B, addend=_MIS), _ALIGN),
+    ("misaligned_Z", dict(Z=_MIS), _ALIGN),
+    ("misaligned_y_mcast", dict(Z=_B, y_mcast=_MIS), _ALIGN),
+    ("misaligned_y_peer", dict(Z=_B, y_peers_host=_peers(_A, _MIS), n_y_peers=2), _ALIGN),
+    ("misaligned_pub_src", dict(Z=_B, pub_src=_MIS, pub_mcast=_B), _ALIGN),
+    ("misaligned_pub_mcast", dict(Z=_B, pub_src=_A, pub_mcast=_MIS), _ALIGN),
+    ("misaligned_pub_peer", dict(Z=_B, pub_src=_A, pub_peers_host=_peers(_MIS), n_pub_peers=1), _ALIGN),
+    ("misaligned_adam_p", dict(_ADAM, adam_p=_MIS), _ALIGN),
+    ("misaligned_adam_m", dict(_ADAM, adam_m=_MIS), _ALIGN),
+    ("misaligned_adam_v", dict(_ADAM, adam_v=_MIS), _ALIGN),
+]
+
+
+@pytest.mark.parametrize("fields,expected", [c[1:] for c in _EPILOGUE_CASES], ids=[c[0] for c in _EPILOGUE_CASES])
+@pytest.mark.parametrize("n_sel", [-1, 0], ids=["all_rows", "empty_subset"])
+def test_spmm_layer_validates_the_epilogue_descriptor(fields, expected, n_sel):
+    """spex_spmm_layer_f32 checks every spex_spmm_epilogue rule before anything else, also for an empty row list."""
+    from spex_b200 import _capi
+
+    ep = _capi.SpmmEpilogue(**fields)
+    rc = _capi.lib.spex_spmm_layer_f32(_A, _A, _A, _A, 0, 64, _A if n_sel == 0 else None, n_sel, None, 0, None, 0,
+                                       None, ctypes.byref(ep), None, None)
+    assert rc == expected, _capi.error_string(rc)
+    assert _capi.lib.spex_spmm_layer_f32(_A, _A, _A, _A, 0, 64, None, -1, None, 0, None, 0, None, None, None,
+                                         None) == _BADARG      # no descriptor
 
 
 def test_product_path_refuses_cpu():
