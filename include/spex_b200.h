@@ -442,6 +442,41 @@ int spex_score_candidates_f32(const float* U, const float* I, int32_t D,
                               int32_t n_c, float* score, void* stream);
 
 /*
+ * Full-ranking metrics of one block of top-k lists, at up to SPEX_METRICS_MAX_CUTOFFS cutoffs, with the
+ * definitions of spex_b200/metrics.py: fullrank_recall_ndcg (upstream LightGCN).  For user u and cutoff K:
+ *   hits      = number of topk_idx[u, :K] entries found in the user's truth row (np.isin semantics)
+ *   recall    = hits / |truth| (0 for an empty row)    precision = hits / K    hit = (hits > 0)
+ *   ndcg      = DCG / idcg[min(|truth|, K)] (0 where that is 0), DCG = sum of disc[i] over the hit ranks i < K,
+ *               summed in ascending i
+ *   topk_idx     int32 [B, k], best first, -1 padding (the output of any scorer above); 1 <= k <= 512
+ *   truth_rowptr int64 [B + 1], truth_col int32: the held-out items of the users as a CSR over their POSITIONS in
+ *                this block, each row ascending (duplicates allowed); the positions are absolute in truth_col, so a
+ *                caller ranking users [s, s + b) of a longer list passes truth_rowptr + s
+ *   cutoffs_host n_cut (1..8) cutoffs, strictly ascending, each in [1, k]
+ *   disc         fp64 [k]: 1 / log2(i + 2);  idcg fp64 [k + 1]: 0 followed by the running sums of disc (both
+ *                computed by the caller, so the device never evaluates a logarithm)
+ *   per_user     fp64 [B, n_cut, 4] (recall, precision, ndcg, hit) per user and cutoff; NULL: not written
+ *   chunk_sums   fp64 [ceil(B / SPEX_METRICS_CHUNK), n_cut, 4]: the sums over each chunk of SPEX_METRICS_CHUNK
+ *                consecutive users, in a fixed order that depends only on that chunk's per-user values
+ * spex_fullrank_metrics_reduce sums n_chunks chunk sums in ascending chunk order into sums fp64 [n_cut, 4]
+ * (n_chunks == 0 writes zeros).  No atomics: the same inputs give the same bits on every run.
+ * Errors, before anything is launched: SPEX_E_TOOBIG for k > 512 or n_cut > 8; SPEX_E_BADARG for k < 1, n_cut < 1,
+ * B < 0, cutoffs not strictly ascending or outside [1, k], NULL cutoffs, disc or idcg, and (B > 0) NULL topk_idx,
+ * truth or chunk_sums.  B == 0 reads and writes nothing.
+ * Replaces the per-user np.isin loop over a [B, k] id matrix copied to the host (metrics.py: fullrank_recall_ndcg,
+ * called by dist.ShardedEvaluator.recall_ndcg and batch_test.test_fullrank).
+ */
+#define SPEX_METRICS_MAX_CUTOFFS 8
+#define SPEX_METRICS_CHUNK 1024
+int spex_fullrank_metrics(const int32_t* topk_idx, int64_t B, int32_t k,
+                          const int64_t* truth_rowptr, const int32_t* truth_col,
+                          const int32_t* cutoffs_host, int32_t n_cut,
+                          const double* disc, const double* idcg,
+                          double* per_user, double* chunk_sums, void* stream);
+int spex_fullrank_metrics_reduce(const double* chunk_sums, int64_t n_chunks, int32_t n_cut,
+                                 double* sums, void* stream);
+
+/*
  * NGCF layer epilogue (configs[2], NGCF_SPEX/code/main_rec.py:76-85), D == 64:
  *   out = lrelu(side·W1^T + b1) + lrelu((ego*side)·W2^T + b2);  norm = out / max(|out|_2, 1e-12)
  * side = A·ego comes from spex_spmm_csr_f32.  W row-major [64,64] (nn.Linear.weight layout).

@@ -689,6 +689,7 @@ class ShardedEvaluator:
         self.U, self.I = U_all, I_all
         self.mrp, self.mcol = mask_rowptr, mask_col
         self.k, self.group, self.scorer = int(k), group, scorer
+        self._requested, self._f16_ranker = scorer, None
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         if (scorer == "f16" and self.k <= ops.F32_MAX_K
@@ -719,3 +720,38 @@ class ShardedEvaluator:
             dist.all_reduce(s, group=self.group)
         n = max(float(s[2]), 1.0)
         return {"recall": float(s[0]) / n, "ndcg": float(s[1]) / n, "users": int(s[2])}
+
+    def evaluate(self, users: torch.Tensor, truth_rowptr, truth_col, cutoffs, block: int = 148 * 2 * 128 * 4):
+        """Mean Recall, precision, NDCG and hit rate over ALL of `users` at each of `cutoffs` (truth: CSR over the
+        positions of `users`, rows ascending), the result dict of ops.FullRanker.evaluate: this rank's shard is
+        ranked at k = max(cutoffs) and scored on the device (FullRanker.evaluate), then ONE all-reduce of the
+        n_cut * 4 metric sums and the user count.  Neither the ids nor a [users, k] matrix reach the host."""
+        from . import ops
+
+        cutoffs = ops.check_cutoffs(cutoffs)
+        dev = self.I.device
+        users = torch.as_tensor(users, device=dev).to(torch.int64)
+        lo, hi = shard_range(users.numel(), self.rank, self.world)
+        trp = ops._i64c(truth_rowptr, dev)
+        if trp.numel() != users.numel() + 1:
+            raise ValueError(f"truth_rowptr must have {users.numel() + 1} entries (users + 1), got {trp.numel()}")
+        sums, _ = self._ranker_for(cutoffs[-1]).metric_sums(self.U, users[lo:hi].contiguous(), cutoffs,
+                                                             trp[lo: hi + 1], truth_col, self.mrp, self.mcol, block)
+        s = torch.cat([sums.flatten(), torch.tensor([float(hi - lo)], dtype=torch.float64, device=dev)])
+        if self.world > 1:
+            if dist.get_backend(self.group) != "nccl":
+                s = s.cpu()
+            dist.all_reduce(s, group=self.group)
+        s = s.cpu().numpy()
+        return ops.metric_means(s[:-1], int(s[-1]))
+
+    def _ranker_for(self, k: int):
+        """The ranker for top-k: above F32_MAX_K, tables that the near-tie probe sent to the exact fp32 scorer are
+        ranked by the f16 scorer, as LightGCN.rank_topk does."""
+        from . import ops
+
+        if self.scorer == "fp32" and self._requested == "f16" and k > ops.F32_MAX_K:
+            if self._f16_ranker is None:
+                self._f16_ranker = ops.FullRanker(self.I, "f16")
+            return self._f16_ranker
+        return self.ranker

@@ -137,6 +137,18 @@ def build_interaction_csr(users: np.ndarray, items: np.ndarray, n_rows: int, m_i
     return rowptr, i
 
 
+def truth_csr(users, truth):
+    """(rowptr int64 [len(users) + 1], col int32) of the held-out items of `users` from a {user: [items]} dict
+    such as dataset.testRatings: a CSR over the POSITIONS in `users` (a user missing from the dict gets an empty
+    row), each row ascending and de-duplicated (build_interaction_csr) - the truth argument of
+    ops.FullRanker.evaluate and dist.ShardedEvaluator.evaluate."""
+    rows = [truth.get(int(u), []) for u in users]
+    pos = np.repeat(np.arange(len(rows), dtype=np.int64), [len(r) for r in rows])
+    items = np.fromiter((i for r in rows for i in r), dtype=np.int64, count=int(pos.size))
+    m = int(items.max()) + 1 if items.size else 1
+    return build_interaction_csr(pos, items, len(rows), m)
+
+
 def csr_from_coo(rows: np.ndarray, cols: np.ndarray, vals: np.ndarray, n_rows: int, n_cols: int,
                  assume_sorted: bool = False, with_tpos: bool = False) -> CSRGraph:
     """CSR from COO triplets.  A coalesced torch sparse tensor is already (row, col)-sorted."""

@@ -28,7 +28,12 @@ _FLAGS = (
     ("hiddenSize", int, 64, "hidden width of the path-prediction task"),
     ("nonhybrid", None, False, "path task: global preference only"),
     ("act", int, 1, "activation selector of the path task"),
+    ("test_mode", str, "sampled", "Test() of main_rec: sampled = the reference's 99 negatives + 1 held-out item, "
+                                  "fullrank = every item ranked, training items masked (single GPU)"),
 )
+# flags the reference does not have: only in the namespace when given, so that a run without them sees the
+# reference's namespace; readers use getattr(args, name, default)
+_ADDED_CHOICES = {"test_mode": ("sampled", "fullrank")}
 
 
 def build_parser() -> argparse.ArgumentParser:
@@ -36,6 +41,9 @@ def build_parser() -> argparse.ArgumentParser:
     for name, kind, default, doc in _FLAGS:
         if kind is None:
             parser.add_argument("--" + name, action="store_true", help=doc)
+        elif name in _ADDED_CHOICES:
+            parser.add_argument("--" + name, type=kind, choices=_ADDED_CHOICES[name], default=argparse.SUPPRESS,
+                                help=f"{doc} (default: {default})")
         elif name == "data_path":
             parser.add_argument("--" + name, nargs="?", default=default, help=doc)
         else:

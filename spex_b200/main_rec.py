@@ -9,6 +9,8 @@ draw DataLoader(shuffle=True)'s RandomSampler makes, so a shared seed visits the
 loss is accumulated on the device and read once per epoch instead of `.item()` per step
 (main_rec.py:36), Test() propagates once instead of once per user (batch_test.py:33), and the
 optimiser is the fused dense Adam.
+`--test_mode fullrank` (single GPU) replaces the sampled 99+1 Test() by a full ranking of every item with the
+training items masked, Recall/NDCG@[10, 20, 50] computed on the device; the printed lines keep their format.
 """
 from __future__ import annotations
 
@@ -57,10 +59,30 @@ def Train(train_dataset, recommend_model, epoch, optimizer, device, batch=BATCH)
     return total_loss
 
 
-def Test(dataset, Recmodel, epoch, best_recall, best_ndcg, best_iter):
+def fullrank_test(Recmodel, testRatings, Ks=batch_test.Ks):
+    """Full-ranking Recall / NDCG at Ks of every user in testRatings, training items masked: {'recall', 'ndcg':
+    float64 [len(Ks)]} like batch_test.test().  One ShardedEvaluator (one GPU) over computer() and the training
+    mask; the metrics are computed on the device (dist.ShardedEvaluator.evaluate)."""
+    from .dist import ShardedEvaluator
+    from .graph import truth_csr
+
+    users = np.fromiter(testRatings.keys(), dtype=np.int64, count=len(testRatings))
+    all_users, all_items = Recmodel.computer()
+    mrp, mcol = Recmodel.train_mask_csr()
+    scorer = "f16" if all_items.shape[1] in (64, 128) else "fp32"
+    ev = ShardedEvaluator(all_users, all_items, mrp, mcol, k=max(Ks), scorer=scorer)
+    trp, tcol = truth_csr(users, testRatings)
+    ret = ev.evaluate(torch.from_numpy(users).to(all_items.device), trp, tcol, Ks)
+    return {"recall": ret["recall"], "ndcg": ret["ndcg"]}
+
+
+def Test(dataset, Recmodel, epoch, best_recall, best_ndcg, best_iter, test_mode="sampled"):
     Recmodel = Recmodel.eval()
     with torch.no_grad():
-        ret = batch_test.test(Recmodel, dataset.testRatings, dataset.testNegatives)
+        if test_mode == "fullrank":
+            ret = fullrank_test(Recmodel, dataset.testRatings)
+        else:
+            ret = batch_test.test(Recmodel, dataset.testRatings, dataset.testNegatives)
     perf_str = "Rec:  Epoch %d : recall=[%.4f, %.4f, %.4f],  ndcg=[%.4f, %.4f, %.4f]" % (
         epoch, ret["recall"][0], ret["recall"][1], ret["recall"][2], ret["ndcg"][0], ret["ndcg"][1],
         ret["ndcg"][2])
@@ -100,6 +122,8 @@ def main_distributed(args):
 
     if args.dropout:
         raise SystemExit(f"--dropout {args.dropout} is not supported with torchrun (row-partitioned backward needs the symmetric graph)")
+    if getattr(args, "test_mode", "sampled") != "sampled":
+        raise SystemExit("--test_mode fullrank is not supported with torchrun: run it on one GPU")
     rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
     local_rank = int(os.environ.get("LOCAL_RANK", rank))
     torch.cuda.set_device(local_rank)
@@ -176,7 +200,8 @@ def main(argv=None):
         for epoch in range(args.epochs):
             start = time.time()
             Train(train_dataset, Recmodel, epoch, optimizer, device)
-            best_recall, best_ndcg, best_iter = Test(dataset, Recmodel, epoch, best_recall, best_ndcg, best_iter)
+            best_recall, best_ndcg, best_iter = Test(dataset, Recmodel, epoch, best_recall, best_ndcg, best_iter,
+                                                     getattr(args, "test_mode", "sampled"))
             _ = time.time() - start
     finally:
         ops.enable_persistent_workspaces(False)

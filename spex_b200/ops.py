@@ -745,15 +745,15 @@ def score_candidates(U, I, users, cand):
     return score
 
 
-def score_topk_f32(U, I, users, k, mask_rowptr=None, mask_col=None):
+def score_topk_f32(U, I, users, k, mask_rowptr=None, mask_col=None, out_idx=None, out_val=None):
     """Exact fp32 full-ranking top-k (score desc, ties by ascending item id)."""
     _need_cuda(U, I)
     U, I = _f32c(U), _f32c(I)
     dev = U.device
     users = _i64c(users, dev)
     B = users.numel()
-    idx = torch.empty(B, k, dtype=torch.int32, device=dev)
-    val = torch.empty(B, k, dtype=torch.float32, device=dev)
+    idx = torch.empty(B, k, dtype=torch.int32, device=dev) if out_idx is None else out_idx
+    val = torch.empty(B, k, dtype=torch.float32, device=dev) if out_val is None else out_val
     call("spex_score_topk_f32", ptr(U), ptr(I), U.shape[1], ptr(users), B, I.shape[0],
          ptr(mask_rowptr), ptr(mask_col), int(k), ptr(idx), ptr(val), stream_ptr())
     return idx, val
@@ -948,20 +948,28 @@ class FullRanker:
         scale 2^s, chosen over all of them, rounds every user's operands (a per-block scale would round a user's
         fp16 subnormal components differently depending on its block-mates); each block is a slice of that
         buffer, `user_block` rounded up to a multiple of 128 rows."""
-        dev, m, D = self.device, self.m_items, self.D
         check_k(self.precision, k)
-        users = _i64c(users, dev)
+        users = _i64c(users, self.device)
         B = users.numel()
-        idx = torch.empty(B, k, dtype=torch.int32, device=dev)
-        val = torch.empty(B, k, dtype=torch.float32, device=dev)
-        step = user_block or max(B, 1)
+        idx = torch.empty(B, k, dtype=torch.int32, device=self.device)
+        val = torch.empty(B, k, dtype=torch.float32, device=self.device)
+        for _ in self._ranked_blocks(U_all, users, k, mask_rowptr, mask_col, user_block or max(B, 1),
+                                     lambda s, n: (idx[s: s + n], val[s: s + n])):
+            pass
+        return idx, val
+
+    def _ranked_blocks(self, U_all, users, k, mask_rowptr, mask_col, step, dest):
+        """Rank users[s: s + step] for s = 0, step, 2 step, ... into the (idx, val) [n, k] views dest(s, n) and
+        yield (s, idx view) after each block's launches."""
+        m, D = self.m_items, self.D
+        B = users.numel()
         if self.precision == "f16":
             step = (step + TC_USER_MULTIPLE - 1) // TC_USER_MULTIPLE * TC_USER_MULTIPLE
             if B:
                 Uh_all, _, umeta = pack_f16(U_all, users, TC_USER_MULTIPLE)
         for s in range(0, B, step):
             ub = users[s: s + step]
-            o_i, o_v = idx[s: s + ub.numel()], val[s: s + ub.numel()]
+            o_i, o_v = dest(s, ub.numel())
             if self.precision == "f16":
                 # the canonical layout keeps every 8-row group contiguous: rows [s, s + b_pad) are one slice
                 b_pad = (ub.numel() + TC_USER_MULTIPLE - 1) // TC_USER_MULTIPLE * TC_USER_MULTIPLE
@@ -974,10 +982,119 @@ class FullRanker:
                 score_topk_bf16(Ub, ub.numel(), b_pad, self._Ib, m, self._m_pad, k, ub, mask_rowptr, mask_col,
                                 o_i, o_v)
             else:
-                i32, v32 = score_topk_f32(U_all, self._I, ub, k, mask_rowptr, mask_col)
-                o_i.copy_(i32)
-                o_v.copy_(v32)
-        return idx, val
+                score_topk_f32(U_all, self._I, ub, k, mask_rowptr, mask_col, o_i, o_v)
+            yield s, o_i
+
+    def metric_sums(self, U_all, users, cutoffs, truth_rowptr, truth_col, mask_rowptr=None, mask_col=None,
+                    user_block=None, per_user=False):
+        """(sums fp64 [n_cut, 4], per-user fp64 [B, n_cut, 4] or None) of evaluate(), on the device; the last
+        axis is METRIC_NAMES.  The sums are over users, each chunk of METRICS_CHUNK users summed on its own and
+        the chunks in ascending order, so they do not depend on `user_block`."""
+        cutoffs = check_cutoffs(cutoffs)
+        k = cutoffs[-1]
+        check_k(self.precision, k)
+        dev = self.device
+        users = _i64c(users, dev)
+        B = users.numel()
+        trp = _i64c(truth_rowptr, dev)
+        tcol = torch.as_tensor(np.asarray(truth_col) if not torch.is_tensor(truth_col) else truth_col)
+        tcol = tcol.to(device=dev, dtype=torch.int32).contiguous()
+        check_truth_csr(trp, tcol, B)
+        if tcol.numel() == 0:
+            tcol = torch.zeros(1, dtype=torch.int32, device=dev)   # all rows empty: never read, but not NULL
+        n_cut = len(cutoffs)
+        cut_host = (C.c_int32 * n_cut)(*cutoffs)
+        disc, idcg = rank_discounts(k)
+        disc = torch.from_numpy(disc).to(dev)
+        idcg = torch.from_numpy(idcg).to(dev)
+        step = user_block or EVAL_USER_BLOCK
+        step = (step + METRICS_CHUNK - 1) // METRICS_CHUNK * METRICS_CHUNK     # also a multiple of TC_USER_MULTIPLE
+        n_chunks = (B + METRICS_CHUNK - 1) // METRICS_CHUNK
+        chunk_sums = torch.empty(n_chunks, n_cut, 4, dtype=torch.float64, device=dev)
+        pu = torch.empty(B, n_cut, 4, dtype=torch.float64, device=dev) if per_user else None
+        nb = min(step, B)
+        bi = torch.empty(nb, k, dtype=torch.int32, device=dev)      # one [block, k] buffer for every block
+        bv = torch.empty(nb, k, dtype=torch.float32, device=dev)
+        for s, o_i in self._ranked_blocks(U_all, users, k, mask_rowptr, mask_col, step,
+                                          lambda s, n: (bi[:n], bv[:n])):
+            n = o_i.shape[0]
+            call("spex_fullrank_metrics", ptr(o_i), n, k, ptr(trp[s:]), ptr(tcol), cut_host, n_cut, ptr(disc),
+                 ptr(idcg), ptr(None if pu is None else pu[s:]), ptr(chunk_sums[s // METRICS_CHUNK:]), stream_ptr())
+        sums = torch.empty(n_cut, 4, dtype=torch.float64, device=dev)
+        call("spex_fullrank_metrics_reduce", ptr(chunk_sums), n_chunks, n_cut, ptr(sums), stream_ptr())
+        return sums, pu
+
+    def evaluate(self, U_all, users, cutoffs, truth_rowptr, truth_col, mask_rowptr=None, mask_col=None,
+                 user_block=None, per_user=False):
+        """Recall, precision, NDCG and hit rate of the full ranking of U_all[users] at each of `cutoffs` (1 to 8
+        strictly ascending k): {"recall", "precision", "ndcg", "hit": float64 [n_cut], "users": B}, means over all
+        B users (an empty truth row counts as zeros), and with per_user=True "per_user": fp64 [B, n_cut, 4] on the
+        device (last axis METRIC_NAMES).  Definitions of metrics.fullrank_recall_ndcg, precision = hits / K.
+
+        truth_rowptr int64 [B + 1] / truth_col: the held-out items as a CSR over the POSITIONS in `users`, every
+        row ascending (ValueError otherwise; graph.truth_csr builds one).  The users are ranked at
+        k = max(cutoffs) through the same scorers as topk(), in blocks of `user_block` users rounded up to a
+        multiple of METRICS_CHUNK (None: EVAL_USER_BLOCK); each block's ids stay on the device in one reused
+        [block, k] buffer and go straight into spex_fullrank_metrics.  The result does not depend on
+        `user_block`."""
+        users = _i64c(users, self.device)
+        sums, pu = self.metric_sums(U_all, users, cutoffs, truth_rowptr, truth_col, mask_rowptr, mask_col,
+                                    user_block, per_user)
+        return metric_means(sums.cpu().numpy(), users.numel(), pu)
+
+
+METRICS_CHUNK = 1024           # SPEX_METRICS_CHUNK in include/spex_b200.h: users per partial sum
+METRICS_MAX_CUTOFFS = 8        # SPEX_METRICS_MAX_CUTOFFS
+METRIC_NAMES = ("recall", "precision", "ndcg", "hit")
+EVAL_USER_BLOCK = 148 * METRICS_CHUNK   # users ranked per block by FullRanker.evaluate (None)
+
+
+def check_cutoffs(cutoffs):
+    """The cutoffs as a list of ints; ValueError unless 1 to METRICS_MAX_CUTOFFS of them, strictly ascending, >= 1."""
+    cutoffs = [int(c) for c in cutoffs]
+    if not 1 <= len(cutoffs) <= METRICS_MAX_CUTOFFS:
+        raise ValueError(f"1 to {METRICS_MAX_CUTOFFS} cutoffs, got {len(cutoffs)}")
+    if cutoffs[0] < 1 or any(b <= a for a, b in zip(cutoffs, cutoffs[1:])):
+        raise ValueError(f"cutoffs must be >= 1 and strictly ascending, got {cutoffs}")
+    return cutoffs
+
+
+def rank_discounts(k: int):
+    """(disc fp64 [k], idcg fp64 [k + 1]) of spex_fullrank_metrics, computed as metrics.fullrank_recall_ndcg
+    computes its disc and cum: the ideal DCGs are bit-equal to the host's by construction."""
+    disc = 1.0 / np.log2(np.arange(2, k + 2))
+    return disc, np.concatenate([[0.0], np.cumsum(disc)])
+
+
+def check_truth_csr(truth_rowptr: torch.Tensor, truth_col: torch.Tensor, B: int):
+    """ValueError unless truth_rowptr (int64 [B + 1]) is non-decreasing inside [0, len(truth_col)] and every row
+    of truth_col is ascending: the kernel's binary search relies on it.  Checked on the device."""
+    if truth_rowptr.numel() != B + 1:
+        raise ValueError(f"truth_rowptr must have {B + 1} entries (users + 1), got {truth_rowptr.numel()}")
+    if B == 0:
+        return
+    rp = truth_rowptr
+    if bool((rp[1:] < rp[:-1]).any() | (rp[0] < 0) | (rp[-1] > truth_col.numel())):
+        raise ValueError("truth_rowptr must be non-decreasing and inside truth_col")
+    a, b = int(rp[0]), int(rp[-1])
+    if b - a < 2:
+        return
+    c = truth_col[a:b]
+    starts = rp[:-1]
+    first = torch.zeros(b - a, dtype=torch.bool, device=c.device)
+    first[starts[starts < b] - a] = True
+    if bool(((c[1:] < c[:-1]) & ~first[1:]).any()):
+        raise ValueError("every truth row must be sorted ascending (graph.build_interaction_csr sorts)")
+
+
+def metric_means(sums: np.ndarray, n_users: int, per_user=None) -> dict:
+    """The result dict of FullRanker.evaluate from metric sums [n_cut, 4] over n_users users."""
+    mean = np.asarray(sums, dtype=np.float64).reshape(-1, 4) / max(float(n_users), 1.0)
+    out = {name: mean[:, j].copy() for j, name in enumerate(METRIC_NAMES)}
+    out["users"] = int(n_users)
+    if per_user is not None:
+        out["per_user"] = per_user
+    return out
 
 
 GATE_BWD_BLOCKS = 1184  # SPEX_GATE_BWD_BLOCKS in include/spex_b200.h
