@@ -464,7 +464,7 @@ int spex_score_candidates_f32(const float* U, const float* I, int32_t D,
  * B < 0, cutoffs not strictly ascending or outside [1, k], NULL cutoffs, disc or idcg, and (B > 0) NULL topk_idx,
  * truth or chunk_sums.  B == 0 reads and writes nothing.
  * Replaces the per-user np.isin loop over a [B, k] id matrix copied to the host (metrics.py: fullrank_recall_ndcg,
- * called by dist.ShardedEvaluator.recall_ndcg and batch_test.test_fullrank).
+ * called by batch_test.test_fullrank).
  */
 #define SPEX_METRICS_MAX_CUTOFFS 8
 #define SPEX_METRICS_CHUNK 1024

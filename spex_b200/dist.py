@@ -41,7 +41,6 @@ from __future__ import annotations
 import ctypes as C
 from typing import Callable, List, Optional, Sequence
 
-import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -679,47 +678,33 @@ def shard_range(n: int, rank: int, world: int):
 
 
 class ShardedEvaluator:
-    """Full-ranking top-k + Recall/NDCG over a user shard per rank.  The propagated item table is
-    replicated (5 M x 64 fp16 = 640 MB), every rank ranks users [lo, hi) of the list it is given with the
-    tcgen05 scorer, metrics are summed over ranks with ONE all-reduce of three numbers."""
+    """Full-ranking top-k and Recall, precision, NDCG and hit rate over a user shard per rank.  The propagated
+    item table is replicated (5 M x 64 fp16 = 640 MB), every rank ranks users [lo, hi) of the list it is given
+    through one ops.FullRanker(probe=True), metrics are summed over ranks with ONE all-reduce."""
 
     def __init__(self, U_all, I_all, mask_rowptr=None, mask_col=None, k: int = 20, group=None, scorer: str = "f16"):
         from . import ops
 
         self.U, self.I = U_all, I_all
         self.mrp, self.mcol = mask_rowptr, mask_col
-        self.k, self.group, self.scorer = int(k), group, scorer
-        self._requested, self._f16_ranker = scorer, None
+        self.k, self.group = int(k), group
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
-        if (scorer == "f16" and self.k <= ops.F32_MAX_K
-                and not ops.f16_filter_is_selective(U_all, I_all, torch.arange(U_all.shape[0], device=I_all.device))):
-            scorer = self.scorer = "fp32"      # near-equal scores: the exact scorer is the faster exact path
-        self.ranker = ops.FullRanker(I_all, scorer)
+        self.ranker = ops.FullRanker(I_all, scorer, probe=True)
+        # the near-tie probe samples all users, whatever this rank's shard: every rank picks the same scorer
+        self._probe_users = torch.arange(U_all.shape[0], device=I_all.device)
+
+    @property
+    def scorer(self) -> str:
+        """The scorer that ranks top-k (rank_topk)."""
+        return self.ranker.scorer_for(self.k, self.U, self._probe_users)
 
     def rank_topk(self, users: torch.Tensor, block: int = 148 * 2 * 128 * 4):
         """(idx int32 [n_local, k], val fp32 [n_local, k], (lo, hi)) for this rank's shard of `users`."""
         lo, hi = shard_range(users.numel(), self.rank, self.world)
         mine = users[lo:hi].to(torch.int64).contiguous()
-        idx, val = self.ranker.topk(self.U, mine, self.k, self.mrp, self.mcol, block)
+        idx, val = self.ranker.topk(self.U, mine, self.k, self.mrp, self.mcol, block, self._probe_users)
         return idx, val, (lo, hi)
-
-    def recall_ndcg(self, users: torch.Tensor, truth_rowptr, truth_col):
-        """Mean Recall@k / NDCG@k over ALL of `users` (truth: CSR over the positions of `users`): local
-        metrics on the host, one all-reduce of (sum recall, sum ndcg, count)."""
-        from . import metrics
-
-        idx, _, (lo, hi) = self.rank_topk(users)
-        trp = np.asarray(truth_rowptr)
-        rec, ndcg = metrics.fullrank_recall_ndcg(idx.cpu().numpy(), trp[lo: hi + 1] - trp[lo],
-                                                 np.asarray(truth_col)[trp[lo]: trp[hi]], self.k)
-        s = torch.tensor([float(rec.sum()), float(ndcg.sum()), float(hi - lo)], dtype=torch.float64,
-                         device=self.I.device if dist.is_initialized() and dist.get_backend(self.group) == "nccl"
-                         else "cpu")
-        if self.world > 1:
-            dist.all_reduce(s, group=self.group)
-        n = max(float(s[2]), 1.0)
-        return {"recall": float(s[0]) / n, "ndcg": float(s[1]) / n, "users": int(s[2])}
 
     def evaluate(self, users: torch.Tensor, truth_rowptr, truth_col, cutoffs, block: int = 148 * 2 * 128 * 4):
         """Mean Recall, precision, NDCG and hit rate over ALL of `users` at each of `cutoffs` (truth: CSR over the
@@ -735,8 +720,8 @@ class ShardedEvaluator:
         trp = ops._i64c(truth_rowptr, dev)
         if trp.numel() != users.numel() + 1:
             raise ValueError(f"truth_rowptr must have {users.numel() + 1} entries (users + 1), got {trp.numel()}")
-        sums, _ = self._ranker_for(cutoffs[-1]).metric_sums(self.U, users[lo:hi].contiguous(), cutoffs,
-                                                             trp[lo: hi + 1], truth_col, self.mrp, self.mcol, block)
+        sums, _ = self.ranker.metric_sums(self.U, users[lo:hi].contiguous(), cutoffs, trp[lo: hi + 1], truth_col,
+                                          self.mrp, self.mcol, block, probe_users=self._probe_users)
         s = torch.cat([sums.flatten(), torch.tensor([float(hi - lo)], dtype=torch.float64, device=dev)])
         if self.world > 1:
             if dist.get_backend(self.group) != "nccl":
@@ -744,14 +729,3 @@ class ShardedEvaluator:
             dist.all_reduce(s, group=self.group)
         s = s.cpu().numpy()
         return ops.metric_means(s[:-1], int(s[-1]))
-
-    def _ranker_for(self, k: int):
-        """The ranker for top-k: above F32_MAX_K, tables that the near-tie probe sent to the exact fp32 scorer are
-        ranked by the f16 scorer, as LightGCN.rank_topk does."""
-        from . import ops
-
-        if self.scorer == "fp32" and self._requested == "f16" and k > ops.F32_MAX_K:
-            if self._f16_ranker is None:
-                self._f16_ranker = ops.FullRanker(self.I, "f16")
-            return self._f16_ranker
-        return self.ranker

@@ -19,7 +19,7 @@ import time
 import numpy as np
 import torch
 
-from . import batch_test, dataloader, utils
+from . import batch_test, dataloader, ops, utils
 from .lg_parser import parse_args_r
 from .model import LightGCN
 from .optim import FusedAdam
@@ -69,8 +69,7 @@ def fullrank_test(Recmodel, testRatings, Ks=batch_test.Ks):
     users = np.fromiter(testRatings.keys(), dtype=np.int64, count=len(testRatings))
     all_users, all_items = Recmodel.computer()
     mrp, mcol = Recmodel.train_mask_csr()
-    scorer = "f16" if all_items.shape[1] in (64, 128) else "fp32"
-    ev = ShardedEvaluator(all_users, all_items, mrp, mcol, k=max(Ks), scorer=scorer)
+    ev = ShardedEvaluator(all_users, all_items, mrp, mcol, k=max(Ks), scorer=ops.default_precision(all_items.shape[1]))
     trp, tcol = truth_csr(users, testRatings)
     ret = ev.evaluate(torch.from_numpy(users).to(all_items.device), trp, tcol, Ks)
     return {"recall": ret["recall"], "ndcg": ret["ndcg"]}

@@ -259,28 +259,22 @@ class LightGCN(BasicModel):
         """Full-ranking top-k items per user: (idx int32 [B,k], score fp32 [B,k]).
 
         precision "f16":  tcgen05 fp16-accumulator filter + exact fp32 re-score of the survivors
-                          (operands fp16(x 2^s); recdim 64 or 128; k <= 512) - the default; for k <= 128
-                          a probe (ops.f16_filter_is_selective) routes tables with near-equal scores to
-                          "fp32", above that the f16 scorer serves them too (exact, slow);
+                          (operands fp16(x 2^s); recdim 64 or 128; k <= 512) - the default;
         precision "bf16": round 1's tcgen05 GEMM, bf16 operands / fp32 accumulators (recdim 64; k <= 64);
         precision "fp32": exact CUDA-core scorer (bit-exact ordering, any recdim; k <= 128).
+        probe: the near-tie probe may send "f16" to "fp32" for k <= 128 (ops.FullRanker.scorer_for, where every
+        caller's scorer is chosen); same ranking, faster on tables with near-equal scores.
         Ordering: score descending, ties by ascending item id; masked = the user's train items.
         """
-        ops.check_k(precision, k)
         all_users, all_items = self.computer()
-        dev = all_users.device
-        users = torch.as_tensor(users, device=dev).long().contiguous()
         mrp = mcol = None
         if exclude_train:
             mrp, mcol = self.train_mask_csr()
-        # the packed item table is reused across eval-mode calls; fp32 reads the current table as it is
+        # the ranker and the item operands it packs are reused across eval-mode calls, in which propagation gives
+        # the same bits every time; fp32 reads the current table as it is
         r = self._ranker
-        if r is None or self.training or r.precision != precision or precision == "fp32":
-            r = self._ranker = ops.FullRanker(all_items, precision)
-        if (precision == "f16" and probe and k <= ops.F32_MAX_K
-                and not ops.f16_filter_is_selective(all_users, all_items, users)):
-            # degenerate score distribution (near-ties everywhere): the exact scorer is the faster exact path
-            return ops.score_topk_f32(all_users, all_items, users, k, mrp, mcol)
+        if r is None or self.training or (r.precision, r.probe) != (precision, probe) or precision == "fp32":
+            r = self._ranker = ops.FullRanker(all_items, precision, probe=probe)
         return r.topk(all_users, users, k, mrp, mcol, user_block)
 
 

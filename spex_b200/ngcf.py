@@ -202,20 +202,16 @@ class Model_Wrapper(nn.Module):
     def rank_topk(self, users, k: int = 20, mask_rowptr=None, mask_col=None, precision: str = "f16",
                   probe: bool = True):
         """Top-k items per user over the concatenated layer outputs (utility/batch_test.py:158 followed by
-        the ranking): tcgen05 fp16-accumulator filter + exact fp32 re-score at D = 64 (L + 1), or the exact
-        fp32 CUDA-core scorer (precision "fp32", k <= 128).  k <= 512 with the f16 scorer; near-equal scores
-        (see ops.f16_filter_is_selective) go to the fp32 scorer when k <= 128.  Returns (idx int32 [B, k],
+        the ranking) through ops.FullRanker: tcgen05 fp16-accumulator filter + exact fp32 re-score at
+        D = 64 (L + 1) in {64, 128}, k <= 512, or the exact fp32 CUDA-core scorer (precision "fp32", or "f16" at
+        any other D; k <= 128).  probe: near-equal scores (an untrained NGCF's normalised outputs are almost
+        parallel) go to the fp32 scorer when k <= 128 (ops.FullRanker.scorer_for).  Returns (idx int32 [B, k],
         score fp32 [B, k])."""
-        ops.check_k(precision, k)
         ua, ia = self.propagate()
         ua, ia = ua.contiguous(), ia.contiguous()
-        users = torch.as_tensor(users, device=ua.device).long().contiguous()
-        Dk = ua.shape[1]
-        if precision == "fp32" or Dk not in (64, 128) or (probe and k <= ops.F32_MAX_K and
-                                                           not ops.f16_filter_is_selective(ua, ia, users)):
-            # (an untrained NGCF's normalised outputs are almost parallel: near-ties everywhere, no filter helps)
-            return ops.score_topk_f32(ua, ia, users, k, mask_rowptr, mask_col)
-        return ops.FullRanker(ia, "f16").topk(ua, users, k, mask_rowptr, mask_col)
+        if precision == "f16":
+            precision = ops.default_precision(ua.shape[1])
+        return ops.FullRanker(ia, precision, probe=probe).topk(ua, users, k, mask_rowptr, mask_col)
 
     @torch.no_grad()
     def rate_all_items(self, users):

@@ -782,8 +782,8 @@ def f16_filter_is_selective(U, I, users, n_users: int = 64, n_items: int = 8192,
     measured 99 ms against 1.7 ms for random tables of the same shape and 7 ms for the exact fp32 scorer - that
     band holds most items and the filter degenerates.  The probe scores a sample (n_users x n_items, exact fp32,
     spex_rating_f32) and compares the band with the spread of each user's scores: selective iff the median of
-    2 eps / (max - median score) stays below 0.1 (random / trained tables: ~0.01).  Callers fall back to the exact
-    fp32 scorer otherwise; the result is the same ranking either way."""
+    2 eps / (max - median score) stays below 0.1 (random / trained tables: ~0.01).  FullRanker(probe=True) falls
+    back to the exact fp32 scorer otherwise; the result is the same ranking either way."""
     _need_cuda(U, I)
     dev = U.device
     users = _i64c(users, dev)
@@ -806,6 +806,14 @@ TC_MAX_K = 64            # larger k: score_topk_f16_wide (or score_topk_f32 up t
 F32_MAX_K = 128          # k limit of score_topk_f32
 WIDE_MAX_K = 512         # k limit of score_topk_f16_wide
 TC_ITEM_MULTIPLE = 128   # items per tile (UMMA N)
+# precision -> (the D its full-ranking scorer is built for, None: any; its largest k).  f16 ranks k <= TC_MAX_K with
+# score_topk_f16 and larger k with score_topk_f16_wide.
+SCORER_LIMITS = {"f16": ((64, 128), WIDE_MAX_K), "bf16": ((64,), TC_MAX_K), "fp32": (None, F32_MAX_K)}
+
+
+def default_precision(D: int) -> str:
+    """The full-ranking precision for D: "f16" where its scorer is built for D, else "fp32" (any D)."""
+    return "f16" if D in SCORER_LIMITS["f16"][0] else "fp32"
 
 
 def pack_bf16(src, rows=None, row_multiple: int = 8, out=None):
@@ -829,8 +837,9 @@ def score_topk_bf16(Ub, B, B_pad, Ib, m_items, m_pad, k, user_ids=None, mask_row
                     mask_col=None, out_idx=None, out_val=None):
     """tcgen05 bf16 scoring GEMM fused with train-item masking and per-row top-k (D = 64)."""
     _need_cuda(Ub, Ib)
-    if not 1 <= k <= TC_MAX_K:
-        raise ValueError(f"score_topk_bf16: k must be in [1, {TC_MAX_K}] (use score_topk_f32 beyond)")
+    max_k = SCORER_LIMITS["bf16"][1]
+    if not 1 <= k <= max_k:
+        raise ValueError(f"score_topk_bf16: k must be in [1, {max_k}] (use score_topk_f32 beyond)")
     dev = Ub.device
     if out_idx is None:
         out_idx = torch.empty(B, k, dtype=torch.int32, device=dev)
@@ -868,7 +877,7 @@ def score_topk_f16(Uh, u_meta, B, B_pad, Ih, i_meta, m_items, m_pad, D, k, user_
     _need_cuda(Uh, Ih)
     if not 1 <= k <= TC_MAX_K:
         raise ValueError(f"score_topk_f16: k must be in [1, {TC_MAX_K}] (use score_topk_f32 beyond)")
-    if D not in (64, 128):
+    if D not in SCORER_LIMITS["f16"][0]:
         raise ValueError("score_topk_f16: D must be 64 or 128 (use score_topk_f32 otherwise)")
     dev = Uh.device
     if out_idx is None:
@@ -888,9 +897,10 @@ def score_topk_f16_wide(Uh, u_meta, B, B_pad, Ih, i_meta, m_items, m_pad, D, k, 
     candidate buffer in a device workspace (allocated here, B_pad * (2k + 64) * 8 bytes) instead of shared
     memory."""
     _need_cuda(Uh, Ih)
-    if not 1 <= k <= WIDE_MAX_K:
-        raise ValueError(f"score_topk_f16_wide: k must be in [1, {WIDE_MAX_K}]")
-    if D not in (64, 128):
+    dims, max_k = SCORER_LIMITS["f16"]
+    if not 1 <= k <= max_k:
+        raise ValueError(f"score_topk_f16_wide: k must be in [1, {max_k}]")
+    if D not in dims:
         raise ValueError("score_topk_f16_wide: D must be 64 or 128 (use score_topk_f32 otherwise)")
     dev = Uh.device
     if out_idx is None:
@@ -907,11 +917,11 @@ def score_topk_f16_wide(Uh, u_meta, B, B_pad, Ih, i_meta, m_items, m_pad, D, k, 
 
 
 def check_k(precision: str, k: int):
-    """ValueError unless `precision` serves top-`k`: f16 up to WIDE_MAX_K, bf16 up to TC_MAX_K, fp32 up to
-    F32_MAX_K; the message names the precision that serves a k beyond the limit."""
-    limit = {"bf16": TC_MAX_K, "fp32": F32_MAX_K}.get(precision, WIDE_MAX_K)
+    """ValueError unless `precision` serves top-`k` (SCORER_LIMITS); the message names the precision that serves a k
+    beyond the limit."""
+    limit, wide = SCORER_LIMITS[precision][1], SCORER_LIMITS["f16"][1]
     if not 1 <= k <= limit:
-        hint = f"; precision 'f16' serves k <= {WIDE_MAX_K}" if precision != "f16" and 1 <= k <= WIDE_MAX_K else ""
+        hint = f"; precision 'f16' serves k <= {wide}" if precision != "f16" and 1 <= k <= wide else ""
         raise ValueError(f"precision '{precision}' serves 1 <= k <= {limit}, got k = {k}{hint}")
 
 
@@ -923,61 +933,74 @@ class FullRanker:
                       k <= TC_MAX_K, score_topk_f16_wide up to WIDE_MAX_K;
     precision "bf16": tcgen05 bf16 operands / fp32 accumulators (score_topk_bf16; D = 64; k <= TC_MAX_K);
     precision "fp32": exact CUDA-core scorer (score_topk_f32; any D; k <= F32_MAX_K).
-    The item table is packed once, here (the fp32 scorer reads it as it is); the users are packed in topk()."""
+    probe=True lets the near-tie probe send "f16" rankings to "fp32" (scorer_for): the one place where any caller's
+    scorer is chosen.  The item table is packed on the first call that needs it packed (the fp32 scorer reads it as
+    it is); the users are packed per call."""
 
-    def __init__(self, I_all, precision: str = "f16"):
-        D = I_all.shape[1]
-        if precision not in ("f16", "bf16", "fp32"):
+    def __init__(self, I_all, precision: str = "f16", probe: bool = False):
+        if precision not in SCORER_LIMITS:
             raise ValueError("precision must be 'f16', 'bf16' or 'fp32'")
-        if precision == "bf16" and D != 64:
-            raise RuntimeError("the bf16 tcgen05 scorer is built for recdim == 64")
-        if precision == "f16" and D not in (64, 128):
-            raise RuntimeError("the f16 tcgen05 scorer is built for recdim 64 or 128")
-        self.precision, self.device = precision, I_all.device
+        dims = SCORER_LIMITS[precision][0]
+        if dims is not None and I_all.shape[1] not in dims:
+            built = " or ".join(map(str, dims)) if len(dims) > 1 else f"== {dims[0]}"
+            raise RuntimeError(f"the {precision} tcgen05 scorer is built for recdim {built}")
+        self.precision, self.probe, self.device = precision, probe, I_all.device
         self.m_items, self.D = I_all.shape
-        self._I = I_all if precision == "fp32" else None
-        if precision == "f16":
-            self._Ih, self._m_pad, self._imeta = pack_f16(I_all, None, TC_ITEM_MULTIPLE)
-        elif precision == "bf16":
-            self._Ib, self._m_pad = pack_bf16(I_all, None, TC_ITEM_MULTIPLE)
+        self._I, self._m_pad = I_all, None      # _m_pad: set when the item table is packed
 
-    def topk(self, U_all, users, k, mask_rowptr=None, mask_col=None, user_block=None):
-        """Rank U_all[users] in blocks of `user_block` users (None: one block).
+    def scorer_for(self, k: int, U_all, probe_users) -> str:
+        """The precision that ranks top-k: ValueError unless this ranker's precision serves k (check_k).  With
+        probe=True, "f16" becomes "fp32" for k <= F32_MAX_K when f16_filter_is_selective(U_all, I_all, probe_users)
+        is False: near-equal scores, on which the exact scorer is the faster exact path (above F32_MAX_K only the
+        f16 scorer serves k)."""
+        check_k(self.precision, k)
+        if (self.precision == "f16" and self.probe and k <= F32_MAX_K
+                and not f16_filter_is_selective(U_all, self._I, probe_users)):
+            return "fp32"
+        return self.precision
+
+    def topk(self, U_all, users, k, mask_rowptr=None, mask_col=None, user_block=None, probe_users=None):
+        """Rank U_all[users] in blocks of `user_block` users (None: one block) with the scorer of
+        scorer_for(k, U_all, probe_users) (None: `users`).
 
         f16: the result does not depend on `user_block`.  The users of the call are packed once, so one user
         scale 2^s, chosen over all of them, rounds every user's operands (a per-block scale would round a user's
         fp16 subnormal components differently depending on its block-mates); each block is a slice of that
         buffer, `user_block` rounded up to a multiple of 128 rows."""
-        check_k(self.precision, k)
         users = _i64c(users, self.device)
+        scorer = self.scorer_for(k, U_all, users if probe_users is None else probe_users)
         B = users.numel()
         idx = torch.empty(B, k, dtype=torch.int32, device=self.device)
         val = torch.empty(B, k, dtype=torch.float32, device=self.device)
-        for _ in self._ranked_blocks(U_all, users, k, mask_rowptr, mask_col, user_block or max(B, 1),
+        for _ in self._ranked_blocks(scorer, U_all, users, k, mask_rowptr, mask_col, user_block or max(B, 1),
                                      lambda s, n: (idx[s: s + n], val[s: s + n])):
             pass
         return idx, val
 
-    def _ranked_blocks(self, U_all, users, k, mask_rowptr, mask_col, step, dest):
-        """Rank users[s: s + step] for s = 0, step, 2 step, ... into the (idx, val) [n, k] views dest(s, n) and
-        yield (s, idx view) after each block's launches."""
+    def _ranked_blocks(self, scorer, U_all, users, k, mask_rowptr, mask_col, step, dest):
+        """Rank users[s: s + step] for s = 0, step, 2 step, ... with `scorer` into the (idx, val) [n, k] views
+        dest(s, n) and yield (s, idx view) after each block's launches."""
         m, D = self.m_items, self.D
         B = users.numel()
-        if self.precision == "f16":
+        if scorer == "f16" and self._m_pad is None:
+            self._Ih, self._m_pad, self._imeta = pack_f16(self._I, None, TC_ITEM_MULTIPLE)
+        elif scorer == "bf16" and self._m_pad is None:
+            self._Ib, self._m_pad = pack_bf16(self._I, None, TC_ITEM_MULTIPLE)
+        if scorer == "f16":
             step = (step + TC_USER_MULTIPLE - 1) // TC_USER_MULTIPLE * TC_USER_MULTIPLE
             if B:
                 Uh_all, _, umeta = pack_f16(U_all, users, TC_USER_MULTIPLE)
         for s in range(0, B, step):
             ub = users[s: s + step]
             o_i, o_v = dest(s, ub.numel())
-            if self.precision == "f16":
+            if scorer == "f16":
                 # the canonical layout keeps every 8-row group contiguous: rows [s, s + b_pad) are one slice
                 b_pad = (ub.numel() + TC_USER_MULTIPLE - 1) // TC_USER_MULTIPLE * TC_USER_MULTIPLE
                 Uh = Uh_all[s * D: (s + b_pad) * D]
                 f16 = score_topk_f16 if k <= TC_MAX_K else score_topk_f16_wide
                 f16(Uh, umeta, ub.numel(), b_pad, self._Ih, self._imeta, m, self._m_pad, D, k, ub, mask_rowptr,
                     mask_col, o_i, o_v)
-            elif self.precision == "bf16":
+            elif scorer == "bf16":
                 Ub, b_pad = pack_bf16(U_all, ub, TC_USER_MULTIPLE)
                 score_topk_bf16(Ub, ub.numel(), b_pad, self._Ib, m, self._m_pad, k, ub, mask_rowptr, mask_col,
                                 o_i, o_v)
@@ -986,13 +1009,12 @@ class FullRanker:
             yield s, o_i
 
     def metric_sums(self, U_all, users, cutoffs, truth_rowptr, truth_col, mask_rowptr=None, mask_col=None,
-                    user_block=None, per_user=False):
+                    user_block=None, per_user=False, probe_users=None):
         """(sums fp64 [n_cut, 4], per-user fp64 [B, n_cut, 4] or None) of evaluate(), on the device; the last
         axis is METRIC_NAMES.  The sums are over users, each chunk of METRICS_CHUNK users summed on its own and
         the chunks in ascending order, so they do not depend on `user_block`."""
         cutoffs = check_cutoffs(cutoffs)
         k = cutoffs[-1]
-        check_k(self.precision, k)
         dev = self.device
         users = _i64c(users, dev)
         B = users.numel()
@@ -1000,6 +1022,7 @@ class FullRanker:
         tcol = torch.as_tensor(np.asarray(truth_col) if not torch.is_tensor(truth_col) else truth_col)
         tcol = tcol.to(device=dev, dtype=torch.int32).contiguous()
         check_truth_csr(trp, tcol, B)
+        scorer = self.scorer_for(k, U_all, users if probe_users is None else probe_users)
         if tcol.numel() == 0:
             tcol = torch.zeros(1, dtype=torch.int32, device=dev)   # all rows empty: never read, but not NULL
         n_cut = len(cutoffs)
@@ -1015,7 +1038,7 @@ class FullRanker:
         nb = min(step, B)
         bi = torch.empty(nb, k, dtype=torch.int32, device=dev)      # one [block, k] buffer for every block
         bv = torch.empty(nb, k, dtype=torch.float32, device=dev)
-        for s, o_i in self._ranked_blocks(U_all, users, k, mask_rowptr, mask_col, step,
+        for s, o_i in self._ranked_blocks(scorer, U_all, users, k, mask_rowptr, mask_col, step,
                                           lambda s, n: (bi[:n], bv[:n])):
             n = o_i.shape[0]
             call("spex_fullrank_metrics", ptr(o_i), n, k, ptr(trp[s:]), ptr(tcol), cut_host, n_cut, ptr(disc),
@@ -1025,7 +1048,7 @@ class FullRanker:
         return sums, pu
 
     def evaluate(self, U_all, users, cutoffs, truth_rowptr, truth_col, mask_rowptr=None, mask_col=None,
-                 user_block=None, per_user=False):
+                 user_block=None, per_user=False, probe_users=None):
         """Recall, precision, NDCG and hit rate of the full ranking of U_all[users] at each of `cutoffs` (1 to 8
         strictly ascending k): {"recall", "precision", "ndcg", "hit": float64 [n_cut], "users": B}, means over all
         B users (an empty truth row counts as zeros), and with per_user=True "per_user": fp64 [B, n_cut, 4] on the
@@ -1033,13 +1056,13 @@ class FullRanker:
 
         truth_rowptr int64 [B + 1] / truth_col: the held-out items as a CSR over the POSITIONS in `users`, every
         row ascending (ValueError otherwise; graph.truth_csr builds one).  The users are ranked at
-        k = max(cutoffs) through the same scorers as topk(), in blocks of `user_block` users rounded up to a
-        multiple of METRICS_CHUNK (None: EVAL_USER_BLOCK); each block's ids stay on the device in one reused
-        [block, k] buffer and go straight into spex_fullrank_metrics.  The result does not depend on
+        k = max(cutoffs) by the scorer topk() would use (probe_users as there), in blocks of `user_block` users
+        rounded up to a multiple of METRICS_CHUNK (None: EVAL_USER_BLOCK); each block's ids stay on the device in
+        one reused [block, k] buffer and go straight into spex_fullrank_metrics.  The result does not depend on
         `user_block`."""
         users = _i64c(users, self.device)
         sums, pu = self.metric_sums(U_all, users, cutoffs, truth_rowptr, truth_col, mask_rowptr, mask_col,
-                                    user_block, per_user)
+                                    user_block, per_user, probe_users)
         return metric_means(sums.cpu().numpy(), users.numel(), pu)
 
 

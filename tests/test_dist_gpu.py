@@ -228,9 +228,9 @@ def _train_worker(rank, world, port, q):
         from spex_b200 import metrics
         from spex_b200.graph import build_interaction_csr
         trp, tcol = build_interaction_csr(tu, ti, ds.n_users, ds.m_items)
-        mm = ev.recall_ndcg(users_all, trp, tcol)
+        mm = ev.evaluate(users_all, trp, tcol, [20])
         r1g, n1g = metrics.fullrank_recall_ndcg(i_ref.cpu().numpy(), trp, tcol, 20)
-        res["eval"] = (same, abs(mm["recall"] - float(r1g.mean())), abs(mm["ndcg"] - float(n1g.mean())))
+        res["eval"] = (same, abs(mm["recall"][0] - float(r1g.mean())), abs(mm["ndcg"][0] - float(n1g.mean())))
         q.put((rank, res))
     finally:
         dist.destroy_process_group()

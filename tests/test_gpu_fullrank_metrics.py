@@ -159,8 +159,8 @@ def test_sharded_evaluate_matches_recall_ndcg_and_test_fullrank(cuda_device, pre
     trp, tcol = graph.truth_csr(users, truth)
     users_d = torch.from_numpy(users).to(cuda_device)
     got = ev.evaluate(users_d, trp, tcol, [20])
-    ref = ev.recall_ndcg(users_d, trp, tcol)
-    assert got["users"] == ref["users"] == ds.n_users
+    ref = batch_test.test_fullrank(model, users, truth, k=20, precision=precision)
+    assert got["users"] == ds.n_users
     assert abs(got["recall"][0] - ref["recall"]) < 1e-12 and abs(got["ndcg"][0] - ref["ndcg"]) < 1e-12
     wide = [64, 100] if precision == "f16" else []          # f16 at k = 100: the wide kernel
     for cutoffs in ([10, 20, 50], wide):
@@ -286,11 +286,13 @@ def test_main_rec_fullrank_test_mode(tmp_path, capsys, monkeypatch):
     def spy(dataset, Recmodel, epoch, *a, **kw):
         out = orig(dataset, Recmodel, epoch, *a, **kw)
         # the reference at the same weights: the host metrics of test_fullrank on the scorer the evaluator picks
+        # (its probe samples all users; test_fullrank's, through rank_topk, the test users)
         au, ai = Recmodel.computer()
         users = np.fromiter(dataset.testRatings.keys(), np.int64)
-        prec = "f16" if ops.f16_filter_is_selective(au, ai, torch.arange(au.shape[0], device=au.device)) else "fp32"
+        ranker = ops.FullRanker(ai, ops.default_precision(ai.shape[1]), probe=True)
+        prec = ranker.scorer_for(max(batch_test.Ks), au, torch.arange(au.shape[0], device=au.device))
         if prec == "f16":
-            assert ops.f16_filter_is_selective(au, ai, torch.from_numpy(users).to(au.device))
+            assert ranker.scorer_for(max(batch_test.Ks), au, torch.from_numpy(users).to(au.device)) == "f16"
         seen.append([batch_test.test_fullrank(Recmodel, users, dataset.testRatings, k=K, precision=prec)
                      for K in batch_test.Ks])
         return out

@@ -351,7 +351,7 @@ def test_sharded_evaluator_k100_matches_test_fullrank(cuda_device):
     idx, _, _ = ev.rank_topk(torch.from_numpy(users).to(cuda_device))
     i_ref, _ = model.rank_topk(users, k=100)
     assert torch.equal(idx, i_ref)
-    got = ev.recall_ndcg(torch.from_numpy(users).to(cuda_device), trp, tcol)
+    got = ev.evaluate(torch.from_numpy(users).to(cuda_device), trp, tcol, [100])
     ref = batch_test.test_fullrank(model, users, truth, k=100, precision="f16")
     assert got["users"] == ds.n_users
-    assert abs(got["recall"] - ref["recall"]) < 1e-12 and abs(got["ndcg"] - ref["ndcg"]) < 1e-12, (got, ref)
+    assert abs(got["recall"][0] - ref["recall"]) < 1e-12 and abs(got["ndcg"][0] - ref["ndcg"]) < 1e-12, (got, ref)
