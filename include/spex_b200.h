@@ -434,6 +434,37 @@ int spex_score_topk_f16_wide(const void* Uh, const void* Ih, int32_t D, int64_t 
                              void* work, int64_t work_bytes, void* stream);
 
 /*
+ * Full-ranking rank of held-out pairs.  Pair p = (user u_p, item t_p); its rank is
+ *   r_p = #{ i in [0, m_items) : i not in mask row of u_p, i != t_p, s(u_p, i) > s(u_p, t_p)
+ *                                or (s(u_p, i) == s(u_p, t_p) and i < t_p) }
+ * with s the exact score of the precision: the position of t_p in that precision's top-k list when it is there,
+ * >= k otherwise; t_p may be masked (its rank is still defined).  A mask row may repeat an id (it is
+ * excluded once).  out_rank int32 [P], in pair order; one store per
+ * pair, no atomics: the same inputs give the same bits.  Item ids must lie in [0, m_items) (not checked here).
+ *
+ * spex_rank_pairs_f16 (D == 64 or 128): s = the fp32 FMA chain over the fp16 operands of spex_score_topk_f16.  Uh is
+ * a table packed by spex_pack_f16 (the users' rows, any order), a_rows int64 [P] the row of Uh of each pair (NULL:
+ * row p); Ih / i_meta the packed item table; user_ids int64 [P] the mask row of each pair (NULL: row p); mask as
+ * spex_score_topk_f16.  P_pad >= P and m_pad are multiples of 128.  The tensor core computes the fp16 filter
+ * value of every (pair, item); only items within the filter's error bound of s(u_p, t_p) are re-scored exactly.
+ * Errors, before anything is launched: SPEX_E_BADDIM for D not 64 or 128; SPEX_E_BADARG for P_pad or m_pad not a
+ * multiple of 128, half a mask, NULL operands, items or out_rank, m_items == 0 with P > 0; SPEX_E_TOOBIG for
+ * m_pad >= 2^31; SPEX_E_ALIGN for Uh or Ih misaligned.
+ *
+ * spex_rank_pairs_f32 (D a multiple of 4, <= 512): s = the dot product of spex_score_topk_f32 in its accumulation
+ * order, over U [.., D] / I [m_items, D] fp32; users int64 [P] are the rows of U and the mask rows.
+ * Errors, before anything is launched: SPEX_E_BADDIM for D; SPEX_E_BADARG for half a mask, NULL operands, users,
+ * items or out_rank, m_items == 0 with P > 0; SPEX_E_TOOBIG for m_items >= 2^31; SPEX_E_ALIGN for U or I.
+ */
+int spex_rank_pairs_f16(const void* Uh, const void* Ih, int32_t D, const int64_t* a_rows,
+                        const int64_t* user_ids, const int32_t* items, int64_t P, int64_t P_pad,
+                        int64_t m_items, int64_t m_pad, const float* i_meta, const int64_t* mask_rowptr,
+                        const int32_t* mask_col, int32_t* out_rank, void* stream);
+int spex_rank_pairs_f32(const float* U, const float* I, int32_t D, const int64_t* users,
+                        const int32_t* items, int64_t P, int64_t m_items, const int64_t* mask_rowptr,
+                        const int32_t* mask_col, int32_t* out_rank, void* stream);
+
+/*
  * Sampled-candidate scoring for the reference Test() (batch_test.py:28-40, hoisted):
  *   score[u,c] = <U[users[u]], I[cand[u,c]]>,  cand int32 [n_u, n_c]  ->  score fp32 [n_u, n_c]
  */
@@ -475,6 +506,34 @@ int spex_fullrank_metrics(const int32_t* topk_idx, int64_t B, int32_t k,
                           double* per_user, double* chunk_sums, void* stream);
 int spex_fullrank_metrics_reduce(const double* chunk_sums, int64_t n_chunks, int32_t n_cut,
                                  double* sums, void* stream);
+
+/*
+ * The same metrics from the ranks of the held-out items (spex_rank_pairs_*) instead of top-k lists, at cutoffs up
+ * to m_items, plus MRR and AUC.  ranks int32 is aligned with truth_col: ranks[j] is the rank of truth_col[j] for
+ * its user.  A held-out item in the user's mask row, or a repeat of the item before it in its truth row, is never a
+ * hit, as in spex_fullrank_metrics, where it cannot appear in a list.  For user u with truth row T:
+ *   hits, recall, precision, hit, ndcg as spex_fullrank_metrics with "rank < K" for "in topk[:K]"; the DCG sums
+ *               disc[r] over the hit ranks in ascending r (the same bits as the top-k path);
+ *               disc fp64 [max cutoff], idcg fp64 [max cutoff + 1] as there
+ *   mrr       = 1 / (1 + min r) over the hits at any rank (0 when there is none)
+ *   auc       = mean over the entries t of T of 1 - (r_t - #{live t' : r_t' < r_t}) / n_neg, n_neg = m_items -
+ *               #{distinct ids of the mask row in [0, m_items)} - #{live t'}; a masked entry contributes 0;
+ *               n_neg == 0 gives 1 (no negative outranks t)
+ * (live = not masked and not a repeat; an empty truth row contributes zeros).  users int64 [B] gives each
+ * position's mask row (needed only with a mask).  chunk_sums fp64 [n_chunks, n_cut, 4] as spex_fullrank_metrics,
+ * chunk_extra fp64 [n_chunks, 4] = (mrr, auc, 0, 0) sums per chunk: both go through spex_fullrank_metrics_reduce
+ * (chunk_extra with n_cut = 1).  No atomics.  One warp per user; a user with T held-out items costs O(T^2 / 32)
+ * steps (each entry is compared with every other, and the hit walk scans the row once per hit), which suits
+ * leave-one-out and short truth rows, not rows of thousands of items.
+ * Errors, before anything is launched: SPEX_E_TOOBIG for n_cut > 8 or m_items >= 2^31; SPEX_E_BADARG for B < 0,
+ * m_items < 1, n_cut < 1, cutoffs not strictly ascending or outside [1, m_items], half a mask, NULL cutoffs, disc or
+ * idcg and (B > 0) NULL ranks, truth, sums or (with a mask) users.
+ */
+int spex_rank_metrics(const int32_t* ranks, int64_t B, const int64_t* truth_rowptr,
+                      const int32_t* truth_col, const int64_t* users, const int64_t* mask_rowptr,
+                      const int32_t* mask_col, int64_t m_items, const int32_t* cutoffs_host,
+                      int32_t n_cut, const double* disc, const double* idcg, double* chunk_sums,
+                      double* chunk_extra, void* stream);
 
 /*
  * NGCF layer epilogue (configs[2], NGCF_SPEX/code/main_rec.py:76-85), D == 64:

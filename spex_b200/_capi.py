@@ -86,9 +86,12 @@ SIGNATURES = {
     "spex_score_topk_f16_wide_workspace_bytes": (_i64, [_i64, _i32]),
     "spex_score_topk_f16_wide": (C.c_int, [_p, _p, _i32, _i64, _i64, _i64, _i64, _p, _p, _p, _p, _p, _i32, _p, _p, _p,
                                            _i64, _p]),
+    "spex_rank_pairs_f16": (C.c_int, [_p, _p, _i32, _p, _p, _p, _i64, _i64, _i64, _i64, _p, _p, _p, _p, _p]),
+    "spex_rank_pairs_f32": (C.c_int, [_p, _p, _i32, _p, _p, _i64, _i64, _p, _p, _p, _p]),
     "spex_score_candidates_f32": (C.c_int, [_p, _p, _i32, _p, _p, _i64, _i32, _p, _p]),
     "spex_fullrank_metrics": (C.c_int, [_p, _i64, _i32, _p, _p, _p, _i32, _p, _p, _p, _p, _p]),
     "spex_fullrank_metrics_reduce": (C.c_int, [_p, _i64, _i32, _p, _p]),
+    "spex_rank_metrics": (C.c_int, [_p, _i64, _p, _p, _p, _p, _p, _i64, _p, _i32, _p, _p, _p, _p, _p]),
     "spex_ngcf_epilogue_f32": (C.c_int, [_p, _p, _p, _p, _p, _p, _i64, _i32, _f, _p, _p, _i64, _p]),
     "spex_ngcf_layer_fwd_f32": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _i64, _i32, _f, _p, _p, _i64, _p]),
     "spex_ngcf_layer_bwd_f32": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _i64, _i32, _f, _p, _p, _p, _p,

@@ -120,9 +120,154 @@ fullrank_metrics_reduce_kernel(const double* __restrict__ chunk_sums, int64_t n_
   sums[l] = s;
 }
 
+// Metrics from the ranks of the held-out items (spex_rank_pairs_*), one warp per user, chunks and summation order
+// as fullrank_metrics_kernel: the hit ranks are walked in ascending order by a warp minimum per step, so the DCG
+// is summed in the order the top-k path sums it.  A held-out item in the user's mask, or a repeat of the previous
+// item of its truth row, is never a hit (its effective rank is INT_MAX).  Lanes 0 and 1 of each warp also sum MRR
+// and AUC, into chunk_extra (mrr, auc, 0, 0) per chunk.
+__global__ void __launch_bounds__(kMetricsWarps * kWarp)
+rank_metrics_kernel(const int32_t* __restrict__ ranks, int64_t B, const int64_t* __restrict__ rowptr,
+                    const int32_t* __restrict__ tcol, const int64_t* __restrict__ users,
+                    const int64_t* __restrict__ mask_rowptr, const int32_t* __restrict__ mask_col, int64_t m_items,
+                    MetricsCutoffs cuts, int32_t n_cut, const double* __restrict__ disc,
+                    const double* __restrict__ idcg, double* __restrict__ chunk_sums,
+                    double* __restrict__ chunk_extra) {
+  __shared__ int32_t s_cut[SPEX_METRICS_MAX_CUTOFFS];
+  __shared__ double s_part[kMetricsWarps][kWarp];
+  __shared__ double s_extra[kMetricsWarps][2];
+  if (threadIdx.x < SPEX_METRICS_MAX_CUTOFFS) s_cut[threadIdx.x] = cuts.c[threadIdx.x];
+  __syncthreads();
+  const int lane = threadIdx.x & (kWarp - 1);
+  const int warp = threadIdx.x >> 5;
+  const int nv = n_cut * 4;
+  const int my_c = lane >> 2, my_m = lane & 3;
+  const int my_K = s_cut[my_c < n_cut ? my_c : 0];
+  const int Kmax = s_cut[n_cut - 1];
+  const int64_t u0 = (int64_t)blockIdx.x * SPEX_METRICS_CHUNK + warp * kUsersPerWarp;
+  double sum = 0.0, extra = 0.0;
+  for (int t = 0; t < kUsersPerWarp; ++t) {
+    const int64_t u = u0 + t;
+    if (u >= B) break;
+    const int64_t lo = __ldg(rowptr + u), hi = __ldg(rowptr + u + 1);
+    int64_t mlo = 0, mhi = 0;
+    if (mask_rowptr) {
+      const int64_t uid = users[u];
+      mlo = __ldg(mask_rowptr + uid);
+      mhi = __ldg(mask_rowptr + uid + 1);
+    }
+    auto masked = [&](int64_t j) { return mask_rowptr && truth_has(mask_col, mlo, mhi, __ldg(tcol + j)); };
+    // effective rank: INT_MAX for a masked item or a repeat
+    auto eff = [&](int64_t j) {
+      const bool rep = j > lo && __ldg(tcol + j) == __ldg(tcol + j - 1);
+      return (rep || masked(j)) ? INT_MAX : __ldg(ranks + j);
+    };
+    int e_min = INT_MAX, n_live = 0;
+    for (int64_t j = lo + lane; j < hi; j += kWarp) {
+      const int e = eff(j);
+      e_min = min(e_min, e);
+      n_live += e != INT_MAX ? 1 : 0;
+    }
+    e_min = __reduce_min_sync(kFull, e_min);
+    n_live = (int)__reduce_add_sync(kFull, (unsigned)n_live);
+    double acc = 0.0, my_dcg = 0.0;
+    int h = 0, c = 0, my_h = 0, prev = -1, next = e_min;
+    while (next < Kmax) {
+      for (; c < n_cut && next >= s_cut[c]; ++c)
+        if (c == my_c) my_h = h, my_dcg = acc;
+      acc += __ldg(disc + next);
+      ++h;
+      prev = next;
+      int nx = INT_MAX;
+      for (int64_t j = lo + lane; j < hi; j += kWarp) {
+        const int e = eff(j);
+        if (e > prev && e < nx) nx = e;
+      }
+      next = __reduce_min_sync(kFull, nx);
+    }
+    for (; c < n_cut; ++c)
+      if (c == my_c) my_h = h, my_dcg = acc;
+    const int64_t T = hi - lo;
+    if (lane < nv) {
+      double v;
+      if (my_m == 0) {
+        v = T > 0 ? (double)my_h / (double)T : 0.0;
+      } else if (my_m == 1) {
+        v = (double)my_h / (double)my_K;
+      } else if (my_m == 2) {
+        const double id = __ldg(idcg + (T < my_K ? T : (int64_t)my_K));
+        v = id > 0.0 ? my_dcg / id : 0.0;
+      } else {
+        v = my_h > 0 ? 1.0 : 0.0;
+      }
+      sum += v;
+    }
+    // AUC of each held-out item: 1 - (negatives above it) / n_neg, negatives = items outside mask and truth
+    int n_mask = 0;                                     // distinct mask ids in [0, m_items): a repeat counts once
+    for (int64_t k = mlo + lane; k < mhi; k += kWarp) {
+      const int32_t id = __ldg(mask_col + k);
+      n_mask += (id >= 0 && id < m_items && (k == mlo || __ldg(mask_col + k - 1) != id)) ? 1 : 0;
+    }
+    n_mask = (int)__reduce_add_sync(kFull, (unsigned)n_mask);
+    const int64_t n_neg = m_items - n_mask - n_live;
+    double auc = 0.0;
+    for (int64_t j = lo + lane; j < hi; j += kWarp) {
+      if (masked(j)) continue;
+      const int r = __ldg(ranks + j);
+      int above = 0;
+      for (int64_t j2 = lo; j2 < hi; ++j2) above += eff(j2) < r ? 1 : 0;
+      auc += n_neg > 0 ? 1.0 - (double)(r - above) / (double)n_neg : 1.0;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) auc += __shfl_xor_sync(kFull, auc, o);
+    if (lane == 0) extra += e_min != INT_MAX ? 1.0 / (1.0 + (double)e_min) : 0.0;
+    if (lane == 1) extra += T > 0 ? auc / (double)T : 0.0;
+  }
+  s_part[warp][lane] = sum;
+  if (lane < 2) s_extra[warp][lane] = extra;
+  __syncthreads();
+  if (threadIdx.x < nv) {
+    double s = 0.0;
+#pragma unroll
+    for (int w = 0; w < kMetricsWarps; ++w) s += s_part[w][threadIdx.x];
+    chunk_sums[(int64_t)blockIdx.x * nv + threadIdx.x] = s;
+  }
+  if (threadIdx.x < 4) {
+    double s = 0.0;
+    if (threadIdx.x < 2)
+      for (int w = 0; w < kMetricsWarps; ++w) s += s_extra[w][threadIdx.x];
+    chunk_extra[(int64_t)blockIdx.x * 4 + threadIdx.x] = s;
+  }
+}
+
 }  // namespace spex
 
 using namespace spex;
+
+extern "C" int spex_rank_metrics(const int32_t* ranks, int64_t B, const int64_t* truth_rowptr,
+                                 const int32_t* truth_col, const int64_t* users, const int64_t* mask_rowptr,
+                                 const int32_t* mask_col, int64_t m_items, const int32_t* cutoffs_host, int32_t n_cut,
+                                 const double* disc, const double* idcg, double* chunk_sums, double* chunk_extra,
+                                 void* stream) {
+  SPEX_RETURN_IF(n_cut > SPEX_METRICS_MAX_CUTOFFS || m_items > 0x7fffffffLL, SPEX_E_TOOBIG);
+  SPEX_RETURN_IF(B < 0 || m_items < 1 || n_cut < 1 || !cutoffs_host || !disc || !idcg, SPEX_E_BADARG);
+  SPEX_RETURN_IF((mask_rowptr == nullptr) != (mask_col == nullptr), SPEX_E_BADARG);
+  MetricsCutoffs cuts = {};
+  for (int i = 0; i < n_cut; ++i) {
+    const int32_t K = cutoffs_host[i];
+    SPEX_RETURN_IF(K < 1 || K > m_items || (i > 0 && K <= cutoffs_host[i - 1]), SPEX_E_BADARG);
+    cuts.c[i] = K;
+  }
+  if (B == 0) return 0;
+  SPEX_RETURN_IF(!ranks || !truth_rowptr || !truth_col || !chunk_sums || !chunk_extra ||
+                     (mask_rowptr && !users),
+                 SPEX_E_BADARG);
+  const int64_t n_chunks = (B + SPEX_METRICS_CHUNK - 1) / SPEX_METRICS_CHUNK;
+  rank_metrics_kernel<<<(unsigned)n_chunks, kMetricsWarps * kWarp, 0, (cudaStream_t)stream>>>(
+      ranks, B, truth_rowptr, truth_col, users, mask_rowptr, mask_col, m_items, cuts, n_cut, disc, idcg, chunk_sums,
+      chunk_extra);
+  count_launch();
+  return check_last();
+}
 
 extern "C" int spex_fullrank_metrics(const int32_t* topk_idx, int64_t B, int32_t k, const int64_t* truth_rowptr,
                                      const int32_t* truth_col, const int32_t* cutoffs_host, int32_t n_cut,

@@ -820,6 +820,221 @@ static int launch_k(const void* Uh, const void* Ih, int64_t B, int64_t B_pad, in
   return launch<DK, 3>(Uh, Ih, B, B_pad, m_items, m_pad, u_meta, i_meta, user_ids, mask_rowptr, mask_col, k, out_idx, out_val, nullptr, 0, st);
 }
 
+// ---- rank of held-out pairs -----------------------------------------------------------------------------------
+// Row p of a launch is the pair (user row a_rows[p] of Uh, item items[p]); its rank is the number of items
+// i != t, i < m, outside the user's mask row, with exact score s_i above s_t under (score desc, id asc).
+// The epilogue thread of the row computes s_t = exact_score(row, t) and the row's filter margin eps as the
+// top-k kernel does; with |f - s| <= eps (header comment) every item whose fp16 filter value f is above
+// hi = RU(s_t + eps) is above t, every item below lo = RD(s_t - eps) is below, and only the band [lo, hi] is
+// re-scored exactly.  Per tile: a warp-wide reject when every lane's max is below lo, a lane-wide accept when
+// its min is above hi, else two packed compares per register summed in fp16 (integers <= 64: exact).  The
+// masked items above t are subtracted after the sweep, re-scored exactly: the sweep's count is exact, so the
+// subtraction is too.  Counts live in registers; one store per pair.
+__device__ __forceinline__ uint32_t hmin2(uint32_t a, uint32_t b) {
+  uint32_t d;
+  asm("min.f16x2 %0, %1, %2;" : "=r"(d) : "r"(a), "r"(b));
+  return d;
+}
+__device__ __forceinline__ __half2 as_h2(uint32_t x) { return *reinterpret_cast<const __half2*>(&x); }
+
+template <int DK>
+__global__ void __launch_bounds__(kThreads, DK == 64 ? 2 : 1)
+rank_pairs_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict__ Ih, int64_t P, int m_items,
+                      int n_item_tiles, const float* __restrict__ i_meta, const int64_t* __restrict__ a_rows,
+                      const int64_t* __restrict__ user_ids, const int32_t* __restrict__ items,
+                      const int64_t* __restrict__ mask_rowptr, const int32_t* __restrict__ mask_col,
+                      int32_t* __restrict__ out_rank, int stages) {
+  constexpr int A_BYTES = BM * DK * 2;
+  extern __shared__ uint8_t smem_raw[];
+  __shared__ __align__(8) uint64_t bar_full[kMaxStages];
+  __shared__ __align__(8) uint64_t bar_empty[kMaxStages];
+  __shared__ __align__(8) uint64_t bar_tfull[2];
+  __shared__ __align__(8) uint64_t bar_tempty[2];
+  __shared__ __align__(8) uint64_t bar_a;
+  __shared__ uint32_t tmem_slot;
+
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 127) & ~(uintptr_t)127);
+  uint8_t* sA = smem;                 // [128 pairs][DK] fp16, gathered by the epilogue
+  uint8_t* sB = smem + A_BYTES;       // stages x [128 items][DK]
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int64_t tile_m = blockIdx.x;
+  const uint32_t tmem_base =
+      pipeline_init(warp, stages, bar_full, bar_empty, bar_tfull, bar_tempty, &bar_a, &tmem_slot);
+
+  if (warp == 0) {
+    if (elect_one()) produce_item_tiles<DK>(Ih, n_item_tiles, stages, sB, bar_full, bar_empty);
+  } else if (warp == 1) {
+    constexpr uint32_t idesc = ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);   // as the top-k kernel
+    mma_role<DK>(idesc, sA, sB, tmem_base, n_item_tiles, stages, bar_full, bar_empty, bar_tfull, bar_tempty, &bar_a);
+  } else {
+    const int q = warp & 3;
+    const int row = q * 32 + lane;
+    const int64_t grow = tile_m * BM + row;
+    const bool live = grow < P;
+    // gather this pair's user row into the A tile (zeros past P), then publish the tile to the tensor core
+    uint8_t* a_row = sA + (size_t)(row >> 3) * (16 * DK) + (size_t)(row & 7) * 16;
+    {
+      const int64_t ur = live ? (a_rows ? a_rows[grow] : grow) : 0;
+      const uint8_t* src = Uh + (size_t)(ur >> 3) * (16 * DK) + (size_t)(ur & 7) * 16;
+#pragma unroll
+      for (int kc = 0; kc < DK / 8; ++kc)
+        *reinterpret_cast<uint4*>(a_row + kc * 128) =
+            live ? __ldg(reinterpret_cast<const uint4*>(src + kc * 128)) : make_uint4(0u, 0u, 0u, 0u);
+    }
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    asm volatile("bar.sync 1, 128;" ::: "memory");   // the four epilogue warps
+    if (row == 0) mbar_arrive(&bar_a);
+    float un2 = 0.f;
+#pragma unroll
+    for (int kc = 0; kc < DK / 8; ++kc) {
+      const uint4 a = *reinterpret_cast<const uint4*>(a_row + kc * 128);
+      const uint32_t aw[4] = {a.x, a.y, a.z, a.w};
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&aw[j]));
+        un2 = fmaf(f.x, f.x, un2);
+        un2 = fmaf(f.y, f.y, un2);
+      }
+    }
+    const float eps = kEpsRel<DK> * sqrtf(un2) * i_meta[2] * 1.0001f + kEpsAbs;
+    const int tid = live ? items[grow] : -1;
+    const float st = live ? exact_score<DK>(a_row, Ih, tid) : 0.f;
+    // padded rows: lo = hi = +inf, nothing is counted
+    const __half lo = live ? __float2half_rd(__fsub_rd(st, eps)) : __ushort_as_half((unsigned short)0x7c00u);
+    const __half hi = live ? __float2half_ru(__fadd_ru(st, eps)) : __ushort_as_half((unsigned short)0x7c00u);
+    const __half2 lo2 = __half2half2(lo), hi2 = __half2half2(hi);
+    int cnt = 0;
+    const uint32_t tq = tmem_base + ((uint32_t)(q * 32) << 16);
+    uint32_t r[64];
+    for (int t = 0; t < n_item_tiles; ++t) {
+      const int buf = t & 1;
+      mbar_wait(&bar_tfull[buf], (uint32_t)(t >> 1) & 1u);
+      tc_fence_after();
+      __syncwarp();
+      tmem_ld128h_issue(tq + (uint32_t)(buf * BN), r);
+      tmem_wait64(r);
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&bar_tempty[buf]);
+      uint32_t mx[8];
+#pragma unroll
+      for (int b = 0; b < 8; ++b) {
+        mx[b] = r[8 * b];
+#pragma unroll
+        for (int i = 1; i < 8; ++i) mx[b] = hmax2(mx[b], r[8 * b + i]);
+      }
+      const uint32_t mm = hmax2(hmax2(hmax2(mx[0], mx[1]), hmax2(mx[2], mx[3])),
+                                hmax2(hmax2(mx[4], mx[5]), hmax2(mx[6], mx[7])));
+      const bool any_ge = __hge(__hmax(lo_half(mm), hi_half(mm)), lo);
+      if (!__any_sync(kFull, any_ge)) continue;           // every lane: the whole tile is below t
+      if (!any_ge) continue;
+      const int id0 = t * BN;
+      const bool full = id0 + BN <= m_items;
+      uint32_t mn[8];
+#pragma unroll
+      for (int b = 0; b < 8; ++b) {
+        mn[b] = r[8 * b];
+#pragma unroll
+        for (int i = 1; i < 8; ++i) mn[b] = hmin2(mn[b], r[8 * b + i]);
+      }
+      const uint32_t nn = hmin2(hmin2(hmin2(mn[0], mn[1]), hmin2(mn[2], mn[3])),
+                                hmin2(hmin2(mn[4], mn[5]), hmin2(mn[6], mn[7])));
+      if (full && __hgt(__hmin(lo_half(nn), hi_half(nn)), hi)) {
+        cnt += BN;                                        // the whole tile is above t (t itself is in the band)
+        continue;
+      }
+      // per column: [f > hi] and [f >= lo], summed in fp16 over four independent chains
+      __half2 c_hi[4], c_lo[4];
+#pragma unroll
+      for (int c = 0; c < 4; ++c) c_hi[c] = c_lo[c] = __float2half2_rn(0.f);
+#pragma unroll
+      for (int i = 0; i < 64; ++i) {
+        c_hi[i & 3] = __hadd2(c_hi[i & 3], __hgt2(as_h2(r[i]), hi2));
+        c_lo[i & 3] = __hadd2(c_lo[i & 3], __hge2(as_h2(r[i]), lo2));
+      }
+      const __half2 s_hi = __hadd2(__hadd2(c_hi[0], c_hi[1]), __hadd2(c_hi[2], c_hi[3]));
+      const __half2 s_lo = __hadd2(__hadd2(c_lo[0], c_lo[1]), __hadd2(c_lo[2], c_lo[3]));
+      const int n_hi = (int)__half2float(__hadd(__low2half(s_hi), __high2half(s_hi)));
+      const int n_lo = (int)__half2float(__hadd(__low2half(s_lo), __high2half(s_lo)));
+      if (full && n_lo == n_hi) {
+        cnt += n_hi;                                      // no column in the band
+        continue;
+      }
+      // band columns (or the zero-padded last tile): 16 columns at a time, exact re-score of the band
+#pragma unroll 1
+      for (int bi = 0; bi < 8; ++bi) {
+        uint32_t p0, p1, p2, p3, p4, p5, p6, p7;
+#define SPEX_PICK(b)                                                                                   \
+  case b:                                                                                              \
+    p0 = r[8 * b]; p1 = r[8 * b + 1]; p2 = r[8 * b + 2]; p3 = r[8 * b + 3];                             \
+    p4 = r[8 * b + 4]; p5 = r[8 * b + 5]; p6 = r[8 * b + 6]; p7 = r[8 * b + 7];                         \
+    break;
+        switch (bi) {
+          SPEX_PICK(0) SPEX_PICK(1) SPEX_PICK(2) SPEX_PICK(3) SPEX_PICK(4) SPEX_PICK(5) SPEX_PICK(6)
+          default: SPEX_PICK(7)
+        }
+#undef SPEX_PICK
+        const uint32_t p[8] = {p0, p1, p2, p3, p4, p5, p6, p7};
+        const int b0 = id0 + bi * 16;
+        const unsigned valid = (b0 + 16 <= m_items) ? 0xffffu : (b0 < m_items ? (1u << (m_items - b0)) - 1u : 0u);
+        unsigned above = 0, band = 0;
+#pragma unroll
+        for (int j = 0; j < 16; ++j) {
+          const __half a = (j & 1) ? hi_half(p[j >> 1]) : lo_half(p[j >> 1]);
+          above |= __hgt(a, hi) ? (1u << j) : 0u;
+          band |= __hge(a, lo) ? (1u << j) : 0u;
+        }
+        above &= valid;
+        band &= valid & ~above;
+        cnt += __popc(above);
+#pragma unroll 1
+        while (band) {
+          const int id = b0 + __ffs(band) - 1;
+          band &= band - 1;
+          if (id != tid && beats(exact_score<DK>(a_row, Ih, id), id, st, tid)) ++cnt;
+        }
+      }
+    }
+    if (live) {
+      if (mask_rowptr) {
+        const int64_t uid = user_ids ? user_ids[grow] : grow;
+        const int64_t e = mask_rowptr[uid + 1];
+        int prev = -1;                                    // a repeated mask id is subtracted once
+        for (int64_t c = mask_rowptr[uid]; c < e; ++c) {
+          const int id = __ldg(mask_col + c);
+          if (id != prev && id != tid && id >= 0 && id < m_items &&
+              beats(exact_score<DK>(a_row, Ih, id), id, st, tid))
+            --cnt;
+          prev = id;
+        }
+      }
+      out_rank[grow] = cnt;
+    }
+  }
+  pipeline_teardown(warp, tmem_base);
+}
+
+template <int DK>
+static int launch_rank(const void* Uh, const void* Ih, int64_t P, int64_t P_pad, int64_t m_items, int64_t m_pad,
+                       const float* i_meta, const int64_t* a_rows, const int64_t* user_ids, const int32_t* items,
+                       const int64_t* mask_rowptr, const int32_t* mask_col, int32_t* out_rank, cudaStream_t st) {
+  // no candidate buffers: the ring takes kMaxStages stages at both D, with two CTAs per SM at D = 64 (80 KB each)
+  // and one at D = 128 (160 KB), the occupancy of the top-k kernel
+  const int stages = choose_stages(DK, 0, (DK == 64) ? 115712 - 7600 : 227 * 1024 - 7600);
+  const size_t smem = smem_bytes(DK, 0, stages);
+  cudaError_t e = cudaFuncSetAttribute(rank_pairs_f16_kernel<DK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)smem);
+  if (e != cudaSuccess) return (int)e;
+  const int64_t grid = P_pad / BM;
+  SPEX_RETURN_IF(grid > 0x7fffffffLL, SPEX_E_TOOBIG);
+  rank_pairs_f16_kernel<DK><<<(unsigned)grid, kThreads, smem, st>>>(
+      (const uint8_t*)Uh, (const uint8_t*)Ih, P, (int)m_items, (int)(m_pad / BN), i_meta, a_rows, user_ids, items,
+      mask_rowptr, mask_col, out_rank, stages);
+  count_launch();
+  return check_last();
+}
+
 }  // namespace tf
 }  // namespace spex
 
@@ -871,6 +1086,27 @@ extern "C" int spex_score_topk_f16(const void* Uh, const void* Ih, int32_t D, in
   if (D == 64)
     return tf::launch_k<64>(Uh, Ih, B, B_pad, m_items, m_pad, u_meta, i_meta, user_ids, mask_rowptr, mask_col, k, out_idx, out_val, st);
   return tf::launch_k<128>(Uh, Ih, B, B_pad, m_items, m_pad, u_meta, i_meta, user_ids, mask_rowptr, mask_col, k, out_idx, out_val, st);
+}
+
+extern "C" int spex_rank_pairs_f16(const void* Uh, const void* Ih, int32_t D, const int64_t* a_rows,
+                                   const int64_t* user_ids, const int32_t* items, int64_t P, int64_t P_pad,
+                                   int64_t m_items, int64_t m_pad, const float* i_meta, const int64_t* mask_rowptr,
+                                   const int32_t* mask_col, int32_t* out_rank, void* stream) {
+  SPEX_RETURN_IF(D != 64 && D != 128, SPEX_E_BADDIM);
+  SPEX_RETURN_IF(!Uh || !Ih || !i_meta || !items || !out_rank || P < 0 || P_pad < P || m_items < 0 ||
+                     m_pad < m_items || (P > 0 && m_items == 0),
+                 SPEX_E_BADARG);
+  SPEX_RETURN_IF((P_pad % tf::BM) || (m_pad % tf::BN), SPEX_E_BADARG);
+  SPEX_RETURN_IF((mask_rowptr == nullptr) != (mask_col == nullptr), SPEX_E_BADARG);
+  SPEX_RETURN_IF(m_pad > 0x7fffffffLL, SPEX_E_TOOBIG);
+  SPEX_RETURN_IF(!aligned16(Uh) || !aligned16(Ih), SPEX_E_ALIGN);
+  if (P == 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (D == 64)
+    return tf::launch_rank<64>(Uh, Ih, P, P_pad, m_items, m_pad, i_meta, a_rows, user_ids, items, mask_rowptr,
+                               mask_col, out_rank, st);
+  return tf::launch_rank<128>(Uh, Ih, P, P_pad, m_items, m_pad, i_meta, a_rows, user_ids, items, mask_rowptr,
+                              mask_col, out_rank, st);
 }
 
 extern "C" int64_t spex_score_topk_f16_wide_workspace_bytes(int64_t B_pad, int32_t k) {

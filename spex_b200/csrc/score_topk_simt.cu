@@ -154,9 +154,133 @@ rating_dense_kernel(const float* __restrict__ U, const float* __restrict__ I, in
   }
 }
 
+// Rank of held-out pairs, exact fp32: CTA = TU pairs, items streamed through the threads as in the top-k kernel
+// above, with the same FMA chain (item element times user element, d ascending), so a pair's rank is the
+// position of its item in the fp32 top-k list bit for bit.  Each thread counts, per pair, the items it scored
+// that beat the held-out item t (score desc, id asc; t itself excluded) and un-counts the masked items of the
+// user that beat it; the counts are reduced per pair in a fixed order (integers: order-free anyway).
+__device__ __forceinline__ float dot_f32(const float* __restrict__ item_row, const float* su_row, int D4) {
+  const float4* row = reinterpret_cast<const float4*>(item_row);
+  float acc = 0.f;
+#pragma unroll 4
+  for (int d4 = 0; d4 < D4; ++d4) {
+    const float4 x = __ldg(row + d4);
+    const float4 w = *reinterpret_cast<const float4*>(su_row + d4 * 4);
+    acc = fmaf(x.x, w.x, acc);
+    acc = fmaf(x.y, w.y, acc);
+    acc = fmaf(x.z, w.z, acc);
+    acc = fmaf(x.w, w.w, acc);
+  }
+  return acc;
+}
+
+__global__ void __launch_bounds__(TILE)
+rank_pairs_f32_kernel(const float* __restrict__ U, const float* __restrict__ I, int D,
+                      const int64_t* __restrict__ users, const int32_t* __restrict__ items, int64_t P,
+                      int64_t m_items, const int64_t* __restrict__ mask_rowptr, const int32_t* __restrict__ mask_col,
+                      int32_t* __restrict__ out_rank) {
+  extern __shared__ __align__(16) float smem[];
+  float* su = smem;                                   // [TU][D]
+  __shared__ float s_st[TU];
+  __shared__ int s_t[TU];
+  __shared__ int part[TILE / 32][TU];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int64_t p0 = (int64_t)blockIdx.x * TU;
+  const int np = (int)((P - p0) < TU ? (P - p0) : TU);
+  for (int i = tid; i < TU * D; i += TILE) {
+    const int u = i / D, d = i - u * D;
+    su[i] = (u < np) ? U[users[p0 + u] * D + d] : 0.f;
+  }
+  __syncthreads();
+  const int D4 = D >> 2;
+  if (tid < TU) {
+    const int t = tid < np ? items[p0 + tid] : -1;
+    s_t[tid] = t;
+    s_st[tid] = t >= 0 ? dot_f32(I + (int64_t)t * D, su + tid * D, D4) : INFINITY;
+  }
+  __syncthreads();
+  float st[TU];
+  int tt[TU], cnt[TU];
+#pragma unroll
+  for (int u = 0; u < TU; ++u) {
+    st[u] = s_st[u];
+    tt[u] = s_t[u];
+    cnt[u] = 0;
+  }
+  for (int64_t j = tid; j < m_items; j += TILE) {
+    float acc[TU];
+#pragma unroll
+    for (int u = 0; u < TU; ++u) acc[u] = 0.f;
+    const float4* row = reinterpret_cast<const float4*>(I + j * D);
+#pragma unroll 4
+    for (int d4 = 0; d4 < D4; ++d4) {
+      const float4 x = __ldg(row + d4);
+#pragma unroll
+      for (int u = 0; u < TU; ++u) {
+        const float4 w = *reinterpret_cast<const float4*>(su + u * D + d4 * 4);
+        acc[u] = fmaf(x.x, w.x, acc[u]);
+        acc[u] = fmaf(x.y, w.y, acc[u]);
+        acc[u] = fmaf(x.z, w.z, acc[u]);
+        acc[u] = fmaf(x.w, w.w, acc[u]);
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < TU; ++u) cnt[u] += ((int)j != tt[u] && beats(acc[u], (int)j, st[u], tt[u])) ? 1 : 0;
+  }
+#pragma unroll
+  for (int u = 0; u < TU; ++u) {
+    const int c = (int)__reduce_add_sync(kFull, (unsigned)cnt[u]);
+    if (lane == 0) part[warp][u] = c;
+  }
+  if (mask_rowptr) {
+    for (int u = 0; u < np; ++u) {
+      const int64_t uid = users[p0 + u];
+      const int64_t e = mask_rowptr[uid + 1];
+      const int t = s_t[u];
+      const float s = s_st[u];
+      int c = 0;
+      const int64_t b = mask_rowptr[uid];
+      for (int64_t k = b + tid; k < e; k += TILE) {
+        const int id = __ldg(mask_col + k);
+        const bool first = k == b || __ldg(mask_col + k - 1) != id;   // a repeated mask id is subtracted once
+        if (first && id != t && id >= 0 && id < m_items &&
+            beats(dot_f32(I + (int64_t)id * D, su + u * D, D4), id, s, t))
+          ++c;
+      }
+      c = (int)__reduce_add_sync(kFull, (unsigned)c);
+      if (lane == 0) part[warp][u] -= c;
+    }
+  }
+  __syncthreads();
+  if (tid < np) {
+    int c = 0;
+#pragma unroll
+    for (int w = 0; w < TILE / 32; ++w) c += part[w][tid];
+    out_rank[p0 + tid] = c;
+  }
+}
+
 }  // namespace spex
 
 using namespace spex;
+
+extern "C" int spex_rank_pairs_f32(const float* U, const float* I, int32_t D, const int64_t* users,
+                                   const int32_t* items, int64_t P, int64_t m_items, const int64_t* mask_rowptr,
+                                   const int32_t* mask_col, int32_t* out_rank, void* stream) {
+  SPEX_RETURN_IF(D <= 0 || (D & 3) || D > 512, SPEX_E_BADDIM);
+  SPEX_RETURN_IF(!U || !I || !users || !items || !out_rank || P < 0 || m_items < 0 || (P > 0 && m_items == 0),
+                 SPEX_E_BADARG);
+  SPEX_RETURN_IF((mask_rowptr == nullptr) != (mask_col == nullptr), SPEX_E_BADARG);
+  SPEX_RETURN_IF(m_items > 0x7fffffffLL, SPEX_E_TOOBIG);
+  SPEX_RETURN_IF(!aligned16(U) || !aligned16(I), SPEX_E_ALIGN);
+  if (P == 0) return 0;
+  const int64_t grid = (P + TU - 1) / TU;
+  SPEX_RETURN_IF(grid > 0x7fffffffLL, SPEX_E_TOOBIG);
+  rank_pairs_f32_kernel<<<(unsigned)grid, TILE, (size_t)TU * D * 4, (cudaStream_t)stream>>>(
+      U, I, D, users, items, P, m_items, mask_rowptr, mask_col, out_rank);
+  count_launch();
+  return check_last();
+}
 
 extern "C" int spex_score_topk_f32(const float* U, const float* I, int32_t D, const int64_t* users,
                                    int64_t B, int64_t m_items, const int64_t* mask_rowptr,

@@ -143,27 +143,35 @@ __device__ __forceinline__ uint32_t pipeline_init(int warp, int stages, uint64_t
   return *tmem_slot;
 }
 
+// Item half of the producer, run by the elected thread: every item tile through the ring.
+template <int DK>
+__device__ __forceinline__ void produce_item_tiles(const uint8_t* Ig, int n_item_tiles, int stages, uint8_t* sB,
+                                                   uint64_t* bar_full, uint64_t* bar_empty) {
+  constexpr int B_BYTES = BN * DK * 2;
+  int t = 0;
+  uint32_t ph = 0;
+  int s = 0;
+  for (; t < n_item_tiles; ++t) {
+    mbar_wait(&bar_empty[s], ph ^ 1u);
+    mbar_arrive_expect_tx(&bar_full[s], B_BYTES);
+    bulk_g2s(sB + (size_t)s * B_BYTES, Ig + (size_t)t * B_BYTES, B_BYTES, &bar_full[s]);
+    if (++s == stages) {
+      s = 0;
+      ph ^= 1u;
+    }
+  }
+}
+
 // Producer (warp 0): one thread streams the user tile `tile_m` once, then every item tile.
 template <int DK>
 __device__ __forceinline__ void producer_role(const uint8_t* Ug, const uint8_t* Ig, int64_t tile_m,
                                               int n_item_tiles, int stages, uint8_t* sA, uint8_t* sB,
                                               uint64_t* bar_full, uint64_t* bar_empty, uint64_t* bar_a) {
-  constexpr int A_BYTES = BM * DK * 2, B_BYTES = BN * DK * 2;
+  constexpr int A_BYTES = BM * DK * 2;
   if (elect_one()) {
     mbar_arrive_expect_tx(bar_a, A_BYTES);
     bulk_g2s(sA, Ug + tile_m * A_BYTES, A_BYTES, bar_a);
-    int t = 0;
-    uint32_t ph = 0;
-    int s = 0;
-    for (; t < n_item_tiles; ++t) {
-      mbar_wait(&bar_empty[s], ph ^ 1u);
-      mbar_arrive_expect_tx(&bar_full[s], B_BYTES);
-      bulk_g2s(sB + (size_t)s * B_BYTES, Ig + (size_t)t * B_BYTES, B_BYTES, &bar_full[s]);
-      if (++s == stages) {
-        s = 0;
-        ph ^= 1u;
-      }
-    }
+    produce_item_tiles<DK>(Ig, n_item_tiles, stages, sB, bar_full, bar_empty);
   }
 }
 

@@ -270,12 +270,27 @@ class LightGCN(BasicModel):
         mrp = mcol = None
         if exclude_train:
             mrp, mcol = self.train_mask_csr()
+        return self._full_ranker(all_items, precision, probe).topk(all_users, users, k, mrp, mcol, user_block)
+
+    @torch.no_grad()
+    def item_ranks(self, users, items, exclude_train: bool = True, precision: str = "f16", probe: bool = True):
+        """Full-ranking rank of item items[p] for user users[p] (int32 [P] on the device): its 0-based position in
+        rank_topk's order (score descending, ties by ascending id, the user's train items excluded when
+        exclude_train) among all items, however far down.  Same ranker, precisions and probe as rank_topk, except
+        that "bf16" has no rank kernel (ValueError)."""
+        all_users, all_items = self.computer()
+        mrp = mcol = None
+        if exclude_train:
+            mrp, mcol = self.train_mask_csr()
+        return self._full_ranker(all_items, precision, probe).ranks(all_users, users, items, mrp, mcol)
+
+    def _full_ranker(self, all_items, precision: str, probe: bool):
         # the ranker and the item operands it packs are reused across eval-mode calls, in which propagation gives
         # the same bits every time; fp32 reads the current table as it is
         r = self._ranker
         if r is None or self.training or (r.precision, r.probe) != (precision, probe) or precision == "fp32":
             r = self._ranker = ops.FullRanker(all_items, precision, probe=probe)
-        return r.topk(all_users, users, k, mrp, mcol, user_block)
+        return r
 
 
 def dropout_seed() -> int:

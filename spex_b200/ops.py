@@ -916,6 +916,40 @@ def score_topk_f16_wide(Uh, u_meta, B, B_pad, Ih, i_meta, m_items, m_pad, D, k, 
     return out_idx, out_val
 
 
+def rank_pairs_f16(Uh, a_rows, user_ids, items, Ih, i_meta, m_items, m_pad, D, mask_rowptr=None, mask_col=None,
+                   out=None):
+    """Rank of each held-out pair (user row a_rows[p] of the packed table Uh, item items[p]) among the items outside
+    mask row user_ids[p], under the exact score of the f16 scorer (spex_rank_pairs_f16): int32 [P]."""
+    _need_cuda(Uh, Ih)
+    if D not in SCORER_LIMITS["f16"][0]:
+        raise ValueError("rank_pairs_f16: D must be 64 or 128 (use rank_pairs_f32 otherwise)")
+    dev = Uh.device
+    items = items.to(device=dev, dtype=torch.int32).contiguous()
+    P = items.numel()
+    out = torch.empty(P, dtype=torch.int32, device=dev) if out is None else out
+    p_pad = (P + TC_USER_MULTIPLE - 1) // TC_USER_MULTIPLE * TC_USER_MULTIPLE
+    a_rows = None if a_rows is None else _i64c(a_rows, dev)
+    user_ids = None if user_ids is None else _i64c(user_ids, dev)
+    call("spex_rank_pairs_f16", ptr(Uh), ptr(Ih), int(D), ptr(a_rows), ptr(user_ids),
+         ptr(items), P, p_pad, int(m_items), int(m_pad), ptr(i_meta), ptr(mask_rowptr), ptr(mask_col), ptr(out),
+         stream_ptr())
+    return out
+
+
+def rank_pairs_f32(U, I, users, items, mask_rowptr=None, mask_col=None, out=None):
+    """Rank of each held-out pair (U[users[p]], item items[p]) among the items outside mask row users[p], under the
+    exact fp32 score of score_topk_f32 (spex_rank_pairs_f32): int32 [P]."""
+    _need_cuda(U, I)
+    U, I = _f32c(U), _f32c(I)
+    dev = U.device
+    users = _i64c(users, dev)
+    items = items.to(device=dev, dtype=torch.int32).contiguous()
+    out = torch.empty(items.numel(), dtype=torch.int32, device=dev) if out is None else out
+    call("spex_rank_pairs_f32", ptr(U), ptr(I), U.shape[1], ptr(users), ptr(items), items.numel(), I.shape[0],
+         ptr(mask_rowptr), ptr(mask_col), ptr(out), stream_ptr())
+    return out
+
+
 def check_k(precision: str, k: int):
     """ValueError unless `precision` serves top-`k` (SCORER_LIMITS); the message names the precision that serves a k
     beyond the limit."""
@@ -948,11 +982,21 @@ class FullRanker:
         self.m_items, self.D = I_all.shape
         self._I, self._m_pad = I_all, None      # _m_pad: set when the item table is packed
 
-    def scorer_for(self, k: int, U_all, probe_users) -> str:
+    def scorer_for(self, k, U_all, probe_users) -> str:
         """The precision that ranks top-k: ValueError unless this ranker's precision serves k (check_k).  With
         probe=True, "f16" becomes "fp32" for k <= F32_MAX_K when f16_filter_is_selective(U_all, I_all, probe_users)
         is False: near-equal scores, on which the exact scorer is the faster exact path (above F32_MAX_K only the
-        f16 scorer serves k)."""
+        f16 scorer serves k).
+
+        k=None asks for the precision of a rank query (ranks, rank_metrics), which has no k: "f16" (turned into
+        "fp32" by the same probe when probe=True) or "fp32"; ValueError for "bf16", which has no rank kernel."""
+        if k is None:
+            if self.precision == "bf16":
+                raise ValueError("precision 'bf16' has no rank kernel; use 'f16' or 'fp32'")
+            if (self.precision == "f16" and self.probe
+                    and not f16_filter_is_selective(U_all, self._I, probe_users)):
+                return "fp32"
+            return self.precision
         check_k(self.precision, k)
         if (self.precision == "f16" and self.probe and k <= F32_MAX_K
                 and not f16_filter_is_selective(U_all, self._I, probe_users)):
@@ -1065,11 +1109,107 @@ class FullRanker:
                                     user_block, per_user, probe_users)
         return metric_means(sums.cpu().numpy(), users.numel(), pu)
 
+    def _check_items(self, items):
+        items = torch.as_tensor(items).to(device=self.device, dtype=torch.int64)
+        if items.numel() and bool((items.min() < 0) | (items.max() >= self.m_items)):
+            raise ValueError(f"item ids must lie in [0, {self.m_items})")
+        return items.to(torch.int32).contiguous()
+
+    def _rank(self, scorer, U_all, urows, a_rows, pair_users, items, mask_rowptr, mask_col):
+        """Ranks of the pairs (U_all[pair_users[p]], items[p]) with `scorer`, in launches of RANK_PAIR_BLOCK pairs.
+        f16: the users `urows` are packed once (one scale 2^s over all of them, as topk() packs its users) and
+        pair p reads packed row a_rows[p]."""
+        P = items.numel()
+        out = torch.empty(P, dtype=torch.int32, device=self.device)
+        if P == 0:
+            return out
+        if scorer == "f16":
+            if self._m_pad is None:
+                self._Ih, self._m_pad, self._imeta = pack_f16(self._I, None, TC_ITEM_MULTIPLE)
+            Uh, _, _ = pack_f16(U_all, urows)
+        for s in range(0, P, RANK_PAIR_BLOCK):
+            e = min(s + RANK_PAIR_BLOCK, P)
+            if scorer == "f16":
+                rank_pairs_f16(Uh, a_rows[s:e], pair_users[s:e], items[s:e], self._Ih, self._imeta, self.m_items,
+                               self._m_pad, self.D, mask_rowptr, mask_col, out[s:e])
+            else:
+                rank_pairs_f32(U_all, self._I, pair_users[s:e], items[s:e], mask_rowptr, mask_col, out[s:e])
+        return out
+
+    def ranks(self, U_all, users, items, mask_rowptr=None, mask_col=None, probe_users=None):
+        """Rank of item items[p] for user users[p], int32 [P] on the device: the number of items outside the user's
+        mask row, other than items[p], that come before it in the order of topk() (score descending, ties by
+        ascending id) under the exact score of scorer_for(None, U_all, probe_users) (None: `users`).  It is the
+        item's position in topk(...) when the item is listed there, >= k otherwise; a masked item still has one.
+        ValueError for an item outside [0, m_items).  The result does not depend on RANK_PAIR_BLOCK."""
+        users = _i64c(users, self.device)
+        items = self._check_items(items)
+        if users.numel() != items.numel():
+            raise ValueError(f"{users.numel()} users but {items.numel()} items")
+        scorer = self.scorer_for(None, U_all, users if probe_users is None else probe_users)
+        if scorer == "f16" and users.numel():
+            urows, a_rows = torch.unique(users, return_inverse=True)
+        else:
+            urows, a_rows = users, None
+        return self._rank(scorer, U_all, urows, a_rows, users, items, mask_rowptr, mask_col)
+
+    def rank_metrics(self, U_all, users, cutoffs, truth_rowptr, truth_col, mask_rowptr=None, mask_col=None,
+                     probe_users=None):
+        """Recall, precision, NDCG and hit rate at `cutoffs` (1 to 8 strictly ascending K, 1 <= K <= m_items), MRR
+        and AUC of the full ranking of U_all[users], from the rank of every held-out item (ranks()):
+        {"recall", "precision", "ndcg", "hit": float64 [n_cut], "mrr", "auc": float, "users": B}.
+
+        The truth CSR is evaluate()'s; so are the definitions, with "rank < K" for "in the top K": a held-out item
+        in the user's mask is never a hit.  MRR = 1 / (1 + the best rank among the user's hits), AUC = the mean over
+        the held-out items of the fraction of the user's negatives (items outside the mask and the truth row) that
+        score below the item (1 when the user has no negative; 0 for a masked item); spex_rank_metrics has the
+        exact rules.  Means over all users, an empty truth row counting as zeros.  The users are packed as
+        evaluate() packs them, so the ranks are the positions evaluate() ranks by; sums run per chunk of
+        METRICS_CHUNK users in a fixed order on the device."""
+        cutoffs = check_cutoffs(cutoffs)
+        if cutoffs[-1] > self.m_items:
+            raise ValueError(f"cutoffs must be <= m_items = {self.m_items}, got {cutoffs[-1]}")
+        dev = self.device
+        users = _i64c(users, dev)
+        B = users.numel()
+        trp = _i64c(truth_rowptr, dev)
+        tcol = torch.as_tensor(np.asarray(truth_col) if not torch.is_tensor(truth_col) else truth_col)
+        tcol = tcol.to(device=dev, dtype=torch.int32).contiguous()
+        check_truth_csr(trp, tcol, B)
+        scorer = self.scorer_for(None, U_all, users if probe_users is None else probe_users)
+        a = int(trp[0]) if B else 0
+        tcol = self._check_items(tcol[a: int(trp[-1])] if B else tcol[:0])
+        trp = (trp - a).contiguous()
+        pos = torch.repeat_interleave(torch.arange(B, device=dev), trp[1:] - trp[:-1])
+        ranks = self._rank(scorer, U_all, users, pos, users[pos], tcol, mask_rowptr, mask_col)
+        n_cut = len(cutoffs)
+        disc, idcg = rank_discounts(cutoffs[-1])
+        disc = torch.from_numpy(disc).to(dev)
+        idcg = torch.from_numpy(idcg).to(dev)
+        n_chunks = (B + METRICS_CHUNK - 1) // METRICS_CHUNK
+        chunk_sums = torch.empty(n_chunks, n_cut, 4, dtype=torch.float64, device=dev)
+        chunk_extra = torch.empty(n_chunks, 4, dtype=torch.float64, device=dev)
+        if tcol.numel() == 0:
+            tcol = torch.zeros(1, dtype=torch.int32, device=dev)       # all rows empty: never read, but not NULL
+            ranks = torch.zeros(1, dtype=torch.int32, device=dev)
+        call("spex_rank_metrics", ptr(ranks), B, ptr(trp), ptr(tcol), ptr(users), ptr(mask_rowptr), ptr(mask_col),
+             self.m_items, (C.c_int32 * n_cut)(*cutoffs), n_cut, ptr(disc), ptr(idcg), ptr(chunk_sums),
+             ptr(chunk_extra), stream_ptr())
+        sums = torch.empty(n_cut, 4, dtype=torch.float64, device=dev)
+        extra = torch.empty(1, 4, dtype=torch.float64, device=dev)
+        call("spex_fullrank_metrics_reduce", ptr(chunk_sums), n_chunks, n_cut, ptr(sums), stream_ptr())
+        call("spex_fullrank_metrics_reduce", ptr(chunk_extra), n_chunks, 1, ptr(extra), stream_ptr())
+        out = metric_means(sums.cpu().numpy(), B)
+        ex = extra.cpu().numpy()[0] / max(float(B), 1.0)
+        out["mrr"], out["auc"] = float(ex[0]), float(ex[1])
+        return out
+
 
 METRICS_CHUNK = 1024           # SPEX_METRICS_CHUNK in include/spex_b200.h: users per partial sum
 METRICS_MAX_CUTOFFS = 8        # SPEX_METRICS_MAX_CUTOFFS
 METRIC_NAMES = ("recall", "precision", "ndcg", "hit")
 EVAL_USER_BLOCK = 148 * METRICS_CHUNK   # users ranked per block by FullRanker.evaluate (None)
+RANK_PAIR_BLOCK = 1 << 22      # pairs per rank launch of FullRanker.ranks / rank_metrics
 
 
 def check_cutoffs(cutoffs):
