@@ -37,6 +37,33 @@ __device__ __forceinline__ bool truth_has(const int32_t* __restrict__ col, int64
   return false;
 }
 
+// metric my_m (recall, precision, ndcg, hit) at cutoff my_K of a user with T held-out items, my_h of them in the
+// top my_K with DCG my_dcg
+__device__ __forceinline__ double metric_value(int my_m, int my_h, double my_dcg, int my_K, int64_t T,
+                                               const double* idcg) {
+  double v;
+  if (my_m == 0) {
+    v = T > 0 ? (double)my_h / (double)T : 0.0;
+  } else if (my_m == 1) {
+    v = (double)my_h / (double)my_K;
+  } else if (my_m == 2) {
+    const double id = __ldg(idcg + (T < my_K ? T : (int64_t)my_K));
+    v = id > 0.0 ? my_dcg / id : 0.0;
+  } else {
+    v = my_h > 0 ? 1.0 : 0.0;
+  }
+  return v;
+}
+
+// The walk of a user's hit ranks in ascending order reaches rank i with h hits and DCG acc before it: every cutoff
+// c <= i is passed (c advances), and the lane that owns cutoff my_c keeps (h, acc) as its (my_h, my_dcg).
+// i = INT_MAX passes the cutoffs left after the last hit.
+__device__ __forceinline__ void pass_cutoffs(int i, int& c, int n_cut, const int32_t* s_cut, int my_c, int h,
+                                             double acc, int& my_h, double& my_dcg) {
+  for (; c < n_cut && i >= s_cut[c]; ++c)
+    if (c == my_c) my_h = h, my_dcg = acc;
+}
+
 __global__ void __launch_bounds__(kMetricsWarps * kWarp)
 fullrank_metrics_kernel(const int32_t* __restrict__ topk, int64_t B, int32_t k,
                         const int64_t* __restrict__ rowptr, const int32_t* __restrict__ tcol,
@@ -73,28 +100,15 @@ fullrank_metrics_kernel(const int32_t* __restrict__ topk, int64_t B, int32_t k,
       unsigned m = __ballot_sync(kFull, hit);
       while (m) {
         const int i = j * kWarp + __ffs(m) - 1;
-        for (; c < n_cut && i >= s_cut[c]; ++c)
-          if (c == my_c) my_h = h, my_dcg = acc;
+        pass_cutoffs(i, c, n_cut, s_cut, my_c, h, acc, my_h, my_dcg);
         acc += __ldg(disc + i);
         ++h;
         m &= m - 1;
       }
     }
-    for (; c < n_cut; ++c)
-      if (c == my_c) my_h = h, my_dcg = acc;
+    pass_cutoffs(INT_MAX, c, n_cut, s_cut, my_c, h, acc, my_h, my_dcg);
     if (lane < nv) {
-      const int64_t T = hi - lo;
-      double v;
-      if (my_m == 0) {
-        v = T > 0 ? (double)my_h / (double)T : 0.0;
-      } else if (my_m == 1) {
-        v = (double)my_h / (double)my_K;
-      } else if (my_m == 2) {
-        const double id = __ldg(idcg + (T < my_K ? T : (int64_t)my_K));
-        v = id > 0.0 ? my_dcg / id : 0.0;
-      } else {
-        v = my_h > 0 ? 1.0 : 0.0;
-      }
+      const double v = metric_value(my_m, my_h, my_dcg, my_K, hi - lo, idcg);
       if (per_user) per_user[u * nv + lane] = v;
       sum += v;
     }
@@ -172,8 +186,7 @@ rank_metrics_kernel(const int32_t* __restrict__ ranks, int64_t B, const int64_t*
     double acc = 0.0, my_dcg = 0.0;
     int h = 0, c = 0, my_h = 0, prev = -1, next = e_min;
     while (next < Kmax) {
-      for (; c < n_cut && next >= s_cut[c]; ++c)
-        if (c == my_c) my_h = h, my_dcg = acc;
+      pass_cutoffs(next, c, n_cut, s_cut, my_c, h, acc, my_h, my_dcg);
       acc += __ldg(disc + next);
       ++h;
       prev = next;
@@ -184,23 +197,9 @@ rank_metrics_kernel(const int32_t* __restrict__ ranks, int64_t B, const int64_t*
       }
       next = __reduce_min_sync(kFull, nx);
     }
-    for (; c < n_cut; ++c)
-      if (c == my_c) my_h = h, my_dcg = acc;
+    pass_cutoffs(INT_MAX, c, n_cut, s_cut, my_c, h, acc, my_h, my_dcg);
     const int64_t T = hi - lo;
-    if (lane < nv) {
-      double v;
-      if (my_m == 0) {
-        v = T > 0 ? (double)my_h / (double)T : 0.0;
-      } else if (my_m == 1) {
-        v = (double)my_h / (double)my_K;
-      } else if (my_m == 2) {
-        const double id = __ldg(idcg + (T < my_K ? T : (int64_t)my_K));
-        v = id > 0.0 ? my_dcg / id : 0.0;
-      } else {
-        v = my_h > 0 ? 1.0 : 0.0;
-      }
-      sum += v;
-    }
+    if (lane < nv) sum += metric_value(my_m, my_h, my_dcg, my_K, T, idcg);
     // AUC of each held-out item: 1 - (negatives above it) / n_neg, negatives = items outside mask and truth
     int n_mask = 0;                                     // distinct mask ids in [0, m_items): a repeat counts once
     for (int64_t k = mlo + lane; k < mhi; k += kWarp) {
@@ -243,6 +242,17 @@ rank_metrics_kernel(const int32_t* __restrict__ ranks, int64_t B, const int64_t*
 
 using namespace spex;
 
+// the n_cut host cutoffs into `cuts`: SPEX_E_BADARG unless they are strictly ascending in [1, bound]
+static int read_cutoffs(const int32_t* cutoffs_host, int32_t n_cut, int64_t bound, MetricsCutoffs* cuts) {
+  *cuts = {};
+  for (int i = 0; i < n_cut; ++i) {
+    const int32_t K = cutoffs_host[i];
+    SPEX_RETURN_IF(K < 1 || K > bound || (i > 0 && K <= cutoffs_host[i - 1]), SPEX_E_BADARG);
+    cuts->c[i] = K;
+  }
+  return 0;
+}
+
 extern "C" int spex_rank_metrics(const int32_t* ranks, int64_t B, const int64_t* truth_rowptr,
                                  const int32_t* truth_col, const int64_t* users, const int64_t* mask_rowptr,
                                  const int32_t* mask_col, int64_t m_items, const int32_t* cutoffs_host, int32_t n_cut,
@@ -251,12 +261,8 @@ extern "C" int spex_rank_metrics(const int32_t* ranks, int64_t B, const int64_t*
   SPEX_RETURN_IF(n_cut > SPEX_METRICS_MAX_CUTOFFS || m_items > 0x7fffffffLL, SPEX_E_TOOBIG);
   SPEX_RETURN_IF(B < 0 || m_items < 1 || n_cut < 1 || !cutoffs_host || !disc || !idcg, SPEX_E_BADARG);
   SPEX_RETURN_IF((mask_rowptr == nullptr) != (mask_col == nullptr), SPEX_E_BADARG);
-  MetricsCutoffs cuts = {};
-  for (int i = 0; i < n_cut; ++i) {
-    const int32_t K = cutoffs_host[i];
-    SPEX_RETURN_IF(K < 1 || K > m_items || (i > 0 && K <= cutoffs_host[i - 1]), SPEX_E_BADARG);
-    cuts.c[i] = K;
-  }
+  MetricsCutoffs cuts;
+  if (const int rc = read_cutoffs(cutoffs_host, n_cut, m_items, &cuts)) return rc;
   if (B == 0) return 0;
   SPEX_RETURN_IF(!ranks || !truth_rowptr || !truth_col || !chunk_sums || !chunk_extra ||
                      (mask_rowptr && !users),
@@ -275,12 +281,8 @@ extern "C" int spex_fullrank_metrics(const int32_t* topk_idx, int64_t B, int32_t
                                      void* stream) {
   SPEX_RETURN_IF(k > kMaxK || n_cut > SPEX_METRICS_MAX_CUTOFFS, SPEX_E_TOOBIG);
   SPEX_RETURN_IF(B < 0 || k < 1 || n_cut < 1 || !cutoffs_host || !disc || !idcg, SPEX_E_BADARG);
-  MetricsCutoffs cuts = {};
-  for (int i = 0; i < n_cut; ++i) {
-    const int32_t K = cutoffs_host[i];
-    SPEX_RETURN_IF(K < 1 || K > k || (i > 0 && K <= cutoffs_host[i - 1]), SPEX_E_BADARG);
-    cuts.c[i] = K;
-  }
+  MetricsCutoffs cuts;
+  if (const int rc = read_cutoffs(cutoffs_host, n_cut, k, &cuts)) return rc;
   if (B == 0) return 0;
   SPEX_RETURN_IF(!topk_idx || !truth_rowptr || !truth_col || !chunk_sums, SPEX_E_BADARG);
   const int64_t n_chunks = (B + SPEX_METRICS_CHUNK - 1) / SPEX_METRICS_CHUNK;

@@ -104,6 +104,35 @@ __device__ __forceinline__ uint32_t hmax2(uint32_t a, uint32_t b) {
 __device__ __forceinline__ __half lo_half(uint32_t x) { return __ushort_as_half((unsigned short)(x & 0xffffu)); }
 __device__ __forceinline__ __half hi_half(uint32_t x) { return __ushort_as_half((unsigned short)(x >> 16)); }
 
+// the maxima m[b] of the eight 16-column blocks of a quarter tile row (8 registers each) as eight independent chains,
+// and their max: 63 HMNMX2 in all
+__device__ __forceinline__ uint32_t block_max(const uint32_t (&r)[64], uint32_t (&m)[8]) {
+#pragma unroll
+  for (int b = 0; b < 8; ++b) {
+    m[b] = r[8 * b];
+#pragma unroll
+    for (int i = 1; i < 8; ++i) m[b] = hmax2(m[b], r[8 * b + i]);
+  }
+  return hmax2(hmax2(hmax2(m[0], m[1]), hmax2(m[2], m[3])), hmax2(hmax2(m[4], m[5]), hmax2(m[6], m[7])));
+}
+
+// the eight packed registers p of 16-column block bi (warp-uniform) of r: a switch over named scalars (an array
+// written in a switch is placed in local memory by the compiler)
+__device__ __forceinline__ void pick_block(const uint32_t (&r)[64], int bi, uint32_t (&p)[8]) {
+  uint32_t p0, p1, p2, p3, p4, p5, p6, p7;
+#define SPEX_PICK(b)                                                                                   \
+  case b:                                                                                              \
+    p0 = r[8 * b]; p1 = r[8 * b + 1]; p2 = r[8 * b + 2]; p3 = r[8 * b + 3];                             \
+    p4 = r[8 * b + 4]; p5 = r[8 * b + 5]; p6 = r[8 * b + 6]; p7 = r[8 * b + 7];                         \
+    break;
+  switch (bi) {
+    SPEX_PICK(0) SPEX_PICK(1) SPEX_PICK(2) SPEX_PICK(3) SPEX_PICK(4) SPEX_PICK(5) SPEX_PICK(6)
+    default: SPEX_PICK(7)
+  }
+#undef SPEX_PICK
+  p[0] = p0, p[1] = p1, p[2] = p2, p[3] = p3, p[4] = p4, p[5] = p5, p[6] = p6, p[7] = p7;
+}
+
 // Per-row mask cursor (shared memory; only the survivor path touches it).  Items are offered to a
 // row in strictly ascending id order and the row's training items (CSR row of R) are ascending
 // too, so the mask test is a merge: the cursor only moves forward.
@@ -112,10 +141,35 @@ struct MaskCursor {
   const int32_t* end[BM];
 };
 
+// byte offset of row r of a packed fp16 table in the canonical layout (pack_rows); element block kc at + kc * 128
+template <int DK, class Row>
+__device__ __forceinline__ size_t packed_off(Row r) {
+  return (size_t)(r >> 3) * (16 * DK) + (size_t)(r & 7) * 16;
+}
+
+// filter margin eps of a row (header comment) from its resident A row and the max scaled item-row norm vmax
+// (i_meta[2]): the one rule of the top-k filter and of the rank kernel's band
+template <int DK>
+__device__ __forceinline__ float row_eps(const uint8_t* a_row, float vmax) {
+  float un2 = 0.f;
+#pragma unroll
+  for (int kc = 0; kc < DK / 8; ++kc) {
+    const uint4 a = *reinterpret_cast<const uint4*>(a_row + kc * 128);
+    const uint32_t aw[4] = {a.x, a.y, a.z, a.w};
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&aw[j]));
+      un2 = fmaf(f.x, f.x, un2);
+      un2 = fmaf(f.y, f.y, un2);
+    }
+  }
+  return kEpsRel<DK> * sqrtf(un2) * vmax * 1.0001f + kEpsAbs;
+}
+
 // exact score of (this row, item id): fp32 FMA chain over the fp16 operands, d = 0 .. DK-1
 template <int DK>
 __device__ __forceinline__ float exact_score(const uint8_t* a_row, const uint8_t* Ib, int id) {
-  const uint8_t* b_row = Ib + (size_t)(id >> 3) * (16 * DK) + (size_t)(id & 7) * 16;
+  const uint8_t* b_row = Ib + packed_off<DK>(id);
   float s = 0.f;
 #pragma unroll
   for (int kc = 0; kc < DK / 8; ++kc) {
@@ -258,8 +312,7 @@ __device__ __noinline__ unsigned long long tf_compact(unsigned need, int n, int 
       }
     }
     if (exact) {
-      const int rr = row0 + src;
-      const uint8_t* a_row = sA + (size_t)(rr >> 3) * (16 * DK) + (size_t)(rr & 7) * 16;
+      const uint8_t* a_row = sA + packed_off<DK>(row0 + src);
 #pragma unroll
       for (int e = 0; e < EPL; ++e) {
         if (ef[e] && lane + 32 * e < ns) ev[e] = exact_score<DK>(a_row, Ib, ei[e]);
@@ -398,8 +451,7 @@ __device__ __noinline__ unsigned long long tf_compact_ws(unsigned need, int n, f
       }
     }
     if (exact) {
-      const int rr = row0 + src;
-      const uint8_t* a_row = sA + (size_t)(rr >> 3) * (16 * DK) + (size_t)(rr & 7) * 16;
+      const uint8_t* a_row = sA + packed_off<DK>(row0 + src);
       for (int p = lane; p < ns; p += 32) {
         const uint2 e = sc[p];
         if (e.y & (unsigned)kApprox) {
@@ -540,21 +592,8 @@ score_topk_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict_
     }
     // the row's norm (scaled units) from the resident A tile -> filter margin
     mbar_wait(&bar_a, 0);
-    const uint8_t* a_row = sA + (size_t)(row >> 3) * (16 * DK) + (size_t)(row & 7) * 16;
-    float un2 = 0.f;
-#pragma unroll
-    for (int kc = 0; kc < DK / 8; ++kc) {
-      const uint4 a = *reinterpret_cast<const uint4*>(a_row + kc * 128);
-      const uint32_t aw[4] = {a.x, a.y, a.z, a.w};
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&aw[j]));
-        un2 = fmaf(f.x, f.x, un2);
-        un2 = fmaf(f.y, f.y, un2);
-      }
-    }
-    const float vmax = i_meta[2];                       // max scaled item-row norm
-    const float eps = kEpsRel<DK> * sqrtf(un2) * vmax * 1.0001f + kEpsAbs;
+    const uint8_t* a_row = sA + packed_off<DK>(row);
+    const float eps = row_eps<DK>(a_row, i_meta[2]);
     float* cv_row = cv_warp + lane * CAP;
     int* ci_row = ci_warp + lane * CAP;
     uint2* ws_warp = kWide ? ws + (size_t)(tile_m * BM + q * 32) * CAP : nullptr;
@@ -582,14 +621,7 @@ score_topk_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict_
       // fast reject: eight independent max chains over blocks of 8 registers (16 columns each),
       // 63 HMNMX2 in all, one compare, one vote
       uint32_t m[8];
-#pragma unroll
-      for (int b = 0; b < 8; ++b) {
-        m[b] = r[8 * b];
-#pragma unroll
-        for (int i = 1; i < 8; ++i) m[b] = hmax2(m[b], r[8 * b + i]);
-      }
-      const uint32_t mm = hmax2(hmax2(hmax2(m[0], m[1]), hmax2(m[2], m[3])),
-                                hmax2(hmax2(m[4], m[5]), hmax2(m[6], m[7])));
+      const uint32_t mm = block_max(r, m);
       if (__any_sync(kFull, __hge(__hmax(lo_half(mm), hi_half(mm)), thr))) {
         // slow path: which 16-column blocks hold a hit in any lane
         const long long c0 = stats ? clock64() : 0;
@@ -602,20 +634,8 @@ score_topk_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict_
         while (blocks) {
           const int bi = __ffs(blocks) - 1;
           blocks &= blocks - 1;
-          // warp-uniform pick of the block's eight packed registers (named scalars: an array written in
-          // a switch is placed in local memory by the compiler)
-          uint32_t p0, p1, p2, p3, p4, p5, p6, p7;
-#define SPEX_PICK(b)                                                                                   \
-  case b:                                                                                              \
-    p0 = r[8 * b]; p1 = r[8 * b + 1]; p2 = r[8 * b + 2]; p3 = r[8 * b + 3];                             \
-    p4 = r[8 * b + 4]; p5 = r[8 * b + 5]; p6 = r[8 * b + 6]; p7 = r[8 * b + 7];                         \
-    break;
-          switch (bi) {
-            SPEX_PICK(0) SPEX_PICK(1) SPEX_PICK(2) SPEX_PICK(3) SPEX_PICK(4) SPEX_PICK(5) SPEX_PICK(6)
-            default: SPEX_PICK(7)
-          }
-#undef SPEX_PICK
-          const uint32_t p[8] = {p0, p1, p2, p3, p4, p5, p6, p7};
+          uint32_t p[8];
+          pick_block(r, bi, p);
           // this lane's hits among the block's 16 columns, and the columns that hold a hit in any lane
           const int id0 = t * BN + bi * 16;
           unsigned mine = 0;
@@ -790,19 +810,12 @@ static int launch(const void* Uh, const void* Ih, int64_t B, int64_t B_pad, int6
   SPEX_RETURN_IF(stages < 2 || stages > kMaxStages, SPEX_E_BADARG);
   const size_t smem = smem_bytes(DK, cand, stages);
   SPEX_RETURN_IF(smem > 227 * 1024 - 7600, SPEX_E_TOOBIG);
-  cudaError_t e = cudaFuncSetAttribute(score_topk_f16_kernel<DK, EPL>,
-                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return (int)e;
-  const int64_t grid = B_pad / BM;
-  SPEX_RETURN_IF(grid > 0x7fffffffLL, SPEX_E_TOOBIG);
   int dbg = 0;
   if (!kWide)
     if (const char* e = getenv("SPEX_TF_DBG")) dbg = atoi(e);   // bring-up experiment
-  score_topk_f16_kernel<DK, EPL><<<(unsigned)grid, kThreads, smem, st>>>(
-      (const uint8_t*)Uh, (const uint8_t*)Ih, B, (int)m_items, (int)(m_pad / BN), u_meta, i_meta,
-      user_ids, mask_rowptr, mask_col, k, out_idx, out_val, stages, g_stats, dbg, ws, cap);
-  count_launch();
-  return check_last();
+  return launch_tiles(score_topk_f16_kernel<DK, EPL>, smem, B_pad, st, (const uint8_t*)Uh, (const uint8_t*)Ih, B,
+                      (int)m_items, (int)(m_pad / BN), u_meta, i_meta, user_ids, mask_rowptr, mask_col, k, out_idx,
+                      out_val, stages, g_stats, dbg, ws, cap);
 }
 
 template <int DK>
@@ -873,10 +886,10 @@ rank_pairs_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict_
     const int64_t grow = tile_m * BM + row;
     const bool live = grow < P;
     // gather this pair's user row into the A tile (zeros past P), then publish the tile to the tensor core
-    uint8_t* a_row = sA + (size_t)(row >> 3) * (16 * DK) + (size_t)(row & 7) * 16;
+    uint8_t* a_row = sA + packed_off<DK>(row);
     {
       const int64_t ur = live ? (a_rows ? a_rows[grow] : grow) : 0;
-      const uint8_t* src = Uh + (size_t)(ur >> 3) * (16 * DK) + (size_t)(ur & 7) * 16;
+      const uint8_t* src = Uh + packed_off<DK>(ur);
 #pragma unroll
       for (int kc = 0; kc < DK / 8; ++kc)
         *reinterpret_cast<uint4*>(a_row + kc * 128) =
@@ -885,19 +898,7 @@ rank_pairs_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict_
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     asm volatile("bar.sync 1, 128;" ::: "memory");   // the four epilogue warps
     if (row == 0) mbar_arrive(&bar_a);
-    float un2 = 0.f;
-#pragma unroll
-    for (int kc = 0; kc < DK / 8; ++kc) {
-      const uint4 a = *reinterpret_cast<const uint4*>(a_row + kc * 128);
-      const uint32_t aw[4] = {a.x, a.y, a.z, a.w};
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&aw[j]));
-        un2 = fmaf(f.x, f.x, un2);
-        un2 = fmaf(f.y, f.y, un2);
-      }
-    }
-    const float eps = kEpsRel<DK> * sqrtf(un2) * i_meta[2] * 1.0001f + kEpsAbs;
+    const float eps = row_eps<DK>(a_row, i_meta[2]);
     const int tid = live ? items[grow] : -1;
     const float st = live ? exact_score<DK>(a_row, Ih, tid) : 0.f;
     // padded rows: lo = hi = +inf, nothing is counted
@@ -918,14 +919,7 @@ rank_pairs_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict_
       __syncwarp();
       if (lane == 0) mbar_arrive(&bar_tempty[buf]);
       uint32_t mx[8];
-#pragma unroll
-      for (int b = 0; b < 8; ++b) {
-        mx[b] = r[8 * b];
-#pragma unroll
-        for (int i = 1; i < 8; ++i) mx[b] = hmax2(mx[b], r[8 * b + i]);
-      }
-      const uint32_t mm = hmax2(hmax2(hmax2(mx[0], mx[1]), hmax2(mx[2], mx[3])),
-                                hmax2(hmax2(mx[4], mx[5]), hmax2(mx[6], mx[7])));
+      const uint32_t mm = block_max(r, mx);
       const bool any_ge = __hge(__hmax(lo_half(mm), hi_half(mm)), lo);
       if (!__any_sync(kFull, any_ge)) continue;           // every lane: the whole tile is below t
       if (!any_ge) continue;
@@ -964,18 +958,8 @@ rank_pairs_f16_kernel(const uint8_t* __restrict__ Uh, const uint8_t* __restrict_
       // band columns (or the zero-padded last tile): 16 columns at a time, exact re-score of the band
 #pragma unroll 1
       for (int bi = 0; bi < 8; ++bi) {
-        uint32_t p0, p1, p2, p3, p4, p5, p6, p7;
-#define SPEX_PICK(b)                                                                                   \
-  case b:                                                                                              \
-    p0 = r[8 * b]; p1 = r[8 * b + 1]; p2 = r[8 * b + 2]; p3 = r[8 * b + 3];                             \
-    p4 = r[8 * b + 4]; p5 = r[8 * b + 5]; p6 = r[8 * b + 6]; p7 = r[8 * b + 7];                         \
-    break;
-        switch (bi) {
-          SPEX_PICK(0) SPEX_PICK(1) SPEX_PICK(2) SPEX_PICK(3) SPEX_PICK(4) SPEX_PICK(5) SPEX_PICK(6)
-          default: SPEX_PICK(7)
-        }
-#undef SPEX_PICK
-        const uint32_t p[8] = {p0, p1, p2, p3, p4, p5, p6, p7};
+        uint32_t p[8];
+        pick_block(r, bi, p);
         const int b0 = id0 + bi * 16;
         const unsigned valid = (b0 + 16 <= m_items) ? 0xffffu : (b0 < m_items ? (1u << (m_items - b0)) - 1u : 0u);
         unsigned above = 0, band = 0;
@@ -1022,17 +1006,9 @@ static int launch_rank(const void* Uh, const void* Ih, int64_t P, int64_t P_pad,
   // no candidate buffers: the ring takes kMaxStages stages at both D, with two CTAs per SM at D = 64 (80 KB each)
   // and one at D = 128 (160 KB), the occupancy of the top-k kernel
   const int stages = choose_stages(DK, 0, (DK == 64) ? 115712 - 7600 : 227 * 1024 - 7600);
-  const size_t smem = smem_bytes(DK, 0, stages);
-  cudaError_t e = cudaFuncSetAttribute(rank_pairs_f16_kernel<DK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)smem);
-  if (e != cudaSuccess) return (int)e;
-  const int64_t grid = P_pad / BM;
-  SPEX_RETURN_IF(grid > 0x7fffffffLL, SPEX_E_TOOBIG);
-  rank_pairs_f16_kernel<DK><<<(unsigned)grid, kThreads, smem, st>>>(
-      (const uint8_t*)Uh, (const uint8_t*)Ih, P, (int)m_items, (int)(m_pad / BN), i_meta, a_rows, user_ids, items,
-      mask_rowptr, mask_col, out_rank, stages);
-  count_launch();
-  return check_last();
+  return launch_tiles(rank_pairs_f16_kernel<DK>, smem_bytes(DK, 0, stages), P_pad, st, (const uint8_t*)Uh,
+                      (const uint8_t*)Ih, P, (int)m_items, (int)(m_pad / BN), i_meta, a_rows, user_ids, items,
+                      mask_rowptr, mask_col, out_rank, stages);
 }
 
 }  // namespace tf
@@ -1073,14 +1049,11 @@ extern "C" int spex_score_topk_f16(const void* Uh, const void* Ih, int32_t D, in
                                    const float* i_meta, const int64_t* user_ids,
                                    const int64_t* mask_rowptr, const int32_t* mask_col, int32_t k,
                                    int32_t* out_idx, float* out_val, void* stream) {
-  SPEX_RETURN_IF(!Uh || !Ih || !u_meta || !i_meta || !out_idx || !out_val || B < 0 || B_pad < B ||
-                     m_items < 0 || m_pad < m_items,
-                 SPEX_E_BADARG);
-  SPEX_RETURN_IF((mask_rowptr == nullptr) != (mask_col == nullptr), SPEX_E_BADARG);
-  SPEX_RETURN_IF((B_pad % tf::BM) || (m_pad % tf::BN), SPEX_E_BADARG);
+  const int rc = tcgen05::check_operands(Uh, Ih, B, B_pad, m_items, m_pad, mask_rowptr, mask_col);
+  SPEX_RETURN_IF(rc == SPEX_E_BADARG || !u_meta || !i_meta || !out_idx || !out_val, SPEX_E_BADARG);
   SPEX_RETURN_IF(D != 64 && D != 128, SPEX_E_BADDIM);
-  SPEX_RETURN_IF(k < 1 || k > tf::KMAX_TC || m_pad > 0x7fffffffLL, SPEX_E_TOOBIG);
-  SPEX_RETURN_IF(!aligned16(Uh) || !aligned16(Ih), SPEX_E_ALIGN);
+  SPEX_RETURN_IF(k < 1 || k > tf::KMAX_TC, SPEX_E_TOOBIG);
+  if (rc) return rc;
   if (B == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   if (D == 64)
@@ -1093,13 +1066,8 @@ extern "C" int spex_rank_pairs_f16(const void* Uh, const void* Ih, int32_t D, co
                                    int64_t m_items, int64_t m_pad, const float* i_meta, const int64_t* mask_rowptr,
                                    const int32_t* mask_col, int32_t* out_rank, void* stream) {
   SPEX_RETURN_IF(D != 64 && D != 128, SPEX_E_BADDIM);
-  SPEX_RETURN_IF(!Uh || !Ih || !i_meta || !items || !out_rank || P < 0 || P_pad < P || m_items < 0 ||
-                     m_pad < m_items || (P > 0 && m_items == 0),
-                 SPEX_E_BADARG);
-  SPEX_RETURN_IF((P_pad % tf::BM) || (m_pad % tf::BN), SPEX_E_BADARG);
-  SPEX_RETURN_IF((mask_rowptr == nullptr) != (mask_col == nullptr), SPEX_E_BADARG);
-  SPEX_RETURN_IF(m_pad > 0x7fffffffLL, SPEX_E_TOOBIG);
-  SPEX_RETURN_IF(!aligned16(Uh) || !aligned16(Ih), SPEX_E_ALIGN);
+  SPEX_RETURN_IF(!i_meta || !items || !out_rank || (P > 0 && m_items == 0), SPEX_E_BADARG);
+  if (const int rc = tcgen05::check_operands(Uh, Ih, P, P_pad, m_items, m_pad, mask_rowptr, mask_col)) return rc;
   if (P == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   if (D == 64)
@@ -1120,15 +1088,12 @@ extern "C" int spex_score_topk_f16_wide(const void* Uh, const void* Ih, int32_t 
                                         const int64_t* mask_rowptr, const int32_t* mask_col, int32_t k,
                                         int32_t* out_idx, float* out_val, void* work, int64_t work_bytes,
                                         void* stream) {
-  SPEX_RETURN_IF(!Uh || !Ih || !u_meta || !i_meta || !out_idx || !out_val || B < 0 || B_pad < B ||
-                     m_items < 0 || m_pad < m_items,
-                 SPEX_E_BADARG);
-  SPEX_RETURN_IF((mask_rowptr == nullptr) != (mask_col == nullptr), SPEX_E_BADARG);
-  SPEX_RETURN_IF((B_pad % tf::BM) || (m_pad % tf::BN), SPEX_E_BADARG);
+  const int rc = tcgen05::check_operands(Uh, Ih, B, B_pad, m_items, m_pad, mask_rowptr, mask_col);
+  SPEX_RETURN_IF(rc == SPEX_E_BADARG || !u_meta || !i_meta || !out_idx || !out_val, SPEX_E_BADARG);
   SPEX_RETURN_IF(D != 64 && D != 128, SPEX_E_BADDIM);
-  SPEX_RETURN_IF(k < 1 || k > tf::KMAX_WIDE || m_pad > 0x7fffffffLL, SPEX_E_TOOBIG);
+  SPEX_RETURN_IF(k < 1 || k > tf::KMAX_WIDE || rc == SPEX_E_TOOBIG, SPEX_E_TOOBIG);
   SPEX_RETURN_IF(!work || work_bytes < spex_score_topk_f16_wide_workspace_bytes(B_pad, k), SPEX_E_WORKSPACE);
-  SPEX_RETURN_IF(!aligned16(Uh) || !aligned16(Ih) || !aligned16(work), SPEX_E_ALIGN);
+  SPEX_RETURN_IF(rc == SPEX_E_ALIGN || !aligned16(work), SPEX_E_ALIGN);
   if (B == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   const int cap = tf::wide_cap(k);

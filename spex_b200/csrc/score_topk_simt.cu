@@ -18,6 +18,43 @@ constexpr int TU = 8;        // users per CTA
 constexpr int TILE = 128;    // items per tile == threads per CTA
 constexpr int KMAX = 128;
 
+// su[u][d] = U[rows[r0 + u]][d] for u < nu, zeros for the rows past nu: the CTA's user rows in shared memory
+__device__ __forceinline__ void stage_user_rows(float* su, const float* U, int D, const int64_t* rows, int64_t r0,
+                                                int nu, int tid) {
+  for (int i = tid; i < TU * D; i += TILE) {
+    const int u = i / D, d = i - u * D;
+    su[i] = (u < nu) ? U[rows[r0 + u] * D + d] : 0.f;
+  }
+}
+
+// acc[u] += <item_row, su + u * D> over D4 float4s, for the NU staged user rows (the callers start from zero): the
+// one fp32 FMA chain of every score of this file (item element times user element, d ascending), so the top-k,
+// rating and rank kernels agree bit for bit
+template <int NU>
+__device__ __forceinline__ void dot_rows(const float* item_row, const float* su, int D, int D4,
+                                         float (&acc)[NU]) {
+  const float4* row = reinterpret_cast<const float4*>(item_row);
+#pragma unroll 4
+  for (int d4 = 0; d4 < D4; ++d4) {
+    const float4 x = __ldg(row + d4);
+#pragma unroll
+    for (int u = 0; u < NU; ++u) {
+      const float4 w = *reinterpret_cast<const float4*>(su + u * D + d4 * 4);
+      acc[u] = fmaf(x.x, w.x, acc[u]);
+      acc[u] = fmaf(x.y, w.y, acc[u]);
+      acc[u] = fmaf(x.z, w.z, acc[u]);
+      acc[u] = fmaf(x.w, w.w, acc[u]);
+    }
+  }
+}
+
+// the score of one item row against one staged user row (one row: no row stride)
+__device__ __forceinline__ float dot_f32(const float* item_row, const float* su_row, int D4) {
+  float acc[1] = {0.f};
+  dot_rows(item_row, su_row, 0, D4, acc);
+  return acc[0];
+}
+
 __global__ void __launch_bounds__(TILE)
 score_topk_simt_kernel(const float* __restrict__ U, const float* __restrict__ I, int D,
                        const int64_t* __restrict__ users, int64_t B, int64_t m_items,
@@ -38,10 +75,7 @@ score_topk_simt_kernel(const float* __restrict__ U, const float* __restrict__ I,
   const int64_t u0 = (int64_t)blockIdx.x * TU;
   const int nu = (int)((B - u0) < TU ? (B - u0) : TU);
 
-  for (int i = tid; i < TU * D; i += TILE) {
-    const int u = i / D, d = i - u * D;
-    su[i] = (u < nu) ? U[users[u0 + u] * D + d] : 0.f;
-  }
+  stage_user_rows(su, U, D, users, u0, nu, tid);
   if (tid < TU) {
     cnt[tid] = 0;
     ln[tid] = 0;
@@ -64,19 +98,7 @@ score_topk_simt_kernel(const float* __restrict__ U, const float* __restrict__ I,
       float acc[TU];
 #pragma unroll
       for (int u = 0; u < TU; ++u) acc[u] = 0.f;
-      const float4* row = reinterpret_cast<const float4*>(I + j * D);
-#pragma unroll 4
-      for (int d4 = 0; d4 < D4; ++d4) {
-        const float4 x = __ldg(row + d4);
-#pragma unroll
-        for (int u = 0; u < TU; ++u) {
-          const float4 w = *reinterpret_cast<const float4*>(su + u * D + d4 * 4);
-          acc[u] = fmaf(x.x, w.x, acc[u]);
-          acc[u] = fmaf(x.y, w.y, acc[u]);
-          acc[u] = fmaf(x.z, w.z, acc[u]);
-          acc[u] = fmaf(x.w, w.w, acc[u]);
-        }
-      }
+      dot_rows(I + j * D, su, D, D4, acc);
 #pragma unroll
       for (int u = 0; u < TU; ++u) {
         if (u < nu && (acc[u] > tau[u] || ln[u] < k)) {
@@ -125,29 +147,14 @@ rating_dense_kernel(const float* __restrict__ U, const float* __restrict__ I, in
   const int tid = threadIdx.x;
   const int64_t u0 = (int64_t)blockIdx.y * TU;
   const int nu = (int)((B - u0) < TU ? (B - u0) : TU);
-  for (int i = tid; i < TU * D; i += TILE) {
-    const int u = i / D, d = i - u * D;
-    su[i] = (u < nu) ? U[users[u0 + u] * D + d] : 0.f;
-  }
+  stage_user_rows(su, U, D, users, u0, nu, tid);
   __syncthreads();
   const int D4 = D >> 2;
   for (int64_t j = (int64_t)blockIdx.x * TILE + tid; j < m_items; j += (int64_t)gridDim.x * TILE) {
     float acc[TU];
 #pragma unroll
     for (int u = 0; u < TU; ++u) acc[u] = 0.f;
-    const float4* row = reinterpret_cast<const float4*>(I + j * D);
-#pragma unroll 4
-    for (int d4 = 0; d4 < D4; ++d4) {
-      const float4 x = __ldg(row + d4);
-#pragma unroll
-      for (int u = 0; u < TU; ++u) {
-        const float4 w = *reinterpret_cast<const float4*>(su + u * D + d4 * 4);
-        acc[u] = fmaf(x.x, w.x, acc[u]);
-        acc[u] = fmaf(x.y, w.y, acc[u]);
-        acc[u] = fmaf(x.z, w.z, acc[u]);
-        acc[u] = fmaf(x.w, w.w, acc[u]);
-      }
-    }
+    dot_rows(I + j * D, su, D, D4, acc);
 #pragma unroll
     for (int u = 0; u < TU; ++u)
       if (u < nu) out[(u0 + u) * m_items + j] = apply_sigmoid ? 1.f / (1.f + expf(-acc[u])) : acc[u];
@@ -155,25 +162,10 @@ rating_dense_kernel(const float* __restrict__ U, const float* __restrict__ I, in
 }
 
 // Rank of held-out pairs, exact fp32: CTA = TU pairs, items streamed through the threads as in the top-k kernel
-// above, with the same FMA chain (item element times user element, d ascending), so a pair's rank is the
-// position of its item in the fp32 top-k list bit for bit.  Each thread counts, per pair, the items it scored
-// that beat the held-out item t (score desc, id asc; t itself excluded) and un-counts the masked items of the
-// user that beat it; the counts are reduced per pair in a fixed order (integers: order-free anyway).
-__device__ __forceinline__ float dot_f32(const float* __restrict__ item_row, const float* su_row, int D4) {
-  const float4* row = reinterpret_cast<const float4*>(item_row);
-  float acc = 0.f;
-#pragma unroll 4
-  for (int d4 = 0; d4 < D4; ++d4) {
-    const float4 x = __ldg(row + d4);
-    const float4 w = *reinterpret_cast<const float4*>(su_row + d4 * 4);
-    acc = fmaf(x.x, w.x, acc);
-    acc = fmaf(x.y, w.y, acc);
-    acc = fmaf(x.z, w.z, acc);
-    acc = fmaf(x.w, w.w, acc);
-  }
-  return acc;
-}
-
+// above.  Every score is dot_rows' FMA chain, as in the top-k kernel, so a pair's rank is the position of its
+// item in the fp32 top-k list bit for bit.  Each thread counts, per pair, the items it scored that beat the
+// held-out item t (score desc, id asc; t itself excluded) and un-counts the masked items of the user that beat
+// it; the counts are reduced per pair in a fixed order (integers: order-free anyway).
 __global__ void __launch_bounds__(TILE)
 rank_pairs_f32_kernel(const float* __restrict__ U, const float* __restrict__ I, int D,
                       const int64_t* __restrict__ users, const int32_t* __restrict__ items, int64_t P,
@@ -187,10 +179,7 @@ rank_pairs_f32_kernel(const float* __restrict__ U, const float* __restrict__ I, 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int64_t p0 = (int64_t)blockIdx.x * TU;
   const int np = (int)((P - p0) < TU ? (P - p0) : TU);
-  for (int i = tid; i < TU * D; i += TILE) {
-    const int u = i / D, d = i - u * D;
-    su[i] = (u < np) ? U[users[p0 + u] * D + d] : 0.f;
-  }
+  stage_user_rows(su, U, D, users, p0, np, tid);
   __syncthreads();
   const int D4 = D >> 2;
   if (tid < TU) {
@@ -211,19 +200,7 @@ rank_pairs_f32_kernel(const float* __restrict__ U, const float* __restrict__ I, 
     float acc[TU];
 #pragma unroll
     for (int u = 0; u < TU; ++u) acc[u] = 0.f;
-    const float4* row = reinterpret_cast<const float4*>(I + j * D);
-#pragma unroll 4
-    for (int d4 = 0; d4 < D4; ++d4) {
-      const float4 x = __ldg(row + d4);
-#pragma unroll
-      for (int u = 0; u < TU; ++u) {
-        const float4 w = *reinterpret_cast<const float4*>(su + u * D + d4 * 4);
-        acc[u] = fmaf(x.x, w.x, acc[u]);
-        acc[u] = fmaf(x.y, w.y, acc[u]);
-        acc[u] = fmaf(x.z, w.z, acc[u]);
-        acc[u] = fmaf(x.w, w.w, acc[u]);
-      }
-    }
+    dot_rows(I + j * D, su, D, D4, acc);
 #pragma unroll
     for (int u = 0; u < TU; ++u) cnt[u] += ((int)j != tt[u] && beats(acc[u], (int)j, st[u], tt[u])) ? 1 : 0;
   }

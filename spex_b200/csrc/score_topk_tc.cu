@@ -365,32 +365,19 @@ static int tc_launch(const void* Ub, const void* Ib, int64_t B, int64_t B_pad, i
   const int stages = tcgen05::choose_stages(tc::DK, 32 * EPL, 115712 - 2800);
   const size_t smem = tcgen05::smem_bytes(tc::DK, 32 * EPL, stages);
   SPEX_RETURN_IF(smem > 226 * 1024, SPEX_E_TOOBIG);
-  // per device and per function, and the size depends on `stages`: set on every launch (cheap)
-  {
-    cudaError_t e = cudaFuncSetAttribute(tc::score_topk_tc_kernel<EPL>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (int)e;
-  }
-  const int64_t grid = B_pad / tc::BM;
-  SPEX_RETURN_IF(grid > 0x7fffffffLL, SPEX_E_TOOBIG);
-  tc::score_topk_tc_kernel<EPL><<<(unsigned)grid, tc::kThreads, smem, st>>>(
-      (const uint8_t*)Ub, (const uint8_t*)Ib, B, (int)m_items, (int)(m_pad / tc::BN), user_ids,
-      mask_rowptr, mask_col, k, out_idx, out_val, stages);
-  count_launch();
-  return check_last();
+  return tcgen05::launch_tiles(tc::score_topk_tc_kernel<EPL>, smem, B_pad, st, (const uint8_t*)Ub,
+                               (const uint8_t*)Ib, B, (int)m_items, (int)(m_pad / tc::BN), user_ids, mask_rowptr,
+                               mask_col, k, out_idx, out_val, stages);
 }
 
 extern "C" int spex_score_topk_bf16(const void* Ub, const void* Ib, int64_t B, int64_t B_pad,
                                     int64_t m_items, int64_t m_pad, const int64_t* user_ids,
                                     const int64_t* mask_rowptr, const int32_t* mask_col, int32_t k,
                                     int32_t* out_idx, float* out_val, void* stream) {
-  SPEX_RETURN_IF(!Ub || !Ib || !out_idx || !out_val || B < 0 || B_pad < B || m_items < 0 ||
-                     m_pad < m_items,
-                 SPEX_E_BADARG);
-  SPEX_RETURN_IF((mask_rowptr == nullptr) != (mask_col == nullptr), SPEX_E_BADARG);
-  SPEX_RETURN_IF((B_pad % tc::BM) || (m_pad % tc::BN), SPEX_E_BADARG);
-  SPEX_RETURN_IF(k < 1 || k > tc::KMAX_TC || m_pad > 0x7fffffffLL, SPEX_E_TOOBIG);
-  SPEX_RETURN_IF(!aligned16(Ub) || !aligned16(Ib), SPEX_E_ALIGN);
+  const int rc = tcgen05::check_operands(Ub, Ib, B, B_pad, m_items, m_pad, mask_rowptr, mask_col);
+  SPEX_RETURN_IF(rc == SPEX_E_BADARG || !out_idx || !out_val, SPEX_E_BADARG);
+  SPEX_RETURN_IF(k < 1 || k > tc::KMAX_TC, SPEX_E_TOOBIG);
+  if (rc) return rc;
   if (B == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   // candidate buffer capacity CAP = 32*EPL must hold k kept entries + one group of appends

@@ -283,5 +283,33 @@ static inline int choose_stages(int DK, int cap, size_t budget) {
   return stages;
 }
 
+// The operand contract of a launch over rows_pad packed rows A and m_pad packed items I, first failure first:
+// SPEX_E_BADARG (A or I NULL, negative or inconsistent counts, rows_pad / m_pad not a multiple of 128, one mask
+// array without the other), SPEX_E_TOOBIG (m_pad >= 2^31), SPEX_E_ALIGN (A or I not 16-byte aligned); 0 if it holds.
+// Each entry point interleaves its own checks with these codes in its documented order.
+static inline int check_operands(const void* A, const void* I, int64_t rows, int64_t rows_pad, int64_t m_items,
+                                 int64_t m_pad, const int64_t* mask_rowptr, const int32_t* mask_col) {
+  SPEX_RETURN_IF(!A || !I || rows < 0 || rows_pad < rows || m_items < 0 || m_pad < m_items, SPEX_E_BADARG);
+  SPEX_RETURN_IF((mask_rowptr == nullptr) != (mask_col == nullptr), SPEX_E_BADARG);
+  SPEX_RETURN_IF((rows_pad % BM) || (m_pad % BN), SPEX_E_BADARG);
+  SPEX_RETURN_IF(m_pad > 0x7fffffffLL, SPEX_E_TOOBIG);
+  SPEX_RETURN_IF(!aligned16(A) || !aligned16(I), SPEX_E_ALIGN);
+  return 0;
+}
+
+// Launches `kernel` on rows_pad / BM CTAs of kThreads threads with `smem` bytes of dynamic shared memory.  The
+// attribute is per device and per function, and the size depends on the stage count: it is set on every launch
+// (cheap).
+template <class... P, class... Args>
+static int launch_tiles(void (*kernel)(P...), size_t smem, int64_t rows_pad, cudaStream_t st, Args... args) {
+  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return (int)e;
+  const int64_t grid = rows_pad / BM;
+  SPEX_RETURN_IF(grid > 0x7fffffffLL, SPEX_E_TOOBIG);
+  kernel<<<(unsigned)grid, kThreads, smem, st>>>(args...);
+  count_launch();
+  return check_last();
+}
+
 }  // namespace tcgen05
 }  // namespace spex

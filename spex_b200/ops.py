@@ -874,21 +874,8 @@ def score_topk_f16(Uh, u_meta, B, B_pad, Ih, i_meta, m_items, m_pad, D, k, user_
                    mask_rowptr=None, mask_col=None, out_idx=None, out_val=None):
     """tcgen05 fp16-accumulator filter + exact fp32 re-score, fused mask + per-row top-k
     (D = 64 or 128; NGCF_SPEX/code/utility/batch_test.py:158 semantics + ranking)."""
-    _need_cuda(Uh, Ih)
-    if not 1 <= k <= TC_MAX_K:
-        raise ValueError(f"score_topk_f16: k must be in [1, {TC_MAX_K}] (use score_topk_f32 beyond)")
-    if D not in SCORER_LIMITS["f16"][0]:
-        raise ValueError("score_topk_f16: D must be 64 or 128 (use score_topk_f32 otherwise)")
-    dev = Uh.device
-    if out_idx is None:
-        out_idx = torch.empty(B, k, dtype=torch.int32, device=dev)
-    if out_val is None:
-        out_val = torch.empty(B, k, dtype=torch.float32, device=dev)
-    uid = None if user_ids is None else _i64c(user_ids, dev)
-    call("spex_score_topk_f16", ptr(Uh), ptr(Ih), int(D), B, B_pad, m_items, m_pad, ptr(u_meta),
-         ptr(i_meta), ptr(uid), ptr(mask_rowptr), ptr(mask_col), int(k), ptr(out_idx), ptr(out_val),
-         stream_ptr())
-    return out_idx, out_val
+    return _score_topk_f16(False, Uh, u_meta, B, B_pad, Ih, i_meta, m_items, m_pad, D, k, user_ids, mask_rowptr,
+                           mask_col, out_idx, out_val)
 
 
 def score_topk_f16_wide(Uh, u_meta, B, B_pad, Ih, i_meta, m_items, m_pad, D, k, user_ids=None,
@@ -896,23 +883,33 @@ def score_topk_f16_wide(Uh, u_meta, B, B_pad, Ih, i_meta, m_items, m_pad, D, k, 
     """score_topk_f16 for 1 <= k <= WIDE_MAX_K: the same operands and output contract, each user row's
     candidate buffer in a device workspace (allocated here, B_pad * (2k + 64) * 8 bytes) instead of shared
     memory."""
+    return _score_topk_f16(True, Uh, u_meta, B, B_pad, Ih, i_meta, m_items, m_pad, D, k, user_ids, mask_rowptr,
+                           mask_col, out_idx, out_val)
+
+
+def _score_topk_f16(wide, Uh, u_meta, B, B_pad, Ih, i_meta, m_items, m_pad, D, k, user_ids, mask_rowptr, mask_col,
+                    out_idx, out_val):
+    name = "score_topk_f16_wide" if wide else "score_topk_f16"
     _need_cuda(Uh, Ih)
-    dims, max_k = SCORER_LIMITS["f16"]
+    dims, max_k = SCORER_LIMITS["f16"][0], SCORER_LIMITS["f16"][1] if wide else TC_MAX_K
     if not 1 <= k <= max_k:
-        raise ValueError(f"score_topk_f16_wide: k must be in [1, {max_k}]")
+        raise ValueError(f"{name}: k must be in [1, {max_k}]" + ("" if wide else " (use score_topk_f32 beyond)"))
     if D not in dims:
-        raise ValueError("score_topk_f16_wide: D must be 64 or 128 (use score_topk_f32 otherwise)")
+        raise ValueError(f"{name}: D must be 64 or 128 (use score_topk_f32 otherwise)")
     dev = Uh.device
     if out_idx is None:
         out_idx = torch.empty(B, k, dtype=torch.int32, device=dev)
     if out_val is None:
         out_val = torch.empty(B, k, dtype=torch.float32, device=dev)
     uid = None if user_ids is None else _i64c(user_ids, dev)
-    nbytes = int(call("spex_score_topk_f16_wide_workspace_bytes", int(B_pad), int(k)))
-    work = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=dev)
-    call("spex_score_topk_f16_wide", ptr(Uh), ptr(Ih), int(D), B, B_pad, m_items, m_pad, ptr(u_meta),
-         ptr(i_meta), ptr(uid), ptr(mask_rowptr), ptr(mask_col), int(k), ptr(out_idx), ptr(out_val),
-         ptr(work), nbytes, stream_ptr())
+    args = (ptr(Uh), ptr(Ih), int(D), B, B_pad, m_items, m_pad, ptr(u_meta), ptr(i_meta), ptr(uid), ptr(mask_rowptr),
+            ptr(mask_col), int(k), ptr(out_idx), ptr(out_val))
+    if wide:
+        nbytes = int(call("spex_score_topk_f16_wide_workspace_bytes", int(B_pad), int(k)))
+        work = torch.empty(max(nbytes, 16), dtype=torch.uint8, device=dev)
+        call("spex_score_topk_f16_wide", *args, ptr(work), nbytes, stream_ptr())
+    else:
+        call("spex_score_topk_f16", *args, stream_ptr())
     return out_idx, out_val
 
 
@@ -1021,15 +1018,23 @@ class FullRanker:
             pass
         return idx, val
 
+    def _pack_items(self, scorer):
+        """Pack the item table for `scorer` ("f16" or "bf16", this ranker's precision) on the first call that needs
+        it: self._Ih / self._imeta or self._Ib, and self._m_pad."""
+        if self._m_pad is not None:
+            return
+        if scorer == "f16":
+            self._Ih, self._m_pad, self._imeta = pack_f16(self._I, None, TC_ITEM_MULTIPLE)
+        else:
+            self._Ib, self._m_pad = pack_bf16(self._I, None, TC_ITEM_MULTIPLE)
+
     def _ranked_blocks(self, scorer, U_all, users, k, mask_rowptr, mask_col, step, dest):
         """Rank users[s: s + step] for s = 0, step, 2 step, ... with `scorer` into the (idx, val) [n, k] views
         dest(s, n) and yield (s, idx view) after each block's launches."""
         m, D = self.m_items, self.D
         B = users.numel()
-        if scorer == "f16" and self._m_pad is None:
-            self._Ih, self._m_pad, self._imeta = pack_f16(self._I, None, TC_ITEM_MULTIPLE)
-        elif scorer == "bf16" and self._m_pad is None:
-            self._Ib, self._m_pad = pack_bf16(self._I, None, TC_ITEM_MULTIPLE)
+        if scorer != "fp32":
+            self._pack_items(scorer)
         if scorer == "f16":
             step = (step + TC_USER_MULTIPLE - 1) // TC_USER_MULTIPLE * TC_USER_MULTIPLE
             if B:
@@ -1062,10 +1067,7 @@ class FullRanker:
         dev = self.device
         users = _i64c(users, dev)
         B = users.numel()
-        trp = _i64c(truth_rowptr, dev)
-        tcol = torch.as_tensor(np.asarray(truth_col) if not torch.is_tensor(truth_col) else truth_col)
-        tcol = tcol.to(device=dev, dtype=torch.int32).contiguous()
-        check_truth_csr(trp, tcol, B)
+        trp, tcol = self._truth_csr(truth_rowptr, truth_col, B)
         scorer = self.scorer_for(k, U_all, users if probe_users is None else probe_users)
         if tcol.numel() == 0:
             tcol = torch.zeros(1, dtype=torch.int32, device=dev)   # all rows empty: never read, but not NULL
@@ -1087,9 +1089,7 @@ class FullRanker:
             n = o_i.shape[0]
             call("spex_fullrank_metrics", ptr(o_i), n, k, ptr(trp[s:]), ptr(tcol), cut_host, n_cut, ptr(disc),
                  ptr(idcg), ptr(None if pu is None else pu[s:]), ptr(chunk_sums[s // METRICS_CHUNK:]), stream_ptr())
-        sums = torch.empty(n_cut, 4, dtype=torch.float64, device=dev)
-        call("spex_fullrank_metrics_reduce", ptr(chunk_sums), n_chunks, n_cut, ptr(sums), stream_ptr())
-        return sums, pu
+        return _reduce_chunks(chunk_sums, n_cut), pu
 
     def evaluate(self, U_all, users, cutoffs, truth_rowptr, truth_col, mask_rowptr=None, mask_col=None,
                  user_block=None, per_user=False, probe_users=None):
@@ -1109,6 +1109,15 @@ class FullRanker:
                                     user_block, per_user, probe_users)
         return metric_means(sums.cpu().numpy(), users.numel(), pu)
 
+    def _truth_csr(self, truth_rowptr, truth_col, B):
+        """(rowptr int64, col int32) of a truth CSR over B users on the device; ValueError unless check_truth_csr
+        accepts it."""
+        trp = _i64c(truth_rowptr, self.device)
+        tcol = torch.as_tensor(np.asarray(truth_col) if not torch.is_tensor(truth_col) else truth_col)
+        tcol = tcol.to(device=self.device, dtype=torch.int32).contiguous()
+        check_truth_csr(trp, tcol, B)
+        return trp, tcol
+
     def _check_items(self, items):
         items = torch.as_tensor(items).to(device=self.device, dtype=torch.int64)
         if items.numel() and bool((items.min() < 0) | (items.max() >= self.m_items)):
@@ -1124,8 +1133,7 @@ class FullRanker:
         if P == 0:
             return out
         if scorer == "f16":
-            if self._m_pad is None:
-                self._Ih, self._m_pad, self._imeta = pack_f16(self._I, None, TC_ITEM_MULTIPLE)
+            self._pack_items(scorer)
             Uh, _, _ = pack_f16(U_all, urows)
         for s in range(0, P, RANK_PAIR_BLOCK):
             e = min(s + RANK_PAIR_BLOCK, P)
@@ -1172,10 +1180,7 @@ class FullRanker:
         dev = self.device
         users = _i64c(users, dev)
         B = users.numel()
-        trp = _i64c(truth_rowptr, dev)
-        tcol = torch.as_tensor(np.asarray(truth_col) if not torch.is_tensor(truth_col) else truth_col)
-        tcol = tcol.to(device=dev, dtype=torch.int32).contiguous()
-        check_truth_csr(trp, tcol, B)
+        trp, tcol = self._truth_csr(truth_rowptr, truth_col, B)
         scorer = self.scorer_for(None, U_all, users if probe_users is None else probe_users)
         a = int(trp[0]) if B else 0
         tcol = self._check_items(tcol[a: int(trp[-1])] if B else tcol[:0])
@@ -1195,10 +1200,7 @@ class FullRanker:
         call("spex_rank_metrics", ptr(ranks), B, ptr(trp), ptr(tcol), ptr(users), ptr(mask_rowptr), ptr(mask_col),
              self.m_items, (C.c_int32 * n_cut)(*cutoffs), n_cut, ptr(disc), ptr(idcg), ptr(chunk_sums),
              ptr(chunk_extra), stream_ptr())
-        sums = torch.empty(n_cut, 4, dtype=torch.float64, device=dev)
-        extra = torch.empty(1, 4, dtype=torch.float64, device=dev)
-        call("spex_fullrank_metrics_reduce", ptr(chunk_sums), n_chunks, n_cut, ptr(sums), stream_ptr())
-        call("spex_fullrank_metrics_reduce", ptr(chunk_extra), n_chunks, 1, ptr(extra), stream_ptr())
+        sums, extra = _reduce_chunks(chunk_sums, n_cut), _reduce_chunks(chunk_extra, 1)
         out = metric_means(sums.cpu().numpy(), B)
         ex = extra.cpu().numpy()[0] / max(float(B), 1.0)
         out["mrr"], out["auc"] = float(ex[0]), float(ex[1])
@@ -1210,6 +1212,14 @@ METRICS_MAX_CUTOFFS = 8        # SPEX_METRICS_MAX_CUTOFFS
 METRIC_NAMES = ("recall", "precision", "ndcg", "hit")
 EVAL_USER_BLOCK = 148 * METRICS_CHUNK   # users ranked per block by FullRanker.evaluate (None)
 RANK_PAIR_BLOCK = 1 << 22      # pairs per rank launch of FullRanker.ranks / rank_metrics
+
+
+def _reduce_chunks(chunk_sums, n_cut):
+    """fp64 [n_cut, 4]: the [n_chunks, n_cut, 4] chunk sums summed over the chunks in ascending order, on the
+    device."""
+    sums = torch.empty(n_cut, 4, dtype=torch.float64, device=chunk_sums.device)
+    call("spex_fullrank_metrics_reduce", ptr(chunk_sums), chunk_sums.shape[0], n_cut, ptr(sums), stream_ptr())
+    return sums
 
 
 def check_cutoffs(cutoffs):
