@@ -227,6 +227,8 @@ int spex_edge_dropout_f32(const int64_t* rowptr, const int32_t* col, const float
  *   gamma     fp32 [B]   (always written; flag=1 of forward() returns it)
  *   loss      fp32 [1]   (NULL to skip: then labels may be NULL too)
  *   dgamma    fp32 [B]   dloss/dgamma = (sigmoid(gamma)-label)/B   (NULL to skip)
+ * B == 0: loss = NaN (the mean of no terms, as BCEWithLogitsLoss gives), nothing else is written, and the
+ * per-sample arrays (users, items, labels, gamma, dgamma) may be NULL.
  */
 int spex_bce_fwd_f32(const float* U, const float* I, int32_t D,
                      const int64_t* users, const int64_t* items, const float* labels,
@@ -242,6 +244,8 @@ int spex_bce_fwd_f32(const float* U, const float* I, int32_t D,
  * aligned, >= spex_scatter_workspace_bytes(max list length) bytes; list length: B for BCE, 2B for
  * BPR): a stable radix sort of (row, position) pairs + one warp per run, which pays from a few
  * thousand samples on - same summation order (ascending batch position), bit-identical gradients.
+ * B == 0 writes nothing; the per-sample arrays may then be NULL (also in spex_scatter_rows_f32 and
+ * spex_bpr_bwd_ws_f32).
  */
 int64_t spex_scatter_workspace_bytes(int64_t total_entries);
 int spex_bce_bwd_ws_f32(const float* U, const float* I, int32_t D,
@@ -275,6 +279,7 @@ int spex_scatter_rows_f32(const int64_t* dst_rows, const int64_t* src_rows, cons
  *   loss = mean softplus(<u,n> - <u,p>),  reg = 0.5*(|U0[u]|^2+|I0[p]|^2+|I0[n]|^2)/B
  *   out2 fp32 [2] = {loss, reg};  dscore fp32 [B] = sigmoid(<u,n>-<u,p>)/B  (NULL to skip)
  *   work2B fp32 [2*B] workspace (per-sample terms, reduced in a fixed order)
+ * B == 0: out2 = {NaN, NaN} (means of no terms); users, pos, neg, dscore and work2B may be NULL.
  */
 int spex_bpr_fwd_f32(const float* U, const float* I, const float* U0, const float* I0, int32_t D,
                      const int64_t* users, const int64_t* pos, const int64_t* neg, int64_t B,

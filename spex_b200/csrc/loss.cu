@@ -545,18 +545,20 @@ using namespace spex;
 extern "C" int spex_bce_fwd_f32(const float* U, const float* I, int32_t D, const int64_t* users,
                                 const int64_t* items, const float* labels, int64_t B, float* gamma,
                                 float* loss, float* dgamma, void* stream) {
-  SPEX_RETURN_IF(!U || !I || !users || !items || !gamma || B < 0, SPEX_E_BADARG);
-  SPEX_RETURN_IF((loss || dgamma) && !labels, SPEX_E_BADARG);
+  SPEX_RETURN_IF(!U || !I || B < 0, SPEX_E_BADARG);
+  SPEX_RETURN_IF(B > 0 && (!users || !items || !gamma || ((loss || dgamma) && !labels)), SPEX_E_BADARG);
   SPEX_CHECK_TABLE(D);
   SPEX_RETURN_IF(!aligned16(U) || !aligned16(I), SPEX_E_ALIGN);
   SPEX_RETURN_IF(B > 0x7fffffffLL, SPEX_E_TOOBIG);
-  if (B == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
-  if (D <= 128)
-    bce_fwd_kernel<1><<<warp_grid(B), kWarpsPerCta * 32, 0, st>>>(U, I, D, users, items, labels, B, gamma, dgamma);
-  else
-    bce_fwd_kernel<4><<<warp_grid(B), kWarpsPerCta * 32, 0, st>>>(U, I, D, users, items, labels, B, gamma, dgamma);
-  count_launch();
+  // an empty batch still runs the reduce: the mean of no terms is 0/0 = NaN, as in BCEWithLogitsLoss
+  if (B > 0) {
+    if (D <= 128)
+      bce_fwd_kernel<1><<<warp_grid(B), kWarpsPerCta * 32, 0, st>>>(U, I, D, users, items, labels, B, gamma, dgamma);
+    else
+      bce_fwd_kernel<4><<<warp_grid(B), kWarpsPerCta * 32, 0, st>>>(U, I, D, users, items, labels, B, gamma, dgamma);
+    count_launch();
+  }
   if (loss) {
     bce_loss_reduce_kernel<<<1, 1024, 0, st>>>(gamma, labels, B, loss);
     count_launch();
@@ -598,8 +600,8 @@ extern "C" int spex_scatter_rows_f32(const int64_t* dst_rows, const int64_t* src
                                      const float* gscalar, float cconst, int64_t B, const float* src, int32_t D,
                                      float* out, int64_t row_lo, int64_t row_hi, void* work, int64_t work_bytes,
                                      void* stream) {
-  SPEX_RETURN_IF(!dst_rows || !src_rows || !src || !out || B < 0 || row_lo < 0 || (row_hi != 0 && row_hi < row_lo),
-                 SPEX_E_BADARG);
+  SPEX_RETURN_IF(!src || !out || B < 0 || row_lo < 0 || (row_hi != 0 && row_hi < row_lo), SPEX_E_BADARG);
+  SPEX_RETURN_IF(B > 0 && (!dst_rows || !src_rows), SPEX_E_BADARG);
   SPEX_CHECK_TABLE(D);
   SPEX_RETURN_IF(!aligned16(src) || !aligned16(out), SPEX_E_ALIGN);
   ScatterList L{};
@@ -620,7 +622,8 @@ extern "C" int spex_bce_bwd_ws_f32(const float* U, const float* I, int32_t D, co
                                    const int64_t* items, const float* dgamma, const float* grad_loss,
                                    int64_t B, float* gU, float* gI, void* work, int64_t work_bytes,
                                    void* stream) {
-  SPEX_RETURN_IF(!U || !I || !users || !items || !dgamma || !gU || !gI || B < 0, SPEX_E_BADARG);
+  SPEX_RETURN_IF(!U || !I || !gU || !gI || B < 0, SPEX_E_BADARG);
+  SPEX_RETURN_IF(B > 0 && (!users || !items || !dgamma), SPEX_E_BADARG);
   SPEX_CHECK_TABLE(D);
   SPEX_RETURN_IF(!aligned16(U) || !aligned16(I) || !aligned16(gU) || !aligned16(gI), SPEX_E_ALIGN);
   cudaStream_t st = (cudaStream_t)stream;
@@ -646,19 +649,22 @@ extern "C" int spex_bpr_fwd_f32(const float* U, const float* I, const float* U0,
                                 int32_t D, const int64_t* users, const int64_t* pos,
                                 const int64_t* neg, int64_t B, float* out2, float* dscore,
                                 float* work2B, void* stream) {
-  SPEX_RETURN_IF(!U || !I || !U0 || !I0 || !users || !pos || !neg || !out2 || !work2B || B < 0,
-                 SPEX_E_BADARG);
+  SPEX_RETURN_IF(!U || !I || !U0 || !I0 || !out2 || B < 0, SPEX_E_BADARG);
+  SPEX_RETURN_IF(B > 0 && (!users || !pos || !neg || !work2B), SPEX_E_BADARG);
   SPEX_CHECK_TABLE(D);
   SPEX_RETURN_IF(!aligned16(U) || !aligned16(I) || !aligned16(U0) || !aligned16(I0), SPEX_E_ALIGN);
   SPEX_RETURN_IF(B > 0x7fffffffLL, SPEX_E_TOOBIG);
-  if (B == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
-  if (D <= 128)
-    bpr_fwd_kernel<1><<<warp_grid(B), kWarpsPerCta * 32, 0, st>>>(U, I, U0, I0, D, users, pos, neg, B, dscore, work2B);
-  else
-    bpr_fwd_kernel<4><<<warp_grid(B), kWarpsPerCta * 32, 0, st>>>(U, I, U0, I0, D, users, pos, neg, B, dscore, work2B);
+  // an empty batch still runs the reduce: both means of no terms are 0/0 = NaN
+  if (B > 0) {
+    if (D <= 128)
+      bpr_fwd_kernel<1><<<warp_grid(B), kWarpsPerCta * 32, 0, st>>>(U, I, U0, I0, D, users, pos, neg, B, dscore, work2B);
+    else
+      bpr_fwd_kernel<4><<<warp_grid(B), kWarpsPerCta * 32, 0, st>>>(U, I, U0, I0, D, users, pos, neg, B, dscore, work2B);
+    count_launch();
+  }
   pair_mean_reduce_kernel<<<1, 1024, 0, st>>>(work2B, B, out2);
-  count_launch(2);
+  count_launch();
   return check_last();
 }
 
@@ -667,7 +673,8 @@ extern "C" int spex_bpr_bwd_ws_f32(const float* U, const float* I, const float* 
                                    const int64_t* neg, const float* dscore, const float* grad2,
                                    int64_t B, float* gU, float* gI, float* gU0, float* gI0, void* work,
                                    int64_t work_bytes, void* stream) {
-  SPEX_RETURN_IF(!U || !I || !U0 || !I0 || !users || !pos || !neg || !dscore || B < 0, SPEX_E_BADARG);
+  SPEX_RETURN_IF(!U || !I || !U0 || !I0 || B < 0, SPEX_E_BADARG);
+  SPEX_RETURN_IF(B > 0 && (!users || !pos || !neg || !dscore), SPEX_E_BADARG);
   SPEX_RETURN_IF(!gU || !gI || !gU0 || !gI0, SPEX_E_BADARG);
   SPEX_CHECK_TABLE(D);
   SPEX_RETURN_IF(!aligned16(U) || !aligned16(I) || !aligned16(U0) || !aligned16(I0), SPEX_E_ALIGN);
