@@ -88,7 +88,7 @@ class PartitionedPropagator:
         self.timing = None        # set to [] to collect per-phase CUDA-event pairs (bring-up)
         self._mc = None           # multicast pointers of the tables (mode "mcast")
         self._symm = []
-        self._nnz_global = None   # nnz of the whole matrix (receptive_sets)
+        self._nnz_global = None   # nnz of the whole matrix (receptive_plan)
         self._slot = 0            # ring slot that holds / receives E^(0) of the next propagate()
         self._staged = None       # (key, event): E^(0) already published into slot self._slot
         self._side = None         # high-priority stream of the background publish
@@ -320,34 +320,26 @@ class PartitionedPropagator:
         every rank passes before that propagate(): peers push into the slot only afterwards."""
         self._X[(self._slot + j) % self.n_tables].zero_()
 
-    def receptive_sets(self, S: torch.Tensor):
-        """ops.receptive_rows over the partition: R[k] (global row ids, identical on every rank) = the rows of
-        E^(k) that the rows S of the layer mean depend on, or None = all rows.  Every rank expands the rows it
-        owns through its own CSR block (the columns are global ids); the lists are all-gathered."""
+    def receptive_plan(self, S: torch.Tensor):
+        """ops.receptive_plan over the partition: its sets R[k] are global row ids, identical on every rank.  Every
+        rank measures and expands the rows it owns through its own CSR block (the columns are global ids); the
+        degree sums are summed and the neighbour lists all-gathered over the ranks.  Outside the fused modes
+        every set is None."""
         from . import ops
 
-        K = self.K
-        R = [None] * (K + 1)
-        if (K < 1 or self.mode not in ("push", "mcast") or self.local_spmm is not None
+        if (self.K < 1 or self.mode not in ("push", "mcast") or self.local_spmm is not None
                 or self.D not in (32, 64, 128)):
-            return R
+            return ops.ReceptivePlan(self.K, 0)
         if self._nnz_global is None:
             self._nnz_global = self._sum_over_ranks(self.g.nnz)
-        nnz = self._nnz_global
-        d = self._sum_over_ranks(self.g.degree_sum(self._own(S)))
-        if d > ops.SUBSET_MAX_EDGE_FRAC * nnz:
-            return R
-        R[K] = S
-        cur = S
-        for k in range(K - 1, 0, -1):
-            if d > ops.EXPAND_MAX_EDGE_FRAC * nnz:
-                break
-            cand = torch.unique(torch.cat([S, self._all_gather_var(self.g.neighbors(self._own(cur)))]))
-            d = self._sum_over_ranks(self.g.degree_sum(self._own(cand)))
-            if d > ops.SUBSET_MAX_EDGE_FRAC * nnz:
-                break
-            R[k] = cur = cand
-        return R
+        return ops.receptive_plan(S, self.K, self._nnz_global,
+                                  lambda rows: self._sum_over_ranks(self.g.degree_sum(self._own(rows))),
+                                  lambda rows: self._all_gather_var(self.g.neighbors(self._own(rows))))
+
+    def receptive_sets(self, S: torch.Tensor):
+        """R[k] of receptive_plan(S): the rows of E^(k) that the rows S of the layer mean depend on, or None = all
+        rows."""
+        return self.receptive_plan(S).R
 
     def propagate(self, E0_local: torch.Tensor, out: torch.Tensor = None,
                   next_E0_local: torch.Tensor = None, next_ready=None, first_full: torch.Tensor = None,
@@ -606,30 +598,24 @@ class PartitionedTrainer:
         # forward restricted to the batch's receptive field (fused modes; every computed row is bit-identical to
         # the full computer(), so loss, gradients and weights are unchanged): layer K on the batch's rows, layer
         # K-1 on their neighbours, ...; the backward mirrors it (below)
-        sets = p.receptive_sets(torch.unique(rows)) if (self.receptive_field and self.fused) else None
-        out = p.propagate(self.W, out=self.out, row_sets=sets)
+        plan = p.receptive_plan(torch.unique(rows)) if (self.receptive_field and self.fused) else None
+        out = p.propagate(self.W, out=self.out, row_sets=None if plan is None else plan.R)
         R = self.ops.gather_owned(out, rows, r0, r1)
-        # backward mirror of the receptive field: H_j = g + A^T H_{j-1} is non-zero only on sets[K - j], so layer j
-        # (j < K) computes and exchanges those rows into a zeroed table (zeroed here, before the all-reduce that
-        # orders it ahead of every peer's stores)
+        # backward mirror of the receptive field (plan.backward_layer): layer j (j < K) computes and exchanges its
+        # rows into a zeroed table (zeroed here, before the all-reduce that orders it ahead of every peer's stores);
+        # the last layer is the fused Adam kernel: dense and unmasked
         bsets = bmasks = None
-        if sets is not None and self.fused and self.receptive_backward:
+        if plan is not None and self.receptive_backward:
             from . import ops
 
             bsets = [None] * (p.K + 1)
             bmasks = [None] * (p.K + 1)
-            x_rows = sets[p.K]                       # layer 1 reads the gradient table: non-zero on the batch rows
-            for j in range(1, p.K):                  # (the last layer is the fused Adam kernel: dense)
+            for j in range(1, p.K):
+                bsets[j], x_rows = plan.backward_layer(j)
                 if x_rows is not None:
-                    d = p._sum_over_ranks(p.g.degree_sum(p._own(x_rows)))
-                    if d <= ops.SPARSE_INPUT_MAX_EDGE_FRAC * p._nnz_global:
-                        bmasks[j] = ops.nonzero_mask(p.N, x_rows)
-                if sets[p.K - j] is not None:
-                    bsets[j] = sets[p.K - j]
+                    bmasks[j] = ops.nonzero_mask(p.N, x_rows)
+                if bsets[j] is not None:
                     p.zero_slot(j)
-                    x_rows = sets[p.K - j]           # the next layer reads a zeroed table holding these rows
-                else:
-                    x_rows = None
         if p.world > 1:
             dist.all_reduce(R, group=p.group)
         Ru, Ri = R[:B], R[B:]

@@ -477,118 +477,120 @@ SUBSET_MAX_EDGE_FRAC = 0.5
 EXPAND_MAX_EDGE_FRAC = 0.02
 
 
-def receptive_rows(graph: DeviceGraph, S: torch.Tensor, K: int):
-    """R[k], k = 1..K: the rows of E^(k) that the rows S of the layer mean depend on - R[K] = S,
-    R[k] = S + neighbours(R[k+1]) - or None = all rows, from the first set that outgrows the limits on."""
-    R = [None] * (K + 1)
-    if K < 1 or graph.degree_sum(S) > SUBSET_MAX_EDGE_FRAC * graph.nnz:
-        return R
-    R[K] = S
+class ReceptivePlan:
+    """receptive_plan's result.  R[k], k = 1..K: the rows of E^(k) that the rows S = R[K] of the layer mean depend
+    on, or None = all rows; edges[k]: the edge count of R[k].  R[0] and edges[0] are None."""
+
+    def __init__(self, K: int, nnz: int):
+        self.R, self.edges, self.nnz = [None] * (K + 1), [None] * (K + 1), nnz
+
+    def backward_layer(self, j: int):
+        """(rows, x_rows) of backward layer j = 1..K.  H_j = g + A^T H_{j-1} is non-zero only on rows = R[K-j]
+        (None = all; always for j = K).  x_rows = R[K-j+1], the rows of H_{j-1} that may be non-zero, is given only
+        while they hold at most SPARSE_INPUT_MAX_EDGE_FRAC of nnz(A): the layer then skips the other rows' gathers."""
+        k = len(self.R) - j
+        sparse = self.edges[k] is not None and self.edges[k] <= SPARSE_INPUT_MAX_EDGE_FRAC * self.nnz
+        return self.R[k - 1], (self.R[k] if sparse else None)
+
+
+def receptive_plan(S: torch.Tensor, K: int, nnz: int, degree_sum, neighbors) -> ReceptivePlan:
+    """The rows each layer computes when only the rows S (sorted unique int64 ids) of the layer mean are read:
+    R[K] = S, R[k] = S + neighbours(R[k+1]), each set None = all rows from the first one that outgrows the limits
+    on.  `degree_sum(rows) -> int` and `neighbors(rows) -> int64 ids` query one graph, or a row partition's blocks
+    summed / gathered over the ranks; nnz = nnz(A)."""
+    plan = ReceptivePlan(K, nnz)
+    R, edges = plan.R, plan.edges
+    if K < 1 or (d := degree_sum(S)) > SUBSET_MAX_EDGE_FRAC * nnz:
+        return plan
+    R[K], edges[K] = S, d
     for k in range(K - 1, 0, -1):
-        if graph.degree_sum(R[k + 1]) > EXPAND_MAX_EDGE_FRAC * graph.nnz:
+        if edges[k + 1] > EXPAND_MAX_EDGE_FRAC * nnz:
             break
-        cand = torch.unique(torch.cat([S, graph.neighbors(R[k + 1])]))
-        if graph.degree_sum(cand) > SUBSET_MAX_EDGE_FRAC * graph.nnz:
+        cand = torch.unique(torch.cat([S, neighbors(R[k + 1])]))
+        d = degree_sum(cand)
+        if d > SUBSET_MAX_EDGE_FRAC * nnz:
             break
-        R[k] = cand
-    return R
+        R[k], edges[k] = cand, d
+    return plan
 
 
-class _PropagateMeanRows(torch.autograd.Function):
-    """_PropagateMean for a training step whose loss reads only the rows S of the result: every layer is
-    computed on the rows the batch depends on (receptive_rows) with the same kernels and epilogues, so the
-    rows S of `out`, the loss and dE0 are bit-identical to the full computation; the other rows of `out`
-    are NOT valid.  Backward contract: the incoming gradient is zero outside the rows S."""
+def receptive_rows(graph: DeviceGraph, S: torch.Tensor, K: int):
+    """R[k], k = 1..K, of receptive_plan over `graph`."""
+    return receptive_plan(S, K, graph.nnz, graph.degree_sum, graph.neighbors).R
+
+
+class _PropagateMean(torch.autograd.Function):
+    """out = mean_k A^k E0 over the fused [N, D] table (model.py:66-97), backward through A^T.
+
+    With a ReceptivePlan whose R[K] is set (a training step whose loss reads only the rows S = R[K] of the
+    result), every layer is computed on the rows the batch depends on with the same kernels and epilogues, so
+    the rows S of `out`, the loss and dE0 are bit-identical to the full computation; the other rows of `out`
+    are NOT valid.  Backward contract: the incoming gradient is then zero outside the rows S."""
 
     @staticmethod
-    def forward(ctx, table, graph: DeviceGraph, K: int, val, valT, S):
+    def forward(ctx, table, graph: DeviceGraph, K: int, val, valT, plan):
         _need_cuda(table)
         E0 = _f32c(table)
         N, D = E0.shape
-        R = receptive_rows(graph, S, K)
-        subs = [None if r is None else graph.row_subset(r) for r in R]
         out = torch.empty_like(E0) if not workspaces.enabled else workspaces.get("prop_out", E0.shape, E0.device)[0]
         tmp = [workspaces.get("prop_tmp0", E0.shape, E0.device)[0] if K >= 2 else None,
                workspaces.get("prop_tmp1", E0.shape, E0.device)[0] if K >= 3 else None]
         v = graph.val if val is None else val
-        inv = 1.0 / float(K + 1)
-        X = E0
-        for k in range(1, K + 1):
-            last = k == K
-            Y = None if last else tmp[(k - 1) & 1]
-            kw = dict(Y=Y, addend=E0 if k == 1 else out, addend_scale=1.0, Z=out, z_scale=inv if last else 1.0, val=v)
-            if subs[k] is None:
-                spmm(graph, X, **kw)
-            else:
-                spmm_rows(graph, X, subs[k], **kw)
-            X = Y
-        ctx.graph, ctx.K, ctx.valT, ctx.subs, ctx.R = graph, K, (v if valT is None else valT), subs, R
+        # R[K] None: no layer is restricted and no backward input is masked - the two fused calls
+        restricted = plan is not None and plan.R[K] is not None
+        subs = [None if r is None else graph.row_subset(r) for r in plan.R] if restricted else None
+        if subs is None:
+            call("spex_propagate_mean_f32", ptr(graph.rowptr), ptr(graph.col), ptr(v), ptr(E0), N, D, K,
+                 ptr(out), ptr(tmp[0]), ptr(tmp[1]), graph.plan(D), stream_ptr())
+        else:
+            inv = 1.0 / float(K + 1)
+            X = E0
+            for k in range(1, K + 1):
+                last = k == K
+                Y = None if last else tmp[(k - 1) & 1]
+                kw = dict(Y=Y, addend=E0 if k == 1 else out, addend_scale=1.0, Z=out, z_scale=inv if last else 1.0,
+                          val=v)
+                if subs[k] is None:
+                    spmm(graph, X, **kw)
+                else:
+                    spmm_rows(graph, X, subs[k], **kw)
+                X = Y
+        ctx.graph, ctx.K, ctx.valT, ctx.plan, ctx.subs = graph, K, (v if valT is None else valT), plan, subs
         return out
 
     @staticmethod
     def backward(ctx, g):
-        graph, K, subs, R = ctx.graph, ctx.K, ctx.subs, ctx.R
+        graph, K, plan, subs = ctx.graph, ctx.K, ctx.plan, ctx.subs
         g = _f32c(g)
         N, D = g.shape
         dE0 = torch.empty_like(g) if not workspaces.enabled else workspaces.get("prop_dE0", g.shape, g.device)[0]
         tmp = [workspaces.get("prop_tmp0", g.shape, g.device)[0] if K >= 2 else None,
                workspaces.get("prop_tmp1", g.shape, g.device)[0] if K >= 3 else None]
+        if subs is None:
+            call("spex_propagate_mean_bwd_f32", ptr(graph.rowptr), ptr(graph.col), ptr(ctx.valT), ptr(g),
+                 N, D, K, ptr(dE0), ptr(tmp[0]), ptr(tmp[1]), graph.plan(D), stream_ptr())
+            return dE0, None, None, None, None, None
         inv = 1.0 / float(K + 1)
-        # H_0 = g; H_j = g + A^T H_{j-1}, non-zero only on R[K - j]: a restricted layer writes its rows into a
-        # zero table (zero-filled once; afterwards only the rows of the previous step are cleared)
+        # H_0 = g; H_j = g + A^T H_{j-1}: a restricted layer writes its rows into a zero table (zero-filled once;
+        # afterwards only the rows of the previous step are cleared)
         X = g
-        x_rows = R[K]              # rows of X that may be non-zero (None: dense)
         for j in range(1, K + 1):
             last = j == K
-            sub = subs[K - j] if j < K else None
             kw = dict(addend=g, addend_scale=1.0, z_scale=inv if last else 1.0, val=ctx.valT)
-            mask = None
-            if x_rows is not None and graph.degree_sum(x_rows) <= SPARSE_INPUT_MAX_EDGE_FRAC * graph.nnz:
-                mask = nonzero_mask(N, x_rows)       # most gathers of this layer would fetch zero rows: skip them
-            if sub is None:
+            rows, x_rows = plan.backward_layer(j)
+            mask = None if x_rows is None else nonzero_mask(N, x_rows)
+            if rows is None:
                 Z = dE0 if last else tmp[(j - 1) & 1]
                 if mask is None:
                     spmm(graph, X, Z=Z, **kw)
                 else:
                     spmm_rows(graph, X, None, Z=Z, x_nonzero=mask, **kw)
-                x_rows = None
             else:
                 Z, zkey = workspaces.get(f"prop_bwd_rows{j}", g.shape, g.device, zero=True)
-                spmm_rows(graph, X, sub, Z=Z, x_nonzero=mask, **kw)
-                workspaces.mark(zkey, R[K - j])
-                x_rows = R[K - j]
+                spmm_rows(graph, X, subs[K - j], Z=Z, x_nonzero=mask, **kw)
+                workspaces.mark(zkey, rows)
             X = Z
         return dE0, None, None, None, None, None
-
-
-class _PropagateMean(torch.autograd.Function):
-    """out = mean_k A^k E0 over the fused [N, D] table (model.py:66-97), backward through A^T."""
-
-    @staticmethod
-    def forward(ctx, table, graph: DeviceGraph, K: int, val, valT):
-        _need_cuda(table)
-        E0 = _f32c(table)
-        N, D = E0.shape
-        out = torch.empty_like(E0) if not workspaces.enabled else workspaces.get("prop_out", E0.shape, E0.device)[0]
-        tmp0 = workspaces.get("prop_tmp0", E0.shape, E0.device)[0] if K >= 2 else None
-        tmp1 = workspaces.get("prop_tmp1", E0.shape, E0.device)[0] if K >= 3 else None
-        v = graph.val if val is None else val
-        call("spex_propagate_mean_f32", ptr(graph.rowptr), ptr(graph.col), ptr(v), ptr(E0), N, D, K,
-             ptr(out), ptr(tmp0), ptr(tmp1), graph.plan(D), stream_ptr())
-        ctx.graph, ctx.K, ctx.valT = graph, K, (v if valT is None else valT)
-        return out
-
-    @staticmethod
-    def backward(ctx, g):
-        graph, K = ctx.graph, ctx.K
-        g = _f32c(g)
-        N, D = g.shape
-        dE0 = torch.empty_like(g) if not workspaces.enabled else workspaces.get("prop_dE0", g.shape, g.device)[0]
-        tmp0 = workspaces.get("prop_tmp0", g.shape, g.device)[0] if K >= 2 else None
-        tmp1 = workspaces.get("prop_tmp1", g.shape, g.device)[0] if K >= 3 else None
-        call("spex_propagate_mean_bwd_f32", ptr(graph.rowptr), ptr(graph.col), ptr(ctx.valT), ptr(g),
-             N, D, K, ptr(dE0), ptr(tmp0), ptr(tmp1), graph.plan(D), stream_ptr())
-        return dE0, None, None, None, None
 
 
 def propagate_mean(table: torch.Tensor, graph: DeviceGraph, K: int,
@@ -597,13 +599,14 @@ def propagate_mean(table: torch.Tensor, graph: DeviceGraph, K: int,
     """K-layer propagation + layer mean.  `val` overrides the graph values (edge dropout); the
     backward then needs `valT` (values of the transposed matrix) unless the override is symmetric.
     `rows_needed` (int64 row ids): the caller reads - and back-propagates into - only these rows of the
-    result; the layers are then restricted to the rows they depend on (_PropagateMeanRows)."""
+    result; the layers are then restricted to the rows they depend on (receptive_plan)."""
     if graph.n_rows != graph.n_cols or table.shape[0] != graph.n_rows:
         raise ValueError("propagate_mean needs the full square adjacency and an [N, D] table")
+    plan = None
     if rows_needed is not None and int(K) >= 1 and table.shape[1] in (32, 64, 128):
-        S = torch.unique(_i64c(rows_needed, table.device))
-        return _PropagateMeanRows.apply(table, graph, int(K), val, valT, S)
-    return _PropagateMean.apply(table, graph, int(K), val, valT)
+        plan = receptive_plan(torch.unique(_i64c(rows_needed, table.device)), int(K), graph.nnz, graph.degree_sum,
+                              graph.neighbors)
+    return _PropagateMean.apply(table, graph, int(K), val, valT, plan)
 
 
 # ------------------------------------------------------------------------------------------------

@@ -1,6 +1,6 @@
-"""Receptive-field training step (spex_spmm_layer_f32, ops._PropagateMeanRows): restricting every layer to
-the rows a mini-batch depends on must not change a single bit of what the batch sees - its rows of the layer
-mean, the loss, and the gradient of the whole embedding table - against the full computer() of
+"""Receptive-field training step (spex_spmm_layer_f32, ops.receptive_plan + ops._PropagateMean): restricting
+every layer to the rows a mini-batch depends on must not change a single bit of what the batch sees - its rows
+of the layer mean, the loss, and the gradient of the whole embedding table - against the full computer() of
 LightGCN_SPEX/code/utility1/model.py:66-97 + main_rec.py:34-35, which stays the semantics."""
 import numpy as np
 import pytest
