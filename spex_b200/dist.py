@@ -33,8 +33,9 @@ skew at 8 GPUs in round 1, un-overlapped) disappears from the critical path, and
 unnecessary (every slot's previous readers are separated from its next writer by a barrier that
 already exists).
 
-The local multiply is injectable (``local_spmm``) so the orchestration can be tested on CPU with the
-oracle's SpMM under the gloo backend; the default is the CUDA kernel and there is no fallback.
+The local multiply is injectable (``local_spmm(g, X)``, and ``local_spmm(g, X, val)`` for a call with per-call
+edge values) so the orchestration can be tested on CPU with the oracle's SpMM under the gloo backend; the default
+is the CUDA kernel and there is no fallback.
 """
 from __future__ import annotations
 
@@ -197,13 +198,14 @@ class PartitionedPropagator:
 
     # ---- one layer --------------------------------------------------------------------------------
     def _layer(self, X_full, Y_local, addend, Z_local, z_scale, push_buf=None, publish=None, subset=None,
-               x_nonzero=None, adam=None):
+               x_nonzero=None, adam=None, val=None):
         """One layer over the local rows (ops.spmm_rows), restricted to `subset` / reading a table that is zero
-        outside the rows `x_nonzero` marks.  Fused modes: `push_buf` = ring slot into which the Y rows go on every
-        rank; `publish` = (src, slot): the rows of src - or, with `adam` ({p, m, v, lr, beta1, beta2, eps, step},
-        src None), the rows of p updated with the Z rows as gradient - go to ring slot `slot` on every rank."""
+        outside the rows `x_nonzero` marks, with the block's edge values `val` (None = the graph's).  Fused modes:
+        `push_buf` = ring slot into which the Y rows go on every rank; `publish` = (src, slot): the rows of src - or,
+        with `adam` ({p, m, v, lr, beta1, beta2, eps, step}, src None), the rows of p updated with the Z rows as
+        gradient - go to ring slot `slot` on every rank."""
         if self.local_spmm is not None:
-            acc = self.local_spmm(self.g, X_full)
+            acc = self.local_spmm(self.g, X_full) if val is None else self.local_spmm(self.g, X_full, val)
             if Y_local is not None:
                 Y_local.copy_(acc)
             Z_local.copy_((addend + acc) * z_scale)
@@ -220,7 +222,7 @@ class PartitionedPropagator:
         pub_mcast, pub_peers = dest(pub_slot)
         ops.spmm_rows(self.g, X_full, subset, Y=Y_local, addend=addend, Z=Z_local, z_scale=float(z_scale),
                       x_nonzero=x_nonzero, out_row_offset=self.r0, y_mcast=y_mcast, y_peers=y_peers,
-                      pub_src=pub_src, pub_mcast=pub_mcast, pub_peers=pub_peers, adam=adam)
+                      pub_src=pub_src, pub_mcast=pub_mcast, pub_peers=pub_peers, adam=adam, val=val)
 
     def _mark(self, name):
         if self.timing is not None:
@@ -343,7 +345,7 @@ class PartitionedPropagator:
 
     def propagate(self, E0_local: torch.Tensor, out: torch.Tensor = None,
                   next_E0_local: torch.Tensor = None, next_ready=None, first_full: torch.Tensor = None,
-                  adam: dict = None, row_sets=None, x_masks=None) -> torch.Tensor:
+                  adam: dict = None, row_sets=None, x_masks=None, val: torch.Tensor = None) -> torch.Tensor:
         """E0_local: this rank's rows [r0, r1) of the fused table.  Returns mean_k E^(k)[r0:r1]
         (written into `out` if given).  `next_E0_local`: this rank's rows of the table of the NEXT
         call, if the caller already has it (an inference / evaluation sweep over many tables, or
@@ -358,8 +360,13 @@ class PartitionedPropagator:
         `row_sets` (fused modes; from receptive_sets(S)): layer k computes - and exchanges - only the rows
         row_sets[k] (None = all); only the rows S = row_sets[K] of the result are then valid.
         `x_masks` (fused modes): x_masks[k] = uint8 [N] marking the rows of layer k's INPUT table that may be
-        non-zero (None = dense): gathers of the other rows are skipped (bit-identical, see spmm_rows)."""
+        non-zero (None = dense): gathers of the other rows are skipped (bit-identical, see spmm_rows).
+        `val` (fp32 [nnz] of the local block, e.g. one side of DeviceGraph.device_dropout_values): every layer of
+        this call multiplies by these edge values instead of the graph's."""
         K = self.K
+        if val is not None and self.local_spmm is None and (
+                val.dtype != torch.float32 or val.numel() != self.g.nnz or not val.is_contiguous()):
+            raise ValueError("val must be a contiguous fp32 tensor with one value per edge of the local block")
         if out is None:
             out = torch.empty_like(E0_local)
         if K == 0:
@@ -393,7 +400,7 @@ class PartitionedPropagator:
             if last and adam is not None:
                 if not fused:
                     raise ValueError("the fused Adam epilogue needs a fused exchange mode")
-                self._layer(X_full, None, addend, None, inv, publish=(None, (a + K) % nt), adam=adam)
+                self._layer(X_full, None, addend, None, inv, publish=(None, (a + K) % nt), adam=adam, val=val)
                 self._mark(f"layer{k + 1}")
                 done = torch.cuda.Event()
                 done.record()
@@ -420,7 +427,7 @@ class PartitionedPropagator:
                     raise ValueError("x_masks cannot be combined with a published next table")
                 self._layer(X_full, None, addend, out, inv if last else 1.0,
                             push_buf=None if last else (a + k + 1) % nt, publish=publish, subset=subset,
-                            x_nonzero=xm)
+                            x_nonzero=xm, val=val)
                 if publish is not None:
                     done = torch.cuda.Event()
                     done.record()
@@ -432,7 +439,7 @@ class PartitionedPropagator:
             else:
                 if not last and Y is None:
                     Y = torch.empty_like(E0_local)
-                self._layer(X_full, None if last else Y, addend, out, inv if last else 1.0)
+                self._layer(X_full, None if last else Y, addend, out, inv if last else 1.0, val=val)
                 self._mark(f"layer{k + 1}")
                 if not last:
                     self._all_gather_rows(self._X[(a + k + 1) % nt], Y)
@@ -477,10 +484,14 @@ class PartitionedPropagator:
 #   loss      BCE on the compact rows, replicated: bit-identical to the single-GPU loss
 #   backward  dL/d(out) rows are scattered by the same deterministic segmented reduction, each rank
 #             keeping only the rows it owns (row window), into its [rows_p, D] gradient slice;
-#             dL/dW = (1/(K+1)) sum_k (A^T)^k dL/d(out) = propagate(dL/d(out)) because the normalised
-#             adjacency is symmetric: the SAME partitioned propagation, exchange included, on gradients
-#             (sum-of-powers instead of the single-GPU kernel's Horner form: <= 1e-6 relative, not
-#             bit-equal).  Edge dropout (non-symmetric values) is not supported in this mode.
+#             dL/dW = (1/(K+1)) sum_k (A^T)^k dL/d(out): the SAME partitioned propagation, exchange included,
+#             on gradients, with the values of A^T on the structure of A (sum-of-powers instead of the
+#             single-GPU kernel's Horner form: <= 1e-6 relative, not bit-equal).  The normalised adjacency is
+#             symmetric, so without dropout A^T's values are A's.
+#   dropout   keep_prob (--dropout 2): the mask is a function of (seed, global row, column), so every rank
+#             makes val and valT of its own rows (spex_edge_dropout_f32 on its block, no communication) -
+#             the edges the single-GPU model drops under the same seed.  The forward multiplies by val, every
+#             backward layer by valT.
 #   optimiser row-owned dense Adam (spex_adam_f32 on the local slice): no collective.
 # With a fused exchange (push / mcast) the tail of the step is ONE kernel per rank: the last backward layer
 # applies Adam to each owned row in its epilogue and stores the updated row into every rank's table
@@ -490,6 +501,10 @@ class PartitionedPropagator:
 # ---------------------------------------------------------------------------------------------------
 class _CudaTrainOps:
     """The CUDA entry points behind PartitionedTrainer (no fallback: CPU tensors are rejected)."""
+
+    def dropout_values(self, g, seed, keep_prob):
+        """(val, valT) of the local block under the device mask (ops.DeviceGraph.device_dropout_values)."""
+        return g.device_dropout_values(seed, keep_prob)
 
     def gather_owned(self, local, rows, r0, r1):
         from ._capi import call, ptr, stream_ptr
@@ -536,7 +551,8 @@ class _CudaTrainOps:
 
 class _TorchTrainOps:
     """The same five operations in plain torch: used by the gloo CPU test of the orchestration (the
-    oracle's arithmetic; never selected on a GPU)."""
+    oracle's arithmetic; never selected on a GPU).  The sixth, dropout_values(g, seed, keep_prob), has no torch
+    replica here: a test that trains with dropout supplies it."""
 
     def gather_owned(self, local, rows, r0, r1):
         R = torch.zeros(rows.numel(), local.shape[1], dtype=local.dtype)
@@ -565,11 +581,18 @@ class _TorchTrainOps:
 
 class PartitionedTrainer:
     """main_rec.py:30-37 over a row partition: this rank owns rows [r0, r1) of the fused table `W_local`,
-    of its gradient and of the Adam moments.  `prop` is the PartitionedPropagator of the same partition."""
+    of its gradient and of the Adam moments.  `prop` is the PartitionedPropagator of the same partition.
+    `keep_prob` (None = no dropout): edge dropout with the device mask of LightGCN(dropout=2); every step draws its
+    seed with model.dropout_seed(), so a run seeded like a one-GPU run drops the same edges at every step.  The
+    local block must then give its transposed values (DeviceGraph.device_dropout_values)."""
 
     def __init__(self, prop: PartitionedPropagator, W_local: torch.Tensor, n_user_rows: int, lr: float = 1e-3,
-                 betas=(0.9, 0.999), eps: float = 1e-8, train_ops=None, fused_tail: bool = True):
+                 betas=(0.9, 0.999), eps: float = 1e-8, train_ops=None, fused_tail: bool = True,
+                 keep_prob: Optional[float] = None):
+        if keep_prob is not None and not 0.0 < keep_prob <= 1.0:
+            raise ValueError("keep_prob must be in (0, 1]")
         self.prop = prop
+        self.keep_prob = keep_prob
         self.W = W_local
         self.nur = int(n_user_rows)
         self.lr, self.betas, self.eps = lr, betas, eps
@@ -594,12 +617,17 @@ class PartitionedTrainer:
     def step(self, users: torch.Tensor, items: torch.Tensor, labels: torch.Tensor) -> torch.Tensor:
         p, r0, r1 = self.prop, self.prop.r0, self.prop.r1
         B = users.numel()
+        val = valT = None
+        if self.keep_prob is not None:   # one seed per step, where LightGCN._propagate draws it
+            from .model import dropout_seed
+
+            val, valT = self.ops.dropout_values(p.g, dropout_seed(), self.keep_prob)
         rows = torch.cat([users, items + self.nur]).to(torch.int64)
         # forward restricted to the batch's receptive field (fused modes; every computed row is bit-identical to
         # the full computer(), so loss, gradients and weights are unchanged): layer K on the batch's rows, layer
         # K-1 on their neighbours, ...; the backward mirrors it (below)
         plan = p.receptive_plan(torch.unique(rows)) if (self.receptive_field and self.fused) else None
-        out = p.propagate(self.W, out=self.out, row_sets=None if plan is None else plan.R)
+        out = p.propagate(self.W, out=self.out, row_sets=None if plan is None else plan.R, val=val)
         R = self.ops.gather_owned(out, rows, r0, r1)
         # backward mirror of the receptive field (plan.backward_layer): layer j (j < K) computes and exchanges its
         # rows into a zeroed table (zeroed here, before the all-reduce that orders it ahead of every peer's stores);
@@ -636,7 +664,7 @@ class PartitionedTrainer:
                 self.dW.zero_()     # a restricted first layer writes g + A g on its rows only; the rest is 0
             p.propagate(self.G_full[r0:r1], out=self.dW, first_full=self.G_full, row_sets=bsets, x_masks=bmasks,
                         adam={"p": self.W, "m": self.m, "v": self.v, "lr": self.lr, "beta1": self.betas[0],
-                              "beta2": self.betas[1], "eps": self.eps, "step": self.t})
+                              "beta2": self.betas[1], "eps": self.eps, "step": self.t}, val=valT)
             return loss
         if self._dirty is not None:
             self.ops.clear_rows(self.g, self._dirty)
@@ -644,7 +672,7 @@ class PartitionedTrainer:
         self.ops.scatter(rows[B:], Ru, dgamma, self.g, r0, r1)      # gI[items] = sum dgamma * U[users]
         own = (rows >= r0) & (rows < r1)
         self._dirty = (rows[own] - r0).contiguous()
-        dW = p.propagate(self.g, out=self.dW)                        # (1/(K+1)) sum_k A^k g
+        dW = p.propagate(self.g, out=self.dW, val=valT)              # (1/(K+1)) sum_k (A^T)^k g
         self.ops.adam(self.W, dW, self.m, self.v, self.lr, self.betas[0], self.betas[1], self.eps, self.t)
         return loss
 

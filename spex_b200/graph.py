@@ -40,6 +40,12 @@ class CSRGraph:
     tpos: Optional[np.ndarray] = None
     row_offset: int = 0  # first global row when this is a row block of a larger matrix
     meta: dict = field(default_factory=dict)
+    # val of (c, r) == val of (r, c) bit for bit for every edge (r, c) of these rows: the values of A^T on these
+    # rows are `val` itself
+    values_symmetric: bool = False
+    # tval[e] = value of the transposed entry of edge e, for a row block whose values are not symmetric (that
+    # entry usually lives in another block, so `tpos` cannot reach it)
+    tval: Optional[np.ndarray] = None
 
     @property
     def nnz(self) -> int:
@@ -48,17 +54,31 @@ class CSRGraph:
     def degrees(self) -> np.ndarray:
         return np.diff(self.rowptr)
 
-    def row_block(self, r0: int, r1: int) -> "CSRGraph":
-        """Rows [r0, r1) as a standalone CSR whose columns still index the full table."""
+    def row_block(self, r0: int, r1: int, transposed_values: bool = False) -> "CSRGraph":
+        """Rows [r0, r1) as a standalone CSR whose columns still index the full table.  `transposed_values`: the
+        block can also produce the values of A^T on its rows (edge dropout of a row-partitioned training step):
+        it is marked values_symmetric when they equal its own values bit for bit, else it carries them in tval,
+        read once here through the full matrix's transpose map."""
         lo, hi = int(self.rowptr[r0]), int(self.rowptr[r1])
+        val = self.val[lo:hi]
+        sym, tval = False, None
+        if transposed_values:
+            if self.tpos is None:
+                raise ValueError("the transposed values of a row block need the transpose map (tpos)")
+            tval = self.val[self.tpos[lo:hi]]
+            sym = bool(np.array_equal(tval.view(np.uint32), val.view(np.uint32)))
+            if sym:
+                tval = None
         return CSRGraph(
             n_rows=r1 - r0,
             n_cols=self.n_cols,
             rowptr=(self.rowptr[r0 : r1 + 1] - lo).astype(np.int64),
             col=self.col[lo:hi],
-            val=self.val[lo:hi],
+            val=val,
             tpos=None,
             row_offset=self.row_offset + r0,
+            values_symmetric=sym,
+            tval=tval,
         )
 
     def rows_of_entries(self) -> np.ndarray:

@@ -109,8 +109,9 @@ def main_distributed(args):
     """`torchrun --nproc-per-node P -m spex_b200.main_rec ...`: the same epochs with the table, its
     gradient and the Adam moments row-partitioned over P GPUs (spex_b200.dist.PartitionedTrainer).
     Every rank runs the same seeded host-side sampling (replicated, no communication), the batches are
-    visited in the single-GPU order, rank 0 prints the reference's lines.  Edge dropout is not
-    supported in this mode (the partitioned backward relies on the symmetric adjacency)."""
+    visited in the single-GPU order, rank 0 prints the reference's lines.  Edge dropout runs with the
+    device mask (`--dropout 2`): every rank makes the dropped values of its own rows, the same edges a
+    one-GPU run with the same --seed drops."""
     import os
 
     import torch.distributed as dist
@@ -119,8 +120,11 @@ def main_distributed(args):
     from .dist import PartitionedPropagator, PartitionedTrainer
     from .graph import partition_rows_by_nnz
 
-    if args.dropout:
-        raise SystemExit(f"--dropout {args.dropout} is not supported with torchrun (row-partitioned backward needs the symmetric graph)")
+    if args.dropout not in (0, 2):
+        # the reference's mask is one torch.rand(nnz) stream over the whole graph: every rank would need all of
+        # it and the global transpose map
+        raise SystemExit(f"--dropout {args.dropout} is not supported with torchrun: use --dropout 2, the device "
+                         "mask, which every rank generates for its own rows")
     if getattr(args, "test_mode", "sampled") != "sampled":
         raise SystemExit("--test_mode fullrank is not supported with torchrun: run it on one GPU")
     rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
@@ -140,9 +144,10 @@ def main_distributed(args):
     host = dataset.getCSR()
     bounds = partition_rows_by_nnz(host.rowptr, world)
     r0, r1 = bounds[rank], bounds[rank + 1]
-    lg = ops.DeviceGraph.from_host(host.row_block(r0, r1), device, D_hint=D)
+    lg = ops.DeviceGraph.from_host(host.row_block(r0, r1, transposed_values=bool(args.dropout)), device, D_hint=D)
     prop = PartitionedPropagator(lg, bounds, D, K, mode="nccl", device=device)
-    trainer = PartitionedTrainer(prop, model._table[r0:r1].detach().to(device).contiguous(), nur, lr=args.lr)
+    trainer = PartitionedTrainer(prop, model._table[r0:r1].detach().to(device).contiguous(), nur, lr=args.lr,
+                                 keep_prob=args.keepprob if args.dropout else None)
     best_recall, best_ndcg, best_iter = [0, 0, 0], [0, 0, 0], [0, 0]
     for epoch in range(args.epochs):
         train_dataset.ng_sample()

@@ -131,6 +131,7 @@ class DeviceGraph:
         # val of (c, r) == val of (r, c) bit for bit (no tpos needed for the transposed values).  Not implied by
         # `symmetric`: a weighted build computes (d_u*w)*d_i one way and (d_i*w)*d_u the other.
         self.values_symmetric = values_symmetric
+        self._tval_pos = None         # a row block's map to its transposed values (from_host)
         self.device = val.device
         self.seg_len = int(seg_len)
         self._plan_struct = None
@@ -147,9 +148,21 @@ class DeviceGraph:
         dev = torch.device(device)
         rowptr = torch.from_numpy(np.ascontiguousarray(g.rowptr)).to(dev)
         col = torch.from_numpy(np.ascontiguousarray(g.col)).to(dev)
-        val = torch.from_numpy(np.ascontiguousarray(g.val)).to(dev)
         tpos = None if g.tpos is None else torch.from_numpy(np.ascontiguousarray(g.tpos)).to(dev)
-        return cls(rowptr, col, val, g.n_cols, tpos, seg_len, g.row_offset, D_hint=D_hint)
+        if g.tval is None:
+            val = torch.from_numpy(np.ascontiguousarray(g.val)).to(dev)
+            tval_pos = None
+        else:
+            # a row block's transposed values behind its own values in one buffer, [val | tval], and a block-local
+            # map into the second half: spex_edge_dropout_f32 reads the transposed value of edge e at val[tpos[e]],
+            # so they reach the kernel through its existing tpos argument (12 B per edge)
+            nnz = int(g.val.size)
+            val = torch.from_numpy(np.concatenate([g.val, g.tval]).astype(np.float32, copy=False)).to(dev)[:nnz]
+            tval_pos = torch.arange(nnz, 2 * nnz, dtype=torch.int64, device=dev)
+        out = cls(rowptr, col, val, g.n_cols, tpos, seg_len, g.row_offset, D_hint=D_hint,
+                  values_symmetric=g.values_symmetric)
+        out._tval_pos = tval_pos
+        return out
 
     @classmethod
     def from_sparse_coo(cls, A: torch.Tensor, device, seg_len: int = DEFAULT_SEG_LEN):
@@ -387,13 +400,16 @@ class DeviceGraph:
     def device_dropout_values(self, seed: int, keep_prob: float):
         """(val, valT) of the edge-dropped graph under the counter-based mask of spex_edge_dropout_f32: edge (r, c)
         is kept by a hash of (seed, global row, column), so no host random numbers and no mask copy.  Fresh
-        tensors: autograd holds valT until the backward runs."""
-        if self.tpos is None and not self.values_symmetric:
+        tensors: autograd holds valT until the backward runs.  A row block (row_offset = its first global row) gives
+        its slice of the whole graph's pair when it is bit-symmetric or was cut with CSRGraph.row_block(...,
+        transposed_values=True)."""
+        tpos = self.tpos if self.tpos is not None else self._tval_pos
+        if tpos is None and not self.values_symmetric:
             raise RuntimeError("edge dropout needs the transpose map of the adjacency or bit-symmetric values; "
                                "build the graph through spex_b200.dataloader (getCSR) or synthetic.build_norm_adj_device")
         val = torch.empty_like(self.val)
         valT = torch.empty_like(self.val)
-        call("spex_edge_dropout_f32", ptr(self.rowptr), ptr(self.col), ptr(self.val), ptr(self.tpos), self.n_rows,
+        call("spex_edge_dropout_f32", ptr(self.rowptr), ptr(self.col), ptr(self.val), ptr(tpos), self.n_rows,
              self.row_offset, int(seed), float(keep_prob), ptr(val), ptr(valT), stream_ptr())
         return val, valT
 
