@@ -167,6 +167,26 @@ int spex_spmm_layer_f32(const int64_t* rowptr, const int32_t* col, const float* 
                         const spex_spmm_epilogue* ep, const spex_long_plan* plan, void* stream);
 
 /*
+ * spex_spmm_layer_f32 with an ADDED GRADIENT in the epilogue: for every computed row i with z_add_rows[i] != 0
+ *      z[i,:] = (addend[i,:] * addend_scale + acc) * z_scale + z_add[i,:]
+ * (one fp32 add after the scale), and both Z and the fused Adam see that sum; rows whose flag is 0 never read
+ * z_add.  Replaces the autograd sum dE0 = dE0_propagated + d(reg)/dE0 of a BPR step (main_rec.py:35 with upstream
+ * LightGCN's L2 term): the last backward layer of a row-partitioned step takes the ego rows' L2 gradient.
+ *   z_add       fp32 [n_rows, D], 16-byte aligned (SPEX_E_ALIGN)
+ *   z_add_rows  uint8 [n_rows]
+ * z_add and z_add_rows are both NULL (spex_spmm_layer_f32) or both set, and then the descriptor sets Z or Adam
+ * (SPEX_E_BADARG otherwise); everything is checked before anything runs.
+ */
+int spex_spmm_layer_zadd_f32(const int64_t* rowptr, const int32_t* col, const float* val,
+                             const float* X, int64_t n_rows, int32_t D,
+                             const int32_t* rows, int64_t n_sel,
+                             const int32_t* long_slots, int32_t n_long_sel,
+                             const int32_t* seg_ids, int32_t n_seg_sel,
+                             const uint8_t* x_nonzero,
+                             const spex_spmm_epilogue* ep, const float* z_add, const uint8_t* z_add_rows,
+                             const spex_long_plan* plan, void* stream);
+
+/*
  * K-layer propagation + layer mean:  out = (E0 + A·E0 + ... + A^K·E0) / (K+1)
  * E0 [N,D] is the concatenated user+item table (model.py:72); tmp0/tmp1 are [N,D] ping-pong
  * workspaces (K>=2 needs tmp0, K>=3 needs both).  The mean is accumulated in `out` by every

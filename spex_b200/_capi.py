@@ -60,6 +60,8 @@ SIGNATURES = {
     "spex_spmm_csr_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _p, _p, _f, _p, _f, _PLAN, _p]),
     "spex_spmm_layer_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _p, _i64, _p, _i32, _p, _i32, _p,
                                       C.POINTER(SpmmEpilogue), _PLAN, _p]),
+    "spex_spmm_layer_zadd_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _p, _i64, _p, _i32, _p, _i32, _p,
+                                           C.POINTER(SpmmEpilogue), _p, _p, _PLAN, _p]),
     "spex_propagate_mean_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _i32, _p, _p, _p, _PLAN, _p]),
     "spex_propagate_mean_bwd_f32": (C.c_int, [_p, _p, _p, _p, _i64, _i32, _i32, _p, _p, _p, _PLAN, _p]),
     "spex_gather_f32": (C.c_int, [_p, _p, _p, _f, _p, _i64, _p]),

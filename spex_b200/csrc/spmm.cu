@@ -22,7 +22,8 @@
 //     boundaries and listed block-major so that the table window they gather from stays in L2, the other long
 //     rows cut every seg_len edges;
 //   * epilogue: Y = acc (next layer's input) and/or Z = (addend*a + acc)*b (running layer mean forward,
-//     g + A^T G backward), optionally stored into every peer's table (P2P or one NVLS multicast store), with the
+//     g + A^T G backward) plus, on flagged rows, an added gradient (the BPR L2 term of the last backward layer),
+//     optionally stored into every peer's table (P2P or one NVLS multicast store), with the
 //     next call's table or a dense Adam step riding on the last layer (row-partitioned modes);
 //   * a layer can be restricted to a ROW LIST (RowSubset: the receptive field of a mini-batch) and can be told
 //     which rows of X may be non-zero (x_nonzero: the sparse gradient tables of the training backward); both
@@ -405,7 +406,22 @@ struct Epilogue {
   float* adam_m;
   float* adam_v;
   float adam_b1, adam_b2, adam_eps, adam_step_size, adam_bc2_sqrt;
+  // added gradient (spex_spmm_layer_zadd_f32): rows with z_add_rows[i] != 0 get z += z_add[i, :] after the scale,
+  // one fp32 add that Z and the fused Adam both see; the other rows never read z_add
+  const float* z_add;
+  const uint8_t* z_add_rows;
 };
+
+// z += row `row` of z_add (flagged rows only); __fadd_rn: an add of its own, never contracted into the scale's FMA
+__device__ __forceinline__ void add_z_row(const Epilogue& ep, float4& z, int64_t row, int64_t off) {
+  if (ep.z_add && ep.z_add_rows[row]) {
+    const float4 g = ld_f4(ep.z_add + off);
+    z.x = __fadd_rn(z.x, g.x);
+    z.y = __fadd_rn(z.y, g.y);
+    z.z = __fadd_rn(z.z, g.z);
+    z.w = __fadd_rn(z.w, g.w);
+  }
+}
 
 __device__ __forceinline__ void adam_update(float& pp, float gg, float& mm, float& vv, const Epilogue& ep) {
   mm = mm + (gg - mm) * (1.f - ep.adam_b1);               // exp_avg.lerp_(grad, 1-beta1)
@@ -436,6 +452,7 @@ __device__ __forceinline__ void row_epilogue(const Epilogue& ep, float4 acc, int
       z.y = (a.y * ep.addend_scale + acc.y) * ep.z_scale;
       z.z = (a.z * ep.addend_scale + acc.z) * ep.z_scale;
       z.w = (a.w * ep.addend_scale + acc.w) * ep.z_scale;
+      add_z_row(ep, z, row, off);
       if (ep.Z) *reinterpret_cast<float4*>(ep.Z + off) = z;
     }
     float4 pnew = f4_zero();
@@ -687,6 +704,7 @@ spmm_rows_generic_kernel(const int64_t* __restrict__ rowptr, const int32_t* __re
         z.y = (a.y * ep.addend_scale + acc[v].y) * ep.z_scale;
         z.z = (a.z * ep.addend_scale + acc[v].z) * ep.z_scale;
         z.w = (a.w * ep.addend_scale + acc[v].w) * ep.z_scale;
+        add_z_row(ep, z, row, off);
         *reinterpret_cast<float4*>(ep.Z + off) = z;
       }
     }
@@ -1015,20 +1033,35 @@ static int make_epilogue(const spex_spmm_epilogue* d, Epilogue& ep) {
 // duplicates; rows with degree > plan->seg_len are skipped by the rows kernel and must be given again as
 // long_slots (their positions in plan->long_rows) with seg_ids = the ids of all their segments.  Every listed
 // row gets exactly the value the full layer would give it; the other rows of the outputs are not touched.
-extern "C" int spex_spmm_layer_f32(const int64_t* rowptr, const int32_t* col, const float* val, const float* X,
-                                   int64_t n_rows, int32_t D, const int32_t* rows, int64_t n_sel,
-                                   const int32_t* long_slots, int32_t n_long_sel, const int32_t* seg_ids,
-                                   int32_t n_seg_sel, const uint8_t* x_nonzero, const spex_spmm_epilogue* epilogue,
-                                   const spex_long_plan* plan, void* stream) {
+extern "C" int spex_spmm_layer_zadd_f32(const int64_t* rowptr, const int32_t* col, const float* val, const float* X,
+                                        int64_t n_rows, int32_t D, const int32_t* rows, int64_t n_sel,
+                                        const int32_t* long_slots, int32_t n_long_sel, const int32_t* seg_ids,
+                                        int32_t n_seg_sel, const uint8_t* x_nonzero,
+                                        const spex_spmm_epilogue* epilogue, const float* z_add,
+                                        const uint8_t* z_add_rows, const spex_long_plan* plan, void* stream) {
   SPEX_RETURN_IF(n_long_sel < 0 || n_seg_sel < 0 || (n_sel > 0 && !rows), SPEX_E_BADARG);
   SPEX_RETURN_IF(n_long_sel > 0 && (!long_slots || !seg_ids || !plan || n_seg_sel < n_long_sel), SPEX_E_BADARG);
   Epilogue ep{};
   const int rc = make_epilogue(epilogue, ep);
   if (rc) return rc;
+  // the added gradient needs its row flags and a row it is added to (Z or the fused Adam's gradient)
+  SPEX_RETURN_IF(!z_add != !z_add_rows || (z_add && !ep.Z && !ep.adam_p), SPEX_E_BADARG);
+  SPEX_RETURN_IF(!aligned16(z_add), SPEX_E_ALIGN);
+  ep.z_add = z_add;
+  ep.z_add_rows = z_add_rows;
   if (n_sel == 0) return 0;
   RowSubset sub{rows, n_sel, long_slots, n_long_sel, seg_ids, n_seg_sel};
   return spmm_launch(rowptr, col, val, X, n_rows, D, ep, plan, (cudaStream_t)stream, n_sel < 0 ? nullptr : &sub,
                      x_nonzero);
+}
+
+extern "C" int spex_spmm_layer_f32(const int64_t* rowptr, const int32_t* col, const float* val, const float* X,
+                                   int64_t n_rows, int32_t D, const int32_t* rows, int64_t n_sel,
+                                   const int32_t* long_slots, int32_t n_long_sel, const int32_t* seg_ids,
+                                   int32_t n_seg_sel, const uint8_t* x_nonzero, const spex_spmm_epilogue* epilogue,
+                                   const spex_long_plan* plan, void* stream) {
+  return spex_spmm_layer_zadd_f32(rowptr, col, val, X, n_rows, D, rows, n_sel, long_slots, n_long_sel, seg_ids,
+                                  n_seg_sel, x_nonzero, epilogue, nullptr, nullptr, plan, stream);
 }
 
 // n_ctas == 0: the full-speed grid (8 CTAs per SM); > 0: a small grid for a BACKGROUND exchange that

@@ -42,6 +42,7 @@ from __future__ import annotations
 import ctypes as C
 from typing import Callable, List, Optional, Sequence
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -56,6 +57,14 @@ class _CudaArray:
     def __init__(self, ptr: int, shape, typestr="<f4"):
         self.__cuda_array_interface__ = {"data": (int(ptr), False), "shape": tuple(shape),
                                          "typestr": typestr, "version": 3, "strides": None}
+
+
+def _add_flagged(Z: torch.Tensor, z_add):
+    """Z[i] += rows[i] on the rows flags marks (z_add = (rows, flags)): the torch form of the epilogue's added
+    gradient, for K = 0 and the CPU-injected local multiply."""
+    rows, flags = z_add
+    m = flags.bool()
+    Z[m] += rows[m]
 
 
 class PartitionedPropagator:
@@ -198,17 +207,20 @@ class PartitionedPropagator:
 
     # ---- one layer --------------------------------------------------------------------------------
     def _layer(self, X_full, Y_local, addend, Z_local, z_scale, push_buf=None, publish=None, subset=None,
-               x_nonzero=None, adam=None, val=None):
+               x_nonzero=None, adam=None, val=None, z_add=None):
         """One layer over the local rows (ops.spmm_rows), restricted to `subset` / reading a table that is zero
         outside the rows `x_nonzero` marks, with the block's edge values `val` (None = the graph's).  Fused modes:
         `push_buf` = ring slot into which the Y rows go on every rank; `publish` = (src, slot): the rows of src - or,
         with `adam` ({p, m, v, lr, beta1, beta2, eps, step}, src None), the rows of p updated with the Z rows as
-        gradient - go to ring slot `slot` on every rank."""
+        gradient - go to ring slot `slot` on every rank.  `z_add` = (rows [rows_p, D], flags uint8 [rows_p]): the
+        flagged rows of Z (or of Adam's gradient) get the row added after the scale."""
         if self.local_spmm is not None:
             acc = self.local_spmm(self.g, X_full) if val is None else self.local_spmm(self.g, X_full, val)
             if Y_local is not None:
                 Y_local.copy_(acc)
             Z_local.copy_((addend + acc) * z_scale)
+            if z_add is not None:
+                _add_flagged(Z_local, z_add)
             return
         from . import ops
 
@@ -222,7 +234,8 @@ class PartitionedPropagator:
         pub_mcast, pub_peers = dest(pub_slot)
         ops.spmm_rows(self.g, X_full, subset, Y=Y_local, addend=addend, Z=Z_local, z_scale=float(z_scale),
                       x_nonzero=x_nonzero, out_row_offset=self.r0, y_mcast=y_mcast, y_peers=y_peers,
-                      pub_src=pub_src, pub_mcast=pub_mcast, pub_peers=pub_peers, adam=adam, val=val)
+                      pub_src=pub_src, pub_mcast=pub_mcast, pub_peers=pub_peers, adam=adam, val=val,
+                      z_add=None if z_add is None else z_add[0], z_add_rows=None if z_add is None else z_add[1])
 
     def _mark(self, name):
         if self.timing is not None:
@@ -345,7 +358,8 @@ class PartitionedPropagator:
 
     def propagate(self, E0_local: torch.Tensor, out: torch.Tensor = None,
                   next_E0_local: torch.Tensor = None, next_ready=None, first_full: torch.Tensor = None,
-                  adam: dict = None, row_sets=None, x_masks=None, val: torch.Tensor = None) -> torch.Tensor:
+                  adam: dict = None, row_sets=None, x_masks=None, val: torch.Tensor = None,
+                  z_add=None) -> torch.Tensor:
         """E0_local: this rank's rows [r0, r1) of the fused table.  Returns mean_k E^(k)[r0:r1]
         (written into `out` if given).  `next_E0_local`: this rank's rows of the table of the NEXT
         call, if the caller already has it (an inference / evaluation sweep over many tables, or
@@ -362,7 +376,10 @@ class PartitionedPropagator:
         `x_masks` (fused modes): x_masks[k] = uint8 [N] marking the rows of layer k's INPUT table that may be
         non-zero (None = dense): gathers of the other rows are skipped (bit-identical, see spmm_rows).
         `val` (fp32 [nnz] of the local block, e.g. one side of DeviceGraph.device_dropout_values): every layer of
-        this call multiplies by these edge values instead of the graph's."""
+        this call multiplies by these edge values instead of the graph's.
+        `z_add` = (rows fp32 [rows_p, D], flags uint8 [rows_p]): added to the flagged rows of the result after the
+        layer mean's scale - in the last layer's epilogue (and so into the fused Adam's gradient), with K = 0 to the
+        copy (the L2 gradient of a BPR step's ego rows, which the propagation does not carry)."""
         K = self.K
         if val is not None and self.local_spmm is None and (
                 val.dtype != torch.float32 or val.numel() != self.g.nnz or not val.is_contiguous()):
@@ -371,6 +388,8 @@ class PartitionedPropagator:
             out = torch.empty_like(E0_local)
         if K == 0:
             out.copy_(E0_local)
+            if z_add is not None:
+                _add_flagged(out, z_add)
             return out
         inv = 1.0 / (K + 1)
         if self.timing is not None:
@@ -400,7 +419,8 @@ class PartitionedPropagator:
             if last and adam is not None:
                 if not fused:
                     raise ValueError("the fused Adam epilogue needs a fused exchange mode")
-                self._layer(X_full, None, addend, None, inv, publish=(None, (a + K) % nt), adam=adam, val=val)
+                self._layer(X_full, None, addend, None, inv, publish=(None, (a + K) % nt), adam=adam, val=val,
+                            z_add=z_add)
                 self._mark(f"layer{k + 1}")
                 done = torch.cuda.Event()
                 done.record()
@@ -427,7 +447,7 @@ class PartitionedPropagator:
                     raise ValueError("x_masks cannot be combined with a published next table")
                 self._layer(X_full, None, addend, out, inv if last else 1.0,
                             push_buf=None if last else (a + k + 1) % nt, publish=publish, subset=subset,
-                            x_nonzero=xm, val=val)
+                            x_nonzero=xm, val=val, z_add=z_add if last else None)
                 if publish is not None:
                     done = torch.cuda.Event()
                     done.record()
@@ -439,7 +459,8 @@ class PartitionedPropagator:
             else:
                 if not last and Y is None:
                     Y = torch.empty_like(E0_local)
-                self._layer(X_full, None if last else Y, addend, out, inv if last else 1.0, val=val)
+                self._layer(X_full, None if last else Y, addend, out, inv if last else 1.0, val=val,
+                            z_add=z_add if last else None)
                 self._mark(f"layer{k + 1}")
                 if not last:
                     self._all_gather_rows(self._X[(a + k + 1) % nt], Y)
@@ -493,6 +514,11 @@ class PartitionedPropagator:
 #             the edges the single-GPU model drops under the same seed.  The forward multiplies by val, every
 #             backward layer by valT.
 #   optimiser row-owned dense Adam (spex_adam_f32 on the local slice): no collective.
+#   BPR       (bpr_step) the rows gathered are the batch's users, positives and negatives, each propagated AND raw
+#             (ego): one [6B, D] buffer, one all-reduce, and the one-GPU loss kernel on it.  The L2 term's gradient
+#             lives on the ego rows, which the propagation does not carry: each rank scatters it into its own rows
+#             and the last backward layer adds it to the gradient after the layer mean's scale (the epilogue's
+#             z_add), the autograd sum dE0 + g0 of one GPU.
 # With a fused exchange (push / mcast) the tail of the step is ONE kernel per rank: the last backward layer
 # applies Adam to each owned row in its epilogue and stores the updated row into every rank's table
 # (the fused Adam of spex_spmm_layer_f32), so the next forward starts without an E^(0) exchange; and the first
@@ -506,13 +532,11 @@ class _CudaTrainOps:
         """(val, valT) of the local block under the device mask (ops.DeviceGraph.device_dropout_values)."""
         return g.device_dropout_values(seed, keep_prob)
 
-    def gather_owned(self, local, rows, r0, r1):
+    def gather_owned(self, local, rows, r0, r1, R):
         from ._capi import call, ptr, stream_ptr
 
-        R = torch.empty(rows.numel(), local.shape[1], dtype=torch.float32, device=local.device)
         call("spex_gather_owned_rows_f32", ptr(local), ptr(rows), rows.numel(), local.shape[1], r0, r1, ptr(R),
              stream_ptr())
-        return R
 
     def bce(self, Ru, Ri, labels):
         from ._capi import call, ptr, stream_ptr
@@ -526,15 +550,29 @@ class _CudaTrainOps:
              ptr(dgamma), stream_ptr())
         return loss, dgamma
 
-    def scatter(self, dst_rows, src, coef, out_local, r0, r1):
+    def bpr(self, R, B):
+        """(loss, reg, dscore) of spex_bpr_fwd_f32 on R = [users, pos, neg propagated; users, pos, neg ego] rows."""
+        from ._capi import call, ptr, stream_ptr
+
+        D = R.shape[1]
+        ar = torch.arange(B, device=R.device)
+        out2 = torch.empty(2, dtype=torch.float32, device=R.device)
+        dscore = torch.empty(B, dtype=torch.float32, device=R.device)
+        work = torch.empty(2 * B, dtype=torch.float32, device=R.device)
+        ego = R[3 * B:]
+        pos, neg = ar + B, ar + 2 * B      # held until the launch: a freed temporary's memory is reused at once
+        call("spex_bpr_fwd_f32", ptr(R), ptr(R), ptr(ego), ptr(ego), D, ptr(ar), ptr(pos), ptr(neg), B, ptr(out2),
+             ptr(dscore), ptr(work), stream_ptr())
+        return out2[0], out2[1], dscore
+
+    def scatter(self, dst_rows, src_rows, src, coef, gscalar, cconst, out_local, r0, r1):
         from . import ops
         from ._capi import call, ptr, stream_ptr
 
-        B, D = src.shape
-        ar = torch.arange(B, device=src.device)
-        work, wb = ops._scatter_workspace(B, src.device)
-        call("spex_scatter_rows_f32", ptr(dst_rows), ptr(ar), ptr(coef), None, 1.0, B, ptr(src), D, ptr(out_local),
-             r0, r1, ptr(work), wb, stream_ptr())
+        n, D = dst_rows.numel(), src.shape[1]
+        work, wb = ops._scatter_workspace(n, src.device)
+        call("spex_scatter_rows_f32", ptr(dst_rows), ptr(src_rows), ptr(coef), ptr(gscalar), float(cconst), n,
+             ptr(src), D, ptr(out_local), r0, r1, ptr(work), wb, stream_ptr())
 
     def clear_rows(self, table_local, rows_local):
         from ._capi import call, ptr, stream_ptr
@@ -550,24 +588,34 @@ class _CudaTrainOps:
 
 
 class _TorchTrainOps:
-    """The same five operations in plain torch: used by the gloo CPU test of the orchestration (the
-    oracle's arithmetic; never selected on a GPU).  The sixth, dropout_values(g, seed, keep_prob), has no torch
-    replica here: a test that trains with dropout supplies it."""
+    """The same operations in plain torch: used by the gloo CPU test of the orchestration (the oracle's arithmetic;
+    never selected on a GPU).  dropout_values(g, seed, keep_prob) has no torch replica here: a test that trains with
+    dropout supplies it."""
 
-    def gather_owned(self, local, rows, r0, r1):
-        R = torch.zeros(rows.numel(), local.shape[1], dtype=local.dtype)
+    def gather_owned(self, local, rows, r0, r1, R):
+        R.zero_()
         own = (rows >= r0) & (rows < r1)
         R[own] = local[rows[own] - r0]
-        return R
 
     def bce(self, Ru, Ri, labels):
         gamma = (Ru * Ri).sum(1)
         loss = torch.nn.functional.binary_cross_entropy_with_logits(gamma, labels).reshape(1)
         return loss, (torch.sigmoid(gamma) - labels) / labels.numel()
 
-    def scatter(self, dst_rows, src, coef, out_local, r0, r1):
+    def bpr(self, R, B):
+        u, p, n, u0, p0, n0 = R.split(B)
+        x = (u * n).sum(1) - (u * p).sum(1)
+        reg = 0.5 * (u0.square().sum() + p0.square().sum() + n0.square().sum()) / B
+        return torch.nn.functional.softplus(x).mean(), reg, torch.sigmoid(x) / B
+
+    def scatter(self, dst_rows, src_rows, src, coef, gscalar, cconst, out_local, r0, r1):
         own = (dst_rows >= r0) & (dst_rows < r1)
-        out_local.index_add_(0, dst_rows[own] - r0, src[own] * coef[own, None])
+        w = torch.full((dst_rows.numel(),), float(cconst), dtype=src.dtype)
+        if coef is not None:
+            w = w * coef
+        if gscalar is not None:
+            w = w * gscalar
+        out_local.index_add_(0, dst_rows[own] - r0, src[src_rows[own]] * w[own, None])
 
     def clear_rows(self, table_local, rows_local):
         table_local[rows_local] = 0
@@ -584,21 +632,23 @@ class PartitionedTrainer:
     of its gradient and of the Adam moments.  `prop` is the PartitionedPropagator of the same partition.
     `keep_prob` (None = no dropout): edge dropout with the device mask of LightGCN(dropout=2); every step draws its
     seed with model.dropout_seed(), so a run seeded like a one-GPU run drops the same edges at every step.  The
-    local block must then give its transposed values (DeviceGraph.device_dropout_values)."""
+    local block must then give its transposed values (DeviceGraph.device_dropout_values).  `decay`: weight of the L2
+    term of bpr_step's loss."""
 
     def __init__(self, prop: PartitionedPropagator, W_local: torch.Tensor, n_user_rows: int, lr: float = 1e-3,
                  betas=(0.9, 0.999), eps: float = 1e-8, train_ops=None, fused_tail: bool = True,
-                 keep_prob: Optional[float] = None):
+                 keep_prob: Optional[float] = None, decay: float = 1e-4):
         if keep_prob is not None and not 0.0 < keep_prob <= 1.0:
             raise ValueError("keep_prob must be in (0, 1]")
         self.prop = prop
         self.keep_prob = keep_prob
+        self.decay = float(decay)
         self.W = W_local
         self.nur = int(n_user_rows)
         self.lr, self.betas, self.eps = lr, betas, eps
         self.m = torch.zeros_like(W_local)
         self.v = torch.zeros_like(W_local)
-        # fused path (push / mcast exchange on GPUs, K >= 1, D with a vector kernel): see step()
+        # fused path (push / mcast exchange on GPUs, K >= 1, D with a vector kernel): see _step()
         self.fused = (train_ops is None and prop.mode in ("push", "mcast") and prop.K >= 1
                       and prop.D in (32, 64, 128) and fused_tail)
         if self.fused:
@@ -609,26 +659,67 @@ class PartitionedTrainer:
         self.dW = torch.empty_like(W_local)
         self.out = torch.empty_like(W_local)
         self._dirty = None
+        # bpr_step: the L2 gradient of the owned ego rows and their flags (the last backward layer's z_add)
+        self.g0 = self.g0_rows = self._ego_dirty = None
         self.t = 0
         self.receptive_field = True
         self.receptive_backward = True
         self.ops = train_ops if train_ops is not None else _CudaTrainOps()
 
     def step(self, users: torch.Tensor, items: torch.Tensor, labels: torch.Tensor) -> torch.Tensor:
-        p, r0, r1 = self.prop, self.prop.r0, self.prop.r1
+        """One BCE step (main_rec.py:30-37); returns the device loss."""
         B = users.numel()
+        rows = torch.cat([users, items + self.nur]).to(torch.int64)
+        ar = torch.arange(B, device=rows.device)
+
+        def loss_grads(R):
+            loss, dgamma = self.ops.bce(R[:B], R[B:], labels.to(torch.float32))
+            # gU[users] = sum dgamma * I[items];  gI[items] = sum dgamma * U[users]
+            return loss, [(rows[:B], ar + B, dgamma, None), (rows[B:], ar, dgamma, None)], None
+
+        return self._step(rows, False, loss_grads)
+
+    def bpr_step(self, users: torch.Tensor, pos: torch.Tensor, neg: torch.Tensor) -> torch.Tensor:
+        """One BPR step: LightGCN.bpr_loss's (loss, reg) on the batch, then loss + decay * reg back-propagated and
+        Adam (upstream LightGCN's training loss).  Returns the device scalar loss + decay * reg."""
+        B = users.numel()
+        rows = torch.cat([users, pos + self.nur, neg + self.nur]).to(torch.int64)
+        ar = torch.arange(B, device=rows.device)
+        grad2 = torch.tensor([1.0, self.decay], dtype=torch.float32, device=rows.device)   # d/d(loss), d/d(reg)
+        cconst = float(np.float32(1.0) / np.float32(B)) if B else 1.0                          # fp32 1/B, as the kernel's
+
+        def loss_grads(R):
+            loss, reg, dscore = self.ops.bpr(R, B)
+            # spex_bpr_bwd_ws_f32's lists in one: per destination row the pos entries in batch order, then the neg
+            # ones; (1 * -d) * gs is ((-1) * d) * gs bit for bit
+            prop = (torch.cat([rows[:B], rows[:B], rows[B:2 * B], rows[2 * B:]]),
+                    torch.cat([ar + B, ar + 2 * B, ar, ar]), torch.cat([-dscore, dscore, -dscore, dscore]), grad2[:1])
+            ego = (rows, torch.arange(3 * B, 6 * B, device=rows.device), grad2[1:], cconst)
+            return loss + self.decay * reg, [prop], ego
+
+        return self._step(rows, True, loss_grads)
+
+    def _step(self, rows, ego, loss_grads):
+        """The step both losses share.  rows: the global rows the loss reads; ego: the loss also reads their raw
+        rows (gathered after the propagated ones).  loss_grads(R) -> (loss, lists, ego_list) on the assembled rows R:
+        lists = [(dst rows, positions in R, coef, gscalar)] of the propagated gradient, ego_list = (dst rows,
+        positions in R, gscalar, cconst) of the ego rows' gradient or None."""
+        p, r0, r1 = self.prop, self.prop.r0, self.prop.r1
         val = valT = None
         if self.keep_prob is not None:   # one seed per step, where LightGCN._propagate draws it
             from .model import dropout_seed
 
             val, valT = self.ops.dropout_values(p.g, dropout_seed(), self.keep_prob)
-        rows = torch.cat([users, items + self.nur]).to(torch.int64)
         # forward restricted to the batch's receptive field (fused modes; every computed row is bit-identical to
         # the full computer(), so loss, gradients and weights are unchanged): layer K on the batch's rows, layer
         # K-1 on their neighbours, ...; the backward mirrors it (below)
         plan = p.receptive_plan(torch.unique(rows)) if (self.receptive_field and self.fused) else None
         out = p.propagate(self.W, out=self.out, row_sets=None if plan is None else plan.R, val=val)
-        R = self.ops.gather_owned(out, rows, r0, r1)
+        n = rows.numel()
+        R = self.W.new_empty(2 * n if ego else n, self.W.shape[1])
+        self.ops.gather_owned(out, rows, r0, r1, R[:n])
+        if ego:
+            self.ops.gather_owned(self.W, rows, r0, r1, R[n:])
         # backward mirror of the receptive field (plan.backward_layer): layer j (j < K) computes and exchanges its
         # rows into a zeroed table (zeroed here, before the all-reduce that orders it ahead of every peer's stores);
         # the last layer is the fused Adam kernel: dense and unmasked
@@ -645,10 +736,10 @@ class PartitionedTrainer:
                 if bsets[j] is not None:
                     p.zero_slot(j)
         if p.world > 1:
-            dist.all_reduce(R, group=p.group)
-        Ru, Ri = R[:B], R[B:]
-        loss, dgamma = self.ops.bce(Ru, Ri, labels.to(torch.float32))
+            dist.all_reduce(R, group=p.group)   # one non-zero term per row: exact
+        loss, lists, ego_list = loss_grads(R)
         self.t += 1
+        z_add = None if ego_list is None else self._ego_grad(R, *ego_list)
         if self.fused:
             # Every rank holds all rows of the batch, so every rank can write ALL gradient rows into its own
             # full-size gradient table (zero elsewhere: zero-filled once, the touched rows cleared per step):
@@ -657,24 +748,39 @@ class PartitionedTrainer:
             # main_rec.py:35-37's backward tail, the optimiser and the next all-gather).
             if self._dirty is not None:
                 self.ops.clear_rows(self.G_full, self._dirty)
-            self.ops.scatter(rows[:B], Ri, dgamma, self.G_full, 0, 0)
-            self.ops.scatter(rows[B:], Ru, dgamma, self.G_full, 0, 0)
+            for dst, src, coef, gs in lists:
+                self.ops.scatter(dst, src, R, coef, gs, 1.0, self.G_full, 0, 0)
             self._dirty = rows
             if bsets is not None and any(b is not None for b in bsets):
                 self.dW.zero_()     # a restricted first layer writes g + A g on its rows only; the rest is 0
             p.propagate(self.G_full[r0:r1], out=self.dW, first_full=self.G_full, row_sets=bsets, x_masks=bmasks,
                         adam={"p": self.W, "m": self.m, "v": self.v, "lr": self.lr, "beta1": self.betas[0],
-                              "beta2": self.betas[1], "eps": self.eps, "step": self.t}, val=valT)
+                              "beta2": self.betas[1], "eps": self.eps, "step": self.t}, val=valT, z_add=z_add)
             return loss
         if self._dirty is not None:
             self.ops.clear_rows(self.g, self._dirty)
-        self.ops.scatter(rows[:B], Ri, dgamma, self.g, r0, r1)      # gU[users] = sum dgamma * I[items]
-        self.ops.scatter(rows[B:], Ru, dgamma, self.g, r0, r1)      # gI[items] = sum dgamma * U[users]
+        for dst, src, coef, gs in lists:
+            self.ops.scatter(dst, src, R, coef, gs, 1.0, self.g, r0, r1)
         own = (rows >= r0) & (rows < r1)
         self._dirty = (rows[own] - r0).contiguous()
-        dW = p.propagate(self.g, out=self.dW, val=valT)              # (1/(K+1)) sum_k (A^T)^k g
+        dW = p.propagate(self.g, out=self.dW, val=valT, z_add=z_add)   # (1/(K+1)) sum_k (A^T)^k g (+ g0)
         self.ops.adam(self.W, dW, self.m, self.v, self.lr, self.betas[0], self.betas[1], self.eps, self.t)
         return loss
+
+    def _ego_grad(self, R, dst, src, gscalar, cconst):
+        """The ego rows' gradient scattered into this rank's rows of g0, and their flags: the last backward layer's
+        z_add.  Both are cleared on the previous step's rows first."""
+        if self.g0 is None:
+            self.g0 = torch.zeros_like(self.W)
+            self.g0_rows = torch.zeros(self.W.shape[0], dtype=torch.uint8, device=self.W.device)
+        if self._ego_dirty is not None:
+            self.ops.clear_rows(self.g0, self._ego_dirty)
+            self.g0_rows[self._ego_dirty] = 0
+        self.ops.scatter(dst, src, R, None, gscalar, cconst, self.g0, self.prop.r0, self.prop.r1)
+        own = (dst >= self.prop.r0) & (dst < self.prop.r1)
+        self._ego_dirty = (dst[own] - self.prop.r0).contiguous()
+        self.g0_rows[self._ego_dirty] = 1
+        return self.g0, self.g0_rows
 
     def gather_table(self, local: torch.Tensor) -> torch.Tensor:
         """The full [N, D] table from the ranks' slices (evaluation: every rank ranks its own users

@@ -30,10 +30,15 @@ _FLAGS = (
     ("act", int, 1, "activation selector of the path task"),
     ("test_mode", str, "sampled", "Test() of main_rec: sampled = the reference's 99 negatives + 1 held-out item, "
                                   "fullrank = every item ranked, training items masked (single GPU)"),
+    ("loss", str, "bce", "training loss of main_rec: bce = the reference's sampled BCE, bpr = upstream LightGCN's "
+                         "BPR loss + decay * L2 over uniformly sampled (user, positive, negative) triples"),
+    ("decay", float, 1e-4, "weight of the L2 term of the BPR loss (--loss bpr)"),
+    ("bpr_batch", int, 2048, "triples per BPR step (--loss bpr)"),
 )
 # flags the reference does not have: only in the namespace when given, so that a run without them sees the
 # reference's namespace; readers use getattr(args, name, default)
-_ADDED_CHOICES = {"test_mode": ("sampled", "fullrank")}
+_ADDED = {"test_mode", "loss", "decay", "bpr_batch"}
+_CHOICES = {"test_mode": ("sampled", "fullrank"), "loss": ("bce", "bpr")}
 
 
 def build_parser() -> argparse.ArgumentParser:
@@ -41,8 +46,8 @@ def build_parser() -> argparse.ArgumentParser:
     for name, kind, default, doc in _FLAGS:
         if kind is None:
             parser.add_argument("--" + name, action="store_true", help=doc)
-        elif name in _ADDED_CHOICES:
-            parser.add_argument("--" + name, type=kind, choices=_ADDED_CHOICES[name], default=argparse.SUPPRESS,
+        elif name in _ADDED:
+            parser.add_argument("--" + name, type=kind, choices=_CHOICES.get(name), default=argparse.SUPPRESS,
                                 help=f"{doc} (default: {default})")
         elif name == "data_path":
             parser.add_argument("--" + name, nargs="?", default=default, help=doc)

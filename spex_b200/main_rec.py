@@ -11,6 +11,9 @@ loss is accumulated on the device and read once per epoch instead of `.item()` p
 optimiser is the fused dense Adam.
 `--test_mode fullrank` (single GPU) replaces the sampled 99+1 Test() by a full ranking of every item with the
 training items masked, Recall/NDCG@[10, 20, 50] computed on the device; the printed lines keep their format.
+`--loss bpr` trains upstream LightGCN's BPR loss instead of the reference's BCE: an epoch is ceil(n_train / bpr_batch)
+steps of bpr_batch (user, positive, negative) triples drawn on the device, each step minimising
+loss + decay * reg (LightGCN.bpr_loss); the printed lines keep their format.
 """
 from __future__ import annotations
 
@@ -51,6 +54,39 @@ def Train(train_dataset, recommend_model, epoch, optimizer, device, batch=BATCH)
         idx = idx.to(device)
         optimizer.zero_grad(set_to_none=True)
         loss = recommend_model(users=users_d[idx], items=items_d[idx], labels=labels_d[idx], flag=0)
+        loss.backward()
+        total += loss.detach().double()
+        optimizer.step()
+    total_loss = float(total.item())
+    print("%d,%.5f" % (epoch, total_loss))
+    return total_loss
+
+
+def bpr_epoch_steps(n_train: int, batch: int):
+    """Triples per step of one BPR epoch: ceil(n_train / batch) steps that together draw n_train triples."""
+    return [min(batch, n_train - s) for s in range(0, n_train, batch)]
+
+
+def bpr_triples(icsr, n_user_rows: int, m_items: int, n: int):
+    """n (user, positive, negative) triples on the device from the training-interaction CSR `icsr` (rowptr, col:
+    user rows over item ids, item offset 0).  The sampler's seed is drawn from torch's default CPU generator, so a
+    seeded run - or every rank of a distributed one - draws the same triples."""
+    from .model import dropout_seed
+
+    rp, col = icsr
+    return dataloader.uniform_sample_bpr_device(rp, col, 0, m_items, n_user_rows, n, seed=dropout_seed())
+
+
+def TrainBPR(dataset, recommend_model, epoch, optimizer, decay, batch):
+    """One BPR epoch: per step a fresh batch of triples, model.bpr_loss, loss + decay * reg, backward, Adam."""
+    recommend_model.train()
+    icsr = recommend_model.train_mask_csr()
+    total = torch.zeros((), dtype=torch.float64, device=icsr[0].device)
+    for n in bpr_epoch_steps(int(np.asarray(dataset.trainUser).size), batch):
+        users, pos, neg = bpr_triples(icsr, recommend_model.n_user_rows, recommend_model.num_items, n)
+        optimizer.zero_grad(set_to_none=True)
+        loss, reg = recommend_model.bpr_loss(users, pos, neg)
+        loss = loss + decay * reg
         loss.backward()
         total += loss.detach().double()
         optimizer.step()
@@ -111,7 +147,8 @@ def main_distributed(args):
     Every rank runs the same seeded host-side sampling (replicated, no communication), the batches are
     visited in the single-GPU order, rank 0 prints the reference's lines.  Edge dropout runs with the
     device mask (`--dropout 2`): every rank makes the dropped values of its own rows, the same edges a
-    one-GPU run with the same --seed drops."""
+    one-GPU run with the same --seed drops.  `--loss bpr`: every rank samples the one-GPU run's triples
+    (same interaction CSR, same seeds) and runs PartitionedTrainer.bpr_step."""
     import os
 
     import torch.distributed as dist
@@ -146,18 +183,27 @@ def main_distributed(args):
     r0, r1 = bounds[rank], bounds[rank + 1]
     lg = ops.DeviceGraph.from_host(host.row_block(r0, r1, transposed_values=bool(args.dropout)), device, D_hint=D)
     prop = PartitionedPropagator(lg, bounds, D, K, mode="nccl", device=device)
+    bpr = getattr(args, "loss", "bce") == "bpr"
     trainer = PartitionedTrainer(prop, model._table[r0:r1].detach().to(device).contiguous(), nur, lr=args.lr,
-                                 keep_prob=args.keepprob if args.dropout else None)
+                                 keep_prob=args.keepprob if args.dropout else None,
+                                 decay=getattr(args, "decay", 1e-4))
+    if bpr:
+        rp, col = dataset.getInteractionCSR()
+        icsr = (torch.as_tensor(rp, dtype=torch.int64).to(device), torch.as_tensor(col, dtype=torch.int32).to(device))
     best_recall, best_ndcg, best_iter = [0, 0, 0], [0, 0, 0], [0, 0]
     for epoch in range(args.epochs):
-        train_dataset.ng_sample()
-        users, items, labels = (torch.from_numpy(a) for a in train_dataset.arrays())
-        users_d, items_d = users.to(device), items.to(device)
-        labels_d = labels.to(device=device, dtype=torch.float32)
         total = torch.zeros((), dtype=torch.float64, device=device)
-        for idx in epoch_batches(users.numel(), BATCH):
-            idx = idx.to(device)
-            total += trainer.step(users_d[idx], items_d[idx], labels_d[idx]).double().reshape(())
+        if bpr:
+            for n in bpr_epoch_steps(int(dataset.trainUser.size), getattr(args, "bpr_batch", 2048)):
+                total += trainer.bpr_step(*bpr_triples(icsr, nur, model.num_items, n)).double().reshape(())
+        else:
+            train_dataset.ng_sample()
+            users, items, labels = (torch.from_numpy(a) for a in train_dataset.arrays())
+            users_d, items_d = users.to(device), items.to(device)
+            labels_d = labels.to(device=device, dtype=torch.float32)
+            for idx in epoch_batches(users.numel(), BATCH):
+                idx = idx.to(device)
+                total += trainer.step(users_d[idx], items_d[idx], labels_d[idx]).double().reshape(())
         if rank == 0:
             print("%d,%.5f" % (epoch, float(total.item())))
         with torch.no_grad():
@@ -203,7 +249,11 @@ def main(argv=None):
     try:
         for epoch in range(args.epochs):
             start = time.time()
-            Train(train_dataset, Recmodel, epoch, optimizer, device)
+            if getattr(args, "loss", "bce") == "bpr":
+                TrainBPR(dataset, Recmodel, epoch, optimizer, getattr(args, "decay", 1e-4),
+                         getattr(args, "bpr_batch", 2048))
+            else:
+                Train(train_dataset, Recmodel, epoch, optimizer, device)
             best_recall, best_ndcg, best_iter = Test(dataset, Recmodel, epoch, best_recall, best_ndcg, best_iter,
                                                      getattr(args, "test_mode", "sampled"))
             _ = time.time() - start

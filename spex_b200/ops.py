@@ -450,7 +450,8 @@ def spmm_rows(g: DeviceGraph, X: torch.Tensor, subset, Y: Optional[torch.Tensor]
               Z: Optional[torch.Tensor] = None, z_scale: float = 1.0, val: Optional[torch.Tensor] = None,
               x_nonzero: Optional[torch.Tensor] = None, out_row_offset: int = 0, y_mcast: Optional[int] = None,
               y_peers=None, pub_src: Optional[torch.Tensor] = None, pub_mcast: Optional[int] = None,
-              pub_peers=None, adam: Optional[dict] = None):
+              pub_peers=None, adam: Optional[dict] = None, z_add: Optional[torch.Tensor] = None,
+              z_add_rows: Optional[torch.Tensor] = None):
     """spmm() restricted to the rows of `subset` (= g.row_subset(rows); None = all rows): the listed rows of
     Y / Z get exactly the values a full layer gives them, the other rows are left untouched.  `x_nonzero`
     (uint8 [n_cols]): X is exactly zero on the rows it marks 0 - those gathers are skipped, the result is
@@ -458,7 +459,8 @@ def spmm_rows(g: DeviceGraph, X: torch.Tensor, subset, Y: Optional[torch.Tensor]
     rows out_row_offset + i they write): the Y rows to every rank's table through the multicast address `y_mcast`
     or the ctypes array of peer tables `y_peers`; the rows of `pub_src` (or, with `adam`, the updated rows of
     adam["p"]) likewise through `pub_mcast` / `pub_peers`; `adam` = {p, m, v, lr, beta1, beta2, eps, step}: dense
-    Adam on the rows of p with the Z row as gradient."""
+    Adam on the rows of p with the Z row as gradient; `z_add` (fp32 [n_rows, D]) with `z_add_rows` (uint8 [n_rows]):
+    the flagged rows of Z / of Adam's gradient get z_add's row added after the scale (spex_spmm_layer_zadd_f32)."""
     _need_cuda(X)
     X = _f32c(X)
     D = X.shape[1]
@@ -470,6 +472,10 @@ def spmm_rows(g: DeviceGraph, X: torch.Tensor, subset, Y: Optional[torch.Tensor]
     v = g.val if val is None else val
     if x_nonzero is not None and (x_nonzero.dtype != torch.uint8 or x_nonzero.numel() != g.n_cols):
         raise ValueError("x_nonzero must be uint8 [n_cols]")
+    if z_add is not None and (z_add.dtype != torch.float32 or tuple(z_add.shape) != (g.n_rows, D)
+                              or not z_add.is_contiguous() or z_add_rows is None or z_add_rows.dtype != torch.uint8
+                              or z_add_rows.numel() != g.n_rows):
+        raise ValueError("z_add must be contiguous fp32 [n_rows, D] with z_add_rows uint8 [n_rows]")
     ep = SpmmEpilogue(Y=ptr(Y), addend=ptr(addend), addend_scale=addend_scale, Z=ptr(Z), z_scale=z_scale,
                       out_row_offset=out_row_offset, y_mcast=y_mcast, y_peers_host=y_peers,
                       n_y_peers=0 if y_peers is None else len(y_peers), pub_src=ptr(pub_src), pub_mcast=pub_mcast,
@@ -478,9 +484,10 @@ def spmm_rows(g: DeviceGraph, X: torch.Tensor, subset, Y: Optional[torch.Tensor]
         ep.adam_p, ep.adam_m, ep.adam_v = ptr(adam["p"]), ptr(adam["m"]), ptr(adam["v"])
         ep.lr, ep.beta1, ep.beta2, ep.eps, ep.step = (adam["lr"], adam["beta1"], adam["beta2"], adam["eps"],
                                                      adam["step"])
-    call("spex_spmm_layer_f32", ptr(g.rowptr), ptr(g.col), ptr(v), ptr(X), g.n_rows, D, ptr(rows),
+    call("spex_spmm_layer_zadd_f32", ptr(g.rowptr), ptr(g.col), ptr(v), ptr(X), g.n_rows, D, ptr(rows),
          -1 if rows is None else rows.numel(), ptr(slots), 0 if slots is None else slots.numel(), ptr(segs),
-         0 if segs is None else segs.numel(), ptr(x_nonzero), C.byref(ep), g.plan(D), stream_ptr())
+         0 if segs is None else segs.numel(), ptr(x_nonzero), C.byref(ep), ptr(z_add), ptr(z_add_rows), g.plan(D),
+         stream_ptr())
 
 
 # A layer's input is treated as sparse (x_nonzero mask, gathers of zero rows skipped) while the rows that may be
